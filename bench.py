@@ -206,6 +206,8 @@ def run_reference(config, steps, warmup):
     """The UNMODIFIED reference on all host cores, one env per process -> cpu_baseline dict, or None if not staged."""
     from oracle import ref_bench
     if ref_bench.available() is None:
+        print("cpu_baseline: no reference tree (build() stages oracle/_ref only when SSD_REFERENCE_ROOT names a checkout "
+              "of the original project); the C restatement (kind 'port') stands in for it", file=sys.stderr)
         return None
     rate, procs, ms, sample = ref_bench.run(config, steps=steps, warmup=warmup)
     out = {"value": rate, "unit": "agent-steps/s", "cores": procs, "kind": "reference", "ms_per_env_step": ms, "sample": sample}
@@ -353,6 +355,44 @@ class Runner:
         if self.stats is not None:
             self.stats.zero_()
 
+    def outputs(self):
+        """what a caller of `substep` receives from the last step: the env's output tensors (rewritten in place every
+        step) and, with the negotiation prologue, the decisions of the envs that negotiated in it"""
+        env = self.env
+        out = {"obs": env.obs, "rew": env.rew, "done": env.done}
+        if self.fam != "car":                      # selfdrive writes info only with extras=True
+            out["info"] = env.info
+        if self.cfg["negotiate"]:
+            out["negotiation_decision"] = self.dec
+        return out
+
+
+DUMP_BYTES = 64 * 10 ** 6                      # npy headers fit in the 4 KB kept aside
+
+
+def dump_outputs(run, stats_total, out_dir):
+    """Write the last timed step's outputs as DIR/<name>.npy (float64 stays float64, everything else becomes float32).
+    Arrays are sampled along the env axis to keep the dump under DUMP_BYTES: the same seeded sample of env indices
+    (written as env_index.npy) for every array, so that two builds run with the same arguments can be compared."""
+    import torch
+    outs = run.outputs()
+    per_env = 8 + sum(t[0].numel() * (8 if t.dtype == torch.float64 else 4) for t in outs.values())
+    S = min(run.E, (DUMP_BYTES - 4096) // per_env)
+    if S < run.E:
+        idx = np.sort(np.random.RandomState(SEED).choice(run.E, S, replace=False))
+    else:
+        idx = np.arange(run.E)
+    sel = torch.as_tensor(idx, device=run.dev)
+    arrays = {"env_index": idx.astype(np.float64)}
+    for name, t in outs.items():
+        a = t.index_select(0, sel).cpu().numpy()
+        arrays[name] = a if a.dtype == np.float64 else a.astype(np.float32)
+    if stats_total is not None:
+        arrays["episode_stats"] = np.asarray(stats_total, dtype=np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
 
 def pin_to_cores(local, world):
     """each rank's host threads on their own block of cores (the ranks share one NUMA node on these boxes)"""
@@ -378,6 +418,9 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=300)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--graph-steps", type=int, default=50, help="env steps per captured CUDA graph (1 = no graphs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (rank 0's envs, a "
+                         "fixed sample of them when they exceed 64 MB)")
     args = ap.parse_args()
     if args.impl == "reference":
         reference_arm(args)
@@ -504,6 +547,8 @@ def main():
         stats_total = g.sum(0)
         stats_total[7] = g[:, 7].max()
         stats_total = stats_total.tolist()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(run, stats_total, args.dump_outputs)
 
     # ---- the step kernels alone (roofline): CUDA events around each step call of an un-graphed stretch -------
     Kk = 200

@@ -1,7 +1,7 @@
 """Generate the golden vectors in tests/golden/ by running the UNMODIFIED reference.
 
-TEST INFRASTRUCTURE (oracle/), container-only: needs /root/reference.  Run as
-    python -m oracle.make_golden
+TEST INFRASTRUCTURE (oracle/): needs a checkout of the original project.  Run as
+    SSD_REFERENCE_ROOT=<checkout> python -m oracle.make_golden
 Each fixture is the reference's own output (oracle/ref_harness.py: reference code + RNG
 injection) for a seeded action sequence: per-step grid, agent state, uint8 observations,
 rewards before/after contract transfers, transfers, infos and feature_obs, plus episode

@@ -3,7 +3,7 @@
 TEST INFRASTRUCTURE (oracle/): imported only by tests/, bench.py's cpu_baseline /
 `--impl reference` leg, `__graft_entry__.smoke()` and the golden-vector generator.
 
-The reference (`/root/reference`) draws from NumPy's / stdlib's global MT19937 at the
+The reference (the original project) draws from NumPy's / stdlib's global MT19937 at the
 call sites of SURVEY.md §8a table R.  For parity every one of those sites is replaced
 by a *counter-based* draw, so that the reference, the C oracle and the CUDA kernels
 all see identical randomness regardless of evaluation order:

@@ -3,7 +3,7 @@
 TEST / MEASUREMENT INFRASTRUCTURE (oracle/).  SURVEY.md §8(d): the reference (stubbed imports, its own MT19937 RNG — no
 injection) stepping the env + SeparateContractSubgameStage wrapper with iid random actions, one env per process,
 P processes via multiprocessing (mirrors RLlib's one env per rollout worker, utils/ray_config_utils.py:140); the rate is
-P envs x n agents x steps over the SLOWEST worker's loop time.  Uses /root/reference when present, else the staged copy
+P envs x n agents x steps over the SLOWEST worker's loop time.  Uses $SSD_REFERENCE_ROOT when set, else the staged copy
 oracle/_ref/ (oracle/stage_reference.py).
 """
 import multiprocessing as mp
@@ -67,7 +67,7 @@ def run(config="cleanup8", steps=200, warmup=5, procs=None):
     """-> (agent-steps/s, procs, ms per env step of the slowest worker, sample description)"""
     root = available()
     if root is None:
-        raise RuntimeError("no reference tree (neither /root/reference nor oracle/_ref)")
+        raise RuntimeError("no reference tree (neither $SSD_REFERENCE_ROOT nor oracle/_ref)")
     procs = procs or (os.cpu_count() or 1)
     n = CONFIGS[config][1]
     ctx = mp.get_context("spawn")                                  # no forked CUDA / OpenMP state in the workers

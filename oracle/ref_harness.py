@@ -1,6 +1,6 @@
 """Run the UNMODIFIED reference env code under counter-based RNG injection.
 
-TEST INFRASTRUCTURE (oracle/), container-only (needs `/root/reference`).  This is the
+TEST INFRASTRUCTURE (oracle/), needs a checkout of the original project (SSD_REFERENCE_ROOT).  This is the
 ground truth that pins both the C oracle (`oracle/ssd_oracle.c`) and the CUDA path: every
 RNG call site of SURVEY.md §8a table R is monkey-patched (no reference source is edited or
 copied) to read from the Philox stream defined in `oracle/philox.py`.  The golden vectors in

@@ -1,29 +1,37 @@
-"""Import stubs that let the UNMODIFIED reference (`/root/reference`) be imported here.
+"""Import stubs that let the UNMODIFIED reference (the original project, a checkout of which SSD_REFERENCE_ROOT names)
+be imported here.
 
 TEST INFRASTRUCTURE (oracle/).  The reference needs gym 0.21, ray 2.2 and matplotlib, none
-of which is in this image (SURVEY.md §8c).  Only the tiny surface the hot path touches is
-stubbed; nothing here re-implements reference logic.  Container-only: `/root/reference`
-does not exist on the GPU box, so nothing under `-m gpu`, `smoke()` or `bench.py` uses it.
+of which this project depends on (SURVEY.md §8c).  Only the tiny surface the hot path touches is
+stubbed; nothing here re-implements reference logic.  Nothing under `-m gpu`, `smoke()` or
+`bench.py`'s GPU arm uses it; the tests that run the reference skip when SSD_REFERENCE_ROOT is not set.
 """
+import os
 import sys
 import types
 
 import numpy as np
 
-REFERENCE_ROOT = "/root/reference"
-# `oracle/stage_reference.py` (run by __graft_entry__.build() in the container) copies the unmodified reference modules
-# the path needs into this git-ignored directory, so that bench.py's CPU-baseline arm can time the REAL reference on the
-# GPU box, where /root/reference does not exist.  Parity tests never use the staged copy.
-STAGED_ROOT = __import__("os").path.join(__import__("os").path.dirname(__import__("os").path.abspath(__file__)), "_ref")
+# a checkout of the original project (its `environments/`, `contract/`, `utils/` at the top level), or None
+REFERENCE_ROOT = os.environ.get("SSD_REFERENCE_ROOT") or None
+# `oracle/stage_reference.py` (run by __graft_entry__.build()) copies the unmodified reference modules the path needs into
+# this git-ignored directory, so that bench.py's CPU-baseline arm can time the REAL reference on a machine that has a built
+# tree but no reference checkout.  Parity tests never use the staged copy.
+STAGED_ROOT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref")
+
+
+def live_reference():
+    """REFERENCE_ROOT when it holds the reference tree, else None (what the parity tests run against)."""
+    if REFERENCE_ROOT and os.path.isdir(os.path.join(REFERENCE_ROOT, "environments")):
+        return REFERENCE_ROOT
+    return None
 
 
 def reference_root():
-    """/root/reference when present (container), else the staged copy (GPU box), else None."""
-    import os
-    for r in (REFERENCE_ROOT, STAGED_ROOT):
-        if os.path.isdir(os.path.join(r, "environments")):
-            return r
-    return None
+    """The reference checkout when present, else the staged copy, else None."""
+    if live_reference():
+        return REFERENCE_ROOT
+    return STAGED_ROOT if os.path.isdir(os.path.join(STAGED_ROOT, "environments")) else None
 
 
 class Space:
@@ -82,10 +90,9 @@ def _mod(name, **attrs):
 
 def install(root=None):
     """Put the stub modules in sys.modules and the reference root on sys.path."""
-    import os
     root = root or REFERENCE_ROOT
-    if not os.path.isdir(root):
-        raise RuntimeError("reference tree %s not present (container-only)" % root)
+    if not root or not os.path.isdir(root):
+        raise RuntimeError("reference tree %r not present: set SSD_REFERENCE_ROOT to a checkout of the original project" % root)
     if "gym" not in sys.modules:
         spaces = _mod("gym.spaces", Space=Space, Box=Box, Discrete=Discrete,
                       MultiDiscrete=MultiDiscrete, Dict=Dict)

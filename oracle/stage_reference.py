@@ -1,10 +1,10 @@
 """Stage the UNMODIFIED reference modules of the hot path into oracle/_ref/ (git-ignored).
 
-TEST / MEASUREMENT INFRASTRUCTURE (oracle/).  `/root/reference` exists only in the build container; the GPU box gets a
-snapshot of this repo.  `__graft_entry__.build()` therefore copies the reference's own files — byte for byte, nothing is
-edited — into `oracle/_ref/`, which is listed in .gitignore (never committed) but not in .gpurunignore (it travels like
-the built .so files).  The only consumer is `oracle/ref_bench.py` (bench.py's cpu_baseline / `--impl reference` arm):
-it times the reference's Python env loop on the GPU box's host cores.
+TEST / MEASUREMENT INFRASTRUCTURE (oracle/).  When SSD_REFERENCE_ROOT names a checkout of the original project,
+`__graft_entry__.build()` copies the reference's own files — byte for byte, nothing is edited — into `oracle/_ref/`, which
+is listed in .gitignore (never committed) and can travel with a built tree to a machine without the checkout.  The only
+consumer is `oracle/ref_bench.py` (bench.py's cpu_baseline / `--impl reference` arm): it times the reference's Python env
+loop on the host cores.
 """
 import os
 import shutil
@@ -19,8 +19,8 @@ FILES = ["__init__.py", "LICENSE", "utils/__init__.py", "utils/env_creator_funct
 
 
 def stage(src=ref_stubs.REFERENCE_ROOT, dst=ref_stubs.STAGED_ROOT):
-    """Returns the staged root, or None when the reference tree is not present (GPU box: keep what travelled)."""
-    if not os.path.isdir(os.path.join(src, "environments")):
+    """Returns the staged root, or None when neither a reference checkout nor an earlier staged copy is present."""
+    if not src or not os.path.isdir(os.path.join(src, "environments")):
         return dst if os.path.isdir(os.path.join(dst, "environments")) else None
     for rel in FILES:
         s = os.path.join(src, rel)

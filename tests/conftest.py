@@ -10,11 +10,12 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (container only)")
+    config.addinivalue_line("markers", "reference: needs a checkout of the original project (SSD_REFERENCE_ROOT)")
 
 
 def has_reference():
-    return os.path.isdir("/root/reference/environments")
+    from oracle import ref_stubs
+    return ref_stubs.live_reference() is not None
 
 
 @pytest.fixture(scope="session")

@@ -8,6 +8,7 @@ A backend adapter exposes, for ONE environment:
 Every comparison is bit-exact (float64 compared through their uint64 bit patterns).
 """
 import glob
+import hashlib
 import os
 
 import numpy as np
@@ -46,11 +47,76 @@ def contract_name(fx):
     return "CleanupContract" if str(fx["kind"]) == "cleanup" else "HarvestFeaturemodLocalContract"
 
 
+class _Stored:
+    """The reference's side of a comparison when the reference does not run: its outputs are only known through the
+    digests stored in tests/golden/reference_tapes.json (see Tape).  Indexing and membership keep the test bodies as they
+    are; every comparison against it is checked through the active tape."""
+
+    def __getitem__(self, key):
+        return self
+
+    def __contains__(self, key):
+        return True
+
+
+STORED = _Stored()
+TAPE = None                 # the active Tape, set by a fixture of the differential tests
+
+
+class Tape:
+    """Ordered digest of every value a reference comparison checks (name, shape and the bits assert_same compares).
+    A checkpoint is taken every EVERY values and at the end; against `stored` checkpoints each one must match, so a
+    divergence is located to within EVERY comparisons."""
+    EVERY = 1000
+
+    def __init__(self, test_id, stored=None):
+        self.test_id, self.stored = test_id, stored
+        self.h, self.count, self.marks, self.last_ctx = hashlib.sha256(), 0, [], None
+        self.diverged = False
+
+    def feed(self, name, got, ctx):
+        got = np.asarray(got)
+        canon = bits(got) if got.dtype.kind == "f" else np.ascontiguousarray(got.astype(np.int64))
+        self.h.update(("%s|%r|" % (name, got.shape)).encode())
+        self.h.update(canon.tobytes())
+        self.count += 1
+        self.last_ctx = ctx
+        if self.count % self.EVERY == 0:
+            self._mark()
+
+    def _mark(self):
+        d = self.h.hexdigest()[:16]
+        i = len(self.marks)
+        self.marks.append(d)
+        if self.stored is not None:
+            self.diverged = True                    # until this checkpoint is found equal
+            assert i < len(self.stored), "%s: more comparisons than the reference's recorded run" % self.test_id
+            assert self.stored[i] == d, ("%s: the values of comparisons %d..%d (the last at %s) differ from the reference's "
+                                         "recorded outputs" % (self.test_id, i * self.EVERY + 1, self.count, self.last_ctx))
+            self.diverged = False
+
+    def finish(self):
+        if self.diverged:                           # already reported by the failing comparison
+            return
+        if self.count % self.EVERY:
+            self._mark()
+        if self.stored is not None:
+            assert len(self.marks) == len(self.stored), "%s: fewer comparisons than the reference's recorded run" % self.test_id
+
+
+def _f64(x):
+    return x if x is STORED else np.float64(x)
+
+
 def bits(x):
     return np.ascontiguousarray(np.asarray(x, dtype=np.float64)).view(np.uint64)
 
 
 def assert_same(name, got, want, ctx):
+    if TAPE is not None:
+        TAPE.feed(name, got, ctx)
+    if want is STORED:
+        return
     got, want = np.asarray(got), np.asarray(want)
     if got.dtype.kind == "f" or want.dtype.kind == "f":
         ok = np.array_equal(bits(got), bits(want)) and got.shape == want.shape
@@ -99,16 +165,16 @@ def check_episode_metrics(kind, n, contract, raw, want, ctx):
     assert raw[5] == 0, "backend error flags %r" % raw[5]
     got = metrics_from_raw(kind, n, contract, raw)
     for k, v in got.items():
-        assert_same("metric " + k, np.float64(v), np.float64(want[k]), ctx)
+        assert_same("metric " + k, np.float64(v), _f64(want[k]), ctx)
     if "equality" in want:          # episode ended: cleanup_new.py:264-266, two_stage_train.py:97-99
         totals, tsums = list(raw[24:24 + n]), list(raw[32:32 + n])
-        assert_same("equality", np.float64(equality(totals)), np.float64(want["equality"]), ctx)
-        assert_same("sustainability", np.float64(sustainability(totals, tsums)), np.float64(want["sustainability"]), ctx)
+        assert_same("equality", np.float64(equality(totals)), _f64(want["equality"]), ctx)
+        assert_same("sustainability", np.float64(sustainability(totals, tsums)), _f64(want["sustainability"]), ctx)
         if "transfer_equality" in want:
             totals, tsums = list(raw[40:40 + n]), list(raw[48:48 + n])
-            assert_same("transfer_equality", np.float64(equality(totals)), np.float64(want["transfer_equality"]), ctx)
+            assert_same("transfer_equality", np.float64(equality(totals)), _f64(want["transfer_equality"]), ctx)
             assert_same("transfer_sustainability", np.float64(sustainability(totals, tsums)),
-                        np.float64(want["transfer_sustainability"]), ctx)
+                        _f64(want["transfer_sustainability"]), ctx)
 
 
 def replay(backend, fx, check_features=True):

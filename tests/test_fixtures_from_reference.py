@@ -1,14 +1,14 @@
-"""Container-only (needs /root/reference): the committed fixtures are what the UNMODIFIED reference produces today —
-a sample of every fixture family is regenerated through oracle/make_golden.py and compared array by array."""
-import os
-
+"""Needs a checkout of the original project (SSD_REFERENCE_ROOT): the committed fixtures are what the UNMODIFIED
+reference produces today — a sample of every fixture family is regenerated through oracle/make_golden.py and compared
+array by array."""
 import numpy as np
 import pytest
 
 import golden_util as gu
+from oracle import ref_stubs
 
-pytestmark = pytest.mark.skipif(not os.path.isdir("/root/reference/environments"),
-                                reason="reference tree not present (GPU box): fixtures were generated in the build container")
+pytestmark = pytest.mark.skipif(ref_stubs.live_reference() is None,
+                                reason="SSD_REFERENCE_ROOT does not name a checkout of the original project")
 
 SAMPLES = [("run_scenario", "cleanup_n5_short_horizon"), ("run_scenario", "harvest_cramped_n6_collective_inequity"),
            ("run_negotiate", "negotiate_cleanup_n2"), ("run_solver", "solver_cleanup_n2_majority"),
