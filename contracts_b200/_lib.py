@@ -54,6 +54,10 @@ class ssd_host_layout(ctypes.Structure):
     ]
 
 
+class ssd_checkpoint_layout(ctypes.Structure):
+    _fields_ = [("row_bytes", ctypes.c_int64), ("config_tag", ctypes.c_uint64)]
+
+
 STATS_LEN = 8
 
 
@@ -94,6 +98,7 @@ EXPORTS = [
     "ssd_global_view", "ssd_concat_obs", "ssd_solver_sample", "ssd_solver_choose", "ssd_policy_inputs", "ssd_record_beams", "ssd_render", "ssd_step_host",
     "ssd_step_host_async", "ssd_step_host_wait", "ssd_host_result_layout", "ssd_host_result_expand", "ssd_set_episode_stats",
     "ssd_feat_step_host_async", "ssd_selfdrive_step_host_async",
+    "ssd_checkpoint_get_layout", "ssd_checkpoint_save", "ssd_checkpoint_load",
 ]
 
 _LIB = None
@@ -155,6 +160,9 @@ def load():
     L.ssd_kernel_launches.restype = i64
     L.ssd_enable_timing.argtypes = [vp, ctypes.c_int32]
     L.ssd_get_step_times.argtypes = [vp, ctypes.POINTER(ctypes.c_double)]
+    L.ssd_checkpoint_get_layout.argtypes = [vp, ctypes.POINTER(ssd_checkpoint_layout)]
+    L.ssd_checkpoint_save.argtypes = [vp, vp, i32, vp, vp]
+    L.ssd_checkpoint_load.argtypes = [vp, ctypes.c_uint64, vp, i32, vp, vp, vp]
     if L.ssd_abi_version() != SSD_ABI_VERSION:
         raise SsdError("libssd_b200.so ABI %d != binding ABI %d" % (L.ssd_abi_version(), SSD_ABI_VERSION))
     _LIB = L

@@ -16,6 +16,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .checkpoint import CheckpointMixin
 from .maps import CLEANUP_MAP, HARVEST_MAP
 
 _DEFAULT_HIGH = {"CleanupContract": 0.2, "HarvestFeaturemodLocalContract": 10.0}
@@ -119,7 +120,7 @@ class HostResultMixin:
         _lib.check(self._h, self.lib.ssd_step_host_wait(self._h, int(ticket)))
 
 
-class BatchedGridEnv(HostResultMixin):
+class BatchedGridEnv(HostResultMixin, CheckpointMixin):
     """E environments of one kind on one device.
 
     kind: 'cleanup_new' | 'harvest_new' (the reference's `environment` strings,

@@ -22,6 +22,7 @@
 #include "ssd_views.cuh"
 #include "ssd_selfdrive.cuh"
 #include "ssd_features.cuh"
+#include "ssd_checkpoint.cuh"
 
 static thread_local char g_create_error[512] = "";
 
@@ -60,6 +61,8 @@ struct ssd_handle {
     uint32_t* d_counter;     // device step counter for SSD_STEP_AUTO: [0] index, [1] CTAs finished
     bool rounds4;            // point lists fit 4 rounds of 32 (selects the observe-kernel variant)
     int64_t launches;
+    CkParams ck;             // ssd_checkpoint_*: where each part of an env's row lives (ssd_checkpoint.cuh)
+    uint64_t config_tag;     // ssd_checkpoint_get_layout: hash of everything that gives a row its meaning
     char err[512];
     std::vector<void*> dev_allocs;
 };
@@ -595,6 +598,81 @@ static int setup_features(ssd_handle* h)
 }
 
 // ---------------------------------------------------------------------------------------------
+// checkpoint rows (include/ssd_b200.h documents the layout per kind)
+static uint64_t fnv1a(uint64_t h, const void* data, size_t bytes)
+{
+    const uint8_t* b = (const uint8_t*)data;
+    for (size_t i = 0; i < bytes; i++) { h ^= b[i]; h *= 1099511628211ull; }
+    return h;
+}
+// every ssd_config field except num_envs, first_env_id, seed, device and struct_size (and the row layout's version)
+static uint64_t config_tag(const ssd_handle* h)
+{
+    const ssd_config& c = h->cfg;
+    uint64_t t = 14695981039346656037ull;
+    const uint32_t version = CK_LAYOUT_VERSION;
+    const int32_t ints[7] = { c.abi_version, c.env_kind, c.num_agents, c.map_h, c.map_w, c.horizon, c.contract_kind };
+    t = fnv1a(t, &version, sizeof(version));
+    t = fnv1a(t, ints, sizeof(ints));
+    t = fnv1a(t, h->ascii.data(), h->ascii.size());
+    const double dbl[3] = { c.theta_low, c.theta_high, c.null_prob };
+    t = fnv1a(t, dbl, sizeof(dbl));
+    t = fnv1a(t, &c.flags, sizeof(c.flags));
+    t = fnv1a(t, c.env_params, sizeof(c.env_params));
+    return t;
+}
+static void ck_col(CkParams& k, void* base, int elem, int row_off)
+{
+    k.col[k.ncol].base = (uint8_t*)base; k.col[k.ncol].elem = elem; k.col[k.ncol].row_off = row_off; k.ncol++;
+}
+static void setup_checkpoint(ssd_handle* h)
+{
+    CkParams& k = h->ck;
+    memset(&k, 0, sizeof(k));
+    const ssd_config& c = h->cfg;
+    const int n = c.num_agents;
+    k.E = c.num_envs; k.n = n;
+    if (c.env_kind == SSD_ENV_SELFDRIVE) {                 // every array is [car][env] / [env]: columns only
+        const CarParams& p = h->cp;
+        k.fam = CK_CAR;
+        for (int a = 0; a < n; a++) ck_col(k, p.pos + (size_t)a * p.E, 8, 8 * a);
+        for (int a = 0; a < n; a++) ck_col(k, p.vel + (size_t)a * p.E, 8, 8 * (n + a));
+        ck_col(k, p.theta, 8, 16 * n);
+        ck_col(k, p.m_transfers, 8, 16 * n + 8);
+        ck_col(k, p.dist_front, 8, 16 * n + 16);
+        k.car_crossed_off = 16 * n + 24; ck_col(k, p.crossed, 4, k.car_crossed_off);
+        k.car_meta_off = 16 * n + 28; ck_col(k, p.meta, 4, k.car_meta_off);
+        ck_col(k, p.t, 4, 16 * n + 32);
+        ck_col(k, p.episode, 4, 16 * n + 36);
+        k.row_bytes = round_up(16 * n + 40, 16);
+        k.zero_fill = 1;
+    } else if (c.env_kind == SSD_ENV_CLEANUP_FEATURES || c.env_kind == SSD_ENV_HARVEST_FEATURES) {   // hot record + lists env-major; metrics / accumulators [k][E]
+        const FeatParams& p = h->fp;
+        k.fam = CK_FEAT;
+        k.H = p.H; k.W = p.W; k.horizon = p.horizon; k.n_apple = p.n_apple; k.n_waste = p.n_waste; k.LA = p.LA; k.LW = p.LW;
+        k.lists_off = round_up(192 + 28 * n, 16);
+        k.nseg = 2;
+        k.seg[0].base = (uint8_t*)p.rec; k.seg[0].stride = 4 * FR_WORDS; k.seg[0].bytes = 4 * FR_WORDS; k.seg[0].row_off = 0;
+        k.seg[1].base = p.lists; k.seg[1].stride = p.LS; k.seg[1].bytes = p.LS; k.seg[1].row_off = k.lists_off;
+        for (int q = 0; q < 8; q++) ck_col(k, p.metrics + (size_t)q * p.E, 8, 128 + 8 * q);
+        for (int a = 0; a < n; a++) ck_col(k, p.tsum_raw + (size_t)a * p.E, 8, 192 + 8 * a);
+        for (int a = 0; a < n; a++) ck_col(k, p.sum_tr + (size_t)a * p.E, 8, 192 + 8 * (n + a));
+        for (int a = 0; a < n; a++) ck_col(k, p.tsum_tr + (size_t)a * p.E, 8, 192 + 8 * (2 * n + a));
+        for (int a = 0; a < n; a++) ck_col(k, p.sum_raw + (size_t)a * p.E, 4, 192 + 24 * n + 4 * a);
+        k.row_bytes = k.lists_off + p.LS;
+        k.zero_fill = 1;
+    } else {                                               // the whole record, padding included
+        const GridParams& p = h->gp;
+        k.fam = CK_GRID;
+        k.H = p.H; k.W = p.W; k.horizon = p.horizon; k.n_apple = p.n_apple; k.n_waste = p.n_waste;
+        k.nseg = 1;
+        k.seg[0].base = p.state; k.seg[0].stride = p.rec_stride; k.seg[0].bytes = p.rec_stride; k.seg[0].row_off = 0;
+        k.row_bytes = p.rec_stride;
+    }
+    h->config_tag = config_tag(h);
+}
+
+// ---------------------------------------------------------------------------------------------
 // small utility kernels
 __global__ void get_state_kernel(GridParams p, uint8_t* map, int32_t* pos, int32_t* ori, int32_t* t, double* theta)
 {
@@ -807,6 +885,7 @@ int ssd_create(const ssd_config* cfg, ssd_handle** out)
     const bool is_feat = cfg->env_kind == SSD_ENV_CLEANUP_FEATURES || cfg->env_kind == SSD_ENV_HARVEST_FEATURES;
     int rc = cfg->env_kind == SSD_ENV_SELFDRIVE ? setup_selfdrive(h) : (is_feat ? setup_features(h) : setup_grid(h));
     if (rc == SSD_OK) rc = dev_zalloc(h, 2, &h->d_counter);
+    if (rc == SSD_OK) setup_checkpoint(h);
     if (rc != SSD_OK) {
         snprintf(g_create_error, sizeof(g_create_error), "%s", h->err);
         ssd_destroy(h);
@@ -1504,6 +1583,52 @@ int ssd_selfdrive_random_actions(ssd_handle* h, uint32_t step_index, float lo, f
     car_random_actions_kernel<<<(h->cp.E + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->cp, step_index, autoidx ? h->d_counter : nullptr,
                                                                                          lo, hi, actions_dev);
     return check_launch(h, "selfdrive_random_actions");
+}
+
+// ---- checkpoint / restore / copy of env state (ssd_checkpoint.cuh) -------------------------------------------------
+int ssd_checkpoint_get_layout(const ssd_handle* h, ssd_checkpoint_layout* out)
+{
+    if (!h || !out) return SSD_EINVAL;
+    out->row_bytes = h->ck.row_bytes;
+    out->config_tag = h->config_tag;
+    return SSD_OK;
+}
+
+static int checkpoint_args(ssd_handle* h, const char* what, const int32_t* env_idx_dev, int32_t count, const void* rows_dev)
+{
+    if (count < 0) return fail(h, SSD_EINVAL, "%s: count %d < 0", what, count);
+    if (!env_idx_dev && count > h->cfg.num_envs)
+        return fail(h, SSD_EINVAL, "%s: count %d exceeds the handle's %d envs (no index list)", what, count, h->cfg.num_envs);
+    if (count > 0 && !rows_dev) return fail(h, SSD_EINVAL, "%s: rows_dev is NULL", what);
+    if (reinterpret_cast<uintptr_t>(rows_dev) & 15) return fail(h, SSD_EINVAL, "%s: rows_dev must be 16-byte aligned", what);
+    return SSD_OK;
+}
+
+int ssd_checkpoint_save(ssd_handle* h, const int32_t* env_idx_dev, int32_t count, uint8_t* rows_dev, void* stream)
+{
+    if (!h) return SSD_EINVAL;
+    ON_DEVICE(h);
+    int rc = checkpoint_args(h, "checkpoint_save", env_idx_dev, count, rows_dev);
+    if (rc || count == 0) return rc;
+    ck_save_kernel<<<(count + CK_ROWS - 1) / CK_ROWS, CK_THREADS, (size_t)CK_ROWS * h->ck.row_bytes, (cudaStream_t)stream>>>(
+        h->ck, env_idx_dev, count, rows_dev);
+    return check_launch(h, "checkpoint_save");
+}
+
+int ssd_checkpoint_load(ssd_handle* h, uint64_t config_tag, const int32_t* env_idx_dev, int32_t count, const uint8_t* rows_dev,
+                        uint8_t* row_ok_dev, void* stream)
+{
+    if (!h) return SSD_EINVAL;
+    ON_DEVICE(h);
+    if (config_tag != h->config_tag)
+        return fail(h, SSD_EINVAL, "checkpoint_load: config_tag %016llx does not match the handle's %016llx (rows saved under "
+                    "another env kind, agent count, map, horizon, contract or reward configuration)",
+                    (unsigned long long)config_tag, (unsigned long long)h->config_tag);
+    int rc = checkpoint_args(h, "checkpoint_load", env_idx_dev, count, rows_dev);
+    if (rc || count == 0) return rc;
+    ck_load_kernel<<<(count + CK_ROWS - 1) / CK_ROWS, CK_THREADS, (size_t)CK_ROWS * h->ck.row_bytes, (cudaStream_t)stream>>>(
+        h->ck, env_idx_dev, count, rows_dev, row_ok_dev);
+    return check_launch(h, "checkpoint_load");
 }
 
 int ssd_enable_timing(ssd_handle* h, int32_t on)

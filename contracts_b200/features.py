@@ -11,6 +11,7 @@ import torch
 
 from . import _lib
 from .batched import HostResultMixin
+from .checkpoint import CheckpointMixin
 from .maps import CLEANUP_MAP, HARVEST_MAP
 
 _DEFAULT_HIGH = {"CleanupContract": 0.2, "HarvestFeaturemodLocalContract": 10.0}
@@ -20,7 +21,7 @@ def _ptr(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
 
-class BatchedFeatureEnv(HostResultMixin):
+class BatchedFeatureEnv(HostResultMixin, CheckpointMixin):
     """kind: 'cleanup' | 'harvest' (the reference's `environment` strings for the feature envs)."""
 
     def __init__(self, kind, num_envs, num_agents, ascii_map=None, horizon=1000, contract=None, theta_low=0.0,
@@ -38,6 +39,7 @@ class BatchedFeatureEnv(HostResultMixin):
         if theta_high is None:
             theta_high = _DEFAULT_HIGH.get(contract, 0.0)
         self._flat = "".join(self.ascii_map).encode("ascii")
+        self.seed, self.first_env_id = int(seed) & 0xFFFFFFFF, int(first_env_id) & 0xFFFFFFFF
         cfg = _lib.make_config(
             env_kind=_lib.ENV_KIND[kind], num_envs=self.E, num_agents=self.n,
             map_h=self.H, map_w=self.W, ascii_map=self._flat, horizon=self.horizon,

@@ -10,13 +10,16 @@ import torch
 
 from . import _lib
 from .batched import HostResultMixin
+from .checkpoint import CheckpointMixin
 
 
 def _ptr(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
 
-class BatchedCarEnv(HostResultMixin):
+class BatchedCarEnv(HostResultMixin, CheckpointMixin):
+    kind = "selfdrive"
+
     def __init__(self, num_envs, num_agents, contract=None, low_bound=-10.0, high_bound=10.0, start_vel=0.2,
                  start_vel_ambulance=0.8, theta_low=0.0, theta_high=100.0, null_prob=0.0, seed=73907, first_env_id=0,
                  device=None):
@@ -28,6 +31,7 @@ class BatchedCarEnv(HostResultMixin):
         self.E, self.n = int(num_envs), int(num_agents)
         self.device = _lib.resolve_device(device)
         self.contract = contract
+        self.seed, self.first_env_id = int(seed) & 0xFFFFFFFF, int(first_env_id) & 0xFFFFFFFF
         cfg = _lib.make_config(
             env_kind=_lib.ENV_KIND["selfdrive"], num_envs=self.E, num_agents=self.n,
             map_h=0, map_w=0, ascii_map=None, horizon=0, contract_kind=_lib.CONTRACT_KIND[contract],

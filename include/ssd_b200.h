@@ -324,6 +324,50 @@ int ssd_feat_get_state(ssd_handle* h, int32_t* pos_dev, int32_t* ori_dev, uint8_
  * per agent: sum r [8], sum t*r [8], sum transferred r [8], sum t * transferred r [8] */
 int ssd_feat_get_metrics(ssd_handle* h, double* out_dev, void* stream);
 
+/* --- checkpoint / restore / copy of env state (every env_kind) ------------------------------------------------
+ * One primitive behind resuming a run, re-sharding it over another number of handles and branching an env into others:
+ * the complete mutable state of an env as one ROW of row_bytes bytes, and rows loaded back.  A row holds every byte a
+ * later step, reset, negotiation, metrics call or auto_reset reads (flags and sticky error bits, the episode counter —
+ * a word of every Philox counter —, the episode accumulators), and nothing the caller owns (observations, rewards,
+ * infos, the episode-statistics vector), nor the per-step scratch, the beam overlay, the SSD_STEP_AUTO counter or the
+ * pipelined host path's copy-size prediction.  A row loaded into env i continues on env i's own random stream
+ * (seed, first_env_id + i): loaded into the env of the same global id it continues exactly as if it had never stopped.
+ *
+ * Row layouts (byte offsets; n = num_agents; unlisted bytes are padding and saved as 0):
+ *   cleanup_new / harvest_new: the env record, row_bytes = 512 (640 with SSD_FLAG_COLLECTIVE_REWARD / _INEQUITY_AVERSE)
+ *     0 u32 agent[8] (row | col << 8 | ori << 16)   32 i32 t   36 u32 episode   40 f64 theta
+ *     48 u32 flags (bit 31 initialised, bit 0 stale apple list, bits 8.. sticky err_flags)   52 u32 #waste cells
+ *     64 u32 apple mask[8]   96 u32 waste mask[8] (bit j = point j of the row-major point list)
+ *     128.. episode accumulators (apples, low density, dirt, transfers, per-agent sums; 440..575 float64 shaped sums)
+ *   cleanup / harvest (feature envs): row_bytes = L + LS, L = round16(192 + 28 n), LS = both list capacities
+ *     0 u32 agent[8]   32 u32 apple list length   36 u32 waste list length   40 i32 t   44 u32 episode | init << 31
+ *     48 f64 theta   64 u32 apple mask[8]   96 u32 waste mask[8]   128 f64 metrics[8]
+ *     192 u64 sum t*r[n]   192+8n f64 sum transferred[n]   192+16n f64 sum t*transferred[n]   192+24n u32 sum r[n]
+ *     L uint8 apple list (point indices, birth order; capacity LA = max(16, round16(#apple points)))   L+LA waste list
+ *     (the bytes behind each list's length are saved as 0)
+ *   selfdrive: row_bytes = round16(16 n + 40)
+ *     0 f64 pos[n]   8n f64 vel[n]   16n f64 theta   16n+8 f64 transfers metric   16n+16 f64 dist_to_front
+ *     16n+24 u32 crossing order (4 bits per entry)   16n+28 u32 n_crossed | done mask << 8 | all_done << 16 | init << 31
+ *     16n+32 i32 t   16n+36 u32 episode
+ * config_tag hashes a layout version and every ssd_config field except num_envs, first_env_id, seed, device and
+ * struct_size: rows move between handles of the same configuration whatever their size or place in a sharded run. */
+typedef struct ssd_checkpoint_layout {
+    int64_t row_bytes;        /* bytes of one env's row, a multiple of 16 */
+    uint64_t config_tag;      /* hash of everything that gives the row its meaning */
+} ssd_checkpoint_layout;
+int ssd_checkpoint_get_layout(const ssd_handle* h, ssd_checkpoint_layout* out);
+/* rows_dev uint8 [count][row_bytes] (16-byte aligned) <- the envs env_idx_dev[0..count) (int32 local indices; NULL: envs
+ * 0..count-1).  A row whose index is outside [0, E) is saved as zeros. */
+int ssd_checkpoint_save(ssd_handle* h, const int32_t* env_idx_dev, int32_t count, uint8_t* rows_dev, void* stream);
+/* rows_dev -> the envs env_idx_dev[0..count) (NULL: 0..count-1).  SSD_EINVAL before any launch when config_tag is not the
+ * handle's.  Each row is validated first — agents inside the map, orientation <= 3, no mask bits beyond the point lists,
+ * #waste = popcount of the waste mask, 0 <= t <= horizon (grid worlds); list lengths <= point counts, entries < point
+ * counts, each list setting exactly the bits of its presence mask (feature envs); n_crossed <= n, crossing-order entries
+ * < n, no entries beyond n_crossed (selfdrive) — and, like a row whose index is outside [0, E), written only when it
+ * passes: row_ok_dev[r] (uint8, nullable) = 1 if row r was loaded, else 0.  Duplicate destinations are the caller's error. */
+int ssd_checkpoint_load(ssd_handle* h, uint64_t config_tag, const int32_t* env_idx_dev, int32_t count, const uint8_t* rows_dev,
+                        uint8_t* row_ok_dev, void* stream);
+
 /* --- utilities ------------------------------------------------------------------------------------------ */
 /* uniform random action ids in [0, num_actions) for benchmark rollouts, uint8 [E][n];
  * drawn from Philox site 13 at counter `step_index` (no reference equivalent: RLlib's policy).
