@@ -58,6 +58,11 @@ class ssd_checkpoint_layout(ctypes.Structure):
     _fields_ = [("row_bytes", ctypes.c_int64), ("config_tag", ctypes.c_uint64)]
 
 
+class ssd_policy_out(ctypes.Structure):
+    _fields_ = [("struct_size", ctypes.c_int32), ("dtype", ctypes.c_int32), ("image_dev", ctypes.c_void_p),
+                ("contract_dev", ctypes.c_void_p)]
+
+
 STATS_LEN = 8
 
 
@@ -98,7 +103,7 @@ EXPORTS = [
     "ssd_global_view", "ssd_concat_obs", "ssd_solver_sample", "ssd_solver_choose", "ssd_policy_inputs", "ssd_record_beams", "ssd_render", "ssd_step_host",
     "ssd_step_host_async", "ssd_step_host_wait", "ssd_host_result_layout", "ssd_host_result_expand", "ssd_set_episode_stats",
     "ssd_feat_step_host_async", "ssd_selfdrive_step_host_async",
-    "ssd_checkpoint_get_layout", "ssd_checkpoint_save", "ssd_checkpoint_load",
+    "ssd_checkpoint_get_layout", "ssd_checkpoint_save", "ssd_checkpoint_load", "ssd_set_policy_output",
 ]
 
 _LIB = None
@@ -152,6 +157,7 @@ def load():
     L.ssd_record_beams.argtypes = [vp, i32]
     L.ssd_render.argtypes = [vp, vp, vp]
     L.ssd_policy_inputs.argtypes = [vp, vp, i64, i32, vp, vp, vp]
+    L.ssd_set_policy_output.argtypes = [vp, ctypes.POINTER(ssd_policy_out)]
     L.ssd_solver_choose.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp]
     L.ssd_feature_dim.argtypes = [vp]
     L.ssd_state_bytes_per_env.argtypes = [vp]

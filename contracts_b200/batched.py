@@ -127,12 +127,19 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin):
     utils/env_creator_functions.py:47-60).  contract: None or the class name from
     contract/contract_list.py.  theta_low/high default to the contract's gym Box bounds, which
     gym stores as float32 (contract_list.py:20,43) — the float32 rounding is part of parity.
+
+    policy_dtype: None (uint8 windows in `obs`, the reference's observation), or torch.float32 / float16 / bfloat16: the
+    env writes the policy's input tensors itself (ssd_set_policy_output) — `policy_image` T [E*n, 3, 15, 15], the value
+    `policy_inputs(T)` would make of the windows, and `policy_contract` T [E*n, 10] (None without a contract) — and keeps
+    no uint8 windows (`obs` is None).  reset / step / step_host return `policy_image` in place of `obs`.  The mode is fixed
+    for the env's lifetime; the methods that read the uint8 windows (host_snapshot(obs=True), concatenated_obs,
+    policy_inputs) raise ValueError in it.
     """
 
     def __init__(self, kind, num_envs, num_agents, ascii_map=None, horizon=1000, contract=None,
                  theta_low=0.0, theta_high=None, null_prob=0.0, seed=73907, first_env_id=0,
                  device=None, padded_obs=False,
-                 use_collective_reward=False, inequity_averse_reward=False, alpha=0.0, beta=0.0):
+                 use_collective_reward=False, inequity_averse_reward=False, alpha=0.0, beta=0.0, policy_dtype=None):
         if kind not in ("cleanup_new", "harvest_new"):
             raise ValueError("BatchedGridEnv kind must be cleanup_new or harvest_new, got %r" % (kind,))
         if not torch.cuda.is_available():
@@ -168,11 +175,25 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin):
         self._h = h
         self.F = self.lib.ssd_feature_dim(self._h)
         E, n, dev = self.E, self.n, self.device
-        # observation batch tensor: dense [E, n, 15, 15, 3], or env stride padded to 16 B
-        dense = n * _lib.OBS_BYTES_PER_AGENT
-        self.obs_stride = (dense + 15) // 16 * 16 if padded_obs else dense
-        self._obs_buf = torch.zeros((E, self.obs_stride), dtype=torch.uint8, device=dev)
-        self.obs = self._obs_buf[:, :dense].view(E, n, 15, 15, 3) if padded_obs else self._obs_buf.view(E, n, 15, 15, 3)
+        self.policy_dtype, self.policy_image, self.policy_contract = policy_dtype, None, None
+        if policy_dtype is not None:
+            if policy_dtype not in self._POLICY_DTYPES:
+                self.close()
+                raise ValueError("policy_dtype must be None, torch.float32, torch.float16 or torch.bfloat16, got %r" % (policy_dtype,))
+            self.policy_image = torch.zeros((E * n, 3, 15, 15), dtype=policy_dtype, device=dev)
+            if contract is not None:
+                self.policy_contract = torch.zeros((E * n, 10), dtype=policy_dtype, device=dev)
+            out = _lib.ssd_policy_out(struct_size=ctypes.sizeof(_lib.ssd_policy_out), dtype=self._POLICY_DTYPES[policy_dtype],
+                                      image_dev=self.policy_image.data_ptr(),
+                                      contract_dev=None if self.policy_contract is None else self.policy_contract.data_ptr())
+            _lib.check(self._h, self.lib.ssd_set_policy_output(self._h, ctypes.byref(out)))
+            self.obs_stride, self._obs_buf, self.obs = 0, None, None
+        else:
+            # observation batch tensor: dense [E, n, 15, 15, 3], or env stride padded to 16 B
+            dense = n * _lib.OBS_BYTES_PER_AGENT
+            self.obs_stride = (dense + 15) // 16 * 16 if padded_obs else dense
+            self._obs_buf = torch.zeros((E, self.obs_stride), dtype=torch.uint8, device=dev)
+            self.obs = self._obs_buf[:, :dense].view(E, n, 15, 15, 3) if padded_obs else self._obs_buf.view(E, n, 15, 15, 3)
         self.rew = torch.zeros((E, n), dtype=torch.float64, device=dev)
         self.base_rew = torch.zeros((E, n), dtype=torch.float64, device=dev)
         self.transfers = torch.zeros((E, n), dtype=torch.float64, device=dev)
@@ -197,12 +218,27 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin):
     def _stream(self):
         return ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
+    @property
+    def observation(self):
+        """what reset / step return: `obs`, or `policy_image` when the env writes the policy's tensors"""
+        return self.obs if self.policy_dtype is None else self.policy_image
+
+    def _need_windows(self, what):
+        if self.policy_dtype is not None:
+            raise ValueError("%s needs the uint8 observation windows; this env writes the policy's tensors instead "
+                             "(policy_dtype=%s)" % (what, self.policy_dtype))
+
+    def _obs_rows(self):
+        """the observation rows checkpoint / restore carry: uint8 [E, n, 15, 15, 3], or T [E, n, 3, 15, 15] in policy mode"""
+        return self.obs if self.policy_dtype is None else self.policy_image.view(self.E, self.n, 3, 15, 15)
+
     def reset(self, mask=None):
-        """Reset all envs (mask None) or those with mask != 0 (uint8 CUDA tensor [E]).  Returns obs."""
+        """Reset all envs (mask None) or those with mask != 0 (uint8 CUDA tensor [E]).  Returns obs (policy_image in
+        policy mode)."""
         if mask is not None:
             mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
         _lib.check(self._h, self.lib.ssd_reset(self._h, _ptr(mask), _ptr(self._obs_buf), self.obs_stride, self._stream()))
-        return self.obs
+        return self.observation
 
     def _auto_reset_io(self, io, auto_reset, negotiation):
         """vectorised-sampler mode of a step: finished envs restart inside the step (+ negotiate, given the policy's
@@ -231,7 +267,7 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin):
             self.feature_obs = torch.zeros((self.E, self.n, self.F), dtype=torch.float64, device=self.device)
         io = self._io
         io.actions_dev = actions.data_ptr()
-        io.obs_dev = self._obs_buf.data_ptr()
+        io.obs_dev = None if self._obs_buf is None else self._obs_buf.data_ptr()
         io.obs_env_stride = self.obs_stride
         io.rew_dev = self.rew.data_ptr()
         io.base_rew_dev = self.base_rew.data_ptr() if extras else None
@@ -241,7 +277,7 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin):
         io.done_dev = self.done.data_ptr()
         self._auto_reset_io(io, auto_reset, negotiation)
         _lib.check(self._h, self.lib.ssd_step(self._h, ctypes.byref(io), self._stream()))
-        return self.obs, self.rew, self.done, self.info
+        return self.observation, self.rew, self.done, self.info
 
     def step_host(self, actions_host, rew_host, done_host=None, want_features=False):
         """One step for a caller holding HOST tensors (pinned for asynchronous copies): uint8 actions [E, n] in,
@@ -256,7 +292,7 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin):
             self.feature_obs = torch.zeros((self.E, self.n, self.F), dtype=torch.float64, device=self.device)
         io = self._io
         io.actions_dev = self._host_actions_dev.data_ptr()
-        io.obs_dev = self._obs_buf.data_ptr()
+        io.obs_dev = None if self._obs_buf is None else self._obs_buf.data_ptr()
         io.obs_env_stride = self.obs_stride
         io.rew_dev = self.rew.data_ptr()
         io.base_rew_dev = None
@@ -269,7 +305,7 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin):
                                                    ctypes.c_void_p(rew_host.data_ptr()),
                                                    ctypes.c_void_p(done_host.data_ptr()) if done_host is not None else None,
                                                    self._stream()))
-        return self.obs, rew_host, done_host
+        return self.observation, rew_host, done_host
 
     # ---- pipelined host-buffer step (RLlib BaseEnv send_actions / poll shape) ---------------------------------
     def step_host_async(self, actions_host, result, want_features=False, dense_rewards=False, auto_reset=False, negotiation=None):
@@ -283,7 +319,7 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin):
             self.feature_obs = torch.zeros((self.E, self.n, self.F), dtype=torch.float64, device=self.device)
         io = self._io
         io.actions_dev = None
-        io.obs_dev = self._obs_buf.data_ptr()
+        io.obs_dev = None if self._obs_buf is None else self._obs_buf.data_ptr()
         io.obs_env_stride = self.obs_stride
         io.rew_dev = self.rew.data_ptr() if dense_rewards else None
         io.base_rew_dev = None
@@ -303,6 +339,8 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin):
         copied to the host with ONE transfer + ONE synchronisation.  Returns numpy views:
         obs uint8 [.., n, 15, 15, 3], rew / base_rew / transfers float64 [.., n], info uint8 [.., n, 4], done uint8 [..],
         feat float64 [.., n, F] (when `features`)."""
+        if obs:
+            self._need_windows("host_snapshot(obs=True)")
         sel = slice(None) if index is None else slice(index, index + 1)
         E = self.E if index is None else 1
         parts = [("rew", self.rew[sel], np.float64, (E, self.n)), ("info", self.info[sel], np.uint8, (E, self.n, 4)),
@@ -382,6 +420,7 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin):
 
     def concatenated_obs(self, out=None):
         """The agents' windows concatenated along the channel axis (two_stage_train.py:527-533): uint8 [E, 15, 15, 3 n]."""
+        self._need_windows("concatenated_obs")
         if out is None:
             out = torch.empty((self.E, 15, 15, 3 * self.n), dtype=torch.uint8, device=self.device)
         _lib.check(self._h, self.lib.ssd_concat_obs(self._h, _ptr(self._obs_buf), self.obs_stride, _ptr(out), self._stream()))
@@ -392,7 +431,9 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin):
 
     def policy_inputs(self, dtype=torch.float32, with_contract=True, image=None, contract=None):
         """The current observations as VisionNetwork.forward feeds its convolutions: image [E*n, 3, 15, 15] =
-        (`curr_obs / 255`).float().permute(0, 3, 1, 2), contract [E*n, 10] = (theta, 0) repeated 5 times."""
+        (`curr_obs / 255`).float().permute(0, 3, 1, 2), contract [E*n, 10] = (theta, 0) repeated 5 times.
+        (With policy_dtype set the env writes these itself: policy_image / policy_contract.)"""
+        self._need_windows("policy_inputs")
         B = self.E * self.n
         if image is None:
             image = torch.empty((B, 3, 15, 15), dtype=dtype, device=self.device)

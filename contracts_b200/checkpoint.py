@@ -27,8 +27,9 @@ _VERSION = 1
 class EnvCheckpoint:
     """Rows of env state with their global ids.  kind: the env kind string; config_tag / row_bytes: the layout the rows
     were saved under (ssd_checkpoint_layout); seed: the handle's seed; env_ids int64 [count]; rows uint8 [count,
-    row_bytes]; obs: the observation rows of those envs or None (uint8 [count, n, 15, 15, 3] for the grid worlds,
-    float64 [count, n, F | D] for the feature envs and selfdrive)."""
+    row_bytes]; obs: the observation rows of those envs or None (uint8 [count, n, 15, 15, 3] for the grid worlds, T
+    [count, n, 3, 15, 15] for a grid world with policy_dtype T, float64 [count, n, F | D] for the feature envs and
+    selfdrive).  The rows themselves do not depend on the observation form."""
 
     def __init__(self, kind, config_tag, row_bytes, seed, env_ids, rows, obs=None):
         self.kind, self.config_tag, self.row_bytes, self.seed = str(kind), int(config_tag), int(row_bytes), int(seed)
@@ -101,7 +102,10 @@ def _index_tensor(envs, E, device, what):
 
 class CheckpointMixin:
     """checkpoint / restore / copy_envs for BatchedGridEnv, BatchedFeatureEnv and BatchedCarEnv.  The host classes
-    provide _h, lib, E, device, kind, seed, first_env_id and obs."""
+    provide _h, lib, E, device, kind, seed, first_env_id and obs (or _obs_rows())."""
+
+    def _obs_rows(self):
+        return self.obs
 
     def checkpoint_layout(self):
         lay = _lib.ssd_checkpoint_layout()
@@ -123,19 +127,27 @@ class CheckpointMixin:
                                                          count, ctypes.c_void_p(rows.data_ptr()), self._stream()))
         obs = None
         if with_obs:
-            obs = self.obs.clone() if envs is None else self.obs.index_select(0, local)
+            rows_obs = self._obs_rows()
+            obs = rows_obs.clone() if envs is None else rows_obs.index_select(0, local)
         return EnvCheckpoint(self.kind, lay.config_tag, lay.row_bytes, self.seed, local + self.first_env_id, rows, obs)
 
     def restore(self, ck, envs=None):
         """Load the rows of `ck`: into the local envs with the same global ids (envs None: same seed required), or into
         the local envs `envs` (one per row, distinct), which continue on their own random streams.  The observation
-        rows, when the checkpoint holds them, are written to self.obs.  Raises SsdError on a configuration mismatch and
-        naming the rows that failed validation (they are not written; the others are)."""
+        rows, when the checkpoint holds them, are written to self.obs (a grid world's policy_image in policy mode; its
+        policy_contract rows follow the loaded theta).  Raises SsdError on a configuration mismatch and naming the rows
+        that failed validation (they are not written; the others are); ValueError when the checkpoint's observation rows
+        are of another form than the env's (with_obs=False checkpoints restore across forms)."""
         lay = self.checkpoint_layout()
         if ck.config_tag != lay.config_tag or ck.row_bytes != lay.row_bytes:
             raise _lib.SsdError("restore: checkpoint of another configuration (kind %r, config_tag %016x, row_bytes %d; this "
                                 "%s handle has config_tag %016x, row_bytes %d)" % (ck.kind, ck.config_tag, ck.row_bytes,
                                                                                  self.kind, lay.config_tag, lay.row_bytes))
+        own = self._obs_rows()
+        if ck.obs is not None and (ck.obs.dtype != own.dtype or tuple(ck.obs.shape[1:]) != tuple(own.shape[1:])):
+            raise ValueError("restore: the checkpoint's observation rows are %s %s, this env's are %s %s (another observation "
+                             "form; restore a checkpoint taken with with_obs=False)" % (ck.obs.dtype, tuple(ck.obs.shape[1:]),
+                                                                                      own.dtype, tuple(own.shape[1:])))
         if envs is None:
             if ck.seed != self.seed:
                 raise _lib.SsdError("restore: checkpoint seed %d != handle seed %d (pass envs= to branch across seeds)"
@@ -164,9 +176,9 @@ class CheckpointMixin:
         if ck.obs is not None:
             obs = ck.obs.to(self.device)
             if all_ok:
-                self.obs[dst] = obs
+                own[dst] = obs
             else:
-                self.obs[dst[good]] = obs[good]
+                own[dst[good]] = obs[good]
         if not all_ok:
             bad = torch.nonzero(~good).reshape(-1).cpu().tolist()
             raise _lib.SsdError("restore: rows %s failed validation (corrupt or not saved from this configuration); they were "

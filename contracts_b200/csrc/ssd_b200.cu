@@ -63,23 +63,53 @@ struct ssd_handle {
     int64_t launches;
     CkParams ck;             // ssd_checkpoint_*: where each part of an env's row lives (ssd_checkpoint.cuh)
     uint64_t config_tag;     // ssd_checkpoint_get_layout: hash of everything that gives a row its meaning
+    int pol_form;            // ssd_set_policy_output: OBS_U8 (none) or 1 + SSD_POLICY_*, the form the observe / reset kernels write
+    uint8_t* pol_image;      //   T [E n][3][15][15]
+    void* pol_contract;      //   T [E n][10] or NULL
     char err[512];
     std::vector<void*> dev_allocs;
 };
 
 typedef void (*obs_kernel_t)(const GridParams, const StepIO, uint32_t*);
-template <int KIND>
+template <int KIND, int FORM>
 static obs_kernel_t obs_pick(bool rounds4, bool feat)
 {
-    if (rounds4) return feat ? grid_obs_kernel<KIND, 4, true, 0> : grid_obs_kernel<KIND, 4, false, 0>;
-    return feat ? grid_obs_kernel<KIND, MAX_POINT_ROUNDS, true, 0> : grid_obs_kernel<KIND, MAX_POINT_ROUNDS, false, 0>;
+    if (rounds4) return feat ? grid_obs_kernel<KIND, 4, true, 0, FORM> : grid_obs_kernel<KIND, 4, false, 0, FORM>;
+    return feat ? grid_obs_kernel<KIND, MAX_POINT_ROUNDS, true, 0, FORM> : grid_obs_kernel<KIND, MAX_POINT_ROUNDS, false, 0, FORM>;
 }
-// lay: 0, or 1 when the handle matches OBS_LAY_CLEANUP8 (stock cleanup map, 8 agents, dense observation tensor, no feature_obs)
-static obs_kernel_t obs_kernel_fn(int kind, bool rounds4, bool feat, int lay = 0)
+template <int FORM>
+static obs_kernel_t obs_form_fn(int kind, bool rounds4, bool feat, int lay)
 {
-    if (lay == 1 && kind == SSD_ENV_CLEANUP && rounds4 && !feat) return grid_obs_kernel<SSD_ENV_CLEANUP, 4, false, 1>;
-    if (lay == 2 && kind == SSD_ENV_HARVEST && !rounds4 && !feat) return grid_obs_kernel<SSD_ENV_HARVEST, MAX_POINT_ROUNDS, false, 2>;
-    return kind == SSD_ENV_CLEANUP ? obs_pick<SSD_ENV_CLEANUP>(rounds4, feat) : obs_pick<SSD_ENV_HARVEST>(rounds4, feat);
+    if (lay == 1 && kind == SSD_ENV_CLEANUP && rounds4 && !feat) return grid_obs_kernel<SSD_ENV_CLEANUP, 4, false, 1, FORM>;
+    if (lay == 2 && kind == SSD_ENV_HARVEST && !rounds4 && !feat) return grid_obs_kernel<SSD_ENV_HARVEST, MAX_POINT_ROUNDS, false, 2, FORM>;
+    return kind == SSD_ENV_CLEANUP ? obs_pick<SSD_ENV_CLEANUP, FORM>(rounds4, feat) : obs_pick<SSD_ENV_HARVEST, FORM>(rounds4, feat);
+}
+// lay: 0, or 1 when the handle matches OBS_LAY_CLEANUP8 (stock cleanup map, 8 agents, dense observation tensor, no feature_obs);
+// form: OBS_U8 or the policy form of ssd_set_policy_output (1 + SSD_POLICY_*)
+static obs_kernel_t obs_kernel_fn(int kind, bool rounds4, bool feat, int lay = 0, int form = OBS_U8)
+{
+    if (form == 1 + POLICY_F32) return obs_form_fn<1 + POLICY_F32>(kind, rounds4, feat, lay);
+    if (form == 1 + POLICY_F16) return obs_form_fn<1 + POLICY_F16>(kind, rounds4, feat, lay);
+    if (form == 1 + POLICY_BF16) return obs_form_fn<1 + POLICY_BF16>(kind, rounds4, feat, lay);
+    return obs_form_fn<OBS_U8>(kind, rounds4, feat, lay);
+}
+typedef void (*reset_kernel_t)(const GridParams, const uint8_t*, uint8_t*, long long, const StepIO, void*);
+template <int KIND>
+static reset_kernel_t reset_pick(int form)
+{
+    if (form == 1 + POLICY_F32) return grid_reset_kernel<KIND, 1 + POLICY_F32>;
+    if (form == 1 + POLICY_F16) return grid_reset_kernel<KIND, 1 + POLICY_F16>;
+    if (form == 1 + POLICY_BF16) return grid_reset_kernel<KIND, 1 + POLICY_BF16>;
+    return grid_reset_kernel<KIND, OBS_U8>;
+}
+static reset_kernel_t reset_kernel_fn(int kind, int form)
+{
+    return kind == SSD_ENV_CLEANUP ? reset_pick<SSD_ENV_CLEANUP>(form) : reset_pick<SSD_ENV_HARVEST>(form);
+}
+// bytes of one env's block of the policy image tensor
+static long long policy_env_bytes(const GridParams& p, int form)
+{
+    return (long long)p.n * SSD_OBS_BYTES * (form == 1 + POLICY_F32 ? 4 : 2);
 }
 typedef void (*logic_kernel_t)(const GridParams, const StepIO, uint32_t*);
 static logic_kernel_t logic_kernel_fn(int kind, int lay)
@@ -374,7 +404,7 @@ static int setup_grid(ssd_handle* h)
 
     int sms = 0, per_sm = 0;
     CUDA_TRY(h, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c.device));
-    const void* reset_k = cleanup ? (const void*)grid_reset_kernel<SSD_ENV_CLEANUP> : (const void*)grid_reset_kernel<SSD_ENV_HARVEST>;
+    const void* reset_k = (const void*)reset_kernel_fn(c.env_kind, OBS_U8);
     CUDA_TRY(h, cudaFuncSetAttribute(reset_k, cudaFuncAttributeMaxDynamicSharedMemorySize, p.g2_smem_bytes));
     CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, reset_k, GRID_THREADS, p.g2_smem_bytes));
     if (per_sm < 1) return fail(h, SSD_EUNSUPPORTED, "reset kernel does not fit on an SM (smem %d B)", p.g2_smem_bytes);
@@ -741,11 +771,24 @@ __global__ void set_state_kernel(GridParams p, const uint8_t* map, const int32_t
     *reinterpret_cast<uint32_t*>(hdr + RO_FLAGS) = ((f | 0x80000000u) & ~RF_STALE_EMPTY) | (bad << RF_ERR_SHIFT);
 }
 
-__global__ void set_theta_kernel(GridParams p, const double* theta)
+// pcontract (nullable): the policy output's contract rows (ssd_set_policy_output), kept current
+__global__ void set_theta_kernel(GridParams p, const double* theta, void* pcontract, int pdtype)
 {
     int env = blockIdx.x * blockDim.x + threadIdx.x;
     if (env >= p.E) return;
     *reinterpret_cast<double*>(p.state + (size_t)env * p.rec_stride + RO_THETA) = theta[env];
+    if (pcontract) policy_contract_env(pcontract, pdtype, p.n, env, theta[env]);
+}
+
+// checkpoint load with a policy output set: the contract rows of the loaded envs from their (new) theta.  Rows that failed
+// validation kept their theta, so rewriting theirs changes nothing.
+__global__ void policy_contract_refresh_kernel(GridParams p, const int32_t* env_idx, int count, void* pcontract, int pdtype)
+{
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= count) return;
+    const int env = env_idx ? env_idx[r] : r;
+    if (env < 0 || env >= p.E) return;
+    policy_contract_env(pcontract, pdtype, p.n, env, *reinterpret_cast<const double*>(p.state + (size_t)env * p.rec_stride + RO_THETA));
 }
 
 __global__ void get_metrics_kernel(GridParams p, double* out)
@@ -787,8 +830,10 @@ __global__ void negotiate_kernel(SolverParams p, const uint8_t* mask, const doub
     if (mask && !mask[env]) return;
     const uint32_t episode = *reinterpret_cast<const uint32_t*>(p.episode + (size_t)env * p.episode_stride) & p.episode_mask;
     const bool dec = negotiate_agreement(p.seed, p.first_env_id + (uint32_t)env, episode, p.n, accept + (size_t)env * p.n);
-    *reinterpret_cast<double*>(p.theta + (size_t)env * p.theta_stride) = dec ? proposals[env] : 0.0;
+    const double theta = dec ? proposals[env] : 0.0;
+    *reinterpret_cast<double*>(p.theta + (size_t)env * p.theta_stride) = theta;
     if (decision) decision[env] = dec ? 1 : 0;
+    if (p.pol_contract) policy_contract_env(p.pol_contract, p.pol_dtype, p.n, env, theta);
 }
 
 // step_index == SSD_STEP_AUTO: take the index from the handle's device counter (bumped by the last CTA to finish,
@@ -939,13 +984,16 @@ int ssd_reset(ssd_handle* h, const uint8_t* mask_dev, uint8_t* obs_dev, int64_t 
     REQUIRE_GRID(h);
     const GridParams& p = h->gp;
     long long stride = obs_env_stride ? obs_env_stride : (long long)p.n * SSD_OBS_BYTES;
+    if (h->pol_form) {                                   // one observation form per handle: the policy output's
+        if (obs_dev) return fail(h, SSD_EINVAL, "reset: obs_dev must be NULL while a policy output is set (ssd_set_policy_output)");
+        obs_dev = h->pol_image;
+        stride = policy_env_bytes(p, h->pol_form);
+    }
     if (stride < (long long)p.n * SSD_OBS_BYTES) return fail(h, SSD_EINVAL, "obs_env_stride too small");
     cudaStream_t s = (cudaStream_t)stream;
     if (p.beam) beam_clear_kernel<<<(p.E + 3) / 4, 128, 0, s>>>(p, mask_dev);                 // self.beam_pos = [] (map_env.py:316)
-    if (p.kind == SSD_ENV_CLEANUP)
-        grid_reset_kernel<SSD_ENV_CLEANUP><<<h->grid_blocks, GRID_THREADS, p.g2_smem_bytes, s>>>(p, mask_dev, obs_dev, stride, StepIO());
-    else
-        grid_reset_kernel<SSD_ENV_HARVEST><<<h->grid_blocks, GRID_THREADS, p.g2_smem_bytes, s>>>(p, mask_dev, obs_dev, stride, StepIO());
+    reset_kernel_fn(p.kind, h->pol_form)<<<h->grid_blocks, GRID_THREADS, p.g2_smem_bytes, s>>>(p, mask_dev, obs_dev, stride, StepIO(),
+                                                                                                h->pol_contract);
     return check_launch(h, "reset");
 }
 
@@ -953,12 +1001,18 @@ static int make_step_io(ssd_handle* h, const ssd_step_io* io, StepIO& k, bool as
 {
     memset(&k, 0, sizeof(k));
     if (!async_host && (!io->actions_dev || !io->rew_dev)) return fail(h, SSD_EINVAL, "actions_dev, obs_dev and rew_dev are required");
-    if (!io->obs_dev) return fail(h, SSD_EINVAL, "obs_dev is required");
     const GridParams& p = h->gp;
+    if (h->pol_form) {                                   // one observation form per handle: the policy output's
+        if (io->obs_dev) return fail(h, SSD_EINVAL, "obs_dev must be NULL while a policy output is set (ssd_set_policy_output)");
+        k.obs = h->pol_image;
+        k.obs_stride = policy_env_bytes(p, h->pol_form);
+    } else {
+        if (!io->obs_dev) return fail(h, SSD_EINVAL, "obs_dev is required");
+        k.obs = io->obs_dev;
+        k.obs_stride = io->obs_env_stride ? io->obs_env_stride : (long long)p.n * SSD_OBS_BYTES;
+        if (k.obs_stride < (long long)p.n * SSD_OBS_BYTES) return fail(h, SSD_EINVAL, "obs_env_stride too small");
+    }
     k.actions = (const uint8_t*)io->actions_dev;
-    k.obs = io->obs_dev;
-    k.obs_stride = io->obs_env_stride ? io->obs_env_stride : (long long)p.n * SSD_OBS_BYTES;
-    if (k.obs_stride < (long long)p.n * SSD_OBS_BYTES) return fail(h, SSD_EINVAL, "obs_env_stride too small");
     k.rew = io->rew_dev; k.base_rew = io->base_rew_dev; k.transfers = io->transfers_dev;
     k.info = io->info_dev; k.feat = io->feature_obs_dev; k.done = io->done_dev;
     if (k.info && (reinterpret_cast<uintptr_t>(k.info) & 3)) return fail(h, SSD_EINVAL, "info_dev must be 4-byte aligned");
@@ -1028,8 +1082,9 @@ static int launch_step(ssd_handle* h, const StepIO& k, cudaStream_t s, const Hos
     if (hc && hc->slot >= 0) CUDA_TRY(h, cudaEventRecord(h->slot[hc->slot].ev_logic, s));   // the slot's actions were read
     if (p.kind == SSD_ENV_CLEANUP) { int rc = copy_rewards(h, k, s, hc); if (rc) return rc; }
     // programmatic dependent launch: the observe CTAs become resident (tables, tiles) as the one-wave logic grid drains
-    const int lay = (h->obs_lay != 0 && k.obs_stride == (long long)p.n * SSD_OBS_BYTES && !k.feat) ? h->obs_lay : 0;
-    const obs_kernel_t obs_k = obs_kernel_fn(p.kind, h->rounds4, k.feat != nullptr, lay);
+    const bool dense = h->pol_form || k.obs_stride == (long long)p.n * SSD_OBS_BYTES;       // a policy image is always dense
+    const int lay = (h->obs_lay != 0 && dense && !k.feat) ? h->obs_lay : 0;
+    const obs_kernel_t obs_k = obs_kernel_fn(p.kind, h->rounds4, k.feat != nullptr, lay, h->pol_form);
     if (h->pdl && !h->timing) CUDA_TRY(h, launch_pdl(obs_k, dim3(h->obs_blocks), dim3(OBS_WARPS * 32), (size_t)p.g2_smem_bytes, s, p, k, h->d_res));
     else obs_k<<<h->obs_blocks, OBS_WARPS * 32, p.g2_smem_bytes, s>>>(p, k, h->d_res);
     if (p.kind == SSD_ENV_HARVEST) {
@@ -1042,14 +1097,11 @@ static int launch_step(ssd_handle* h, const StepIO& k, cudaStream_t s, const Hos
         h->launches++;
         // (the copy_rewards event record of the host paths sits between the harvest reward kernel and this launch: plain launch then)
         const bool pdl_ok = h->pdl && !h->timing && (p.kind == SSD_ENV_CLEANUP || !hc);
-        if (p.kind == SSD_ENV_CLEANUP && pdl_ok)
-            CUDA_TRY(h, launch_pdl(grid_reset_kernel<SSD_ENV_CLEANUP>, dim3(h->grid_blocks), dim3(GRID_THREADS), (size_t)p.g2_smem_bytes, s,
-                                   p, (const uint8_t*)k.done, k.obs, k.obs_stride, k));
-        else if (pdl_ok)
-            CUDA_TRY(h, launch_pdl(grid_reset_kernel<SSD_ENV_HARVEST>, dim3(h->grid_blocks), dim3(GRID_THREADS), (size_t)p.g2_smem_bytes, s,
-                                   p, (const uint8_t*)k.done, k.obs, k.obs_stride, k));
-        else if (p.kind == SSD_ENV_CLEANUP) grid_reset_kernel<SSD_ENV_CLEANUP><<<h->grid_blocks, GRID_THREADS, p.g2_smem_bytes, s>>>(p, k.done, k.obs, k.obs_stride, k);
-        else grid_reset_kernel<SSD_ENV_HARVEST><<<h->grid_blocks, GRID_THREADS, p.g2_smem_bytes, s>>>(p, k.done, k.obs, k.obs_stride, k);
+        const reset_kernel_t reset_k = reset_kernel_fn(p.kind, h->pol_form);
+        if (pdl_ok)
+            CUDA_TRY(h, launch_pdl(reset_k, dim3(h->grid_blocks), dim3(GRID_THREADS), (size_t)p.g2_smem_bytes, s,
+                                   p, (const uint8_t*)k.done, k.obs, k.obs_stride, k, h->pol_contract));
+        else reset_k<<<h->grid_blocks, GRID_THREADS, p.g2_smem_bytes, s>>>(p, k.done, k.obs, k.obs_stride, k, h->pol_contract);
     }
     if (h->timing) cudaEventRecord(h->tev[2], s);
     return check_launch(h, "step");
@@ -1272,7 +1324,7 @@ int ssd_set_contract_params(ssd_handle* h, const double* theta_dev, void* stream
     else if (IS_FEAT(h))
         feat_set_theta_kernel<<<(h->fp.E + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->fp, theta_dev);
     else
-        SMALL_LAUNCH(set_theta_kernel, theta_dev);
+        SMALL_LAUNCH(set_theta_kernel, theta_dev, h->pol_contract, h->pol_form - 1);
     return check_launch(h, "set_contract_params");
 }
 
@@ -1363,6 +1415,37 @@ int ssd_policy_inputs(ssd_handle* h, const uint8_t* obs_dev, int64_t obs_env_str
     return check_launch(h, "policy_inputs");
 }
 
+int ssd_set_policy_output(ssd_handle* h, const ssd_policy_out* out)
+{
+    if (!h) return SSD_EINVAL;
+    ON_DEVICE(h);
+    REQUIRE_GRID(h);
+    if (!out) { h->pol_form = OBS_U8; h->pol_image = nullptr; h->pol_contract = nullptr; return SSD_OK; }
+    if (out->struct_size < (int32_t)sizeof(ssd_policy_out))
+        return fail(h, SSD_EINVAL, "ssd_policy_out.struct_size %d < %d: the caller's declaration of ssd_policy_out is out of date",
+                    out->struct_size, (int)sizeof(ssd_policy_out));
+    if (out->dtype != POLICY_F32 && out->dtype != POLICY_F16 && out->dtype != POLICY_BF16)
+        return fail(h, SSD_EINVAL, "set_policy_output: dtype %d is not SSD_POLICY_F32, _F16 or _BF16", out->dtype);
+    if (!out->image_dev || (reinterpret_cast<uintptr_t>(out->image_dev) & 15))
+        return fail(h, SSD_EINVAL, "set_policy_output: image_dev must be a 16-byte aligned device pointer");
+    const uintptr_t esize = out->dtype == POLICY_F32 ? 4 : 2;
+    if (reinterpret_cast<uintptr_t>(out->contract_dev) & (esize - 1))
+        return fail(h, SSD_EINVAL, "set_policy_output: contract_dev must be aligned to its element size");
+    const int form = 1 + out->dtype;
+    const GridParams& p = h->gp;
+    for (int feat = 0; feat < 2; feat++)
+        CUDA_TRY(h, cudaFuncSetAttribute((const void*)obs_kernel_fn(p.kind, h->rounds4, feat != 0, 0, form),
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, p.g2_smem_bytes));
+    if (h->obs_lay) CUDA_TRY(h, cudaFuncSetAttribute((const void*)obs_kernel_fn(p.kind, h->rounds4, false, h->obs_lay, form),
+                                                     cudaFuncAttributeMaxDynamicSharedMemorySize, p.g2_smem_bytes));
+    CUDA_TRY(h, cudaFuncSetAttribute((const void*)reset_kernel_fn(p.kind, form), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                     p.g2_smem_bytes));
+    h->pol_form = form;
+    h->pol_image = (uint8_t*)out->image_dev;
+    h->pol_contract = out->contract_dev;
+    return SSD_OK;
+}
+
 // ---- NegotiationSolver (two_stage_train.py:619-776) ------------------------------------------------
 static SolverParams solver_params(ssd_handle* h)
 {
@@ -1381,6 +1464,7 @@ static SolverParams solver_params(ssd_handle* h)
         const GridParams& p = h->gp;
         s.episode = p.state + RO_EPISODE; s.episode_stride = p.rec_stride; s.episode_mask = 0xFFFFFFFFu;
         s.theta = p.state + RO_THETA; s.theta_stride = p.rec_stride;
+        s.pol_contract = h->pol_contract; s.pol_dtype = h->pol_form - 1;
     }
     return s;
 }
@@ -1628,7 +1712,13 @@ int ssd_checkpoint_load(ssd_handle* h, uint64_t config_tag, const int32_t* env_i
     if (rc || count == 0) return rc;
     ck_load_kernel<<<(count + CK_ROWS - 1) / CK_ROWS, CK_THREADS, (size_t)CK_ROWS * h->ck.row_bytes, (cudaStream_t)stream>>>(
         h->ck, env_idx_dev, count, rows_dev, row_ok_dev);
-    return check_launch(h, "checkpoint_load");
+    if ((rc = check_launch(h, "checkpoint_load"))) return rc;
+    if (h->pol_contract) {                                // theta came with the rows: the policy's contract rows follow it
+        policy_contract_refresh_kernel<<<(count + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->gp, env_idx_dev, count, h->pol_contract,
+                                                                                              h->pol_form - 1);
+        return check_launch(h, "checkpoint_load");
+    }
+    return SSD_OK;
 }
 
 int ssd_enable_timing(ssd_handle* h, int32_t on)

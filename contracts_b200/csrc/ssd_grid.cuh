@@ -17,7 +17,28 @@
 //   environments/harvest_new.py  step :181-239, spawn_apples :284-317, count_apples_in_radius :326-336
 //   contract/contract_list.py :22-27, :45-54 ; environments/two_stage_train.py :62-121, :159-187
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include "ssd_common.cuh"
+
+// element types of the policy's input tensors (SSD_POLICY_*: ssd_policy_inputs, ssd_set_policy_output)
+#define POLICY_F32 0
+#define POLICY_F16 1
+#define POLICY_BF16 2
+
+template <typename T> __device__ __forceinline__ T policy_cast(float v);
+template <> __device__ __forceinline__ float policy_cast<float>(float v) { return v; }
+template <> __device__ __forceinline__ __half policy_cast<__half>(float v) { return __float2half_rn(v); }
+template <> __device__ __forceinline__ __nv_bfloat16 policy_cast<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+
+// Observation form written by the observe / reset kernels: OBS_U8 = the uint8 windows [E][n][15][15][3]; 1 + POLICY_* = the
+// policy's image tensor T [E n][3][15][15] (ssd_set_policy_output), the values ssd_policy_inputs would make of the windows.
+#define OBS_U8 0
+template <int FORM> struct ObsForm;
+template <> struct ObsForm<OBS_U8> { typedef uint8_t T; };
+template <> struct ObsForm<1 + POLICY_F32> { typedef float T; };
+template <> struct ObsForm<1 + POLICY_F16> { typedef __half T; };
+template <> struct ObsForm<1 + POLICY_BF16> { typedef __nv_bfloat16 T; };
 
 #ifndef GRID_WARPS
 #define GRID_WARPS 8
@@ -696,6 +717,51 @@ __device__ __forceinline__ void obs_stream_store(int lane, uint8_t* stage, int s
 }
 
 
+// view descriptor of an agent at tile offset ao for byte-step reads over T (gather_obs): {out[0][0], pixel step, row step, 0}
+__device__ __forceinline__ int4 view_desc(int ao, int ori, int S)
+{
+    const int origin = ao - SSD_VIEW * S - SSD_VIEW;     // V[0][0] of this lane's agent
+    const int last = SSD_OBSW - 1;
+    int start0 = origin, step = 1, rs = S;               // UP
+    if (ori == ORI_RIGHT) { start0 = origin + last * S; step = -S; rs = 1; }
+    else if (ori == ORI_DOWN) { start0 = origin + last * S + last; step = -1; rs = -S; }
+    else if (ori == ORI_LEFT) { start0 = origin + last; step = S; rs = -1; }
+    return make_int4(start0, step, rs, 0);
+}
+
+// view descriptor for word reads over T and its transpose T2 (gather_obs2, see there): {lowest byte of out row 0's run, row
+// step, backwards, 0}
+__device__ __forceinline__ int4 view_desc2(const GridParams& p, int ao, int ori)
+{
+    const int S = p.S, S2 = p.S2;
+    const uint32_t trow = __umulhi((uint32_t)ao, p.s_magic);            // ao / S
+    const int row = (int)trow - SSD_VIEW, col = ao - (int)trow * S - 8;
+    const int origin = ao - SSD_VIEW * S - SSD_VIEW;                     // V[0][0] in T
+    const int origin2 = p.tile2_off + (col + SSD_VIEW) * S2 + 8 + row - SSD_VIEW * S2 - SSD_VIEW;   // V[0][0] in T2
+    const int last = SSD_OBSW - 1;
+    int lo0 = origin, rstep = S, back = 0;                                // UP
+    if (ori == ORI_DOWN) { lo0 = origin + last * S; rstep = -S; back = 1; }
+    else if (ori == ORI_LEFT) { lo0 = origin2 + last * S2; rstep = -S2; }
+    else if (ori == ORI_RIGHT) { lo0 = origin2; rstep = S2; back = 1; }
+    return make_int4(lo0, rstep, back, 0);
+}
+// the 15-byte run whose lowest byte is tile[lo], from 5 aligned words: pixel j is byte j & 3 of bw[j >> 2] (back: the run
+// read backwards, pixel j = byte 14 - j)
+__device__ __forceinline__ void run_bytes15(const uint8_t* tile, int lo, int back, uint32_t (&bw)[4])
+{
+    const uint32_t* wsrc = reinterpret_cast<const uint32_t*>(tile + (lo & ~3));
+    const uint32_t w0 = wsrc[0], w1 = wsrc[1], w2 = wsrc[2], w3 = wsrc[3], w4 = wsrc[4];
+    const uint32_t sh = (uint32_t)(lo & 3) * 8u;
+    uint32_t b0 = __funnelshift_r(w0, w1, sh), b1 = __funnelshift_r(w1, w2, sh);
+    uint32_t b2 = __funnelshift_r(w2, w3, sh), b3 = __funnelshift_r(w3, w4, sh);   // bytes lo .. lo + 15
+    if (back) {
+        const uint32_t r0 = __byte_perm(b2, b3, 0x3456), r1 = __byte_perm(b1, b2, 0x3456);
+        const uint32_t r2 = __byte_perm(b0, b1, 0x3456), r3 = __byte_perm(b0, b0, 0x0012);
+        b0 = r0; b1 = r1; b2 = r2; b3 = r3;
+    }
+    bw[0] = b0; bw[1] = b1; bw[2] = b2; bw[3] = b3;
+}
+
 // PENDING: bulk groups of this lane-0 that may stay in flight while `stage` is rewritten
 template <int PENDING>
 __device__ __forceinline__ void gather_obs(const GridParams& p, int lane, const uint8_t* tile, uint8_t* stage,
@@ -707,15 +773,7 @@ __device__ __forceinline__ void gather_obs(const GridParams& p, int lane, const 
     const bool word_ok = (gaddr & 3u) == 0;
     const int shift = word_ok ? (int)gaddr : 0;          // staged stream is congruent to gdst modulo 16
     uint32_t* sw = reinterpret_cast<uint32_t*>(stage + shift);
-    if (lane < n) {
-        const int origin = ao - SSD_VIEW * S - SSD_VIEW;     // V[0][0] of this lane's agent
-        const int last = SSD_OBSW - 1;
-        int start0 = origin, step = 1, rs = S;               // UP
-        if (ori == ORI_RIGHT) { start0 = origin + last * S; step = -S; rs = 1; }
-        else if (ori == ORI_DOWN) { start0 = origin + last * S + last; step = -1; rs = -S; }
-        else if (ori == ORI_LEFT) { start0 = origin + last; step = S; rs = -1; }
-        vdesc[lane] = make_int4(start0, step, rs, 0);
-    }
+    if (lane < n) vdesc[lane] = view_desc(ao, ori, S);
     if (lane == 0) bulk_wait_read<PENDING>();                // the previous env's store has drained `stage`
     __syncwarp();
     if (lane < p.obs_items) {
@@ -737,6 +795,116 @@ __device__ __forceinline__ void gather_obs(const GridParams& p, int lane, const 
         for (int g4 = 0; g4 < 15; g4++) pack4(dst + 3 * g4, col[4 * g4], col[4 * g4 + 1], col[4 * g4 + 2], col[4 * g4 + 3]);
     }
     obs_stream_store(lane, stage, shift, word_ok, L, gdst);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Policy forms of the observation (ssd_set_policy_output): the windows as VisionNetwork.forward feeds them to its first
+// convolution, T [n][3][15][15] per env, value T(float32(float64(byte) / 255)) — what ssd_policy_inputs makes of the uint8
+// windows, written directly.
+//
+// Per-CTA palette of a policy form: element b of it, for a tile byte b = palette index << 2, is channel 0 of that colour,
+// b + 1 / b + 2 channels 1 / 2 (b + 3 unused), so one 16-byte (float) or 8-byte (half types) shared load gives a pixel.
+// Static shared memory, addressed where it is read (a pointer kept in a register across the env loop would spill).
+template <typename T>
+__device__ __forceinline__ T* policy_palette()
+{
+    __shared__ __align__(16) T s_ppal[64];
+    return s_ppal;
+}
+// (visible after the caller's next __syncthreads)
+template <typename T>
+__device__ __forceinline__ void load_policy_palette(const GridParams& p)
+{
+    T* pal = policy_palette<T>();
+    for (int i = threadIdx.x; i < 64; i += blockDim.x) {
+        const uint32_t c = (uint32_t)i & 3u, rgb = __ldg(p.pal + (i >> 2));
+        const uint32_t v = c < 3u ? (rgb >> (8u * c)) & 255u : 0u;
+        pal[i] = policy_cast<T>(__double2float_rn(__ddiv_rn((double)v, 255.0)));
+    }
+}
+// pixel j of an image row: its three channel planes are 225 elements apart
+__device__ __forceinline__ void put_pixel(float* o, const float* e, int j)
+{
+    const float4 v = *reinterpret_cast<const float4*>(e);
+    o[j] = v.x; o[SSD_OBS_PIX + j] = v.y; o[2 * SSD_OBS_PIX + j] = v.z;
+}
+template <typename H>
+__device__ __forceinline__ void put_pixel(H* o, const H* e, int j)
+{
+    const uint2 v = *reinterpret_cast<const uint2*>(e);
+    uint16_t* o16 = reinterpret_cast<uint16_t*>(o);
+    o16[j] = (uint16_t)v.x; o16[SSD_OBS_PIX + j] = (uint16_t)(v.x >> 16); o16[2 * SSD_OBS_PIX + j] = (uint16_t)v.y;
+}
+// a staged chunk (L bytes at stage + shift, shift = gdst mod 16; gdst and L even) -> HBM: one bulk async store for the
+// 16-byte aligned middle, halfword stores for the head / tail (an env block of n 675 sizeof(T) bytes starts on any even
+// address when n is odd)
+__device__ __forceinline__ void policy_stream_store(int lane, uint8_t* stage, int shift, int L, uint8_t* gdst)
+{
+    const uint16_t* sh = reinterpret_cast<const uint16_t*>(stage + shift);
+    __syncwarp();
+    const int a0 = (16 - shift) & 15;                  // head bytes up to the first 16-B boundary (L >= 1350 > a0)
+    const int mid = (L - a0) & ~15;
+    const int tail0 = a0 + mid;
+    if (lane < (a0 >> 1)) reinterpret_cast<uint16_t*>(gdst)[lane] = sh[lane];
+    if (lane < ((L - tail0) >> 1)) reinterpret_cast<uint16_t*>(gdst + tail0)[lane] = sh[(tail0 >> 1) + lane];
+    if (mid > 0) {
+        fence_async_smem();
+        __syncwarp();
+        if (lane == 0) bulk_store(gdst + a0, stage + shift + a0, (uint32_t)mid);
+    }
+}
+// One env's windows in policy form T at gdst.  The staging area holds `per` agents' planes (stage_r16 = g2_misc - g2_stage
+// bytes: cleanup n = 8 gives 2 agents of float or 4 of a half type, 5400 B), so the env goes out in ceil(n / per) chunks,
+// each staged and shipped like the uint8 stream.  A lane builds whole image rows: row (a, i) is a run of 15 tile bytes,
+// read as gather_obs2 reads it (TWO: 5 aligned words of T or T2) or as gather_obs does (byte steps over T, the reset kernel).
+template <int FORM, bool TWO>
+__device__ __forceinline__ void gather_policy(const GridParams& p, int lane, const uint8_t* tile, uint8_t* stage,
+                                              int4* vdesc, int ao, int ori, uint8_t* gdst)
+{
+    typedef typename ObsForm<FORM>::T T;
+    const T* ppal = policy_palette<T>();
+    const int n = p.n;
+    if (lane < n) vdesc[lane] = TWO ? view_desc2(p, ao, ori) : view_desc(ao, ori, p.S);
+    const int per = (p.g2_misc - p.g2_stage - 16) / (SSD_OBS_BYTES * (int)sizeof(T));
+    for (int a0 = 0; a0 < n; a0 += per) {
+        const int k = min(per, n - a0);
+        uint8_t* g = gdst + (size_t)a0 * SSD_OBS_BYTES * sizeof(T);
+        const int shift = (int)(reinterpret_cast<uintptr_t>(g) & 15u);
+        T* st = reinterpret_cast<T*>(stage + shift);
+        if (lane == 0) bulk_wait_read<0>();              // the previous chunk's (env's) store has drained `stage`
+        __syncwarp();
+        for (int r = lane; r < SSD_OBSW * k; r += 32) {
+            const int ar = (int)(((uint32_t)r * 0x8889u) >> 19), i = r - SSD_OBSW * ar;     // r / 15, r % 15
+            const int4 d = vdesc[a0 + ar];
+            T* o = st + ar * SSD_OBS_BYTES + i * SSD_OBSW;
+            if (TWO) {
+                uint32_t bw[4];
+                run_bytes15(tile, d.x + i * d.y, d.z, bw);
+#pragma unroll
+                for (int j = 0; j < SSD_OBSW; j++) put_pixel(o, ppal + __byte_perm(bw[j >> 2], 0u, 0x4440u + (uint32_t)(j & 3)), j);
+            } else {
+                const uint8_t* src = tile + (d.x + i * d.z);
+#pragma unroll
+                for (int j = 0; j < SSD_OBSW; j++) put_pixel(o, ppal + src[j * d.y], j);
+            }
+        }
+        policy_stream_store(lane, stage, shift, k * SSD_OBS_BYTES * (int)sizeof(T), g);
+    }
+}
+// the contract rows of one env: (theta, 0) x 5 per agent, T [n][10] (vision_net.py:160-161, as ssd_policy_inputs)
+template <typename T>
+__device__ __forceinline__ void policy_contract_rows(T* c, int n, double theta, int lane, int lanes)
+{
+    const T v = policy_cast<T>(__double2float_rn(theta)), z = policy_cast<T>(0.0f);
+    for (int k = lane; k < n * 10; k += lanes) c[k] = (k & 1) ? z : v;
+}
+// runtime-dtype form for the thread-per-env kernels (negotiation, contract parameters, checkpoint load)
+__device__ __forceinline__ void policy_contract_env(void* c, int dtype, int n, int env, double theta)
+{
+    const size_t o = (size_t)env * n * 10;
+    if (dtype == POLICY_F32) policy_contract_rows(reinterpret_cast<float*>(c) + o, n, theta, 0, 1);
+    else if (dtype == POLICY_F16) policy_contract_rows(reinterpret_cast<__half*>(c) + o, n, theta, 0, 1);
+    else policy_contract_rows(reinterpret_cast<__nv_bfloat16*>(c) + o, n, theta, 0, 1);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -784,10 +952,12 @@ __device__ __forceinline__ void apply_masks(const GridParams& p, uint8_t* tile, 
 // costs the hot loop registers (12 -> 68 B of spills), out of line it forces spills around the call, and a warp that
 // resets an env finishes ~10 us after the others of the one-wave persistent grid: observe kernel 0.204 -> 0.223 ms, more
 // than the launch it saves.  ssd_step_io.auto_reset therefore launches the masked reset kernel behind the step.)
-template <int KIND, int MW>
+// FORM: the observation form written to obs_dst (OBS_U8, or a policy form and, when pcontract is given, the env's contract
+// rows there).
+template <int KIND, int MW, int FORM>
 __device__ __forceinline__ void reset_env(const GridParams& p, const SharedTables& tb, int lane, uint8_t* tile, uint8_t* stage, int4* vdesc,
                                           const PointRegs<MW>& pr, int env, uint8_t* obs_dst, const double* neg_prop,
-                                          const double* neg_acc, uint8_t* neg_dec)
+                                          const double* neg_acc, uint8_t* neg_dec, void* pcontract)
 {
     const int n = p.n, S = p.S;
     const bool act_lane = lane < n;
@@ -870,7 +1040,10 @@ __device__ __forceinline__ void reset_env(const GridParams& p, const SharedTable
     __syncwarp();
     if (act_lane) tile[ao] &= CODE_MASK;              // MapEnv.reset never paints agents into the colour grid; the tile is clean again
     __syncwarp();
-    if (obs_dst) gather_obs<0>(p, lane, tile, stage, tb.pal, vdesc, ao, ori, obs_dst);
+    if (obs_dst) {
+        if constexpr (FORM == OBS_U8) gather_obs<0>(p, lane, tile, stage, tb.pal, vdesc, ao, ori, obs_dst);
+        else gather_policy<FORM, false>(p, lane, tile, stage, vdesc, ao, ori, obs_dst);
+    }
 
     // ---- SeparateContractSubgameStage.reset (two_stage_train.py:163-168)
     double theta = 0.0;
@@ -885,6 +1058,12 @@ __device__ __forceinline__ void reset_env(const GridParams& p, const SharedTable
         const bool dec = negotiate_agreement(g.seed, g.env_id, episode, n, neg_acc + (size_t)env * n);
         theta = dec ? neg_prop[env] : 0.0;
         if (neg_dec) neg_dec[env] = dec ? 1 : 0;
+    }
+    if constexpr (FORM != OBS_U8) {
+        if (pcontract) {                                  // lane 0 holds the negotiated theta
+            typedef typename ObsForm<FORM>::T T;
+            policy_contract_rows(reinterpret_cast<T*>(pcontract) + (size_t)env * n * 10, n, __shfl_sync(FULL, theta, 0), lane, 32);
+        }
     }
     // ---- record: zero everything, then the hot line
     for (int i = lane; i < p.hdr_bytes / 4; i += 32) reinterpret_cast<uint32_t*>(hdr)[i] = 0u;
@@ -911,9 +1090,10 @@ __device__ __forceinline__ void reset_env(const GridParams& p, const SharedTable
 // RESET kernel: one warp per env; the warp's envs are env0 + i * estride, their mask bytes are read 32 at a time (one round
 // trip, one ballot), so a sparse mask — a vectorised sampler in steady state resets ~E / horizon envs per step — costs a
 // few loads per warp.
-template <int KIND>
+// FORM (see OBS_U8): obs is a policy image tensor T for the policy forms, pcontract its contract rows (nullable; unused for OBS_U8).
+template <int KIND, int FORM = OBS_U8>
 __global__ void __launch_bounds__(GRID_THREADS) grid_reset_kernel(const GridParams p, const uint8_t* mask,
-                                                                  uint8_t* obs, long long obs_stride, const StepIO io)
+                                                                  uint8_t* obs, long long obs_stride, const StepIO io, void* pcontract)
 {
     constexpr int MW = MAX_POINT_ROUNDS;
     extern __shared__ __align__(16) uint8_t smem[];
@@ -927,6 +1107,7 @@ __global__ void __launch_bounds__(GRID_THREADS) grid_reset_kernel(const GridPara
         if (!__syncthreads_or(any)) return;
     }
     const SharedTables tb = load_shared_tables(p, smem, false);
+    if constexpr (FORM != OBS_U8) load_policy_palette<typename ObsForm<FORM>::T>(p);
     uint8_t* tile = smem + p.sm_warp0 + warp * p.g2_warp_bytes;
     uint8_t* stage = tile + p.g2_stage;
     int4* vdesc = reinterpret_cast<int4*>(tile + p.g2_misc + MISC_VDESC);
@@ -939,8 +1120,8 @@ __global__ void __launch_bounds__(GRID_THREADS) grid_reset_kernel(const GridPara
         while (todo) {
             const int env = env0 + (i0 + __ffs(todo) - 1) * estride;
             todo &= todo - 1;
-            reset_env<KIND, MW>(p, tb, lane, tile, stage, vdesc, pr, env, obs ? obs + (size_t)env * (size_t)obs_stride : nullptr,
-                                io.neg_prop, io.neg_acc, io.neg_dec);
+            reset_env<KIND, MW, FORM>(p, tb, lane, tile, stage, vdesc, pr, env, obs ? obs + (size_t)env * (size_t)obs_stride : nullptr,
+                                      io.neg_prop, io.neg_acc, io.neg_dec, pcontract);
         }
     }
     if (lane == 0) bulk_wait_read<0>();

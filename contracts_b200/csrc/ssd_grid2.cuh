@@ -594,24 +594,13 @@ __global__ void __launch_bounds__(LOGIC_THREADS) grid_reward_kernel(const GridPa
 __device__ __forceinline__ void gather_obs2(const GridParams& p, int lane, const uint8_t* tile, uint8_t* stage,
                                             const uint32_t* sm_pal, int4* vdesc, int ao, int ori, uint8_t* gdst)
 {
-    const int n = p.n, S = p.S, S2 = p.S2;
+    const int n = p.n;
     const int L = n * SSD_OBS_BYTES;
     const uint32_t gaddr = (uint32_t)(reinterpret_cast<uintptr_t>(gdst) & 15u);
     const bool word_ok = (gaddr & 3u) == 0;
     const int shift = word_ok ? (int)gaddr : 0;          // staged stream is congruent to gdst modulo 16
     uint32_t* sw = reinterpret_cast<uint32_t*>(stage + shift);
-    if (lane < n) {
-        const uint32_t trow = __umulhi((uint32_t)ao, p.s_magic);            // ao / S
-        const int row = (int)trow - SSD_VIEW, col = ao - (int)trow * S - 8;
-        const int origin = ao - SSD_VIEW * S - SSD_VIEW;                     // V[0][0] in T
-        const int origin2 = p.tile2_off + (col + SSD_VIEW) * S2 + 8 + row - SSD_VIEW * S2 - SSD_VIEW;   // V[0][0] in T2
-        const int last = SSD_OBSW - 1;
-        int lo0 = origin, rstep = S, back = 0;                                // UP
-        if (ori == ORI_DOWN) { lo0 = origin + last * S; rstep = -S; back = 1; }
-        else if (ori == ORI_LEFT) { lo0 = origin2 + last * S2; rstep = -S2; }
-        else if (ori == ORI_RIGHT) { lo0 = origin2; rstep = S2; back = 1; }
-        vdesc[lane] = make_int4(lo0, rstep, back, 0);
-    }
+    if (lane < n) vdesc[lane] = view_desc2(p, ao, ori);
     if (lane == 0) bulk_wait_read<0>();                  // the previous env's store has drained `stage`
     __syncwarp();
     if (lane < p.obs_items) {
@@ -623,18 +612,8 @@ __device__ __forceinline__ void gather_obs2(const GridParams& p, int lane, const
             int i = r - 15 * a;
             if (a >= n) { a = n - 1; i = SSD_OBSW - 1; }     // rows past the stream end: harmless in-bounds reads
             const int4 d = vdesc[a];
-            const int lo = d.x + i * d.y;                     // lowest byte of the 15-byte run
-            const uint32_t* wsrc = reinterpret_cast<const uint32_t*>(tile + (lo & ~3));
-            const uint32_t w0 = wsrc[0], w1 = wsrc[1], w2 = wsrc[2], w3 = wsrc[3], w4 = wsrc[4];
-            const uint32_t sh = (uint32_t)(lo & 3) * 8u;
-            uint32_t b0 = __funnelshift_r(w0, w1, sh), b1 = __funnelshift_r(w1, w2, sh);
-            uint32_t b2 = __funnelshift_r(w2, w3, sh), b3 = __funnelshift_r(w3, w4, sh);   // bytes lo .. lo + 15
-            if (d.z) {                                        // backwards: pixel j is byte 14 - j
-                const uint32_t r0 = __byte_perm(b2, b3, 0x3456), r1 = __byte_perm(b1, b2, 0x3456);
-                const uint32_t r2 = __byte_perm(b0, b1, 0x3456), r3 = __byte_perm(b0, b0, 0x0012);
-                b0 = r0; b1 = r1; b2 = r2; b3 = r3;
-            }
-            const uint32_t bw[4] = { b0, b1, b2, b3 };
+            uint32_t bw[4];
+            run_bytes15(tile, d.x + i * d.y, d.z, bw);        // the row's 15-byte run (lowest byte d.x + i d.y)
 #pragma unroll
             for (int j = 0; j < SSD_OBSW; j++)               // a tile byte IS the byte offset of its palette entry
                 col[15 * q + j] = *reinterpret_cast<const uint32_t*>(
@@ -661,7 +640,8 @@ __device__ __forceinline__ void gather_obs2(const GridParams& p, int lane, const
 #define OBS_LAY_HARVEST4(F) F(S, 56) F(S2, 32) F(tile2_off, 1696) F(g2_stage, 3440) F(g2_misc, 6512) F(g2_warp_bytes, 6640) \
     F(sm_thr, 64) F(sm_won, 80) F(sm_apple_rc, 96) F(sm_waste_rc, 416) F(sm_warp0, 416) F(n, 4) F(obs_items, 15) \
     F(n_apple, 155) F(n_waste, 0) F(rec_stride, 512) F(H, 16) F(W, 38) F(Wp, 40)
-template <int KIND, int MW, bool FEAT, int LAY>
+// FORM: the observation form (OBS_U8: uint8 windows at io.obs; a policy form: the policy's image tensor, io.obs_stride bytes per env).
+template <int KIND, int MW, bool FEAT, int LAY, int FORM = OBS_U8>
 __global__ void __maxnreg__(OBS_MAXREG) grid_obs_kernel(const GridParams p_in, const StepIO io_in, uint32_t* __restrict__ res_g)
 {
     GridParams p_pin; StepIO io_pin;                  // LAY == 1: a copy (scalar-replaced by the compiler) with the layout fields pinned
@@ -671,7 +651,7 @@ __global__ void __maxnreg__(OBS_MAXREG) grid_obs_kernel(const GridParams p_in, c
         OBS_LAY_CLEANUP8(OBS_PIN)
 #undef OBS_PIN
         p_pin.s_magic = 119304648u;
-        io_pin.obs_stride = 5400;
+        io_pin.obs_stride = 5400 * (int)sizeof(typename ObsForm<FORM>::T);
     }
     if (LAY == 2) {
         p_pin = p_in; io_pin = io_in;
@@ -679,12 +659,13 @@ __global__ void __maxnreg__(OBS_MAXREG) grid_obs_kernel(const GridParams p_in, c
         OBS_LAY_HARVEST4(OBS_PIN)
 #undef OBS_PIN
         p_pin.s_magic = 76695845u;
-        io_pin.obs_stride = 2700;
+        io_pin.obs_stride = 2700 * (int)sizeof(typename ObsForm<FORM>::T);
     }
     const GridParams& p = LAY != 0 ? p_pin : p_in;
     const StepIO& io = LAY != 0 ? io_pin : io_in;
     extern __shared__ __align__(16) uint8_t smem[];
     const SharedTables tb = load_shared_tables(p, smem, FEAT);
+    if constexpr (FORM != OBS_U8) load_policy_palette<typename ObsForm<FORM>::T>(p);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     uint8_t* tile = smem + p.sm_warp0 + warp * p.g2_warp_bytes;
     uint8_t* tile2 = tile + p.tile2_off;
@@ -792,11 +773,12 @@ __global__ void __maxnreg__(OBS_MAXREG) grid_obs_kernel(const GridParams p_in, c
         __syncwarp();
         if (act_lane && lane == 31 - __clz(grp)) { tile[ao] = (uint8_t)PAINT_CODE(lane); tile2[ao2] = (uint8_t)PAINT_CODE(lane); }
         __syncwarp();
-        // gather_obs2 waits (lane 0) until the previous observation store has drained `stage`, then syncs the warp
+        // gather_obs2 / gather_policy wait (lane 0) until the previous observation store has drained `stage`, then sync the warp
 #ifndef OBS_SKIP_GATHER
-        gather_obs2(p, lane, tile, stage, tb.pal, vdesc, ao, ori, g_obs);
+        if constexpr (FORM == OBS_U8) gather_obs2(p, lane, tile, stage, tb.pal, vdesc, ao, ori, g_obs);
+        else gather_policy<FORM, true>(p, lane, tile, stage, vdesc, ao, ori, g_obs);
 #endif
-        // the agents' cells back to their code (gather_obs2 ends behind a warp barrier after its last tile read)
+        // the agents' cells back to their code (the gather ends behind a warp barrier after its last tile read)
         if (act_lane) { tile[ao] = (uint8_t)old; tile2[ao2] = (uint8_t)old; }
         __syncwarp();
     }

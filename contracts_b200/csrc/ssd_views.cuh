@@ -162,6 +162,7 @@ struct SolverParams {
     double low, high;
     const uint8_t* episode; long long episode_stride; uint32_t episode_mask;
     uint8_t* theta; long long theta_stride;
+    void* pol_contract; int pol_dtype;       // gridworld with a policy output (ssd_set_policy_output): its contract rows, else NULL
 };
 #define SOLVER_RULE_MAX 0
 #define SOLVER_RULE_MAJORITY 1
@@ -215,6 +216,7 @@ __global__ void solver_choose_kernel(const SolverParams p, int S, int rule, cons
     if (best_param) best_param[env] = theta;
     if (best_idx) best_idx[env] = src;
     *reinterpret_cast<double*>(p.theta + (size_t)env * p.theta_stride) = theta;
+    if (p.pol_contract) policy_contract_env(p.pol_contract, p.pol_dtype, n, env, theta);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -226,17 +228,7 @@ __global__ void solver_choose_kernel(const SolverParams p, int S, int rule, cons
 //   contract `orig_obs["contract"].float().repeat(1, 5)` (vision_net.py:160-161): (theta, 0) five times, T [E n][10].
 // T = float32, float16 or bfloat16 (POLICY_F32 / F16 / BF16).  HBM-bound: 675 B read, 675 sizeof(T) written per agent.
 // One CTA per env; the windows are staged in shared memory, the outputs leave as coalesced element runs.
-#include <cuda_bf16.h>
-#include <cuda_fp16.h>
-#define POLICY_F32 0
-#define POLICY_F16 1
-#define POLICY_BF16 2
-
-template <typename T> __device__ __forceinline__ T policy_cast(float v);
-template <> __device__ __forceinline__ float policy_cast<float>(float v) { return v; }
-template <> __device__ __forceinline__ __half policy_cast<__half>(float v) { return __float2half_rn(v); }
-template <> __device__ __forceinline__ __nv_bfloat16 policy_cast<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
-
+// (POLICY_* and policy_cast are in ssd_grid.cuh: the observe / reset kernels write the same tensor with a policy output set.)
 template <typename T>
 __global__ void __launch_bounds__(VIEW_THREADS) policy_inputs_kernel(const GridParams p, const uint8_t* __restrict__ obs, long long obs_stride,
                                                                      T* __restrict__ image, T* __restrict__ contract)

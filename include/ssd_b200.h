@@ -231,6 +231,25 @@ int ssd_render(ssd_handle* h, uint8_t* out_dev, void* stream);
  * contract_dev (nullable) T [E*n][10] = (theta, 0) repeated 5 times (:160-161).  T by `dtype`. */
 int ssd_policy_inputs(ssd_handle* h, const uint8_t* obs_dev, int64_t obs_env_stride, int32_t dtype, void* image_dev,
                       void* contract_dev, void* stream);
+/* The same tensors written by the environment itself instead of by a second pass over the uint8 windows. */
+typedef struct ssd_policy_out {
+    int32_t struct_size;    /* sizeof(ssd_policy_out) (a smaller value is rejected) */
+    int32_t dtype;          /* SSD_POLICY_F32 / _F16 / _BF16 */
+    void*   image_dev;      /* T [E*n][3][15][15], 16-byte aligned: the tensor ssd_policy_inputs writes */
+    void*   contract_dev;   /* T [E*n][10] = (theta, 0) x 5, nullable */
+} ssd_policy_out;
+/* Gridworld kinds.  While set (sticky, like ssd_set_episode_stats / ssd_record_beams; NULL switches it off), the handle
+ * has one observation form, the policy's:
+ *   - every call that writes uint8 windows — ssd_step, ssd_step_host, ssd_step_host_async, ssd_reset (masked or not) and
+ *     the auto_reset behind a step — writes the image rows of the same envs instead, with exactly the values
+ *     ssd_policy_inputs(dtype) would produce from the windows.  obs_dev must be NULL in these calls (else SSD_EINVAL);
+ *   - every call that changes theta leaves the contract rows of the envs it changes current: ssd_reset, auto_reset with
+ *     negotiation, ssd_negotiate, ssd_set_contract_params, ssd_solver_choose and ssd_checkpoint_load.  ssd_set_state, a
+ *     parity tool, does not (call ssd_set_contract_params afterwards when it changed theta).
+ * Validates before storing anything: SSD_EINVAL for a struct_size too small, an unknown dtype, a NULL or misaligned
+ * image_dev, a contract_dev not aligned to its element, or a feature-env or selfdrive handle.  The caller keeps both
+ * tensors alive while they are set. */
+int ssd_set_policy_output(ssd_handle* h, const ssd_policy_out* out);
 
 /* --- NegotiationSolver (environments/two_stage_train.py:619-776); every env kind ------------------- */
 #define SSD_SOLVER_RULE_MAX 0        /* decision_rule 'max'      (:751-757) */
