@@ -278,3 +278,30 @@ def random_map(rng, kind, n):
     for i, (r, c) in enumerate(inner):
         g[r, c] = must[i] if i < len(must) else rng.choice(chars[0], p=chars[1])
     return ["".join(row) for row in g]
+
+
+def big_map(kind, H, W, seed):
+    """A random walled map near the size limits (48 x 64, 200+ apple / waste points: the 8-word mask variants of the kernels)."""
+    rng = np.random.RandomState(seed)
+    g = np.full((H, W), " ", dtype="<U1")
+    g[0, :] = g[-1, :] = g[:, 0] = g[:, -1] = "@"
+    inner = [(r, c) for r in range(1, H - 1) for c in range(1, W - 1)]
+    rng.shuffle(inner)
+    kinds = (("P", 24), ("@", 60), ("B", 200), ("H", 90), ("R", 120), ("S", 30)) if kind == "cleanup" else (("P", 24), ("@", 60), ("A", 240))
+    k = 0
+    for ch, cnt in kinds:
+        for r, c in inner[k:k + cnt]:
+            g[r, c] = ch
+        k += cnt
+    return ["".join(row) for row in g]
+
+
+def policy_image(want_u8, dtype, chunk=8192):
+    """the reference's windows uint8 [E, n, 15, 15, 3] (a device tensor) as the policy image T [E n, 3, 15, 15], in chunks
+    of envs so that the float64 intermediate stays small"""
+    import torch
+    out = []
+    for e0 in range(0, want_u8.shape[0], chunk):
+        x = want_u8[e0:e0 + chunk]
+        out.append((x.double() / 255).float().to(dtype).reshape(-1, 15, 15, 3).permute(0, 3, 1, 2))
+    return torch.cat(out)

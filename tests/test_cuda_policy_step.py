@@ -211,14 +211,19 @@ def test_policy_mode_replays_reference_negotiation(logic_variant, dt):
         assert torch.equal(img[rows].cpu(), _planar(fx["obs3"][ep], dtype)), "final obs ep %d" % ep
 
 
-def test_policy_mode_full_size_steady_state():
+def test_policy_mode_full_size_steady_state(oracle_lib):
     """E = 131072, cleanup n = 8, bf16: staggered episodes, auto-reset + negotiation in every step (the observe kernel's
-    dynamic tail scheduler at the benchmark's size)"""
+    dynamic tail scheduler at the benchmark's size); the image and rewards of every env also against a full-size oracle
+    driven through the same steps (step, reset(done), negotiate, theta of the finished envs from the negotiation)"""
+    from contracts_b200.maps import CLEANUP_MAP
     E, n = 131072, 8
     tw = Twins("cleanup_new", E, n, torch.bfloat16, horizon=1000, seed=73907, first_env_id=0)
+    orc = oracle_lib.GridOracle("cleanup", E, n, CLEANUP_MAP, horizon=1000, contract=CONTRACT["cleanup_new"], seed=73907)
     tw.both(lambda e: e.reset())
+    orc.reset()
     phase = (torch.arange(E, dtype=torch.int32) % 1000).cuda()
     tw.both(lambda e: e.set_state(t=phase))          # staggered episodes: ~131 envs finish in every step
+    orc.set_state(t=phase.cpu().numpy())
     dec_u, dec_q = (torch.zeros(E, dtype=torch.uint8, device="cuda") for _ in range(2))
     for t in range(20):
         a = tw.u.random_actions(1000 + t, 8)
@@ -230,6 +235,25 @@ def test_policy_mode_full_size_steady_state():
         for name in ("rew", "info", "done"):
             assert torch.equal(getattr(tw.u, name), getattr(tw.q, name)), name
         assert torch.equal(dec_u, dec_q)
+        o = orc.step(a.cpu().numpy(), want_features=False)
+        done = o["done"].astype(bool)
+        want = o["obs"]
+        want[done] = orc.reset(o["done"])[done]
+        old = orc.get_state()["theta"]
+        want_dec = orc.negotiate(prop.cpu().numpy(), acc.cpu().numpy())
+        orc.set_state(theta=np.where(done, orc.get_state()["theta"], old))
+        ctx = "full-size step %d" % t
+        assert np.array_equal(tw.q.done.cpu().numpy(), o["done"]), ctx
+        gu.assert_same("rew", tw.q.rew.cpu().numpy(), o["rew"], ctx)
+        gu.assert_same("decisions", dec_q.cpu().numpy()[done], want_dec[done], ctx)
+        img = tw.q.policy_image
+        want_d = torch.from_numpy(want).cuda()
+        for e0 in range(0, E, 16384):                 # the reference image, converted on the device 16384 envs at a time
+            got = img[e0 * n:(e0 + 16384) * n]
+            ref = gu.policy_image(want_d[e0:e0 + 16384], torch.bfloat16)
+            if not torch.equal(got, ref):
+                bad = (got != ref).reshape(-1, n * 675).any(1).nonzero().flatten()
+                raise AssertionError("image differs from the oracle at %s in envs %r" % (ctx, (bad[:10] + e0).tolist()))
 
 
 def test_policy_mode_graph_replay_matches_eager():

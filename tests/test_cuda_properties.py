@@ -1,5 +1,5 @@
 """GPU: size-independent properties at the full benchmark size (BASELINE configs: 131072 envs x 8 agents cleanup,
-16384 envs x 4 agents harvest), where the CPU oracle is only used on a slice."""
+16384 envs x 4 agents harvest), and the whole batch against the CPU oracle."""
 import numpy as np
 import pytest
 
@@ -22,9 +22,11 @@ def test_full_size_rollout_properties(oracle_lib, kind, E, n, nact, contract):
     k0, ks = E - 77, 64                                   # a slice near the end of the batch
     small = BatchedGridEnv(kind + "_new", ks, n, horizon=40, contract=contract, seed=73907, first_env_id=k0)
     orc = oracle_lib.GridOracle(kind, ks, n, amap, horizon=40, contract=contract, seed=73907, first_env_id=k0)
+    orc_big = oracle_lib.GridOracle(kind, E, n, amap, horizon=40, contract=contract, seed=73907)      # every env of the batch
     ob, osm = big.reset(), small.reset()
     assert torch.equal(ob[k0:k0 + ks], osm)
     assert np.array_equal(osm.cpu().numpy(), orc.reset())
+    assert torch.equal(ob, torch.from_numpy(orc_big.reset()).to(ob.device))
     cleaned_total = torch.zeros((), dtype=torch.float64, device=big.device)
     for t in range(90):                                    # crosses the horizon twice (masked re-resets)
         a = big.random_actions(t, nact)
@@ -36,6 +38,14 @@ def test_full_size_rollout_properties(oracle_lib, kind, E, n, nact, contract):
         assert torch.equal(obs[k0:k0 + ks], o2) and torch.equal(rew[k0:k0 + ks], r2) and torch.equal(info[k0:k0 + ks], i2)
         o = orc.step(a_small.cpu().numpy(), want_features=False)
         assert np.array_equal(o2.cpu().numpy(), o["obs"]) and np.array_equal(r2.cpu().numpy().view(np.uint64), o["rew"].view(np.uint64))
+        # 1b. the whole batch == the oracle (a skipped or doubled env anywhere in the observe kernel's schedule)
+        ob_ = orc_big.step(a.cpu().numpy(), want_features=False)
+        for name, got, want in (("obs", obs, ob_["obs"]), ("rew", rew.view(torch.int64), ob_["rew"].view(np.int64)),
+                                ("base_rew", big.base_rew.view(torch.int64), ob_["base_rew"].view(np.int64)),
+                                ("transfers", big.transfers.view(torch.int64), ob_["transfers"].view(np.int64)),
+                                ("info", info[..., :3].to(torch.int32), ob_["info"][..., :3]), ("done", done, ob_["done"])):
+            bad = (got != torch.from_numpy(np.ascontiguousarray(want)).to(got.device)).reshape(E, -1).any(1).nonzero().flatten()
+            assert bad.numel() == 0, "%s differs from the oracle at step %d in %d envs, first %r" % (name, t, bad.numel(), bad[:10].tolist())
         # 2. transfers redistribute, they do not create reward
         assert float((rew.sum(1) - big.base_rew.sum(1)).abs().max()) < 1e-9
         if kind == "cleanup":
@@ -50,12 +60,17 @@ def test_full_size_rollout_properties(oracle_lib, kind, E, n, nact, contract):
                 assert {tuple(p) for p in np.unique(centre[:, i], axis=0)} <= allowed
         if bool(done.any()):
             assert bool(done.all())                        # equal horizons
-            big.reset(done)
+            ob = big.reset(done)
             small.reset(d2)
             orc.reset(d2.cpu().numpy())
+            assert torch.equal(ob, torch.from_numpy(orc_big.reset(done.cpu().numpy())).to(ob.device))   # all envs are done
             cleaned_total.zero_()
     m = big.metrics_raw()
     assert float(m[:, 5].max()) == 0.0                     # no device error flags
+    assert np.array_equal(m.cpu().numpy().view(np.uint64), orc_big.metrics_raw().view(np.uint64))
+    so, sc = orc_big.get_state(), big.get_state()
+    for k in ("map", "pos", "ori", "t", "theta"):
+        assert np.array_equal(np.asarray(sc[k].cpu().numpy(), dtype=so[k].dtype), so[k]), k
     if kind == "cleanup":
         assert float(m[:, 4].sum()) == float(cleaned_total)          # dirt_cleaned == sum of cleaned_squares infos
         st = big.get_state()

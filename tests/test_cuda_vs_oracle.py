@@ -81,27 +81,11 @@ def test_rollout_matches_oracle(oracle_lib, case):
     gu.assert_same("metrics", env.metrics_raw().cpu().numpy(), orc.metrics_raw(), "end")
 
 
-def _big_map(kind, H, W, seed):
-    """A random walled map near the size limits (48 x 64, 200+ apple / waste points: the 8-word mask variants of the kernels)."""
-    rng = np.random.RandomState(seed)
-    g = np.full((H, W), " ", dtype="<U1")
-    g[0, :] = g[-1, :] = g[:, 0] = g[:, -1] = "@"
-    inner = [(r, c) for r in range(1, H - 1) for c in range(1, W - 1)]
-    rng.shuffle(inner)
-    kinds = (("P", 24), ("@", 60), ("B", 200), ("H", 90), ("R", 120), ("S", 30)) if kind == "cleanup" else (("P", 24), ("@", 60), ("A", 240))
-    k = 0
-    for ch, cnt in kinds:
-        for r, c in inner[k:k + cnt]:
-            g[r, c] = ch
-        k += cnt
-    return ["".join(row) for row in g]
-
-
 @pytest.mark.parametrize("kind,n,H,W", [("cleanup", 8, 44, 60), ("harvest", 6, 40, 63), ("cleanup", 3, 48, 64)])
 def test_big_map_matches_oracle(oracle_lib, kind, n, H, W):
     import torch
     from contracts_b200.batched import BatchedGridEnv
-    amap = _big_map(kind, H, W, H * W)
+    amap = gu.big_map(kind, H, W, H * W)
     contract = "CleanupContract" if kind == "cleanup" else "HarvestFeaturemodLocalContract"
     E, steps = 24, 150
     orc = oracle_lib.GridOracle(kind, E, n, amap, horizon=60, contract=contract, seed=21, first_env_id=3)

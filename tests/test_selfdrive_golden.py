@@ -129,13 +129,18 @@ def test_dropin_selfdrive_dict_api(name):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("n,E,contract", [(8, 4099, True), (3, 515, True), (5, 130, False)])
-def test_cuda_selfdrive_rollout_matches_oracle(oracle_lib, n, E, contract):
+@pytest.mark.parametrize("n,E,contract,params", [
+    pytest.param(8, 4099, True, {}, id="8-4099-True"), pytest.param(3, 515, True, {}, id="3-515-True"),
+    pytest.param(5, 130, False, {}, id="5-130-False"),
+    # the non-default road and speed parameters that test_deep_differential.py pins reference -> oracle
+    pytest.param(5, 777, True, dict(low_bound=-4.5, high_bound=6.25, start_vel=0.35, start_vel_ambulance=0.55), id="5-777-True-params"),
+    pytest.param(3, 301, True, dict(low_bound=-20.0, high_bound=3.0, start_vel=0.05, start_vel_ambulance=1.0), id="3-301-True-params")])
+def test_cuda_selfdrive_rollout_matches_oracle(oracle_lib, n, E, contract, params):
     """Random rollouts, every output, bit-exact, incl. masked re-resets of finished envs."""
     import torch
     from contracts_b200.selfdrive import BatchedCarEnv
-    env = BatchedCarEnv(E, n, contract="SelfdriveContractDistprop" if contract else None, seed=7, first_env_id=123)
-    orc = oracle_lib.CarOracle(E, n, contract=contract, seed=7, first_env_id=123)
+    env = BatchedCarEnv(E, n, contract="SelfdriveContractDistprop" if contract else None, seed=7, first_env_id=123, **params)
+    orc = oracle_lib.CarOracle(E, n, contract=contract, seed=7, first_env_id=123, **params)
     gu.assert_same("reset obs", env.reset().cpu().numpy(), orc.reset(), "reset")
     rng = np.random.RandomState(n)
     for t in range(260):
