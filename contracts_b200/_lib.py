@@ -66,6 +66,16 @@ class ssd_policy_out(ctypes.Structure):
 STATS_LEN = 8
 
 
+class ssd_episode_record(ctypes.Structure):
+    _fields_ = [("env_id", ctypes.c_uint32), ("episode", ctypes.c_uint32), ("t", ctypes.c_int32), ("ended", ctypes.c_uint32),
+                ("theta", ctypes.c_double), ("pad", ctypes.c_double), ("metrics", ctypes.c_double * METRIC_STRIDE)]
+
+
+class ssd_episode_log(ctypes.Structure):
+    _fields_ = [("struct_size", ctypes.c_int32), ("capacity", ctypes.c_int32), ("records_dev", ctypes.c_void_p),
+                ("count_dev", ctypes.c_void_p)]
+
+
 def resolve_device(device):
     """torch.device with an explicit index ('cuda' / None mean torch's CURRENT device, not GPU 0).  The C entry points
     switch to the handle's device themselves (and restore the caller's), so a handle on cuda:1 works whatever the
@@ -104,6 +114,7 @@ EXPORTS = [
     "ssd_step_host_async", "ssd_step_host_wait", "ssd_host_result_layout", "ssd_host_result_expand", "ssd_set_episode_stats",
     "ssd_feat_step_host_async", "ssd_selfdrive_step_host_async",
     "ssd_checkpoint_get_layout", "ssd_checkpoint_save", "ssd_checkpoint_load", "ssd_set_policy_output",
+    "ssd_set_episode_log",
 ]
 
 _LIB = None
@@ -136,6 +147,7 @@ def load():
     L.ssd_host_result_layout.argtypes = [vp, ctypes.POINTER(ssd_host_layout)]
     L.ssd_host_result_expand.argtypes = [vp, vp, vp]
     L.ssd_set_episode_stats.argtypes = [vp, vp]
+    L.ssd_set_episode_log.argtypes = [vp, ctypes.POINTER(ssd_episode_log)]
     L.ssd_get_state.argtypes = [vp, vp, vp, vp, vp, vp, vp]
     L.ssd_set_state.argtypes = [vp, vp, vp, vp, vp, vp, vp]
     L.ssd_get_metrics.argtypes = [vp, vp, vp]

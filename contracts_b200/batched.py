@@ -17,6 +17,7 @@ import torch
 
 from . import _lib
 from .checkpoint import CheckpointMixin
+from .episodes import EpisodeLogMixin
 from .maps import CLEANUP_MAP, HARVEST_MAP
 
 _DEFAULT_HIGH = {"CleanupContract": 0.2, "HarvestFeaturemodLocalContract": 10.0}
@@ -120,7 +121,7 @@ class HostResultMixin:
         _lib.check(self._h, self.lib.ssd_step_host_wait(self._h, int(ticket)))
 
 
-class BatchedGridEnv(HostResultMixin, CheckpointMixin):
+class BatchedGridEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
     """E environments of one kind on one device.
 
     kind: 'cleanup_new' | 'harvest_new' (the reference's `environment` strings,
@@ -154,6 +155,7 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin):
             raise ValueError("ascii_map rows must have equal length")
         self.horizon = int(horizon)
         self.contract = contract
+        self.inequity_averse_reward = bool(inequity_averse_reward)     # env rewards are float64 (map_env.py:293-300)
         if theta_high is None:
             theta_high = _DEFAULT_HIGH.get(contract, 0.0)
         self.theta_low = float(np.float32(theta_low))

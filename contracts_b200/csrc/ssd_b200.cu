@@ -797,29 +797,7 @@ __global__ void get_metrics_kernel(GridParams p, double* out)
     if (env >= p.E) return;
     const uint8_t* hdr = p.state + (size_t)env * p.rec_stride;
     double* o = out + (size_t)env * SSD_METRIC_STRIDE;
-    double raw = 0;
-    for (int a = 0; a < SSD_MAXN; a++) {
-        int sr = reinterpret_cast<const int*>(hdr + RO_SUM_RAW)[a];
-        raw += (double)sr;
-        o[8 + a] = (double)reinterpret_cast<const uint32_t*>(hdr + RO_AGENT_A)[a];
-        o[16 + a] = (double)reinterpret_cast<const uint32_t*>(hdr + RO_AGENT_B)[a];
-        if (p.reward_mode) {                           // shaped rewards: float64 sums in the record extension
-            o[24 + a] = reinterpret_cast<const double*>(hdr + RO_XSUM)[a];
-            o[32 + a] = reinterpret_cast<const double*>(hdr + RO_XTSUM)[a];
-        } else {
-            o[24 + a] = (double)sr;
-            o[32 + a] = (double)reinterpret_cast<const long long*>(hdr + RO_TSUM_RAW)[a];
-        }
-        o[40 + a] = reinterpret_cast<const double*>(hdr + RO_SUM_TR)[a];
-        o[48 + a] = reinterpret_cast<const double*>(hdr + RO_TSUM_TR)[a];
-    }
-    o[0] = (double)*reinterpret_cast<const uint32_t*>(hdr + RO_APPLES);
-    o[1] = (double)*reinterpret_cast<const uint32_t*>(hdr + RO_LOWDENS);
-    o[2] = p.reward_mode ? *reinterpret_cast<const double*>(hdr + RO_XRAW) : raw;
-    o[3] = *reinterpret_cast<const double*>(hdr + RO_TRANSFERS);
-    o[4] = (double)*reinterpret_cast<const uint32_t*>(hdr + RO_DIRT);
-    o[5] = (double)((*reinterpret_cast<const uint32_t*>(hdr + RO_FLAGS) >> RF_ERR_SHIFT) & 0xFFFFu);
-    o[6] = o[7] = 0;
+    for (int q = 0; q < SSD_METRIC_STRIDE; q++) o[q] = grid_metric(p, hdr, q);
 }
 
 // SeparateContractNegotiateStage.step, agreement stage (two_stage_train.py:266-281)
@@ -1309,6 +1287,28 @@ int ssd_set_episode_stats(ssd_handle* h, double* stats_dev)
     if (!h) return SSD_EINVAL;
     REQUIRE_GRID(h);
     h->gp.stats = stats_dev;
+    return SSD_OK;
+}
+
+static_assert(sizeof(ssd_episode_record) == EPREC_VECS * 16, "ssd_episode_record is written as EPREC_VECS 16-byte vectors");
+int ssd_set_episode_log(ssd_handle* h, const ssd_episode_log* log)
+{
+    if (!h) return SSD_EINVAL;
+    EpisodeLog el = { nullptr, nullptr, 0ull };
+    if (log) {
+        if (log->struct_size < (int32_t)sizeof(ssd_episode_log))
+            return fail(h, SSD_EINVAL, "ssd_episode_log.struct_size %d < %d: the caller's declaration of ssd_episode_log is out of date",
+                        log->struct_size, (int)sizeof(ssd_episode_log));
+        if (log->capacity < 1) return fail(h, SSD_EINVAL, "set_episode_log: capacity %d < 1", log->capacity);
+        if (!log->records_dev || (reinterpret_cast<uintptr_t>(log->records_dev) & 15))
+            return fail(h, SSD_EINVAL, "set_episode_log: records_dev must be a 16-byte aligned device pointer");
+        if (!log->count_dev || (reinterpret_cast<uintptr_t>(log->count_dev) & 7))
+            return fail(h, SSD_EINVAL, "set_episode_log: count_dev must be an 8-byte aligned device pointer");
+        el.records = reinterpret_cast<uint4*>(log->records_dev);
+        el.count = log->count_dev;
+        el.capacity = (unsigned long long)log->capacity;
+    }
+    h->gp.elog = el; h->fp.elog = el; h->cp.elog = el;     // (only the params of the handle's kind are ever launched)
     return SSD_OK;
 }
 

@@ -38,6 +38,24 @@ enum { SITE_MOVE_ORDER = 1, SITE_BEAM_ORDER = 2, SITE_SPAWN_DRAWS = 3, SITE_WAST
 #define RF_STALE_EMPTY 1u     // cleanup: current_apple_points is [] until the first step (cleanup_new.py:181 runs before the reset-time spawn)
 #define RF_ERR_SHIFT 8
 
+// ssd_set_episode_log: the ring buffer a reset appends the episode it replaces to (records == nullptr: off).  Part of
+// GridParams / FeatParams / CarParams, a runtime pointer like GridParams::stats.  A record (ssd_episode_record) is EPREC_VECS
+// 16-byte vectors: 0 = {env_id, episode, t, ended}, 1 = {theta, 0}, 2 + j = {metrics[2 j], metrics[2 j + 1]}.
+#define EPREC_VECS 30
+struct EpisodeLog {
+    uint4* records;                  // [capacity][EPREC_VECS]
+    unsigned long long* count;       // records appended so far; record k goes to slot k % capacity
+    unsigned long long capacity;
+};
+__device__ __forceinline__ uint4 eprec_head(uint32_t env_id, uint32_t episode, int t, bool ended)
+{
+    return make_uint4(env_id, episode, (uint32_t)t, ended ? 1u : 0u);
+}
+__device__ __forceinline__ uint4 eprec_pair(double lo, double hi)
+{
+    return make_uint4((uint32_t)__double2loint(lo), (uint32_t)__double2hiint(lo), (uint32_t)__double2loint(hi), (uint32_t)__double2hiint(hi));
+}
+
 struct Philox4 { uint32_t x, y, z, w; };
 
 __host__ __device__ __forceinline__ Philox4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3,

@@ -76,6 +76,7 @@ struct FeatParams {
     unsigned long long* tsum_raw; // [n][E]
     double* sum_tr;             // [n][E]
     double* tsum_tr;            // [n][E]
+    EpisodeLog elog;            // optional: ssd_set_episode_log ring buffer (appended to by the resets of feat_kernel)
 };
 
 struct FeatIO {
@@ -218,6 +219,56 @@ __device__ __noinline__ uint32_t oct_closest(const uint8_t* list, int L, const u
     return rc[list[key & 255u]];
 }
 
+// Element q of env's ssd_feat_get_metrics row (40 doubles; 0 beyond): dirt, raw, transfers, apples, low_density, err_flags,
+// 0, 0, sum_raw[8], tsum_raw[8], sum_tr[8], tsum_tr[8] from the [k][E] accumulators.  What ssd_feat_get_metrics writes and
+// what a reset hands to the episode log.  (Scalar arguments: a FeatParams reference into the non-inlined caller below
+// would copy the kernel parameters to the stack.)
+__device__ __forceinline__ double feat_metric(const double* metrics, const uint32_t* sum_raw, const unsigned long long* tsum_raw,
+                                              const double* sum_tr, const double* tsum_tr, int E, int n, int env, int q)
+{
+    if (q < 8) return q < 6 ? metrics[(size_t)q * E + env] : 0.0;    // [5]: err_flags (unused: no wrapping stamps any more)
+    const int a = q & 7;
+    if (a >= n) return 0.0;
+    const size_t so = (size_t)a * E + env;
+    switch (q >> 3) {
+    case 1: return (double)sum_raw[so];
+    case 2: return (double)tsum_raw[so];
+    case 3: return sum_tr[so];
+    case 4: return tsum_tr[so];
+    default: return 0.0;
+    }
+}
+
+// Episode log of the resets of one feat_kernel round (all 32 lanes; `mine`: this octet resets an initialised env): one
+// atomic for the warp's up to four records, then the octet writes its env's record, lane a the vectors a, a + 8, ...  Reads
+// the accumulators before the reset zeroes them.  Out of line: the step's hot path stays small in the instruction cache
+// (DESIGN §4.5a).
+__device__ __noinline__ void feat_log_episode(EpisodeLog log, const double* metrics, const uint32_t* sum_raw,
+                                              const unsigned long long* tsum_raw, const double* sum_tr, const double* tsum_tr,
+                                              int E, int n, int horizon, int env, uint32_t env_id, bool mine, uint32_t episode,
+                                              int t, double theta, int lane)
+{
+    const int a = lane & 7, obase = lane & 24;
+    const uint32_t lm = __ballot_sync(FULLMASK, mine && a == 0);
+    if (!lm) return;
+    const int leader = __ffs(lm) - 1;
+    unsigned long long base = 0;
+    if (lane == leader) base = atomicAdd(log.count, (unsigned long long)__popc(lm));
+    base = __shfl_sync(FULLMASK, base, leader);
+    if (!mine) return;
+    const unsigned long long slot = (base + (unsigned long long)__popc(lm & ((1u << obase) - 1u))) % log.capacity;
+    uint4* rec = log.records + slot * EPREC_VECS;
+#pragma unroll 1
+    for (int v = a; v < EPREC_VECS; v += 8) {
+        uint4 w;
+        if (v == 0) w = eprec_head(env_id, episode, t, t == horizon);
+        else if (v == 1) w = eprec_pair(theta, 0.0);
+        else w = eprec_pair(feat_metric(metrics, sum_raw, tsum_raw, sum_tr, tsum_tr, E, n, env, 2 * v - 4),
+                            feat_metric(metrics, sum_raw, tsum_raw, sum_tr, tsum_tr, E, n, env, 2 * v - 3));
+        rec[v] = w;
+    }
+}
+
 #ifndef FEAT_MIN_BLOCKS
 #define FEAT_MIN_BLOCKS 4
 #endif
@@ -287,6 +338,9 @@ __global__ void __launch_bounds__(FEAT_THREADS, FEAT_MIN_BLOCKS) feat_kernel(con
 
     // ---- reset (cleanup_features.py:256-284 / harvest_features.py:289-336 + two_stage_train.py:159-187)
     if (__any_sync(FULLMASK, doreset)) {
+        if (p.elog.records)                          // hand the finished episodes over before their accumulators are zeroed
+            feat_log_episode(p.elog, p.metrics, p.sum_raw, p.tsum_raw, p.sum_tr, p.tsum_tr, p.E, n, p.horizon, env, env_id,
+                             doreset && (c3 & 0x80000000u), c3 & 0x7fffffffu, (int)s_rec[FR_T], theta, lane);
         uint32_t sm = (CLEANUP && doreset) ? __ldg(p.waste_start_mask + a) : 0u;
         const int sc = __popc(sm);
         const int sincl = oct_scan_incl(sc, a);
@@ -806,13 +860,7 @@ __global__ void feat_get_metrics_kernel(const FeatParams p, double* out)
     const int env = blockIdx.x * blockDim.x + threadIdx.x;
     if (env >= p.E) return;
     double* o = out + (size_t)env * 40;
-    for (int q = 0; q < 8; q++) o[q] = q < 6 ? p.metrics[(size_t)q * p.E + env] : 0.0;        // [5]: err_flags (unused: no wrapping stamps any more)
-    for (int a = 0; a < SSD_MAXN; a++) {
-        const bool v = a < p.n;
-        const size_t so = (size_t)a * p.E + env;
-        o[8 + a] = v ? (double)p.sum_raw[so] : 0.0; o[16 + a] = v ? (double)p.tsum_raw[so] : 0.0;
-        o[24 + a] = v ? p.sum_tr[so] : 0.0; o[32 + a] = v ? p.tsum_tr[so] : 0.0;
-    }
+    for (int q = 0; q < 40; q++) o[q] = feat_metric(p.metrics, p.sum_raw, p.tsum_raw, p.sum_tr, p.tsum_tr, p.E, p.n, env, q);
 }
 // pos int32 [E][n][2], ori int32 [E][n], cells u8 [E][H][W] (1 apple, 2 waste), theta f64 [E], t int32 [E]
 __global__ void feat_get_state_kernel(const FeatParams p, int32_t* pos, int32_t* ori, uint8_t* cells, double* theta, int32_t* t)

@@ -127,6 +127,7 @@ struct GridParams {
     uint8_t* state;
     uint8_t* beam;               // optional [E][map_bytes]: beam_pos of the last step as a char overlay (render only)
     double* stats;               // optional [8]: ssd_set_episode_stats accumulator (added to by the reset kernel)
+    EpisodeLog elog;             // optional: ssd_set_episode_log ring buffer (appended to by the reset kernel)
     uint32_t* obs_ctr;           // [2] observe kernel: next env of the dynamically scheduled tail, CTAs finished
     int obs_static_iters;        // observe kernel: iterations every warp takes from the static grid-stride schedule
 };
@@ -140,6 +141,40 @@ __device__ __forceinline__ double inequity_term(int ra, int sp, int sn, double a
     const double dis = __dmul_rn(alpha, (double)sp), adv = __dmul_rn(beta, (double)sn);
     return __dsub_rn((double)ra, __ddiv_rn(__dadd_rn(dis, adv), (double)(n - 1)));
 }
+// Element q of the env's ssd_get_metrics row (SSD_METRIC_STRIDE doubles, include/ssd_b200.h) from its record: what
+// ssd_get_metrics writes and what the reset kernel hands to the episode log.
+__device__ __forceinline__ double grid_metric(const GridParams& p, const uint8_t* hdr, int q)
+{
+    if (q >= 8) {
+        const int a = q & 7;
+        switch (q >> 3) {
+        case 1: return (double)reinterpret_cast<const uint32_t*>(hdr + RO_AGENT_A)[a];
+        case 2: return (double)reinterpret_cast<const uint32_t*>(hdr + RO_AGENT_B)[a];
+        case 3: return p.reward_mode ? reinterpret_cast<const double*>(hdr + RO_XSUM)[a]        // shaped rewards: float64 sums
+                                     : (double)reinterpret_cast<const int*>(hdr + RO_SUM_RAW)[a];
+        case 4: return p.reward_mode ? reinterpret_cast<const double*>(hdr + RO_XTSUM)[a]
+                                     : (double)reinterpret_cast<const long long*>(hdr + RO_TSUM_RAW)[a];
+        case 5: return reinterpret_cast<const double*>(hdr + RO_SUM_TR)[a];
+        default: return reinterpret_cast<const double*>(hdr + RO_TSUM_TR)[a];
+        }
+    }
+    switch (q) {
+    case 0: return (double)*reinterpret_cast<const uint32_t*>(hdr + RO_APPLES);
+    case 1: return (double)*reinterpret_cast<const uint32_t*>(hdr + RO_LOWDENS);
+    case 2: {
+        if (p.reward_mode) return *reinterpret_cast<const double*>(hdr + RO_XRAW);
+        double raw = 0;
+#pragma unroll 1
+        for (int a = 0; a < SSD_MAXN; a++) raw += (double)reinterpret_cast<const int*>(hdr + RO_SUM_RAW)[a];
+        return raw;
+    }
+    case 3: return *reinterpret_cast<const double*>(hdr + RO_TRANSFERS);
+    case 4: return (double)*reinterpret_cast<const uint32_t*>(hdr + RO_DIRT);
+    case 5: return (double)((*reinterpret_cast<const uint32_t*>(hdr + RO_FLAGS) >> RF_ERR_SHIFT) & 0xFFFFu);
+    default: return 0.0;
+    }
+}
+
 // thread per env: the int16 rewards sit in the RS_* words rsp[j * rstride] (bits 16-31)
 __device__ __noinline__ double shaped_reward(int mode, double alpha, double beta, int n, const uint32_t* rsp, int rstride, int a)
 {
@@ -985,6 +1020,21 @@ __device__ __forceinline__ void reset_env(const GridParams& p, const SharedTable
             atomicMax(reinterpret_cast<unsigned long long*>(p.stats + 7),
                       (unsigned long long)__double_as_longlong((double)((flags >> RF_ERR_SHIFT) & 0xFFFFu)));
         }
+    }
+    if (p.elog.records && (flags & 0x80000000u)) {   // the same episode as one record of the episode log: lane v writes vector v
+        unsigned long long slot = 0;
+        if (lane == 0) slot = atomicAdd(p.elog.count, 1ull) % p.elog.capacity;
+        slot = __shfl_sync(FULL, slot, 0);
+        uint4 w;
+        if (lane == 0) {
+            const int t = *reinterpret_cast<const int*>(hdr + RO_T);
+            w = eprec_head(p.first_env_id + (uint32_t)env, episode, t, t == p.horizon);
+        } else if (lane == 1) {
+            w = eprec_pair(*reinterpret_cast<const double*>(hdr + RO_THETA), 0.0);
+        } else {
+            w = eprec_pair(grid_metric(p, hdr, 2 * lane - 4), grid_metric(p, hdr, 2 * lane - 3));
+        }
+        if (lane < EPREC_VECS) p.elog.records[slot * EPREC_VECS + lane] = w;
     }
     // the first reset of a record (flags bit 31 clear) is episode 0; later resets increment
     episode = (flags & 0x80000000u) ? episode + 1u : 0u;

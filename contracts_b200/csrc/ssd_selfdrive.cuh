@@ -43,6 +43,7 @@ struct CarParams {
     uint32_t* meta;     // [E]  n_crossed | done mask << 8 | all_done << 16 | initialised << 31
     int32_t* t;         // [E]
     uint32_t* episode;  // [E]
+    EpisodeLog elog;    // optional: ssd_set_episode_log ring buffer (appended to by the resets of car_kernel)
 };
 
 struct CarIO {
@@ -156,6 +157,32 @@ __device__ __noinline__ void car_contract(const CarParams& p, const double* o_po
     if (k == 0) rew = rew0;
 }
 
+// Episode log of the resets of one car_kernel round (all 32 lanes; `mine`: this octet resets an initialised env): one atomic
+// for the warp's up to four records, then the octet writes its env's record — metrics [transfers, 0, ...] —, lane k the
+// vectors k, k + 8, ...  Reads the env's state before the reset rewrites it.  Out of line, off the step's hot path.
+__device__ __noinline__ void car_log_episode(EpisodeLog log, const double* theta, const double* m_transfers, const int32_t* t,
+                                             const uint32_t* episode, int env, uint32_t env_id, bool mine, bool ended, int lane)
+{
+    const int k = lane & 7, obase = lane & 24;
+    const uint32_t lm = __ballot_sync(CAR_FULL, mine && k == 0);
+    if (!lm) return;
+    const int leader = __ffs(lm) - 1;
+    unsigned long long base = 0;
+    if (lane == leader) base = atomicAdd(log.count, (unsigned long long)__popc(lm));
+    base = __shfl_sync(CAR_FULL, base, leader);
+    if (!mine) return;
+    const unsigned long long slot = (base + (unsigned long long)__popc(lm & ((1u << obase) - 1u))) % log.capacity;
+    uint4* rec = log.records + slot * EPREC_VECS;
+#pragma unroll 1
+    for (int v = k; v < EPREC_VECS; v += 8) {
+        uint4 w;
+        if (v == 0) w = eprec_head(env_id, episode[env], t[env], ended);
+        else if (v == 1) w = eprec_pair(theta[env], 0.0);
+        else w = eprec_pair(v == 2 ? m_transfers[env] : 0.0, 0.0);
+        rec[v] = w;
+    }
+}
+
 // One launch = one step (or, RESET_ONLY, one masked reset) of every env.
 // Next-step auto-reset (ssd_selfdrive_io.auto_reset): an env whose episode ended in the previous step starts its next
 // episode in this one — reset observation, zero rewards, dones cleared, the actions of this step ignored.
@@ -210,6 +237,9 @@ __global__ void __launch_bounds__(CAR_THREADS, CAR_MIN_BLOCKS) car_kernel(const 
     const bool stepping = !RESET_ONLY && live && !doreset;
     double x = 0.0, v = 0.0;                            // this car's position / velocity after the step (or the reset)
 
+    if (p.elog.records && __any_sync(CAR_FULL, doreset))     // hand the finished episodes over before the reset rewrites them
+        car_log_episode(p.elog, p.theta, p.m_transfers, p.t, p.episode, env, p.first_env_id + (uint32_t)env,
+                        doreset && (meta0 & 0x80000000u), (meta0 >> 16) & 1u, lane);
     if (doreset) {
         // self_driving_car_accelerate.py:49-79 + two_stage_train.py:159-187
         const uint32_t episode = (meta0 & 0x80000000u) ? p.episode[env] + 1u : 0u;

@@ -10,7 +10,7 @@ import torch
 from .. import spaces
 from ..features import BatchedFeatureEnv
 from ..maps import CLEANUP_MAP, HARVEST_MAP
-from .gridworld import equality, sustainability
+from .gridworld import _num, equality, sustainability
 
 
 class _FeatureEnv:
@@ -69,15 +69,8 @@ class _FeatureEnv:
     @property
     def metrics(self):
         raw = self.batch.metrics_raw()[0].cpu().numpy()
-        n = self.num_agents
-        m = self._metrics_from_raw(raw)
-        if self.timesteps == self.horizon:
-            m["equality"] = equality(list(raw[8:8 + n]))
-            m["sustainability"] = sustainability(list(raw[8:8 + n]), list(raw[16:16 + n]))
-            if self._contract is not None and self._contract[0] is not None:
-                m["transfer_sustainability"] = sustainability(list(raw[24:24 + n]), list(raw[32:32 + n]))
-                m["transfer_equality"] = equality(list(raw[24:24 + n]))
-        return m
+        return feature_metrics(self.KIND, raw, self.num_agents, self.timesteps == self.horizon,
+                               contract=self._contract is not None and self._contract[0] is not None)
 
     def compute_equality(self, reward_dict):
         return equality([sum(v) for v in reward_dict.values()])
@@ -113,9 +106,6 @@ class CleanupFeatures(_FeatureEnv):
     def _agent_info(self, info, obs):
         return {"cleaned_squares": int(info[0])}
 
-    def _metrics_from_raw(self, raw):
-        return {"dirt_cleaned": int(raw[0]), "raw_env_rewards": float(raw[1]) if raw[1] else 0, "transfers": _num(raw[2])}
-
 
 class HarvestFeatures(_FeatureEnv):
     """environments/harvest_features.py HarvestFeatures ('Harvest')."""
@@ -135,10 +125,21 @@ class HarvestFeatures(_FeatureEnv):
     def _agent_info(self, info, obs):
         return {"eaten_apples": int(info[0]), "eaten_close_apples": int(info[1]), "feature_obs": obs.copy()}
 
-    def _metrics_from_raw(self, raw):
-        return {"total_apples_eaten": int(raw[3]), "low_density_apples_eaten": int(raw[4]),
-                "raw_env_rewards": float(raw[1]) if raw[1] else 0, "transfers": _num(raw[2])}
 
-
-def _num(x):
-    return int(x) if float(x).is_integer() else float(x)
+def feature_metrics(kind, raw, n, ended, contract=False):
+    """The `metrics` dict of a CleanupFeatures / HarvestFeatures env (kind 'cleanup' / 'harvest') from its
+    ssd_feat_get_metrics row `raw` (float64 [40] or longer, numpy).  ended: the episode reached its horizon (equality /
+    sustainability are added then, and transfer_* with a contract)."""
+    raw_rew = float(raw[1]) if raw[1] else 0
+    if kind == "cleanup":
+        m = {"dirt_cleaned": int(raw[0]), "raw_env_rewards": raw_rew, "transfers": _num(raw[2])}
+    else:
+        m = {"total_apples_eaten": int(raw[3]), "low_density_apples_eaten": int(raw[4]), "raw_env_rewards": raw_rew,
+             "transfers": _num(raw[2])}
+    if ended:
+        m["equality"] = equality(list(raw[8:8 + n]))
+        m["sustainability"] = sustainability(list(raw[8:8 + n]), list(raw[16:16 + n]))
+        if contract:
+            m["transfer_sustainability"] = sustainability(list(raw[24:24 + n]), list(raw[32:32 + n]))
+            m["transfer_equality"] = equality(list(raw[24:24 + n]))
+    return m

@@ -167,24 +167,9 @@ class _GridWorldEnv:
         raw = self.batch.metrics_raw()[0].cpu().numpy()
         if raw[5] != 0:
             raise RuntimeError("device error flags %d" % int(raw[5]))
-        n = self.num_agents
-        m = self._metrics_from_raw(raw)
-        m["transfers"] = self._num(raw[3])
-        if self.timesteps == self.horizon:
-            m["equality"] = equality([self._rew(x) for x in raw[24:24 + n]])
-            m["sustainability"] = sustainability([self._rew(x) for x in raw[24:24 + n]], [self._rew(x) for x in raw[32:32 + n]])
-            if self._contract is not None and self._contract[0] is not None:
-                m["transfer_sustainability"] = sustainability(list(raw[40:40 + n]), list(raw[48:48 + n]))
-                m["transfer_equality"] = equality(list(raw[40:40 + n]))
-        return m
-
-    def _rew(self, x):
-        """Env rewards are Python ints unless inequity aversion made them float64 (map_env.py:293-300)."""
-        return float(x) if self.inequity_averse_reward else int(x)
-
-    @staticmethod
-    def _num(x):
-        return int(x) if float(x).is_integer() else float(x)
+        return grid_metrics(self.KIND, raw, self.num_agents, self.timesteps == self.horizon,
+                            contract=self._contract is not None and self._contract[0] is not None,
+                            float_rewards=self.inequity_averse_reward)
 
     def compute_equality(self, reward_dict):
         return equality([sum(v) for v in reward_dict.values()])
@@ -214,6 +199,35 @@ class _GridWorldEnv:
         if self._batch is not None:
             self._batch.close()
             self._batch = None
+
+
+def grid_metrics(kind, raw, n, ended, contract=False, float_rewards=False):
+    """The `metrics` dict of a cleanup_new / harvest_new env (cleanup_new.py:186-189,213-232,264-266; harvest_new.py:152-155;
+    two_stage_train.py:92-99) from its ssd_get_metrics row `raw` (float64 [56], numpy).  ended: the episode reached its
+    horizon (the reference adds equality / sustainability then, and transfer_* with a contract).  float_rewards: env
+    rewards are float64 (inequity aversion, map_env.py:293-300), else Python ints."""
+    rew = float if float_rewards else int
+    if kind == "cleanup_new":
+        m = {"total_apples_eaten": int(raw[0]), "raw_env_rewards": rew(raw[2]), "dirt_cleaned": int(raw[4])}
+        for i in range(n):
+            m["a%d-waste_cleaned" % i] = int(raw[8 + i])
+    else:
+        m = {"total_apples_eaten": int(raw[0]), "low_density_apples_eaten": int(raw[1]), "raw_env_rewards": rew(raw[2])}
+        for i in range(n):
+            m["a%d-apples_consumed" % i] = int(raw[8 + i])
+            m["a%d-close_apples_consumed" % i] = int(raw[16 + i])
+    m["transfers"] = _num(raw[3])
+    if ended:
+        m["equality"] = equality([rew(x) for x in raw[24:24 + n]])
+        m["sustainability"] = sustainability([rew(x) for x in raw[24:24 + n]], [rew(x) for x in raw[32:32 + n]])
+        if contract:
+            m["transfer_sustainability"] = sustainability(list(raw[40:40 + n]), list(raw[48:48 + n]))
+            m["transfer_equality"] = equality(list(raw[40:40 + n]))
+    return m
+
+
+def _num(x):
+    return int(x) if float(x).is_integer() else float(x)
 
 
 def equality(totals):
@@ -256,12 +270,6 @@ class CleanupEnv(_GridWorldEnv):
     def _agent_info(self, row):
         return {"eaten_apples": int(row[0]), "cleaned_squares": int(row[1])}
 
-    def _metrics_from_raw(self, raw):
-        m = {"total_apples_eaten": int(raw[0]), "raw_env_rewards": self._rew(raw[2]), "dirt_cleaned": int(raw[4])}
-        for i in range(self.num_agents):
-            m["a%d-waste_cleaned" % i] = int(raw[8 + i])
-        return m
-
     def _reset_feature_obs(self):
         """Feature observation at reset (cleanup_new.py:193-202), computed on the host from the device state."""
         st = self.batch.get_state()
@@ -293,13 +301,6 @@ class HarvestEnv(_GridWorldEnv):
 
     def _agent_info(self, row):
         return {"eaten_apples": int(row[0]), "eaten_close_apples": int(row[1])}
-
-    def _metrics_from_raw(self, raw):
-        m = {"total_apples_eaten": int(raw[0]), "low_density_apples_eaten": int(raw[1]), "raw_env_rewards": self._rew(raw[2])}
-        for i in range(self.num_agents):
-            m["a%d-apples_consumed" % i] = int(raw[8 + i])
-            m["a%d-close_apples_consumed" % i] = int(raw[16 + i])
-        return m
 
     def _reset_feature_obs(self):
         """Feature observation at reset (harvest_new.py:160-168)."""

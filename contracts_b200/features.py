@@ -12,6 +12,7 @@ import torch
 from . import _lib
 from .batched import HostResultMixin
 from .checkpoint import CheckpointMixin
+from .episodes import EpisodeLogMixin
 from .maps import CLEANUP_MAP, HARVEST_MAP
 
 _DEFAULT_HIGH = {"CleanupContract": 0.2, "HarvestFeaturemodLocalContract": 10.0}
@@ -21,7 +22,7 @@ def _ptr(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
 
-class BatchedFeatureEnv(HostResultMixin, CheckpointMixin):
+class BatchedFeatureEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
     """kind: 'cleanup' | 'harvest' (the reference's `environment` strings for the feature envs)."""
 
     def __init__(self, kind, num_envs, num_agents, ascii_map=None, horizon=1000, contract=None, theta_low=0.0,

@@ -11,13 +11,14 @@ import torch
 from . import _lib
 from .batched import HostResultMixin
 from .checkpoint import CheckpointMixin
+from .episodes import EpisodeLogMixin
 
 
 def _ptr(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
 
-class BatchedCarEnv(HostResultMixin, CheckpointMixin):
+class BatchedCarEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
     kind = "selfdrive"
 
     def __init__(self, num_envs, num_agents, contract=None, low_bound=-10.0, high_bound=10.0, start_vel=0.2,

@@ -11,11 +11,16 @@ the dict conventions of the reference's wrappers (`{env_id: {agent_id: ...}}`; o
     requested between two polls run as one masked device reset.
 Arrays are also available without the dict building through `poll_arrays()` — for samplers that batch the policy
 forward themselves the dict layer is pure overhead (INTEGRATION.md §2b has the measured rates).
+
+The envs live on the device, so `get_sub_environments()` has no Python envs to offer an RLlib callback; the metrics the
+reference's MetricsCallback (utils/logger_utils.py:126-151) reads from each env come from `episode_metrics()` instead:
+every adapter keeps an episode log (contracts_b200/episodes.py) and drains it there.
 """
 import numpy as np
 import torch
 
 from .batched import BatchedGridEnv
+from .episodes import EpisodeLog
 
 
 def _upload(v, actions_host):
@@ -33,11 +38,33 @@ def _staging_free(v):
         v._uploaded.synchronize()
 
 
-class SSDVectorEnv:
+def _open_episode_log(v, capacity):
+    """the adapter's episode log (capacity None: 2 E records; 0: none)"""
+    v._episode_log = None
+    if capacity is None or capacity > 0:
+        v._episode_log = EpisodeLog(v.batch, capacity)
+        v.batch.set_episode_log(v._episode_log)
+
+
+class _EpisodeMetricsMixin:
+    def episode_metrics(self):
+        """The metrics of every episode that ended since the last call (a reset of a finished or unfinished env ends it),
+        sorted by (env_id, episode): per episode the dict the drop-in class's `metrics` returns at its last step, plus
+        `env_id` (global) and `episode`.  One device -> host copy and synchronisation; what an RLlib callback calls in
+        place of reading `get_sub_environments()`."""
+        log = self._episode_log
+        if log is None:
+            raise ValueError("this adapter was created with episode_log_capacity=0")
+        rec = log.drain()
+        return [dict(m, env_id=int(e), episode=int(k)) for m, e, k in zip(log.metrics(rec), rec["env_id"], rec["episode"])]
+
+
+class SSDVectorEnv(_EpisodeMetricsMixin):
     def __init__(self, kind, num_envs, num_agents, contract=None, horizon=1000, seed=73907, first_env_id=0, device=None,
-                 ascii_map=None, one_hot_id=False, **batch_kwargs):
+                 ascii_map=None, one_hot_id=False, episode_log_capacity=None, **batch_kwargs):
         self.batch = BatchedGridEnv(kind, num_envs, num_agents, ascii_map=ascii_map, horizon=horizon, contract=contract,
                                     seed=seed, first_env_id=first_env_id, device=device, **batch_kwargs)
+        _open_episode_log(self, episode_log_capacity)
         self.num_envs, self.num_agents, self.contract = int(num_envs), int(num_agents), contract
         self.agent_ids = ["a%d" % i for i in range(self.num_agents)]
         self.one_hot_id = one_hot_id
@@ -134,13 +161,14 @@ class SSDVectorEnv:
         self.batch.close()
 
 
-class _ArrayVectorEnv:
+class _ArrayVectorEnv(_EpisodeMetricsMixin):
     """poll_arrays() / send_action_array() / try_reset() over a feature-env or selfdrive batch (same contract as
     `SSDVectorEnv`: one host -> device copy per send, one packed device -> host copy per poll, resets requested between two
     polls run as one masked device reset and show up as `fresh` envs in the next poll)."""
 
-    def _setup(self, batch, action_dtype, idle_action):
+    def _setup(self, batch, action_dtype, idle_action, episode_log_capacity):
         self.batch = batch
+        _open_episode_log(self, episode_log_capacity)
         self.num_envs, self.num_agents = batch.E, batch.n
         self.agent_ids = ["a%d" % i for i in range(self.num_agents)]
         self._idle = idle_action
@@ -207,11 +235,11 @@ class SSDFeatureVectorEnv(_ArrayVectorEnv):
     observations of the non-convolutional wrapper, features ++ [theta, 0] (two_stage_train.py:104-121)."""
 
     def __init__(self, kind, num_envs, num_agents, contract=None, horizon=1000, seed=73907, first_env_id=0, device=None,
-                 ascii_map=None):
+                 ascii_map=None, episode_log_capacity=None):
         from .features import BatchedFeatureEnv
         self.contract = contract
         self._setup(BatchedFeatureEnv(kind, num_envs, num_agents, ascii_map=ascii_map, horizon=horizon, contract=contract,
-                                      seed=seed, first_env_id=first_env_id, device=device), torch.uint8, 4)
+                                      seed=seed, first_env_id=first_env_id, device=device), torch.uint8, 4, episode_log_capacity)
 
     def send_actions(self, action_dict):
         _staging_free(self)
@@ -243,8 +271,9 @@ class SSDCarVectorEnv(_ArrayVectorEnv):
     """E SelfAcceleratingCarEnv envs behind one rollout worker (arrays only: float32 accelerations [E, n] in; cars that are
     done are flagged in done[:, k] and their actions are ignored)."""
 
-    def __init__(self, num_envs, num_agents, contract=None, seed=73907, first_env_id=0, device=None, **batch_kwargs):
+    def __init__(self, num_envs, num_agents, contract=None, seed=73907, first_env_id=0, device=None, episode_log_capacity=None,
+                 **batch_kwargs):
         from .selfdrive import BatchedCarEnv
         self.contract = contract
         self._setup(BatchedCarEnv(num_envs, num_agents, contract=contract, seed=seed, first_env_id=first_env_id, device=device,
-                                  **batch_kwargs), torch.float32, 0.0)
+                                  **batch_kwargs), torch.float32, 0.0, episode_log_capacity)

@@ -285,6 +285,40 @@ int ssd_get_metrics(ssd_handle* h, double* out_dev, void* stream);
 #define SSD_STATS_LEN 8
 int ssd_set_episode_stats(ssd_handle* h, double* stats_dev);
 
+/* Episode log: one record per finished episode, for every env kind (the per-episode form of the MetricsCallback hand-off,
+ * utils/logger_utils.py:126-151).  While a log is set (sticky; NULL switches it off), the kernel that resets an env whose
+ * episode it replaces appends one record to a caller-owned ring buffer on the device: ssd_reset / ssd_feat_reset /
+ * ssd_selfdrive_reset (masked or not), the grid auto_reset behind a step, the next-step auto_reset of the feature and
+ * selfdrive steps, and the pipelined host-buffer steps, which run the same kernels.  Nothing is read or synchronised per
+ * step, and the appends work inside a captured CUDA graph.
+ *   - only resets append: ssd_checkpoint_load and ssd_set_state are not episode ends;
+ *   - an env that was never reset has no episode to log; a reset at t = 0 logs a zero-length episode (what
+ *     ssd_set_episode_stats counts as an episode too);
+ *   - the order of the records of one launch is unspecified, their contents are deterministic;
+ *   - the caller keeps both buffers alive while the log is set. */
+typedef struct ssd_episode_record {      /* 480 bytes, 16-byte aligned in the buffer */
+    uint32_t env_id;     /* global id (first_env_id + i) */
+    uint32_t episode;    /* number of the finished episode (0 = the env's first) */
+    int32_t  t;          /* steps it ran */
+    uint32_t ended;      /* 1: it ended by itself (grid / feature: t == horizon; selfdrive: every car done); 0: a reset cut it short */
+    double   theta;      /* its contract parameter */
+    double   pad;        /* 0 */
+    double   metrics[SSD_METRIC_STRIDE];   /* grid: the ssd_get_metrics row; feature envs: the ssd_feat_get_metrics row
+                                              (40 values, the rest 0); selfdrive: [0] = the transfers metric, the rest 0 --
+                                              each exactly as the getter would have returned it just before the reset */
+} ssd_episode_record;
+
+typedef struct ssd_episode_log {
+    int32_t struct_size;                 /* sizeof(ssd_episode_log); smaller is rejected */
+    int32_t capacity;                    /* records in records_dev, >= 1 */
+    ssd_episode_record* records_dev;     /* [capacity], 16-byte aligned */
+    unsigned long long* count_dev;       /* records appended since it was zeroed (by the caller); record k lands in slot k % capacity */
+} ssd_episode_log;
+
+/* Every env kind.  Validates before storing anything: SSD_EINVAL for a struct_size too small, capacity < 1, a NULL or
+ * misaligned records_dev (16 bytes) or count_dev (8 bytes). */
+int ssd_set_episode_log(ssd_handle* h, const ssd_episode_log* log);
+
 /* --- SelfAcceleratingCarEnv (env_kind SSD_ENV_SELFDRIVE) -------------------------------------------------
  * environments/self_driving_car_accelerate.py reset :49-79 / step :151-250 (collision_on=False), optionally with
  * SelfdriveContractDistprop (contract/contract_list.py:66-102) + SeparateContractSubgameStage
