@@ -63,6 +63,11 @@ class ssd_policy_out(ctypes.Structure):
                 ("contract_dev", ctypes.c_void_p)]
 
 
+class ssd_flat_policy_out(ctypes.Structure):
+    _fields_ = [("struct_size", ctypes.c_int32), ("dtype", ctypes.c_int32), ("obs_dev", ctypes.c_void_p)]
+
+
+
 STATS_LEN = 8
 
 
@@ -114,7 +119,7 @@ EXPORTS = [
     "ssd_step_host_async", "ssd_step_host_wait", "ssd_host_result_layout", "ssd_host_result_expand", "ssd_set_episode_stats",
     "ssd_feat_step_host_async", "ssd_selfdrive_step_host_async",
     "ssd_checkpoint_get_layout", "ssd_checkpoint_save", "ssd_checkpoint_load", "ssd_set_policy_output",
-    "ssd_set_episode_log",
+    "ssd_set_episode_log", "ssd_set_flat_policy_output",
 ]
 
 _LIB = None
@@ -170,6 +175,7 @@ def load():
     L.ssd_render.argtypes = [vp, vp, vp]
     L.ssd_policy_inputs.argtypes = [vp, vp, i64, i32, vp, vp, vp]
     L.ssd_set_policy_output.argtypes = [vp, ctypes.POINTER(ssd_policy_out)]
+    L.ssd_set_flat_policy_output.argtypes = [vp, ctypes.POINTER(ssd_flat_policy_out)]
     L.ssd_solver_choose.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp]
     L.ssd_feature_dim.argtypes = [vp]
     L.ssd_state_bytes_per_env.argtypes = [vp]

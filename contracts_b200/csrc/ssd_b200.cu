@@ -66,6 +66,8 @@ struct ssd_handle {
     int pol_form;            // ssd_set_policy_output: OBS_U8 (none) or 1 + SSD_POLICY_*, the form the observe / reset kernels write
     uint8_t* pol_image;      //   T [E n][3][15][15]
     void* pol_contract;      //   T [E n][10] or NULL
+    int flat_form;           // ssd_set_flat_policy_output: OBS_F64 (none) or 1 + SSD_POLICY_*, the form the feature / selfdrive kernels write
+    FlatPolicy flat;         //   T [E n][W] (rows NULL: none)
     char err[512];
     std::vector<void*> dev_allocs;
 };
@@ -105,6 +107,34 @@ static reset_kernel_t reset_pick(int form)
 static reset_kernel_t reset_kernel_fn(int kind, int form)
 {
     return kind == SSD_ENV_CLEANUP ? reset_pick<SSD_ENV_CLEANUP>(form) : reset_pick<SSD_ENV_HARVEST>(form);
+}
+typedef void (*feat_kernel_t)(const FeatParams, const FeatIO, const uint8_t*);
+template <bool CLEANUP, bool RESET_ONLY>
+static feat_kernel_t feat_pick(int form)
+{
+    if (form == 1 + POLICY_F32) return feat_kernel<CLEANUP, RESET_ONLY, 1 + POLICY_F32>;
+    if (form == 1 + POLICY_F16) return feat_kernel<CLEANUP, RESET_ONLY, 1 + POLICY_F16>;
+    if (form == 1 + POLICY_BF16) return feat_kernel<CLEANUP, RESET_ONLY, 1 + POLICY_BF16>;
+    return feat_kernel<CLEANUP, RESET_ONLY, OBS_F64>;
+}
+// form: OBS_F64 or the flat policy form of ssd_set_flat_policy_output (1 + SSD_POLICY_*)
+static feat_kernel_t feat_kernel_fn(bool cleanup, bool reset_only, int form)
+{
+    if (cleanup) return reset_only ? feat_pick<true, true>(form) : feat_pick<true, false>(form);
+    return reset_only ? feat_pick<false, true>(form) : feat_pick<false, false>(form);
+}
+typedef void (*car_kernel_t)(const CarParams, const CarIO, const uint8_t*);
+template <bool RESET_ONLY>
+static car_kernel_t car_pick(int form)
+{
+    if (form == 1 + POLICY_F32) return car_kernel<RESET_ONLY, 1 + POLICY_F32>;
+    if (form == 1 + POLICY_F16) return car_kernel<RESET_ONLY, 1 + POLICY_F16>;
+    if (form == 1 + POLICY_BF16) return car_kernel<RESET_ONLY, 1 + POLICY_BF16>;
+    return car_kernel<RESET_ONLY, OBS_F64>;
+}
+static car_kernel_t car_kernel_fn(bool reset_only, int form)
+{
+    return reset_only ? car_pick<true>(form) : car_pick<false>(form);
 }
 // bytes of one env's block of the policy image tensor
 static long long policy_env_bytes(const GridParams& p, int form)
@@ -482,13 +512,13 @@ static int setup_selfdrive(ssd_handle* h)
     if ((rc = dev_zalloc(h, E, &p.episode))) return rc;
     p.warp_doubles = (4 * p.n * p.D + 1) / 2 * 2 + 4 * CAR_OCT_DOUBLES;
     h->car_smem = CAR_WARPS * p.warp_doubles * (int)sizeof(double);
-    CUDA_TRY(h, cudaFuncSetAttribute((const void*)car_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->car_smem));
-    CUDA_TRY(h, cudaFuncSetAttribute((const void*)car_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, h->car_smem));
+    CUDA_TRY(h, cudaFuncSetAttribute((const void*)car_kernel_fn(false, OBS_F64), cudaFuncAttributeMaxDynamicSharedMemorySize, h->car_smem));
+    CUDA_TRY(h, cudaFuncSetAttribute((const void*)car_kernel_fn(true, OBS_F64), cudaFuncAttributeMaxDynamicSharedMemorySize, h->car_smem));
     {   // persistent CTAs: as many as are resident at once
         int dev = 0, sms = 0, per_sm = 0;
         CUDA_TRY(h, cudaGetDevice(&dev));
         CUDA_TRY(h, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-        CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)car_kernel<false>, CAR_THREADS, (size_t)h->car_smem));
+        CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)car_kernel_fn(false, OBS_F64), CAR_THREADS, (size_t)h->car_smem));
         h->grid_blocks = std::max(1, std::min((p.E + CAR_ENVS_PER_CTA - 1) / CAR_ENVS_PER_CTA, sms * std::max(per_sm, 1)));
     }
     return SSD_OK;
@@ -609,18 +639,15 @@ static int setup_features(ssd_handle* h)
     if ((rc = dev_zalloc(h, E * n, &p.tsum_tr))) return rc;
     h->feat_smem = p.sm_static + FEAT_ENVS_PER_CTA * p.oct_bytes;
     if (h->feat_smem > 200 * 1024) return fail(h, SSD_EUNSUPPORTED, "feature envs: %d bytes of shared memory per CTA", h->feat_smem);
-    for (int q = 0; q < 4; q++) {
-        const void* fn = q == 0 ? (const void*)feat_kernel<true, false> : q == 1 ? (const void*)feat_kernel<true, true>
-                       : q == 2 ? (const void*)feat_kernel<false, false> : (const void*)feat_kernel<false, true>;
-        CUDA_TRY(h, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, h->feat_smem));
-    }
+    for (int q = 0; q < 2; q++)
+        CUDA_TRY(h, cudaFuncSetAttribute((const void*)feat_kernel_fn(cleanup, q != 0, OBS_F64), cudaFuncAttributeMaxDynamicSharedMemorySize, h->feat_smem));
     // persistent CTAs: as many as are resident at once (a warp takes four envs per round)
     {
         int dev = 0, sms = 0, per_sm = 0;
         CUDA_TRY(h, cudaGetDevice(&dev));
         CUDA_TRY(h, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-        const void* fn = cleanup ? (const void*)feat_kernel<true, false> : (const void*)feat_kernel<false, false>;
-        CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, FEAT_THREADS, (size_t)h->feat_smem));
+        CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)feat_kernel_fn(cleanup, false, OBS_F64), FEAT_THREADS,
+                                                              (size_t)h->feat_smem));
         const int groups = (p.E + FEAT_ENVS_PER_CTA - 1) / FEAT_ENVS_PER_CTA;
         h->grid_blocks = std::max(1, std::min(groups, sms * std::max(per_sm, 1)));
     }
@@ -800,6 +827,17 @@ __global__ void get_metrics_kernel(GridParams p, double* out)
     for (int q = 0; q < SSD_METRIC_STRIDE; q++) o[q] = grid_metric(p, hdr, q);
 }
 
+// checkpoint load with flat policy rows set (feature envs, selfdrive): their theta column from the loaded envs' theta
+// (addressed like the solver's).  Rows that failed validation kept their theta, so rewriting theirs changes nothing.
+__global__ void flat_theta_refresh_kernel(SolverParams p, const int32_t* env_idx, int count)
+{
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= count) return;
+    const int env = env_idx ? env_idx[r] : r;
+    if (env < 0 || env >= p.E) return;
+    flat_policy_theta(p.flat, p.n, env, *reinterpret_cast<const double*>(p.theta + (size_t)env * p.theta_stride));
+}
+
 // SeparateContractNegotiateStage.step, agreement stage (two_stage_train.py:266-281)
 __global__ void negotiate_kernel(SolverParams p, const uint8_t* mask, const double* proposals, const double* accept, uint8_t* decision)
 {
@@ -812,6 +850,7 @@ __global__ void negotiate_kernel(SolverParams p, const uint8_t* mask, const doub
     *reinterpret_cast<double*>(p.theta + (size_t)env * p.theta_stride) = theta;
     if (decision) decision[env] = dec ? 1 : 0;
     if (p.pol_contract) policy_contract_env(p.pol_contract, p.pol_dtype, p.n, env, theta);
+    flat_policy_theta(p.flat, p.n, env, theta);
 }
 
 // step_index == SSD_STEP_AUTO: take the index from the handle's device counter (bumped by the last CTA to finish,
@@ -954,6 +993,27 @@ static int check_launch(ssd_handle* h, const char* what)
     if (!IS_FEAT(h)) return fail(h, SSD_EINVAL, "%s: handle is not a feature env (env_kind %d)", __func__, (h)->cfg.env_kind)
 #define REQUIRE_CAR(h) \
     if ((h)->cfg.env_kind != SSD_ENV_SELFDRIVE) return fail(h, SSD_EINVAL, "%s: handle is not a selfdrive env", __func__)
+
+// the flat policy rows as the theta refreshes see them: none without a contract (the rows then have no theta column)
+static FlatPolicy flat_theta_rows(const ssd_handle* h)
+{
+    FlatPolicy f = h->flat;
+    if (h->cfg.contract_kind == SSD_CONTRACT_NONE) f.rows = nullptr;
+    return f;
+}
+// the rows a feature-env / selfdrive step or reset writes: obs_dev, or the flat policy rows while they are set (obs_dev
+// must then be NULL: one observation form per handle)
+static int flat_obs_target(ssd_handle* h, const char* what, void* obs_dev, bool required, void** out)
+{
+    if (h->flat_form) {
+        if (obs_dev) return fail(h, SSD_EINVAL, "%s: obs_dev must be NULL while flat policy rows are set (ssd_set_flat_policy_output)", what);
+        *out = h->flat.rows;
+    } else {
+        if (required && !obs_dev) return fail(h, SSD_EINVAL, "actions_dev, obs_dev and rew_dev are required");
+        *out = obs_dev;
+    }
+    return SSD_OK;
+}
 
 int ssd_reset(ssd_handle* h, const uint8_t* mask_dev, uint8_t* obs_dev, int64_t obs_env_stride, void* stream)
 {
@@ -1320,9 +1380,9 @@ int ssd_set_contract_params(ssd_handle* h, const double* theta_dev, void* stream
     if (!h || !theta_dev) return SSD_EINVAL;
     ON_DEVICE(h);
     if (h->cfg.env_kind == SSD_ENV_SELFDRIVE)
-        car_set_theta_kernel<<<(h->cp.E + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->cp, theta_dev);
+        car_set_theta_kernel<<<(h->cp.E + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->cp, theta_dev, flat_theta_rows(h));
     else if (IS_FEAT(h))
-        feat_set_theta_kernel<<<(h->fp.E + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->fp, theta_dev);
+        feat_set_theta_kernel<<<(h->fp.E + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->fp, theta_dev, flat_theta_rows(h));
     else
         SMALL_LAUNCH(set_theta_kernel, theta_dev, h->pol_contract, h->pol_form - 1);
     return check_launch(h, "set_contract_params");
@@ -1446,6 +1506,32 @@ int ssd_set_policy_output(ssd_handle* h, const ssd_policy_out* out)
     return SSD_OK;
 }
 
+int ssd_set_flat_policy_output(ssd_handle* h, const ssd_flat_policy_out* out)
+{
+    if (!h) return SSD_EINVAL;
+    ON_DEVICE(h);
+    if (h->cfg.env_kind != SSD_ENV_SELFDRIVE && !IS_FEAT(h))
+        return fail(h, SSD_EINVAL, "set_flat_policy_output: handle is a gridworld (env_kind %d; see ssd_set_policy_output)", h->cfg.env_kind);
+    if (!out) { h->flat_form = OBS_F64; h->flat = FlatPolicy{ nullptr, 0, 0 }; return SSD_OK; }
+    if (out->struct_size < (int32_t)sizeof(ssd_flat_policy_out))
+        return fail(h, SSD_EINVAL, "ssd_flat_policy_out.struct_size %d < %d: the caller's declaration of ssd_flat_policy_out is out of date",
+                    out->struct_size, (int)sizeof(ssd_flat_policy_out));
+    if (out->dtype != POLICY_F32 && out->dtype != POLICY_F16 && out->dtype != POLICY_BF16)
+        return fail(h, SSD_EINVAL, "set_flat_policy_output: dtype %d is not SSD_POLICY_F32, _F16 or _BF16", out->dtype);
+    if (!out->obs_dev || (reinterpret_cast<uintptr_t>(out->obs_dev) & 15))
+        return fail(h, SSD_EINVAL, "set_flat_policy_output: obs_dev must be a 16-byte aligned device pointer");
+    const int form = 1 + out->dtype;
+    const bool car = h->cfg.env_kind == SSD_ENV_SELFDRIVE;
+    for (int q = 0; q < 2; q++) {
+        const void* fn = car ? (const void*)car_kernel_fn(q != 0, form)
+                             : (const void*)feat_kernel_fn(h->cfg.env_kind == SSD_ENV_CLEANUP_FEATURES, q != 0, form);
+        CUDA_TRY(h, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, car ? h->car_smem : h->feat_smem));
+    }
+    h->flat_form = form;
+    h->flat = FlatPolicy{ out->obs_dev, out->dtype, ssd_feature_dim(h) + (h->cfg.contract_kind != SSD_CONTRACT_NONE ? 2 : 0) };
+    return SSD_OK;
+}
+
 // ---- NegotiationSolver (two_stage_train.py:619-776) ------------------------------------------------
 static SolverParams solver_params(ssd_handle* h)
 {
@@ -1457,9 +1543,11 @@ static SolverParams solver_params(ssd_handle* h)
     if (h->cfg.env_kind == SSD_ENV_SELFDRIVE) {
         s.episode = reinterpret_cast<const uint8_t*>(h->cp.episode); s.episode_stride = 4; s.episode_mask = 0xFFFFFFFFu;
         s.theta = reinterpret_cast<uint8_t*>(h->cp.theta); s.theta_stride = 8;
+        s.flat = flat_theta_rows(h);
     } else if (IS_FEAT(h)) {
         s.episode = reinterpret_cast<const uint8_t*>(h->fp.rec + FR_EPISODE); s.episode_stride = 4 * FR_WORDS; s.episode_mask = 0x7FFFFFFFu;
         s.theta = reinterpret_cast<uint8_t*>(h->fp.rec + FR_THETA); s.theta_stride = 4 * FR_WORDS;
+        s.flat = flat_theta_rows(h);
     } else {
         const GridParams& p = h->gp;
         s.episode = p.state + RO_EPISODE; s.episode_stride = p.rec_stride; s.episode_mask = 0xFFFFFFFFu;
@@ -1543,9 +1631,10 @@ int ssd_feat_reset(ssd_handle* h, const uint8_t* mask_dev, double* obs_dev, void
     ON_DEVICE(h);
     REQUIRE_FEAT(h);
     FeatIO k = {};
-    k.obs = obs_dev;
-    if (h->cfg.env_kind == SSD_ENV_CLEANUP_FEATURES) feat_kernel<true, true><<<h->grid_blocks, FEAT_THREADS, h->feat_smem, (cudaStream_t)stream>>>(h->fp, k, mask_dev);
-    else feat_kernel<false, true><<<h->grid_blocks, FEAT_THREADS, h->feat_smem, (cudaStream_t)stream>>>(h->fp, k, mask_dev);
+    int rc = flat_obs_target(h, "feat_reset", obs_dev, false, &k.obs);
+    if (rc) return rc;
+    feat_kernel_fn(h->cfg.env_kind == SSD_ENV_CLEANUP_FEATURES, true, h->flat_form)<<<h->grid_blocks, FEAT_THREADS, h->feat_smem,
+                                                                                      (cudaStream_t)stream>>>(h->fp, k, mask_dev);
     return check_launch(h, "feat_reset");
 }
 
@@ -1554,32 +1643,38 @@ int ssd_feat_step(ssd_handle* h, const ssd_feat_io* io, void* stream)
     if (!h || !io) return SSD_EINVAL;
     ON_DEVICE(h);
     REQUIRE_FEAT(h);
-    if (!io->actions_dev || !io->obs_dev || !io->rew_dev) return fail(h, SSD_EINVAL, "actions_dev, obs_dev and rew_dev are required");
+    void* obs = nullptr;
+    int rc = flat_obs_target(h, "feat_step", io->obs_dev, true, &obs);
+    if (rc) return rc;
+    if (!io->actions_dev || !io->rew_dev) return fail(h, SSD_EINVAL, "actions_dev, obs_dev and rew_dev are required");
     if (io->info_dev && (reinterpret_cast<uintptr_t>(io->info_dev) & 3)) return fail(h, SSD_EINVAL, "info_dev must be 4-byte aligned");
-    FeatIO k = { io->actions_dev, io->obs_dev, io->rew_dev, io->base_rew_dev, io->transfers_dev, io->info_dev, io->done_dev, io->auto_reset };
-    if (h->cfg.env_kind == SSD_ENV_CLEANUP_FEATURES) feat_kernel<true, false><<<h->grid_blocks, FEAT_THREADS, h->feat_smem, (cudaStream_t)stream>>>(h->fp, k, nullptr);
-    else feat_kernel<false, false><<<h->grid_blocks, FEAT_THREADS, h->feat_smem, (cudaStream_t)stream>>>(h->fp, k, nullptr);
+    FeatIO k = { io->actions_dev, obs, io->rew_dev, io->base_rew_dev, io->transfers_dev, io->info_dev, io->done_dev, io->auto_reset };
+    feat_kernel_fn(h->cfg.env_kind == SSD_ENV_CLEANUP_FEATURES, false, h->flat_form)<<<h->grid_blocks, FEAT_THREADS, h->feat_smem,
+                                                                                       (cudaStream_t)stream>>>(h->fp, k, nullptr);
     return check_launch(h, "feat_step");
 }
 
 int ssd_feat_step_host_async(ssd_handle* h, const ssd_feat_io* io, const void* actions_host, void* result_host, int64_t* ticket_out,
                              void* stream)
 {
-    if (!h || !io || !actions_host || !result_host || !ticket_out || !io->obs_dev) return SSD_EINVAL;
+    if (!h || !io || !actions_host || !result_host || !ticket_out || (!io->obs_dev && !h->flat_form)) return SSD_EINVAL;
     ON_DEVICE(h);
     REQUIRE_FEAT(h);
+    void* obs = nullptr;
+    int rc = flat_obs_target(h, "feat_step_host_async", io->obs_dev, true, &obs);
+    if (rc) return rc;
     if (io->info_dev && (reinterpret_cast<uintptr_t>(io->info_dev) & 3)) return fail(h, SSD_EINVAL, "info_dev must be 4-byte aligned");
     int si = 0;
-    int rc = async_begin(h, actions_host, result_host, (cudaStream_t)stream, &si);
+    rc = async_begin(h, actions_host, result_host, (cudaStream_t)stream, &si);
     if (rc) return rc;
     ssd_handle::Slot& sl = h->slot[si];
-    FeatIO k = { sl.d_actions, io->obs_dev, io->rew_dev, io->base_rew_dev, io->transfers_dev, io->info_dev, io->done_dev, io->auto_reset };
+    FeatIO k = { sl.d_actions, obs, io->rew_dev, io->base_rew_dev, io->transfers_dev, io->info_dev, io->done_dev, io->auto_reset };
     k.c_count = reinterpret_cast<uint32_t*>(sl.d_block + h->lay.count_offset);
     k.c_done = sl.d_block + h->lay.done_offset;
     k.c_rew8 = reinterpret_cast<int8_t*>(sl.d_block + h->lay.rew_i8_offset);
     k.c_rec = sl.d_block + h->lay.records_offset;
-    if (h->cfg.env_kind == SSD_ENV_CLEANUP_FEATURES) feat_kernel<true, false><<<h->grid_blocks, FEAT_THREADS, h->feat_smem, (cudaStream_t)stream>>>(h->fp, k, nullptr);
-    else feat_kernel<false, false><<<h->grid_blocks, FEAT_THREADS, h->feat_smem, (cudaStream_t)stream>>>(h->fp, k, nullptr);
+    feat_kernel_fn(h->cfg.env_kind == SSD_ENV_CLEANUP_FEATURES, false, h->flat_form)<<<h->grid_blocks, FEAT_THREADS, h->feat_smem,
+                                                                                       (cudaStream_t)stream>>>(h->fp, k, nullptr);
     if ((rc = check_launch(h, "feat_step_host_async"))) return rc;
     return async_end(h, si, (cudaStream_t)stream, ticket_out);
 }
@@ -1609,8 +1704,9 @@ int ssd_selfdrive_reset(ssd_handle* h, const uint8_t* mask_dev, double* obs_dev,
     ON_DEVICE(h);
     REQUIRE_CAR(h);
     CarIO k = {};
-    k.obs = obs_dev;
-    car_kernel<true><<<h->grid_blocks, CAR_THREADS, h->car_smem, (cudaStream_t)stream>>>(h->cp, k, mask_dev);
+    int rc = flat_obs_target(h, "selfdrive_reset", obs_dev, false, &k.obs);
+    if (rc) return rc;
+    car_kernel_fn(true, h->flat_form)<<<h->grid_blocks, CAR_THREADS, h->car_smem, (cudaStream_t)stream>>>(h->cp, k, mask_dev);
     return check_launch(h, "selfdrive_reset");
 }
 
@@ -1619,31 +1715,37 @@ int ssd_selfdrive_step(ssd_handle* h, const ssd_selfdrive_io* io, void* stream)
     if (!h || !io) return SSD_EINVAL;
     ON_DEVICE(h);
     REQUIRE_CAR(h);
-    if (!io->actions_dev || !io->obs_dev || !io->rew_dev) return fail(h, SSD_EINVAL, "actions_dev, obs_dev and rew_dev are required");
+    void* obs = nullptr;
+    int rc = flat_obs_target(h, "selfdrive_step", io->obs_dev, true, &obs);
+    if (rc) return rc;
+    if (!io->actions_dev || !io->rew_dev) return fail(h, SSD_EINVAL, "actions_dev, obs_dev and rew_dev are required");
     if (io->info_dev && (reinterpret_cast<uintptr_t>(io->info_dev) & 31)) return fail(h, SSD_EINVAL, "info_dev must be 32-byte aligned");
-    CarIO k = { io->actions_dev, io->obs_dev, io->rew_dev, io->base_rew_dev, io->transfers_dev, io->info_dev, io->done_dev, io->auto_reset };
-    car_kernel<false><<<h->grid_blocks, CAR_THREADS, h->car_smem, (cudaStream_t)stream>>>(h->cp, k, nullptr);
+    CarIO k = { io->actions_dev, obs, io->rew_dev, io->base_rew_dev, io->transfers_dev, io->info_dev, io->done_dev, io->auto_reset };
+    car_kernel_fn(false, h->flat_form)<<<h->grid_blocks, CAR_THREADS, h->car_smem, (cudaStream_t)stream>>>(h->cp, k, nullptr);
     return check_launch(h, "selfdrive_step");
 }
 
 int ssd_selfdrive_step_host_async(ssd_handle* h, const ssd_selfdrive_io* io, const void* actions_host, void* result_host,
                                   int64_t* ticket_out, void* stream)
 {
-    if (!h || !io || !actions_host || !result_host || !ticket_out || !io->obs_dev) return SSD_EINVAL;
+    if (!h || !io || !actions_host || !result_host || !ticket_out || (!io->obs_dev && !h->flat_form)) return SSD_EINVAL;
     ON_DEVICE(h);
     if (h->cfg.env_kind != SSD_ENV_SELFDRIVE) return fail(h, SSD_EINVAL, "selfdrive_step_host_async: handle is not a selfdrive env");
+    void* obs = nullptr;
+    int rc = flat_obs_target(h, "selfdrive_step_host_async", io->obs_dev, true, &obs);
+    if (rc) return rc;
     if (io->info_dev && (reinterpret_cast<uintptr_t>(io->info_dev) & 31)) return fail(h, SSD_EINVAL, "info_dev must be 32-byte aligned");
     int si = 0;
-    int rc = async_begin(h, actions_host, result_host, (cudaStream_t)stream, &si);
+    rc = async_begin(h, actions_host, result_host, (cudaStream_t)stream, &si);
     if (rc) return rc;
     ssd_handle::Slot& sl = h->slot[si];
-    CarIO k = { reinterpret_cast<const float*>(sl.d_actions), io->obs_dev, io->rew_dev, io->base_rew_dev, io->transfers_dev, io->info_dev, io->done_dev,
+    CarIO k = { reinterpret_cast<const float*>(sl.d_actions), obs, io->rew_dev, io->base_rew_dev, io->transfers_dev, io->info_dev, io->done_dev,
                 io->auto_reset };
     k.c_count = reinterpret_cast<uint32_t*>(sl.d_block + h->lay.count_offset);
     k.c_done = sl.d_block + h->lay.done_offset;
     k.c_rew8 = reinterpret_cast<int8_t*>(sl.d_block + h->lay.rew_i8_offset);
     k.c_rec = sl.d_block + h->lay.records_offset;
-    car_kernel<false><<<h->grid_blocks, CAR_THREADS, h->car_smem, (cudaStream_t)stream>>>(h->cp, k, nullptr);
+    car_kernel_fn(false, h->flat_form)<<<h->grid_blocks, CAR_THREADS, h->car_smem, (cudaStream_t)stream>>>(h->cp, k, nullptr);
     if ((rc = check_launch(h, "selfdrive_step_host_async"))) return rc;
     return async_end(h, si, (cudaStream_t)stream, ticket_out);
 }
@@ -1716,6 +1818,11 @@ int ssd_checkpoint_load(ssd_handle* h, uint64_t config_tag, const int32_t* env_i
     if (h->pol_contract) {                                // theta came with the rows: the policy's contract rows follow it
         policy_contract_refresh_kernel<<<(count + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->gp, env_idx_dev, count, h->pol_contract,
                                                                                               h->pol_form - 1);
+        return check_launch(h, "checkpoint_load");
+    }
+    const SolverParams sp = solver_params(h);            // theta came with the rows: the flat policy rows' theta column follows it
+    if (sp.flat.rows) {
+        flat_theta_refresh_kernel<<<(count + 127) / 128, 128, 0, (cudaStream_t)stream>>>(sp, env_idx_dev, count);
         return check_launch(h, "checkpoint_load");
     }
     return SSD_OK;

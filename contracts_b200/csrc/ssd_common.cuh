@@ -4,6 +4,8 @@
 //   u32 = philox4x32_10(ctr = (idx >> 2, site | call << 8, t, episode), key = (seed, env_id))[idx & 3]
 // Site ids follow SURVEY.md §8a table R (reference file:line in oracle/philox.py).
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -119,6 +121,49 @@ __device__ __forceinline__ bool negotiate_agreement(uint32_t seed, uint32_t env_
     }
     const double r = __dmul_rn((double)draw_u32(seed, env_id, episode, 0, SITE_NEGOTIATE, 1, 0), 1.0 / 4294967296.0);
     return r < prod;
+}
+
+// element types of the policy's input tensors (SSD_POLICY_*: ssd_policy_inputs, ssd_set_policy_output,
+// ssd_set_flat_policy_output); an observation form 1 + POLICY_* writes T = PolicyElem<form>::T
+#define POLICY_F32 0
+#define POLICY_F16 1
+#define POLICY_BF16 2
+template <int FORM> struct PolicyElem;
+template <> struct PolicyElem<1 + POLICY_F32> { typedef float T; };
+template <> struct PolicyElem<1 + POLICY_F16> { typedef __half T; };
+template <> struct PolicyElem<1 + POLICY_BF16> { typedef __nv_bfloat16 T; };
+
+template <typename T> __device__ __forceinline__ T policy_cast(float v);
+template <> __device__ __forceinline__ float policy_cast<float>(float v) { return v; }
+template <> __device__ __forceinline__ __half policy_cast<__half>(float v) { return __float2half_rn(v); }
+template <> __device__ __forceinline__ __nv_bfloat16 policy_cast<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+
+// Observation form of the feature-env and selfdrive kernels: OBS_F64 = the float64 rows [E][n][F | D]; 1 + POLICY_* = the
+// policy's flat rows T [E n][W] (ssd_set_flat_policy_output): features ++ [theta, 0] with a contract (W = F + 2), else the
+// features alone (W = F), each value T(float32(x)).
+#define OBS_F64 0
+template <typename T>
+__device__ __forceinline__ void policy_column_rows(T* rows, int n, int width, int col, double theta)
+{
+    const T v = policy_cast<T>(__double2float_rn(theta));
+    for (int a = 0; a < n; a++) rows[(size_t)a * width + col] = v;
+}
+// Column `col` of the n rows of `env` in a policy tensor T [E n][width] (T by dtype = SSD_POLICY_*) set to theta: what
+// the calls that change theta outside a step do to the flat rows (thread-per-env kernels).
+__device__ __forceinline__ void policy_column_env(void* rows, int dtype, int n, int width, int col, int env, double theta)
+{
+    const size_t o = (size_t)env * n * width;
+    if (dtype == POLICY_F32) policy_column_rows(reinterpret_cast<float*>(rows) + o, n, width, col, theta);
+    else if (dtype == POLICY_F16) policy_column_rows(reinterpret_cast<__half*>(rows) + o, n, width, col, theta);
+    else policy_column_rows(reinterpret_cast<__nv_bfloat16*>(rows) + o, n, width, col, theta);
+}
+// The flat policy rows of a feature-env / selfdrive handle as the theta refreshes see them (rows == nullptr: not set).
+struct FlatPolicy {
+    void* rows; int dtype, width;
+};
+__device__ __forceinline__ void flat_policy_theta(const FlatPolicy& f, int n, int env, double theta)
+{
+    if (f.rows) policy_column_env(f.rows, f.dtype, n, f.width, f.width - 2, env, theta);
 }
 
 // SSD_STEP_AUTO (ssd_random_actions & co.): counter[0] = step index, counter[1] = CTAs finished.  Every CTA reads

@@ -81,7 +81,7 @@ struct FeatParams {
 
 struct FeatIO {
     const uint8_t* actions;     // [E][n]
-    double* obs;                // [E][n][F]
+    void* obs;                  // double [E][n][F] (OBS_F64), or the policy's rows T [E n][W] (1 + POLICY_*: feat_policy_row)
     double* rew; double* base_rew; double* transfers;   // [E][n]
     uint8_t* info;              // [E][n][4]: cleanup (cleaned_squares,0,0,0); harvest (eaten_apples, eaten_close_apples,0,0)
     uint8_t* done;              // [E]
@@ -276,10 +276,42 @@ __device__ __noinline__ void feat_log_episode(EpisodeLog log, const double* metr
 #define FEAT_WASTE_DRAWS 8               // waste draws evaluated together with the apple draws (more only when all of them fail)
 #endif
 
+// two policy elements at a 4-byte (T = 16-bit) or 8-byte (T = float) aligned address
+__device__ __forceinline__ void policy_store2(float* o, double x, double y)
+{
+    *reinterpret_cast<float2*>(o) = make_float2(__double2float_rn(x), __double2float_rn(y));
+}
+__device__ __forceinline__ void policy_store2(__half* o, double x, double y)
+{
+    *reinterpret_cast<__half2*>(o) = __halves2half2(__float2half_rn(__double2float_rn(x)), __float2half_rn(__double2float_rn(y)));
+}
+__device__ __forceinline__ void policy_store2(__nv_bfloat16* o, double x, double y)
+{
+    *reinterpret_cast<__nv_bfloat162*>(o) = __halves2bfloat162(__float2bfloat16_rn(__double2float_rn(x)), __float2bfloat16_rn(__double2float_rn(y)));
+}
+
+// The policy form's row of one agent: its F features ++ [theta, 0] with a contract, each T(float32(x)).  Row r starts at
+// byte r W sizeof(T), so it can start on any multiple of 2 bytes: when W is even (then F is even too) every row starts on
+// a pair and goes out in two-element stores, otherwise (cleanup with an odd agent count) element by element.
+template <typename T>
+__device__ __forceinline__ void feat_policy_row(T* o, const double (&v)[FEAT_MAXF], int F, bool contract, double theta)
+{
+    if ((F & 1) == 0) {
+#pragma unroll
+        for (int k = 0; k < FEAT_MAXF; k += 2) if (k < F) policy_store2(o + k, v[k], v[k + 1]);
+        if (contract) policy_store2(o + F, theta, 0.0);
+    } else {
+#pragma unroll
+        for (int k = 0; k < FEAT_MAXF; k++) if (k < F) o[k] = policy_cast<T>(__double2float_rn(v[k]));
+        if (contract) { o[F] = policy_cast<T>(__double2float_rn(theta)); o[F + 1] = policy_cast<T>(0.0f); }
+    }
+}
+
 // One launch = one step (or, RESET_ONLY, one masked reset) of every env.
 // Next-step auto-reset (ssd_feat_io.auto_reset): an env that reached its horizon in the previous step starts its next
 // episode in this one — reset observation, zero rewards, done cleared, the actions of this step ignored.
-template <bool CLEANUP, bool RESET_ONLY>
+// FORM: OBS_F64 (float64 rows [E][n][F]) or 1 + POLICY_* (the policy's rows, feat_policy_row).
+template <bool CLEANUP, bool RESET_ONLY, int FORM>
 __global__ void __launch_bounds__(FEAT_THREADS, FEAT_MIN_BLOCKS) feat_kernel(const FeatParams p, const FeatIO io, const uint8_t* __restrict__ mask)
 {
     extern __shared__ __align__(16) uint8_t fsm[];
@@ -752,13 +784,19 @@ __global__ void __launch_bounds__(FEAT_THREADS, FEAT_MIN_BLOCKS) feat_kernel(con
             for (int i = 10; i < FEAT_MAXF; i++) v[i] = 0.0;
         }
         const int F = p.F;
-        double* o = io.obs + ((size_t)env * n + a) * F;
-        if ((F & 1) == 0) {                                                // rows are 16-byte aligned iff F is even
+        if constexpr (FORM == OBS_F64) {
+            double* o = static_cast<double*>(io.obs) + ((size_t)env * n + a) * F;
+            if ((F & 1) == 0) {                                            // rows are 16-byte aligned iff F is even
 #pragma unroll
-            for (int k = 0; k < FEAT_MAXF; k += 2) if (k < F) reinterpret_cast<double2*>(o)[k >> 1] = make_double2(v[k], v[k + 1]);
+                for (int k = 0; k < FEAT_MAXF; k += 2) if (k < F) reinterpret_cast<double2*>(o)[k >> 1] = make_double2(v[k], v[k + 1]);
+            } else {
+#pragma unroll
+                for (int k = 0; k < FEAT_MAXF; k++) if (k < F) o[k] = v[k];
+            }
         } else {
-#pragma unroll
-            for (int k = 0; k < FEAT_MAXF; k++) if (k < F) o[k] = v[k];
+            const bool con = p.contract != SSD_CONTRACT_NONE;
+            typedef typename PolicyElem<FORM>::T T;
+            feat_policy_row(static_cast<T*>(io.obs) + ((size_t)env * n + a) * (F + (con ? 2 : 0)), v, F, con, theta);
         }
     }
 
@@ -884,10 +922,13 @@ __global__ void feat_get_state_kernel(const FeatParams p, int32_t* pos, int32_t*
     if (theta) theta[env] = *reinterpret_cast<const double*>(rec + FR_THETA);
     if (t) t[env] = (int)rec[FR_T];
 }
-__global__ void feat_set_theta_kernel(const FeatParams p, const double* theta)
+// flat: the policy's rows when they have a theta column (ssd_set_flat_policy_output), kept current
+__global__ void feat_set_theta_kernel(const FeatParams p, const double* theta, const FlatPolicy flat)
 {
     const int env = blockIdx.x * blockDim.x + threadIdx.x;
-    if (env < p.E) *reinterpret_cast<double*>(p.rec + (size_t)env * FR_WORDS + FR_THETA) = theta[env];
+    if (env >= p.E) return;
+    *reinterpret_cast<double*>(p.rec + (size_t)env * FR_WORDS + FR_THETA) = theta[env];
+    flat_policy_theta(flat, p.n, env, theta[env]);
 }
 __global__ void feat_random_actions_kernel(const FeatParams p, uint32_t step_index, uint32_t* counter, int num_actions, uint8_t* actions)
 {

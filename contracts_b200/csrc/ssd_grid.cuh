@@ -17,28 +17,13 @@
 //   environments/harvest_new.py  step :181-239, spawn_apples :284-317, count_apples_in_radius :326-336
 //   contract/contract_list.py :22-27, :45-54 ; environments/two_stage_train.py :62-121, :159-187
 #pragma once
-#include <cuda_bf16.h>
-#include <cuda_fp16.h>
 #include "ssd_common.cuh"
-
-// element types of the policy's input tensors (SSD_POLICY_*: ssd_policy_inputs, ssd_set_policy_output)
-#define POLICY_F32 0
-#define POLICY_F16 1
-#define POLICY_BF16 2
-
-template <typename T> __device__ __forceinline__ T policy_cast(float v);
-template <> __device__ __forceinline__ float policy_cast<float>(float v) { return v; }
-template <> __device__ __forceinline__ __half policy_cast<__half>(float v) { return __float2half_rn(v); }
-template <> __device__ __forceinline__ __nv_bfloat16 policy_cast<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
 
 // Observation form written by the observe / reset kernels: OBS_U8 = the uint8 windows [E][n][15][15][3]; 1 + POLICY_* = the
 // policy's image tensor T [E n][3][15][15] (ssd_set_policy_output), the values ssd_policy_inputs would make of the windows.
 #define OBS_U8 0
-template <int FORM> struct ObsForm;
+template <int FORM> struct ObsForm : PolicyElem<FORM> {};
 template <> struct ObsForm<OBS_U8> { typedef uint8_t T; };
-template <> struct ObsForm<1 + POLICY_F32> { typedef float T; };
-template <> struct ObsForm<1 + POLICY_F16> { typedef __half T; };
-template <> struct ObsForm<1 + POLICY_BF16> { typedef __nv_bfloat16 T; };
 
 #ifndef GRID_WARPS
 #define GRID_WARPS 8

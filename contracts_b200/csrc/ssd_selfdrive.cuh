@@ -48,7 +48,7 @@ struct CarParams {
 
 struct CarIO {
     const float* actions;   // [E][n]
-    double* obs;            // [E][n][D]
+    void* obs;              // double [E][n][D] (OBS_F64), or the policy's rows T [E n][W] (1 + POLICY_*: see car_kernel)
     double* rew; double* base_rew; double* transfers;   // [E][n]
     double* info;           // [E][n][4]: just_passed, active, ambulance_rank, ambulance_dist_to_front (row of the first acting agent)
     uint8_t* done;          // [E][n+1]
@@ -183,10 +183,24 @@ __device__ __noinline__ void car_log_episode(EpisodeLog log, const double* theta
     }
 }
 
+// An env's staged rows, L bytes, to global memory in the widest units that divide L: the staged run and its destination
+// start at multiples of L from 16-byte aligned bases, so both are aligned to the unit (16 bytes for n = 8 in every form).
+__device__ __forceinline__ void car_copy_run(uint8_t* dst, const uint8_t* src, int L, int lane)
+{
+    if ((L & 15) == 0) for (int f = lane; 16 * f < L; f += 32) reinterpret_cast<uint4*>(dst)[f] = reinterpret_cast<const uint4*>(src)[f];
+    else if ((L & 7) == 0) for (int f = lane; 8 * f < L; f += 32) reinterpret_cast<uint2*>(dst)[f] = reinterpret_cast<const uint2*>(src)[f];
+    else if ((L & 3) == 0) for (int f = lane; 4 * f < L; f += 32) reinterpret_cast<uint32_t*>(dst)[f] = reinterpret_cast<const uint32_t*>(src)[f];
+    else for (int f = lane; 2 * f < L; f += 32) reinterpret_cast<uint16_t*>(dst)[f] = reinterpret_cast<const uint16_t*>(src)[f];
+}
+
 // One launch = one step (or, RESET_ONLY, one masked reset) of every env.
 // Next-step auto-reset (ssd_selfdrive_io.auto_reset): an env whose episode ended in the previous step starts its next
 // episode in this one — reset observation, zero rewards, dones cleared, the actions of this step ignored.
-template <bool RESET_ONLY>
+// FORM: OBS_F64 (float64 rows [E][n][D]) or 1 + POLICY_*: the policy's rows T [E n][W], each car's D values ++ [theta, 0]
+// with a contract (W = D + 2), else the D values alone (W = D), each T(float32(x)).  Either form is built in the staging
+// area exactly as it goes out (an env's n rows contiguous, the warp's four envs one after the other) and copied out by
+// car_copy_run.
+template <bool RESET_ONLY, int FORM>
 __global__ void __launch_bounds__(CAR_THREADS, CAR_MIN_BLOCKS) car_kernel(const CarParams p, const CarIO io, const uint8_t* __restrict__ mask)
 {
     extern __shared__ __align__(16) double csm[];
@@ -236,6 +250,7 @@ __global__ void __launch_bounds__(CAR_THREADS, CAR_MIN_BLOCKS) car_kernel(const 
     const bool doreset = RESET_ONLY ? live : (live && io.auto_reset && ((meta0 >> 16) & 1u));
     const bool stepping = !RESET_ONLY && live && !doreset;
     double x = 0.0, v = 0.0;                            // this car's position / velocity after the step (or the reset)
+    double row_theta = theta_in;                        // the policy form's theta column (after a reset: lane 0's new theta)
 
     if (p.elog.records && __any_sync(CAR_FULL, doreset))     // hand the finished episodes over before the reset rewrites them
         car_log_episode(p.elog, p.theta, p.m_transfers, p.t, p.episode, env, p.first_env_id + (uint32_t)env,
@@ -262,6 +277,7 @@ __global__ void __launch_bounds__(CAR_THREADS, CAR_MIN_BLOCKS) car_kernel(const 
                 theta = (u0 > p.null_prob) ? __dadd_rn(p.theta_low, __dmul_rn(__dsub_rn(p.theta_high, p.theta_low), u1)) : p.theta_low;
             }
             p.theta[env] = theta; p.m_transfers[env] = 0.0; p.dist_front[env] = -1.0;
+            row_theta = theta;
             p.crossed[env] = 0u; p.meta[env] = 0x80000000u; p.t[env] = 0; p.episode[env] = episode;
         }
     }
@@ -396,25 +412,50 @@ __global__ void __launch_bounds__(CAR_THREADS, CAR_MIN_BLOCKS) car_kernel(const 
     // ---- observation rows (:244-249): [pos, vel, pos_q - pos (q < n), vel_q (q < n), pos_0 > 0, pos > 0, 0], built by the
     // car's lane in the staging area, then copied out as one contiguous run per env
     if (io.obs) {
-        if (kv) {
-            double* row = w_stage + (size_t)(oct * n + k) * D;
-            row[0] = x; row[1] = v;
-            for (int q = 0; q < n; q++) { row[2 + q] = __dsub_rn(o_pos[q], x); row[2 + n + q] = o_vel[q]; }
-            row[2 + 2 * n] = o_pos[0] > 0 ? 1.0 : 0.0;
-            row[3 + 2 * n] = x > 0 ? 1.0 : 0.0;
-            row[4 + 2 * n] = 0.0;
-        }
-        __syncwarp();
-        const uint32_t lv = __ballot_sync(CAR_FULL, live);
-        for (int q = 0; q < 4; q++) {
-            if (!((lv >> (8 * q)) & 1u)) continue;                        // (uniform)
-            const int e = (grp * CAR_WARPS + warp) * 4 + q;
-            double* dst = io.obs + (size_t)e * nD;
-            const double* src = w_stage + (size_t)q * nD;
-            if ((nD & 1) == 0) {                                           // 16-byte aligned runs
-                for (int f = lane; 2 * f < nD; f += 32) reinterpret_cast<double2*>(dst)[f] = reinterpret_cast<const double2*>(src)[f];
-            } else {
-                for (int f = lane; f < nD; f += 32) dst[f] = src[f];
+        if constexpr (FORM == OBS_F64) {
+            if (kv) {
+                double* row = w_stage + (size_t)(oct * n + k) * D;
+                row[0] = x; row[1] = v;
+                for (int q = 0; q < n; q++) { row[2 + q] = __dsub_rn(o_pos[q], x); row[2 + n + q] = o_vel[q]; }
+                row[2 + 2 * n] = o_pos[0] > 0 ? 1.0 : 0.0;
+                row[3 + 2 * n] = x > 0 ? 1.0 : 0.0;
+                row[4 + 2 * n] = 0.0;
+            }
+            __syncwarp();
+            const uint32_t lv = __ballot_sync(CAR_FULL, live);
+            for (int q = 0; q < 4; q++) {
+                if (!((lv >> (8 * q)) & 1u)) continue;                    // (uniform)
+                const int e = (grp * CAR_WARPS + warp) * 4 + q;
+                double* dst = static_cast<double*>(io.obs) + (size_t)e * nD;
+                const double* src = w_stage + (size_t)q * nD;
+                if ((nD & 1) == 0) {                                       // 16-byte aligned runs
+                    for (int f = lane; 2 * f < nD; f += 32) reinterpret_cast<double2*>(dst)[f] = reinterpret_cast<const double2*>(src)[f];
+                } else {
+                    for (int f = lane; f < nD; f += 32) dst[f] = src[f];
+                }
+            }
+        } else {
+            // the same values as T, and theta (lane 0's of the octet: after a reset the new one) and 0 after them
+            typedef typename PolicyElem<FORM>::T T;
+            const bool con = p.contract != SSD_CONTRACT_NONE;
+            const int W = D + (con ? 2 : 0), L = n * W * (int)sizeof(T);
+            const double th = __shfl_sync(CAR_FULL, row_theta, obase);
+            if (kv) {
+                T* row = reinterpret_cast<T*>(w_stage) + (size_t)(oct * n + k) * W;
+                auto put = [&](int i, double val) { row[i] = policy_cast<T>(__double2float_rn(val)); };
+                put(0, x); put(1, v);
+                for (int q = 0; q < n; q++) { put(2 + q, __dsub_rn(o_pos[q], x)); put(2 + n + q, o_vel[q]); }
+                put(2 + 2 * n, o_pos[0] > 0 ? 1.0 : 0.0);
+                put(3 + 2 * n, x > 0 ? 1.0 : 0.0);
+                put(4 + 2 * n, 0.0);
+                if (con) { put(D, th); put(D + 1, 0.0); }
+            }
+            __syncwarp();
+            const uint32_t lv = __ballot_sync(CAR_FULL, live);
+            for (int q = 0; q < 4; q++) {
+                if (!((lv >> (8 * q)) & 1u)) continue;                    // (uniform)
+                const int e = (grp * CAR_WARPS + warp) * 4 + q;
+                car_copy_run(static_cast<uint8_t*>(io.obs) + (size_t)e * L, reinterpret_cast<const uint8_t*>(w_stage) + (size_t)q * L, L, lane);
             }
         }
     }
@@ -453,8 +494,11 @@ __global__ void car_get_state_kernel(const CarParams p, double* pos, double* vel
     if (m_transfers) m_transfers[env] = p.m_transfers[env];
     if (t) t[env] = p.t[env];
 }
-__global__ void car_set_theta_kernel(const CarParams p, const double* theta)
+// flat: the policy's rows when they have a theta column (ssd_set_flat_policy_output), kept current
+__global__ void car_set_theta_kernel(const CarParams p, const double* theta, const FlatPolicy flat)
 {
     const int env = blockIdx.x * blockDim.x + threadIdx.x;
-    if (env < p.E) p.theta[env] = theta[env];
+    if (env >= p.E) return;
+    p.theta[env] = theta[env];
+    flat_policy_theta(flat, p.n, env, theta[env]);
 }

@@ -163,6 +163,7 @@ struct SolverParams {
     const uint8_t* episode; long long episode_stride; uint32_t episode_mask;
     uint8_t* theta; long long theta_stride;
     void* pol_contract; int pol_dtype;       // gridworld with a policy output (ssd_set_policy_output): its contract rows, else NULL
+    FlatPolicy flat;                         // feature env / selfdrive with flat policy rows that carry theta, else rows NULL
 };
 #define SOLVER_RULE_MAX 0
 #define SOLVER_RULE_MAJORITY 1
@@ -217,6 +218,7 @@ __global__ void solver_choose_kernel(const SolverParams p, int S, int rule, cons
     if (best_idx) best_idx[env] = src;
     *reinterpret_cast<double*>(p.theta + (size_t)env * p.theta_stride) = theta;
     if (p.pol_contract) policy_contract_env(p.pol_contract, p.pol_dtype, n, env, theta);
+    flat_policy_theta(p.flat, n, env, theta);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -2,7 +2,7 @@
 
 Reference: environments/cleanup_features.py:48-336, environments/harvest_features.py:60-364,
 contract/contract_list.py:7-54, environments/two_stage_train.py:62-121,159-187.  Eight lanes per env, one launch per
-step; observations are float64 feature vectors [E, n, F].
+step; observations are float64 feature vectors [E, n, F], or the policy's flat rows (flat_policy.py).
 """
 import ctypes
 
@@ -13,6 +13,7 @@ from . import _lib
 from .batched import HostResultMixin
 from .checkpoint import CheckpointMixin
 from .episodes import EpisodeLogMixin
+from .flat_policy import FlatPolicyMixin
 from .maps import CLEANUP_MAP, HARVEST_MAP
 
 _DEFAULT_HIGH = {"CleanupContract": 0.2, "HarvestFeaturemodLocalContract": 10.0}
@@ -22,11 +23,16 @@ def _ptr(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
 
-class BatchedFeatureEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
-    """kind: 'cleanup' | 'harvest' (the reference's `environment` strings for the feature envs)."""
+class BatchedFeatureEnv(HostResultMixin, FlatPolicyMixin, CheckpointMixin, EpisodeLogMixin):
+    """kind: 'cleanup' | 'harvest' (the reference's `environment` strings for the feature envs).
+
+    policy_dtype: None (float64 `obs` [E, n, F]), or torch.float32 / float16 / bfloat16: the env writes the policy's flat
+    rows `policy_obs` T [E*n, policy_width] instead (features ++ [theta, 0] with a contract, policy_width = F + 2; the
+    features alone without one) and `obs` is None; reset / step / step_host_async return `policy_obs` in its place.  The
+    mode is fixed for the env's lifetime.  (`W` is the map width.)"""
 
     def __init__(self, kind, num_envs, num_agents, ascii_map=None, horizon=1000, contract=None, theta_low=0.0,
-                 theta_high=None, null_prob=0.0, seed=73907, first_env_id=0, device=None):
+                 theta_high=None, null_prob=0.0, seed=73907, first_env_id=0, device=None, policy_dtype=None):
         if kind not in ("cleanup", "harvest"):
             raise ValueError("BatchedFeatureEnv kind must be cleanup or harvest, got %r" % (kind,))
         if not torch.cuda.is_available():
@@ -53,7 +59,7 @@ class BatchedFeatureEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
         self.F = self.lib.ssd_feature_dim(self._h)
         E, n, dev = self.E, self.n, self.device
         f64 = torch.float64
-        self.obs = torch.zeros((E, n, self.F), dtype=f64, device=dev)
+        self.obs = None if self._init_policy_output(policy_dtype, self.F) else torch.zeros((E, n, self.F), dtype=f64, device=dev)
         self.rew = torch.zeros((E, n), dtype=f64, device=dev)
         self.base_rew = torch.zeros((E, n), dtype=f64, device=dev)
         self.transfers = torch.zeros((E, n), dtype=f64, device=dev)
@@ -79,30 +85,30 @@ class BatchedFeatureEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
         if mask is not None:
             mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
         _lib.check(self._h, self.lib.ssd_feat_reset(self._h, _ptr(mask), _ptr(self.obs), self._stream()))
-        return self.obs
+        return self.observation
 
     def step(self, actions, extras=True, auto_reset=False):
-        """actions: uint8 CUDA tensor [E, n].  Returns (obs [E, n, F], rew, done [E], info [E, n, 4])."""
+        """actions: uint8 CUDA tensor [E, n].  Returns (obs [E, n, F] or policy_obs, rew, done [E], info [E, n, 4])."""
         if actions.dtype != torch.uint8 or actions.device != self.device or not actions.is_contiguous():
             actions = actions.to(device=self.device, dtype=torch.uint8).contiguous()
         io = self._io
-        io.actions_dev, io.obs_dev, io.rew_dev = actions.data_ptr(), self.obs.data_ptr(), self.rew.data_ptr()
+        io.actions_dev, io.obs_dev, io.rew_dev = actions.data_ptr(), _ptr(self.obs), self.rew.data_ptr()
         io.base_rew_dev = self.base_rew.data_ptr() if extras else None
         io.transfers_dev = self.transfers.data_ptr() if extras else None
         io.info_dev = self.info.data_ptr()
         io.done_dev = self.done.data_ptr()
         io.auto_reset = 1 if auto_reset else 0       # next-step auto-reset: finished envs restart in the following step
         _lib.check(self._h, self.lib.ssd_feat_step(self._h, ctypes.byref(io), self._stream()))
-        return self.obs, self.rew, self.done, self.info
+        return self.observation, self.rew, self.done, self.info
 
     def step_host_async(self, actions_host, result, dense_rewards=False, auto_reset=False):
         """Submit one step with HOST actions (pinned uint8 [E, n]); returns a ticket without synchronising.  The compact
         result block (int8 rewards + exact float64 records + dones) lands in `result` (a HostResult from new_host_result());
-        `step_host_wait(ticket)` makes it valid.  At most two steps in flight; observations stay in self.obs."""
+        `step_host_wait(ticket)` makes it valid.  At most two steps in flight; observations stay in self.obs (policy_obs)."""
         if actions_host.device.type != "cpu" or actions_host.dtype != torch.uint8 or not actions_host.is_contiguous():
             raise ValueError("step_host_async needs a contiguous CPU uint8 tensor [E, n] (pinned for an asynchronous copy)")
         io = self._io
-        io.actions_dev, io.obs_dev = None, self.obs.data_ptr()
+        io.actions_dev, io.obs_dev = None, _ptr(self.obs)
         io.rew_dev = self.rew.data_ptr() if dense_rewards else None
         io.base_rew_dev = io.transfers_dev = None
         io.info_dev = self.info.data_ptr()

@@ -1,7 +1,8 @@
 """Batched device-resident SelfAcceleratingCarEnv (+ fused SelfdriveContractDistprop subgame wrapper).
 
 Reference: environments/self_driving_car_accelerate.py:18-250, contract/contract_list.py:56-102,
-environments/two_stage_train.py:62-121,159-187.  One kernel launch steps E envs; all values are float64.
+environments/two_stage_train.py:62-121,159-187.  One kernel launch steps E envs; all values are float64 (observations:
+or the policy's flat rows, flat_policy.py).
 """
 import ctypes
 
@@ -12,18 +13,23 @@ from . import _lib
 from .batched import HostResultMixin
 from .checkpoint import CheckpointMixin
 from .episodes import EpisodeLogMixin
+from .flat_policy import FlatPolicyMixin
 
 
 def _ptr(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
 
-class BatchedCarEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
+class BatchedCarEnv(HostResultMixin, FlatPolicyMixin, CheckpointMixin, EpisodeLogMixin):
+    """policy_dtype: None (float64 `obs` [E, n, D]), or torch.float32 / float16 / bfloat16: the env writes the policy's
+    flat rows `policy_obs` T [E*n, policy_width] instead (each car's D values ++ [theta, 0] with a contract,
+    policy_width = D + 2; the D values alone without one) and `obs` is None; reset / step / step_host_async return
+    `policy_obs` in its place.  The mode is fixed for the env's lifetime."""
     kind = "selfdrive"
 
     def __init__(self, num_envs, num_agents, contract=None, low_bound=-10.0, high_bound=10.0, start_vel=0.2,
                  start_vel_ambulance=0.8, theta_low=0.0, theta_high=100.0, null_prob=0.0, seed=73907, first_env_id=0,
-                 device=None):
+                 device=None, policy_dtype=None):
         if contract not in (None, "SelfdriveContractDistprop"):
             raise ValueError("selfdrive supports contract None or 'SelfdriveContractDistprop', got %r" % (contract,))
         if not torch.cuda.is_available():
@@ -46,7 +52,7 @@ class BatchedCarEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
         self.D = self.lib.ssd_feature_dim(self._h)
         E, n, dev = self.E, self.n, self.device
         f64 = torch.float64
-        self.obs = torch.zeros((E, n, self.D), dtype=f64, device=dev)
+        self.obs = None if self._init_policy_output(policy_dtype, self.D) else torch.zeros((E, n, self.D), dtype=f64, device=dev)
         self.rew = torch.zeros((E, n), dtype=f64, device=dev)
         self.base_rew = torch.zeros((E, n), dtype=f64, device=dev)
         self.transfers = torch.zeros((E, n), dtype=f64, device=dev)
@@ -72,21 +78,21 @@ class BatchedCarEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
         if mask is not None:
             mask = mask.to(device=self.device, dtype=torch.uint8).contiguous()
         _lib.check(self._h, self.lib.ssd_selfdrive_reset(self._h, _ptr(mask), _ptr(self.obs), self._stream()))
-        return self.obs
+        return self.observation
 
     def step(self, actions, extras=True, auto_reset=False):
-        """actions: float32 CUDA tensor [E, n].  Returns (obs, rew, done [E, n+1], info [E, n, 4])."""
+        """actions: float32 CUDA tensor [E, n].  Returns (obs or policy_obs, rew, done [E, n+1], info [E, n, 4])."""
         if actions.dtype != torch.float32 or actions.device != self.device or not actions.is_contiguous():
             actions = actions.to(device=self.device, dtype=torch.float32).contiguous()
         io = self._io
-        io.actions_dev, io.obs_dev, io.rew_dev = actions.data_ptr(), self.obs.data_ptr(), self.rew.data_ptr()
+        io.actions_dev, io.obs_dev, io.rew_dev = actions.data_ptr(), _ptr(self.obs), self.rew.data_ptr()
         io.base_rew_dev = self.base_rew.data_ptr() if extras else None
         io.transfers_dev = self.transfers.data_ptr() if extras else None
         io.info_dev = self.info.data_ptr() if extras else None
         io.done_dev = self.done.data_ptr()
         io.auto_reset = 1 if auto_reset else 0       # next-step auto-reset: finished envs restart in the following step
         _lib.check(self._h, self.lib.ssd_selfdrive_step(self._h, ctypes.byref(io), self._stream()))
-        return self.obs, self.rew, self.done, self.info
+        return self.observation, self.rew, self.done, self.info
 
     @property
     def host_done_shape(self):
@@ -99,7 +105,7 @@ class BatchedCarEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
         if actions_host.device.type != "cpu" or actions_host.dtype != torch.float32 or not actions_host.is_contiguous():
             raise ValueError("step_host_async needs a contiguous CPU float32 tensor [E, n] (pinned for an asynchronous copy)")
         io = self._io
-        io.actions_dev, io.obs_dev = None, self.obs.data_ptr()
+        io.actions_dev, io.obs_dev = None, _ptr(self.obs)
         io.rew_dev = self.rew.data_ptr() if dense_rewards else None
         io.base_rew_dev = io.transfers_dev = io.info_dev = None
         io.done_dev = self.done.data_ptr()

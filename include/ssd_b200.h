@@ -250,6 +250,30 @@ typedef struct ssd_policy_out {
  * image_dev, a contract_dev not aligned to its element, or a feature-env or selfdrive handle.  The caller keeps both
  * tensors alive while they are set. */
 int ssd_set_policy_output(ssd_handle* h, const ssd_policy_out* out);
+/* The flat rows a policy on the feature envs and selfdrive consumes (SeparateContractEnv, two_stage_train.py:113-121),
+ * written by the environment itself.  Row e*n + a of obs_dev T [E*n][W] is agent a of env e:
+ *   - with a contract (contract_kind != SSD_CONTRACT_NONE): W = F + 2, the row is features ++ [theta, 0] (theta: the env's
+ *     contract parameter; the last column is the subgame stage, 0 on the device);
+ *   - without a contract: W = F, the features alone.
+ * F = ssd_feature_dim(h): 12 + n (cleanup features), 10 + 2n (harvest features), 2n + 5 (selfdrive).  Each element is
+ * T(float32(x)), x the float64 the step writes without this mode (or theta): float64 -> float32 -> T, round to nearest
+ * even.  Rows are W * sizeof(T) bytes and may start on any multiple of 2 bytes. */
+typedef struct ssd_flat_policy_out {
+    int32_t struct_size;    /* sizeof(ssd_flat_policy_out) (a smaller value is rejected) */
+    int32_t dtype;          /* SSD_POLICY_F32 / _F16 / _BF16 */
+    void*   obs_dev;        /* T [E*n][W], 16-byte aligned */
+} ssd_flat_policy_out;
+/* Feature-env and selfdrive kinds.  While set (sticky; NULL switches it off), the handle has one observation form, the
+ * policy's:
+ *   - every call that writes float64 rows — ssd_feat_step / ssd_selfdrive_step, their _host_async forms, ssd_feat_reset /
+ *     ssd_selfdrive_reset (masked or not) and the auto_reset behind a step — writes the flat rows of the same envs
+ *     instead (selfdrive: the rows of cars that did not act too).  obs_dev must be NULL in these calls (else SSD_EINVAL);
+ *   - every call that changes theta leaves the theta column of the envs it changes current: ssd_set_contract_params,
+ *     ssd_negotiate, ssd_solver_choose and ssd_checkpoint_load.
+ * Validates before storing anything: SSD_EINVAL for a struct_size too small, an unknown dtype, a NULL or not 16-byte
+ * aligned obs_dev, or a gridworld handle (those have ssd_set_policy_output).  The caller keeps the tensor alive while it
+ * is set. */
+int ssd_set_flat_policy_output(ssd_handle* h, const ssd_flat_policy_out* out);
 
 /* --- NegotiationSolver (environments/two_stage_train.py:619-776); every env kind ------------------- */
 #define SSD_SOLVER_RULE_MAX 0        /* decision_rule 'max'      (:751-757) */
