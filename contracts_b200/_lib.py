@@ -7,6 +7,8 @@ point raises.  The library is built in-tree by `contracts_b200.build.build()` /
 import ctypes
 import os
 
+import torch
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 # SSD_LIB_PATH: development only (A/B runs of differently built libraries); the shipped library is the in-tree one
 LIB_PATH = os.environ.get("SSD_LIB_PATH") or os.path.join(_HERE, "libssd_b200.so")
@@ -65,6 +67,16 @@ class ssd_policy_out(ctypes.Structure):
 
 class ssd_flat_policy_out(ctypes.Structure):
     _fields_ = [("struct_size", ctypes.c_int32), ("dtype", ctypes.c_int32), ("obs_dev", ctypes.c_void_p)]
+
+
+POLICY_DTYPE = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}     # SSD_POLICY_F32 / _F16 / _BF16
+
+
+def policy_dtype_code(dtype):
+    """the SSD_POLICY_* code of a policy tensor's torch dtype"""
+    if dtype not in POLICY_DTYPE:
+        raise ValueError("policy_dtype must be None, torch.float32, torch.float16 or torch.bfloat16, got %r" % (dtype,))
+    return POLICY_DTYPE[dtype]
 
 
 

@@ -179,13 +179,15 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
         E, n, dev = self.E, self.n, self.device
         self.policy_dtype, self.policy_image, self.policy_contract = policy_dtype, None, None
         if policy_dtype is not None:
-            if policy_dtype not in self._POLICY_DTYPES:
+            try:
+                code = _lib.policy_dtype_code(policy_dtype)
+            except ValueError:
                 self.close()
-                raise ValueError("policy_dtype must be None, torch.float32, torch.float16 or torch.bfloat16, got %r" % (policy_dtype,))
+                raise
             self.policy_image = torch.zeros((E * n, 3, 15, 15), dtype=policy_dtype, device=dev)
             if contract is not None:
                 self.policy_contract = torch.zeros((E * n, 10), dtype=policy_dtype, device=dev)
-            out = _lib.ssd_policy_out(struct_size=ctypes.sizeof(_lib.ssd_policy_out), dtype=self._POLICY_DTYPES[policy_dtype],
+            out = _lib.ssd_policy_out(struct_size=ctypes.sizeof(_lib.ssd_policy_out), dtype=code,
                                       image_dev=self.policy_image.data_ptr(),
                                       contract_dev=None if self.policy_contract is None else self.policy_contract.data_ptr())
             _lib.check(self._h, self.lib.ssd_set_policy_output(self._h, ctypes.byref(out)))
@@ -429,8 +431,6 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
         return out
 
     # ---- policy-side consumer (environments/Networks/vision_net.py:150-181) -----------------------------
-    _POLICY_DTYPES = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}
-
     def policy_inputs(self, dtype=torch.float32, with_contract=True, image=None, contract=None):
         """The current observations as VisionNetwork.forward feeds its convolutions: image [E*n, 3, 15, 15] =
         (`curr_obs / 255`).float().permute(0, 3, 1, 2), contract [E*n, 10] = (theta, 0) repeated 5 times.
@@ -441,7 +441,7 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
             image = torch.empty((B, 3, 15, 15), dtype=dtype, device=self.device)
         if with_contract and contract is None:
             contract = torch.empty((B, 10), dtype=dtype, device=self.device)
-        _lib.check(self._h, self.lib.ssd_policy_inputs(self._h, _ptr(self._obs_buf), self.obs_stride, self._POLICY_DTYPES[dtype],
+        _lib.check(self._h, self.lib.ssd_policy_inputs(self._h, _ptr(self._obs_buf), self.obs_stride, _lib.policy_dtype_code(dtype),
                                                        _ptr(image), _ptr(contract) if with_contract else None, self._stream()))
         return (image, contract) if with_contract else image
 

@@ -13,6 +13,7 @@
 
 #include <algorithm>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/ssd_b200.h"
@@ -63,83 +64,71 @@ struct ssd_handle {
     int64_t launches;
     CkParams ck;             // ssd_checkpoint_*: where each part of an env's row lives (ssd_checkpoint.cuh)
     uint64_t config_tag;     // ssd_checkpoint_get_layout: hash of everything that gives a row its meaning
-    int pol_form;            // ssd_set_policy_output: OBS_U8 (none) or 1 + SSD_POLICY_*, the form the observe / reset kernels write
-    uint8_t* pol_image;      //   T [E n][3][15][15]
-    void* pol_contract;      //   T [E n][10] or NULL
-    int flat_form;           // ssd_set_flat_policy_output: OBS_F64 (none) or 1 + SSD_POLICY_*, the form the feature / selfdrive kernels write
-    FlatPolicy flat;         //   T [E n][W] (rows NULL: none)
+    // ssd_set_policy_output / ssd_set_flat_policy_output: the one observation form the handle's kernels write
+    int form;                // 0: the native form (OBS_U8 / OBS_F64); else 1 + SSD_POLICY_*
+    void* pol_rows;          //   the policy image T [E n][3][15][15] (grid worlds) or the flat rows T [E n][W]
+    ThetaRows theta_rows;    //   the rows that carry theta: a grid world's contract rows, flat rows under a contract
     char err[512];
     std::vector<void*> dev_allocs;
 };
 
+// f(std::integral_constant<int, FORM>()) for a runtime observation form: 0, the native form (OBS_U8 / OBS_F64), or
+// 1 + SSD_POLICY_*
+template <typename F>
+static auto by_form(int form, F f)
+{
+    if (form == 1 + SSD_POLICY_F32) return f(std::integral_constant<int, 1 + SSD_POLICY_F32>());
+    if (form == 1 + SSD_POLICY_F16) return f(std::integral_constant<int, 1 + SSD_POLICY_F16>());
+    if (form == 1 + SSD_POLICY_BF16) return f(std::integral_constant<int, 1 + SSD_POLICY_BF16>());
+    return f(std::integral_constant<int, 0>());
+}
 typedef void (*obs_kernel_t)(const GridParams, const StepIO, uint32_t*);
-template <int KIND, int FORM>
-static obs_kernel_t obs_pick(bool rounds4, bool feat)
-{
-    if (rounds4) return feat ? grid_obs_kernel<KIND, 4, true, 0, FORM> : grid_obs_kernel<KIND, 4, false, 0, FORM>;
-    return feat ? grid_obs_kernel<KIND, MAX_POINT_ROUNDS, true, 0, FORM> : grid_obs_kernel<KIND, MAX_POINT_ROUNDS, false, 0, FORM>;
-}
-template <int FORM>
-static obs_kernel_t obs_form_fn(int kind, bool rounds4, bool feat, int lay)
-{
-    if (lay == 1 && kind == SSD_ENV_CLEANUP && rounds4 && !feat) return grid_obs_kernel<SSD_ENV_CLEANUP, 4, false, 1, FORM>;
-    if (lay == 2 && kind == SSD_ENV_HARVEST && !rounds4 && !feat) return grid_obs_kernel<SSD_ENV_HARVEST, MAX_POINT_ROUNDS, false, 2, FORM>;
-    return kind == SSD_ENV_CLEANUP ? obs_pick<SSD_ENV_CLEANUP, FORM>(rounds4, feat) : obs_pick<SSD_ENV_HARVEST, FORM>(rounds4, feat);
-}
 // lay: 0, or 1 when the handle matches OBS_LAY_CLEANUP8 (stock cleanup map, 8 agents, dense observation tensor, no feature_obs);
 // form: OBS_U8 or the policy form of ssd_set_policy_output (1 + SSD_POLICY_*)
 static obs_kernel_t obs_kernel_fn(int kind, bool rounds4, bool feat, int lay = 0, int form = OBS_U8)
 {
-    if (form == 1 + POLICY_F32) return obs_form_fn<1 + POLICY_F32>(kind, rounds4, feat, lay);
-    if (form == 1 + POLICY_F16) return obs_form_fn<1 + POLICY_F16>(kind, rounds4, feat, lay);
-    if (form == 1 + POLICY_BF16) return obs_form_fn<1 + POLICY_BF16>(kind, rounds4, feat, lay);
-    return obs_form_fn<OBS_U8>(kind, rounds4, feat, lay);
+    return by_form(form, [&](auto F) -> obs_kernel_t {
+        constexpr int FORM = decltype(F)::value;
+        if (lay == 1 && kind == SSD_ENV_CLEANUP && rounds4 && !feat) return grid_obs_kernel<SSD_ENV_CLEANUP, 4, false, 1, FORM>;
+        if (lay == 2 && kind == SSD_ENV_HARVEST && !rounds4 && !feat) return grid_obs_kernel<SSD_ENV_HARVEST, MAX_POINT_ROUNDS, false, 2, FORM>;
+        if (kind == SSD_ENV_CLEANUP) {
+            if (rounds4) return feat ? grid_obs_kernel<SSD_ENV_CLEANUP, 4, true, 0, FORM> : grid_obs_kernel<SSD_ENV_CLEANUP, 4, false, 0, FORM>;
+            return feat ? grid_obs_kernel<SSD_ENV_CLEANUP, MAX_POINT_ROUNDS, true, 0, FORM> : grid_obs_kernel<SSD_ENV_CLEANUP, MAX_POINT_ROUNDS, false, 0, FORM>;
+        }
+        if (rounds4) return feat ? grid_obs_kernel<SSD_ENV_HARVEST, 4, true, 0, FORM> : grid_obs_kernel<SSD_ENV_HARVEST, 4, false, 0, FORM>;
+        return feat ? grid_obs_kernel<SSD_ENV_HARVEST, MAX_POINT_ROUNDS, true, 0, FORM> : grid_obs_kernel<SSD_ENV_HARVEST, MAX_POINT_ROUNDS, false, 0, FORM>;
+    });
 }
 typedef void (*reset_kernel_t)(const GridParams, const uint8_t*, uint8_t*, long long, const StepIO, void*);
-template <int KIND>
-static reset_kernel_t reset_pick(int form)
-{
-    if (form == 1 + POLICY_F32) return grid_reset_kernel<KIND, 1 + POLICY_F32>;
-    if (form == 1 + POLICY_F16) return grid_reset_kernel<KIND, 1 + POLICY_F16>;
-    if (form == 1 + POLICY_BF16) return grid_reset_kernel<KIND, 1 + POLICY_BF16>;
-    return grid_reset_kernel<KIND, OBS_U8>;
-}
 static reset_kernel_t reset_kernel_fn(int kind, int form)
 {
-    return kind == SSD_ENV_CLEANUP ? reset_pick<SSD_ENV_CLEANUP>(form) : reset_pick<SSD_ENV_HARVEST>(form);
+    return by_form(form, [&](auto F) -> reset_kernel_t {
+        constexpr int FORM = decltype(F)::value;
+        return kind == SSD_ENV_CLEANUP ? grid_reset_kernel<SSD_ENV_CLEANUP, FORM> : grid_reset_kernel<SSD_ENV_HARVEST, FORM>;
+    });
 }
 typedef void (*feat_kernel_t)(const FeatParams, const FeatIO, const uint8_t*);
-template <bool CLEANUP, bool RESET_ONLY>
-static feat_kernel_t feat_pick(int form)
-{
-    if (form == 1 + POLICY_F32) return feat_kernel<CLEANUP, RESET_ONLY, 1 + POLICY_F32>;
-    if (form == 1 + POLICY_F16) return feat_kernel<CLEANUP, RESET_ONLY, 1 + POLICY_F16>;
-    if (form == 1 + POLICY_BF16) return feat_kernel<CLEANUP, RESET_ONLY, 1 + POLICY_BF16>;
-    return feat_kernel<CLEANUP, RESET_ONLY, OBS_F64>;
-}
 // form: OBS_F64 or the flat policy form of ssd_set_flat_policy_output (1 + SSD_POLICY_*)
 static feat_kernel_t feat_kernel_fn(bool cleanup, bool reset_only, int form)
 {
-    if (cleanup) return reset_only ? feat_pick<true, true>(form) : feat_pick<true, false>(form);
-    return reset_only ? feat_pick<false, true>(form) : feat_pick<false, false>(form);
+    return by_form(form, [&](auto F) -> feat_kernel_t {
+        constexpr int FORM = decltype(F)::value;
+        if (cleanup) return reset_only ? feat_kernel<true, true, FORM> : feat_kernel<true, false, FORM>;
+        return reset_only ? feat_kernel<false, true, FORM> : feat_kernel<false, false, FORM>;
+    });
 }
 typedef void (*car_kernel_t)(const CarParams, const CarIO, const uint8_t*);
-template <bool RESET_ONLY>
-static car_kernel_t car_pick(int form)
-{
-    if (form == 1 + POLICY_F32) return car_kernel<RESET_ONLY, 1 + POLICY_F32>;
-    if (form == 1 + POLICY_F16) return car_kernel<RESET_ONLY, 1 + POLICY_F16>;
-    if (form == 1 + POLICY_BF16) return car_kernel<RESET_ONLY, 1 + POLICY_BF16>;
-    return car_kernel<RESET_ONLY, OBS_F64>;
-}
 static car_kernel_t car_kernel_fn(bool reset_only, int form)
 {
-    return reset_only ? car_pick<true>(form) : car_pick<false>(form);
+    return by_form(form, [&](auto F) -> car_kernel_t {
+        constexpr int FORM = decltype(F)::value;
+        return reset_only ? car_kernel<true, FORM> : car_kernel<false, FORM>;
+    });
 }
 // bytes of one env's block of the policy image tensor
 static long long policy_env_bytes(const GridParams& p, int form)
 {
-    return (long long)p.n * SSD_OBS_BYTES * (form == 1 + POLICY_F32 ? 4 : 2);
+    return (long long)p.n * SSD_OBS_BYTES * (form == 1 + SSD_POLICY_F32 ? 4 : 2);
 }
 typedef void (*logic_kernel_t)(const GridParams, const StepIO, uint32_t*);
 static logic_kernel_t logic_kernel_fn(int kind, int lay)
@@ -271,6 +260,30 @@ static int dev_zalloc(ssd_handle* h, size_t count, T** out)
     h->dev_allocs.push_back(d);
     CUDA_TRY(h, cudaMemset(d, 0, (count ? count : 1) * sizeof(T)));
     *out = reinterpret_cast<T*>(d);
+    return SSD_OK;
+}
+
+// the dynamic shared-memory limit of every kernel of the handle's step and reset in observation form `form` (0 at create,
+// the policy form when an output is set)
+static int set_form_smem(ssd_handle* h, int form)
+{
+    const int kind = h->cfg.env_kind;
+    if (kind == SSD_ENV_SELFDRIVE) {
+        for (int q = 0; q < 2; q++)
+            CUDA_TRY(h, cudaFuncSetAttribute((const void*)car_kernel_fn(q != 0, form), cudaFuncAttributeMaxDynamicSharedMemorySize, h->car_smem));
+    } else if (kind == SSD_ENV_CLEANUP_FEATURES || kind == SSD_ENV_HARVEST_FEATURES) {
+        for (int q = 0; q < 2; q++)
+            CUDA_TRY(h, cudaFuncSetAttribute((const void*)feat_kernel_fn(kind == SSD_ENV_CLEANUP_FEATURES, q != 0, form),
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, h->feat_smem));
+    } else {
+        const int smem = h->gp.g2_smem_bytes;
+        CUDA_TRY(h, cudaFuncSetAttribute((const void*)reset_kernel_fn(kind, form), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        for (int feat = 0; feat < 2; feat++)
+            CUDA_TRY(h, cudaFuncSetAttribute((const void*)obs_kernel_fn(kind, h->rounds4, feat != 0, 0, form),
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        if (h->obs_lay) CUDA_TRY(h, cudaFuncSetAttribute((const void*)obs_kernel_fn(kind, h->rounds4, false, h->obs_lay, form),
+                                                         cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    }
     return SSD_OK;
 }
 
@@ -434,21 +447,16 @@ static int setup_grid(ssd_handle* h)
 
     int sms = 0, per_sm = 0;
     CUDA_TRY(h, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c.device));
-    const void* reset_k = (const void*)reset_kernel_fn(c.env_kind, OBS_U8);
-    CUDA_TRY(h, cudaFuncSetAttribute(reset_k, cudaFuncAttributeMaxDynamicSharedMemorySize, p.g2_smem_bytes));
-    CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, reset_k, GRID_THREADS, p.g2_smem_bytes));
+    h->obs_lay = obs_layout_id(p);
+    if ((rc = set_form_smem(h, 0))) return rc;
+    CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)reset_kernel_fn(c.env_kind, OBS_U8), GRID_THREADS,
+                                                              p.g2_smem_bytes));
     if (per_sm < 1) return fail(h, SSD_EUNSUPPORTED, "reset kernel does not fit on an SM (smem %d B)", p.g2_smem_bytes);
     int want = (p.E + GRID_WARPS - 1) / GRID_WARPS;
     h->grid_blocks = want < sms * per_sm ? want : sms * per_sm;
 
     // observe kernel: persistent grid at the achievable occupancy; logic kernel: cell table + per-warp mask copies
     int per_sm2 = 0;
-    h->obs_lay = obs_layout_id(p);
-    for (int feat = 0; feat < 2; feat++)
-        CUDA_TRY(h, cudaFuncSetAttribute((const void*)obs_kernel_fn(c.env_kind, h->rounds4, feat != 0),
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, p.g2_smem_bytes));
-    if (h->obs_lay) CUDA_TRY(h, cudaFuncSetAttribute((const void*)obs_kernel_fn(c.env_kind, h->rounds4, false, h->obs_lay),
-                                                     cudaFuncAttributeMaxDynamicSharedMemorySize, p.g2_smem_bytes));
     CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm2, (const void*)obs_kernel_fn(c.env_kind, h->rounds4, false),
                                                               OBS_WARPS * 32, p.g2_smem_bytes));
     if (per_sm2 < 1) return fail(h, SSD_EUNSUPPORTED, "observe kernel does not fit on an SM (smem %d B)", p.g2_smem_bytes);
@@ -512,8 +520,7 @@ static int setup_selfdrive(ssd_handle* h)
     if ((rc = dev_zalloc(h, E, &p.episode))) return rc;
     p.warp_doubles = (4 * p.n * p.D + 1) / 2 * 2 + 4 * CAR_OCT_DOUBLES;
     h->car_smem = CAR_WARPS * p.warp_doubles * (int)sizeof(double);
-    CUDA_TRY(h, cudaFuncSetAttribute((const void*)car_kernel_fn(false, OBS_F64), cudaFuncAttributeMaxDynamicSharedMemorySize, h->car_smem));
-    CUDA_TRY(h, cudaFuncSetAttribute((const void*)car_kernel_fn(true, OBS_F64), cudaFuncAttributeMaxDynamicSharedMemorySize, h->car_smem));
+    if ((rc = set_form_smem(h, 0))) return rc;
     {   // persistent CTAs: as many as are resident at once
         int dev = 0, sms = 0, per_sm = 0;
         CUDA_TRY(h, cudaGetDevice(&dev));
@@ -639,8 +646,7 @@ static int setup_features(ssd_handle* h)
     if ((rc = dev_zalloc(h, E * n, &p.tsum_tr))) return rc;
     h->feat_smem = p.sm_static + FEAT_ENVS_PER_CTA * p.oct_bytes;
     if (h->feat_smem > 200 * 1024) return fail(h, SSD_EUNSUPPORTED, "feature envs: %d bytes of shared memory per CTA", h->feat_smem);
-    for (int q = 0; q < 2; q++)
-        CUDA_TRY(h, cudaFuncSetAttribute((const void*)feat_kernel_fn(cleanup, q != 0, OBS_F64), cudaFuncAttributeMaxDynamicSharedMemorySize, h->feat_smem));
+    if ((rc = set_form_smem(h, 0))) return rc;
     // persistent CTAs: as many as are resident at once (a warp takes four envs per round)
     {
         int dev = 0, sms = 0, per_sm = 0;
@@ -798,24 +804,24 @@ __global__ void set_state_kernel(GridParams p, const uint8_t* map, const int32_t
     *reinterpret_cast<uint32_t*>(hdr + RO_FLAGS) = ((f | 0x80000000u) & ~RF_STALE_EMPTY) | (bad << RF_ERR_SHIFT);
 }
 
-// pcontract (nullable): the policy output's contract rows (ssd_set_policy_output), kept current
-__global__ void set_theta_kernel(GridParams p, const double* theta, void* pcontract, int pdtype)
+// every env kind: theta where the solver reads it, then the policy output's rows that carry it
+__global__ void set_theta_kernel(SolverParams p, const double* theta)
 {
-    int env = blockIdx.x * blockDim.x + threadIdx.x;
+    const int env = blockIdx.x * blockDim.x + threadIdx.x;
     if (env >= p.E) return;
-    *reinterpret_cast<double*>(p.state + (size_t)env * p.rec_stride + RO_THETA) = theta[env];
-    if (pcontract) policy_contract_env(pcontract, pdtype, p.n, env, theta[env]);
+    *reinterpret_cast<double*>(p.theta + (size_t)env * p.theta_stride) = theta[env];
+    theta_rows_env(p.rows, p.n, env, theta[env]);
 }
 
-// checkpoint load with a policy output set: the contract rows of the loaded envs from their (new) theta.  Rows that failed
-// validation kept their theta, so rewriting theirs changes nothing.
-__global__ void policy_contract_refresh_kernel(GridParams p, const int32_t* env_idx, int count, void* pcontract, int pdtype)
+// checkpoint load with theta rows set: those of the loaded envs from their (new) theta.  Rows that failed validation kept
+// their theta, so rewriting theirs changes nothing.
+__global__ void theta_rows_refresh_kernel(SolverParams p, const int32_t* env_idx, int count)
 {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= count) return;
     const int env = env_idx ? env_idx[r] : r;
     if (env < 0 || env >= p.E) return;
-    policy_contract_env(pcontract, pdtype, p.n, env, *reinterpret_cast<const double*>(p.state + (size_t)env * p.rec_stride + RO_THETA));
+    theta_rows_env(p.rows, p.n, env, *reinterpret_cast<const double*>(p.theta + (size_t)env * p.theta_stride));
 }
 
 __global__ void get_metrics_kernel(GridParams p, double* out)
@@ -825,17 +831,6 @@ __global__ void get_metrics_kernel(GridParams p, double* out)
     const uint8_t* hdr = p.state + (size_t)env * p.rec_stride;
     double* o = out + (size_t)env * SSD_METRIC_STRIDE;
     for (int q = 0; q < SSD_METRIC_STRIDE; q++) o[q] = grid_metric(p, hdr, q);
-}
-
-// checkpoint load with flat policy rows set (feature envs, selfdrive): their theta column from the loaded envs' theta
-// (addressed like the solver's).  Rows that failed validation kept their theta, so rewriting theirs changes nothing.
-__global__ void flat_theta_refresh_kernel(SolverParams p, const int32_t* env_idx, int count)
-{
-    const int r = blockIdx.x * blockDim.x + threadIdx.x;
-    if (r >= count) return;
-    const int env = env_idx ? env_idx[r] : r;
-    if (env < 0 || env >= p.E) return;
-    flat_policy_theta(p.flat, p.n, env, *reinterpret_cast<const double*>(p.theta + (size_t)env * p.theta_stride));
 }
 
 // SeparateContractNegotiateStage.step, agreement stage (two_stage_train.py:266-281)
@@ -849,8 +844,7 @@ __global__ void negotiate_kernel(SolverParams p, const uint8_t* mask, const doub
     const double theta = dec ? proposals[env] : 0.0;
     *reinterpret_cast<double*>(p.theta + (size_t)env * p.theta_stride) = theta;
     if (decision) decision[env] = dec ? 1 : 0;
-    if (p.pol_contract) policy_contract_env(p.pol_contract, p.pol_dtype, p.n, env, theta);
-    flat_policy_theta(p.flat, p.n, env, theta);
+    theta_rows_env(p.rows, p.n, env, theta);
 }
 
 // step_index == SSD_STEP_AUTO: take the index from the handle's device counter (bumped by the last CTA to finish,
@@ -887,6 +881,29 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
+}
+
+// the checks both policy-output setters make: the struct's size, its dtype and a 16-byte aligned output pointer
+template <typename Out>
+static int check_policy_out(ssd_handle* h, const Out* out, const char* type, const char* what, const void* ptr, const char* ptr_name)
+{
+    if (out->struct_size < (int32_t)sizeof(Out))
+        return fail(h, SSD_EINVAL, "%s.struct_size %d < %d: the caller's declaration of %s is out of date", type, out->struct_size,
+                    (int)sizeof(Out), type);
+    if (out->dtype != SSD_POLICY_F32 && out->dtype != SSD_POLICY_F16 && out->dtype != SSD_POLICY_BF16)
+        return fail(h, SSD_EINVAL, "%s: dtype %d is not SSD_POLICY_F32, _F16 or _BF16", what, out->dtype);
+    if (!ptr || (reinterpret_cast<uintptr_t>(ptr) & 15))
+        return fail(h, SSD_EINVAL, "%s: %s must be a 16-byte aligned device pointer", what, ptr_name);
+    return SSD_OK;
+}
+// the handle's observation form and what it writes; form 0 (the native form) clears the policy output
+static int set_form(ssd_handle* h, int form, void* pol_rows, ThetaRows theta_rows)
+{
+    if (form) { int rc = set_form_smem(h, form); if (rc) return rc; }
+    h->form = form;
+    h->pol_rows = pol_rows;
+    h->theta_rows = theta_rows;
+    return SSD_OK;
 }
 
 // =============================================================================================
@@ -994,20 +1011,13 @@ static int check_launch(ssd_handle* h, const char* what)
 #define REQUIRE_CAR(h) \
     if ((h)->cfg.env_kind != SSD_ENV_SELFDRIVE) return fail(h, SSD_EINVAL, "%s: handle is not a selfdrive env", __func__)
 
-// the flat policy rows as the theta refreshes see them: none without a contract (the rows then have no theta column)
-static FlatPolicy flat_theta_rows(const ssd_handle* h)
-{
-    FlatPolicy f = h->flat;
-    if (h->cfg.contract_kind == SSD_CONTRACT_NONE) f.rows = nullptr;
-    return f;
-}
 // the rows a feature-env / selfdrive step or reset writes: obs_dev, or the flat policy rows while they are set (obs_dev
 // must then be NULL: one observation form per handle)
 static int flat_obs_target(ssd_handle* h, const char* what, void* obs_dev, bool required, void** out)
 {
-    if (h->flat_form) {
+    if (h->form) {
         if (obs_dev) return fail(h, SSD_EINVAL, "%s: obs_dev must be NULL while flat policy rows are set (ssd_set_flat_policy_output)", what);
-        *out = h->flat.rows;
+        *out = h->pol_rows;
     } else {
         if (required && !obs_dev) return fail(h, SSD_EINVAL, "actions_dev, obs_dev and rew_dev are required");
         *out = obs_dev;
@@ -1022,16 +1032,16 @@ int ssd_reset(ssd_handle* h, const uint8_t* mask_dev, uint8_t* obs_dev, int64_t 
     REQUIRE_GRID(h);
     const GridParams& p = h->gp;
     long long stride = obs_env_stride ? obs_env_stride : (long long)p.n * SSD_OBS_BYTES;
-    if (h->pol_form) {                                   // one observation form per handle: the policy output's
+    if (h->form) {                                       // one observation form per handle: the policy output's
         if (obs_dev) return fail(h, SSD_EINVAL, "reset: obs_dev must be NULL while a policy output is set (ssd_set_policy_output)");
-        obs_dev = h->pol_image;
-        stride = policy_env_bytes(p, h->pol_form);
+        obs_dev = (uint8_t*)h->pol_rows;
+        stride = policy_env_bytes(p, h->form);
     }
     if (stride < (long long)p.n * SSD_OBS_BYTES) return fail(h, SSD_EINVAL, "obs_env_stride too small");
     cudaStream_t s = (cudaStream_t)stream;
     if (p.beam) beam_clear_kernel<<<(p.E + 3) / 4, 128, 0, s>>>(p, mask_dev);                 // self.beam_pos = [] (map_env.py:316)
-    reset_kernel_fn(p.kind, h->pol_form)<<<h->grid_blocks, GRID_THREADS, p.g2_smem_bytes, s>>>(p, mask_dev, obs_dev, stride, StepIO(),
-                                                                                                h->pol_contract);
+    reset_kernel_fn(p.kind, h->form)<<<h->grid_blocks, GRID_THREADS, p.g2_smem_bytes, s>>>(p, mask_dev, obs_dev, stride, StepIO(),
+                                                                                            h->theta_rows.rows);
     return check_launch(h, "reset");
 }
 
@@ -1040,10 +1050,10 @@ static int make_step_io(ssd_handle* h, const ssd_step_io* io, StepIO& k, bool as
     memset(&k, 0, sizeof(k));
     if (!async_host && (!io->actions_dev || !io->rew_dev)) return fail(h, SSD_EINVAL, "actions_dev, obs_dev and rew_dev are required");
     const GridParams& p = h->gp;
-    if (h->pol_form) {                                   // one observation form per handle: the policy output's
+    if (h->form) {                                       // one observation form per handle: the policy output's
         if (io->obs_dev) return fail(h, SSD_EINVAL, "obs_dev must be NULL while a policy output is set (ssd_set_policy_output)");
-        k.obs = h->pol_image;
-        k.obs_stride = policy_env_bytes(p, h->pol_form);
+        k.obs = (uint8_t*)h->pol_rows;
+        k.obs_stride = policy_env_bytes(p, h->form);
     } else {
         if (!io->obs_dev) return fail(h, SSD_EINVAL, "obs_dev is required");
         k.obs = io->obs_dev;
@@ -1120,9 +1130,9 @@ static int launch_step(ssd_handle* h, const StepIO& k, cudaStream_t s, const Hos
     if (hc && hc->slot >= 0) CUDA_TRY(h, cudaEventRecord(h->slot[hc->slot].ev_logic, s));   // the slot's actions were read
     if (p.kind == SSD_ENV_CLEANUP) { int rc = copy_rewards(h, k, s, hc); if (rc) return rc; }
     // programmatic dependent launch: the observe CTAs become resident (tables, tiles) as the one-wave logic grid drains
-    const bool dense = h->pol_form || k.obs_stride == (long long)p.n * SSD_OBS_BYTES;       // a policy image is always dense
+    const bool dense = h->form || k.obs_stride == (long long)p.n * SSD_OBS_BYTES;       // a policy image is always dense
     const int lay = (h->obs_lay != 0 && dense && !k.feat) ? h->obs_lay : 0;
-    const obs_kernel_t obs_k = obs_kernel_fn(p.kind, h->rounds4, k.feat != nullptr, lay, h->pol_form);
+    const obs_kernel_t obs_k = obs_kernel_fn(p.kind, h->rounds4, k.feat != nullptr, lay, h->form);
     if (h->pdl && !h->timing) CUDA_TRY(h, launch_pdl(obs_k, dim3(h->obs_blocks), dim3(OBS_WARPS * 32), (size_t)p.g2_smem_bytes, s, p, k, h->d_res));
     else obs_k<<<h->obs_blocks, OBS_WARPS * 32, p.g2_smem_bytes, s>>>(p, k, h->d_res);
     if (p.kind == SSD_ENV_HARVEST) {
@@ -1135,11 +1145,11 @@ static int launch_step(ssd_handle* h, const StepIO& k, cudaStream_t s, const Hos
         h->launches++;
         // (the copy_rewards event record of the host paths sits between the harvest reward kernel and this launch: plain launch then)
         const bool pdl_ok = h->pdl && !h->timing && (p.kind == SSD_ENV_CLEANUP || !hc);
-        const reset_kernel_t reset_k = reset_kernel_fn(p.kind, h->pol_form);
+        const reset_kernel_t reset_k = reset_kernel_fn(p.kind, h->form);
         if (pdl_ok)
             CUDA_TRY(h, launch_pdl(reset_k, dim3(h->grid_blocks), dim3(GRID_THREADS), (size_t)p.g2_smem_bytes, s,
-                                   p, (const uint8_t*)k.done, k.obs, k.obs_stride, k, h->pol_contract));
-        else reset_k<<<h->grid_blocks, GRID_THREADS, p.g2_smem_bytes, s>>>(p, k.done, k.obs, k.obs_stride, k, h->pol_contract);
+                                   p, (const uint8_t*)k.done, k.obs, k.obs_stride, k, h->theta_rows.rows));
+        else reset_k<<<h->grid_blocks, GRID_THREADS, p.g2_smem_bytes, s>>>(p, k.done, k.obs, k.obs_stride, k, h->theta_rows.rows);
     }
     if (h->timing) cudaEventRecord(h->tev[2], s);
     return check_launch(h, "step");
@@ -1375,20 +1385,16 @@ int ssd_set_episode_log(ssd_handle* h, const ssd_episode_log* log)
 #define SMALL_LAUNCH(kernel, ...)                                                         \
     kernel<<<(h->gp.E + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->gp, __VA_ARGS__)
 
+static SolverParams solver_params(ssd_handle* h);
 int ssd_set_contract_params(ssd_handle* h, const double* theta_dev, void* stream)
 {
     if (!h || !theta_dev) return SSD_EINVAL;
     ON_DEVICE(h);
-    if (h->cfg.env_kind == SSD_ENV_SELFDRIVE)
-        car_set_theta_kernel<<<(h->cp.E + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->cp, theta_dev, flat_theta_rows(h));
-    else if (IS_FEAT(h))
-        feat_set_theta_kernel<<<(h->fp.E + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->fp, theta_dev, flat_theta_rows(h));
-    else
-        SMALL_LAUNCH(set_theta_kernel, theta_dev, h->pol_contract, h->pol_form - 1);
+    const SolverParams sp = solver_params(h);
+    set_theta_kernel<<<(sp.E + 127) / 128, 128, 0, (cudaStream_t)stream>>>(sp, theta_dev);
     return check_launch(h, "set_contract_params");
 }
 
-static SolverParams solver_params(ssd_handle* h);
 int ssd_negotiate(ssd_handle* h, const uint8_t* mask_dev, const double* proposals_dev, const double* accept_dev, uint8_t* decision_dev,
                   void* stream)
 {
@@ -1468,9 +1474,9 @@ int ssd_policy_inputs(ssd_handle* h, const uint8_t* obs_dev, int64_t obs_env_str
     const dim3 grid(p.E), block(VIEW_THREADS);
     const size_t smem = (size_t)((dense + 15) / 16 * 16);
     cudaStream_t s = (cudaStream_t)stream;
-    if (dtype == POLICY_F32) policy_inputs_kernel<float><<<grid, block, smem, s>>>(p, obs_dev, obs_env_stride, (float*)image_dev, (float*)contract_dev);
-    else if (dtype == POLICY_F16) policy_inputs_kernel<__half><<<grid, block, smem, s>>>(p, obs_dev, obs_env_stride, (__half*)image_dev, (__half*)contract_dev);
-    else if (dtype == POLICY_BF16) policy_inputs_kernel<__nv_bfloat16><<<grid, block, smem, s>>>(p, obs_dev, obs_env_stride, (__nv_bfloat16*)image_dev, (__nv_bfloat16*)contract_dev);
+    if (dtype == SSD_POLICY_F32) policy_inputs_kernel<float><<<grid, block, smem, s>>>(p, obs_dev, obs_env_stride, (float*)image_dev, (float*)contract_dev);
+    else if (dtype == SSD_POLICY_F16) policy_inputs_kernel<__half><<<grid, block, smem, s>>>(p, obs_dev, obs_env_stride, (__half*)image_dev, (__half*)contract_dev);
+    else if (dtype == SSD_POLICY_BF16) policy_inputs_kernel<__nv_bfloat16><<<grid, block, smem, s>>>(p, obs_dev, obs_env_stride, (__nv_bfloat16*)image_dev, (__nv_bfloat16*)contract_dev);
     else return fail(h, SSD_EINVAL, "policy_inputs: dtype must be SSD_POLICY_F32, _F16 or _BF16");
     return check_launch(h, "policy_inputs");
 }
@@ -1480,30 +1486,13 @@ int ssd_set_policy_output(ssd_handle* h, const ssd_policy_out* out)
     if (!h) return SSD_EINVAL;
     ON_DEVICE(h);
     REQUIRE_GRID(h);
-    if (!out) { h->pol_form = OBS_U8; h->pol_image = nullptr; h->pol_contract = nullptr; return SSD_OK; }
-    if (out->struct_size < (int32_t)sizeof(ssd_policy_out))
-        return fail(h, SSD_EINVAL, "ssd_policy_out.struct_size %d < %d: the caller's declaration of ssd_policy_out is out of date",
-                    out->struct_size, (int)sizeof(ssd_policy_out));
-    if (out->dtype != POLICY_F32 && out->dtype != POLICY_F16 && out->dtype != POLICY_BF16)
-        return fail(h, SSD_EINVAL, "set_policy_output: dtype %d is not SSD_POLICY_F32, _F16 or _BF16", out->dtype);
-    if (!out->image_dev || (reinterpret_cast<uintptr_t>(out->image_dev) & 15))
-        return fail(h, SSD_EINVAL, "set_policy_output: image_dev must be a 16-byte aligned device pointer");
-    const uintptr_t esize = out->dtype == POLICY_F32 ? 4 : 2;
+    if (!out) return set_form(h, 0, nullptr, ThetaRows{});
+    int rc = check_policy_out(h, out, "ssd_policy_out", "set_policy_output", out->image_dev, "image_dev");
+    if (rc) return rc;
+    const uintptr_t esize = out->dtype == SSD_POLICY_F32 ? 4 : 2;
     if (reinterpret_cast<uintptr_t>(out->contract_dev) & (esize - 1))
         return fail(h, SSD_EINVAL, "set_policy_output: contract_dev must be aligned to its element size");
-    const int form = 1 + out->dtype;
-    const GridParams& p = h->gp;
-    for (int feat = 0; feat < 2; feat++)
-        CUDA_TRY(h, cudaFuncSetAttribute((const void*)obs_kernel_fn(p.kind, h->rounds4, feat != 0, 0, form),
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, p.g2_smem_bytes));
-    if (h->obs_lay) CUDA_TRY(h, cudaFuncSetAttribute((const void*)obs_kernel_fn(p.kind, h->rounds4, false, h->obs_lay, form),
-                                                     cudaFuncAttributeMaxDynamicSharedMemorySize, p.g2_smem_bytes));
-    CUDA_TRY(h, cudaFuncSetAttribute((const void*)reset_kernel_fn(p.kind, form), cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     p.g2_smem_bytes));
-    h->pol_form = form;
-    h->pol_image = (uint8_t*)out->image_dev;
-    h->pol_contract = out->contract_dev;
-    return SSD_OK;
+    return set_form(h, 1 + out->dtype, out->image_dev, ThetaRows{ out->contract_dev, out->dtype, 10, 0, 5 });
 }
 
 int ssd_set_flat_policy_output(ssd_handle* h, const ssd_flat_policy_out* out)
@@ -1512,24 +1501,12 @@ int ssd_set_flat_policy_output(ssd_handle* h, const ssd_flat_policy_out* out)
     ON_DEVICE(h);
     if (h->cfg.env_kind != SSD_ENV_SELFDRIVE && !IS_FEAT(h))
         return fail(h, SSD_EINVAL, "set_flat_policy_output: handle is a gridworld (env_kind %d; see ssd_set_policy_output)", h->cfg.env_kind);
-    if (!out) { h->flat_form = OBS_F64; h->flat = FlatPolicy{ nullptr, 0, 0 }; return SSD_OK; }
-    if (out->struct_size < (int32_t)sizeof(ssd_flat_policy_out))
-        return fail(h, SSD_EINVAL, "ssd_flat_policy_out.struct_size %d < %d: the caller's declaration of ssd_flat_policy_out is out of date",
-                    out->struct_size, (int)sizeof(ssd_flat_policy_out));
-    if (out->dtype != POLICY_F32 && out->dtype != POLICY_F16 && out->dtype != POLICY_BF16)
-        return fail(h, SSD_EINVAL, "set_flat_policy_output: dtype %d is not SSD_POLICY_F32, _F16 or _BF16", out->dtype);
-    if (!out->obs_dev || (reinterpret_cast<uintptr_t>(out->obs_dev) & 15))
-        return fail(h, SSD_EINVAL, "set_flat_policy_output: obs_dev must be a 16-byte aligned device pointer");
-    const int form = 1 + out->dtype;
-    const bool car = h->cfg.env_kind == SSD_ENV_SELFDRIVE;
-    for (int q = 0; q < 2; q++) {
-        const void* fn = car ? (const void*)car_kernel_fn(q != 0, form)
-                             : (const void*)feat_kernel_fn(h->cfg.env_kind == SSD_ENV_CLEANUP_FEATURES, q != 0, form);
-        CUDA_TRY(h, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, car ? h->car_smem : h->feat_smem));
-    }
-    h->flat_form = form;
-    h->flat = FlatPolicy{ out->obs_dev, out->dtype, ssd_feature_dim(h) + (h->cfg.contract_kind != SSD_CONTRACT_NONE ? 2 : 0) };
-    return SSD_OK;
+    if (!out) return set_form(h, 0, nullptr, ThetaRows{});
+    int rc = check_policy_out(h, out, "ssd_flat_policy_out", "set_flat_policy_output", out->obs_dev, "obs_dev");
+    if (rc) return rc;
+    const bool contract = h->cfg.contract_kind != SSD_CONTRACT_NONE;       // the rows end in [theta, 0] only under a contract
+    const int width = ssd_feature_dim(h) + (contract ? 2 : 0);
+    return set_form(h, 1 + out->dtype, out->obs_dev, ThetaRows{ contract ? out->obs_dev : nullptr, out->dtype, width, width - 2, 1 });
 }
 
 // ---- NegotiationSolver (two_stage_train.py:619-776) ------------------------------------------------
@@ -1540,19 +1517,17 @@ static SolverParams solver_params(ssd_handle* h)
     s.seed = h->cfg.seed; s.first_env_id = h->cfg.first_env_id;
     s.low = h->cfg.theta_low; s.high = h->cfg.theta_high;
     s.E = h->cfg.num_envs; s.n = h->cfg.num_agents;
+    s.rows = h->theta_rows;
     if (h->cfg.env_kind == SSD_ENV_SELFDRIVE) {
         s.episode = reinterpret_cast<const uint8_t*>(h->cp.episode); s.episode_stride = 4; s.episode_mask = 0xFFFFFFFFu;
         s.theta = reinterpret_cast<uint8_t*>(h->cp.theta); s.theta_stride = 8;
-        s.flat = flat_theta_rows(h);
     } else if (IS_FEAT(h)) {
         s.episode = reinterpret_cast<const uint8_t*>(h->fp.rec + FR_EPISODE); s.episode_stride = 4 * FR_WORDS; s.episode_mask = 0x7FFFFFFFu;
         s.theta = reinterpret_cast<uint8_t*>(h->fp.rec + FR_THETA); s.theta_stride = 4 * FR_WORDS;
-        s.flat = flat_theta_rows(h);
     } else {
         const GridParams& p = h->gp;
         s.episode = p.state + RO_EPISODE; s.episode_stride = p.rec_stride; s.episode_mask = 0xFFFFFFFFu;
         s.theta = p.state + RO_THETA; s.theta_stride = p.rec_stride;
-        s.pol_contract = h->pol_contract; s.pol_dtype = h->pol_form - 1;
     }
     return s;
 }
@@ -1633,7 +1608,7 @@ int ssd_feat_reset(ssd_handle* h, const uint8_t* mask_dev, double* obs_dev, void
     FeatIO k = {};
     int rc = flat_obs_target(h, "feat_reset", obs_dev, false, &k.obs);
     if (rc) return rc;
-    feat_kernel_fn(h->cfg.env_kind == SSD_ENV_CLEANUP_FEATURES, true, h->flat_form)<<<h->grid_blocks, FEAT_THREADS, h->feat_smem,
+    feat_kernel_fn(h->cfg.env_kind == SSD_ENV_CLEANUP_FEATURES, true, h->form)<<<h->grid_blocks, FEAT_THREADS, h->feat_smem,
                                                                                       (cudaStream_t)stream>>>(h->fp, k, mask_dev);
     return check_launch(h, "feat_reset");
 }
@@ -1649,7 +1624,7 @@ int ssd_feat_step(ssd_handle* h, const ssd_feat_io* io, void* stream)
     if (!io->actions_dev || !io->rew_dev) return fail(h, SSD_EINVAL, "actions_dev, obs_dev and rew_dev are required");
     if (io->info_dev && (reinterpret_cast<uintptr_t>(io->info_dev) & 3)) return fail(h, SSD_EINVAL, "info_dev must be 4-byte aligned");
     FeatIO k = { io->actions_dev, obs, io->rew_dev, io->base_rew_dev, io->transfers_dev, io->info_dev, io->done_dev, io->auto_reset };
-    feat_kernel_fn(h->cfg.env_kind == SSD_ENV_CLEANUP_FEATURES, false, h->flat_form)<<<h->grid_blocks, FEAT_THREADS, h->feat_smem,
+    feat_kernel_fn(h->cfg.env_kind == SSD_ENV_CLEANUP_FEATURES, false, h->form)<<<h->grid_blocks, FEAT_THREADS, h->feat_smem,
                                                                                        (cudaStream_t)stream>>>(h->fp, k, nullptr);
     return check_launch(h, "feat_step");
 }
@@ -1657,7 +1632,7 @@ int ssd_feat_step(ssd_handle* h, const ssd_feat_io* io, void* stream)
 int ssd_feat_step_host_async(ssd_handle* h, const ssd_feat_io* io, const void* actions_host, void* result_host, int64_t* ticket_out,
                              void* stream)
 {
-    if (!h || !io || !actions_host || !result_host || !ticket_out || (!io->obs_dev && !h->flat_form)) return SSD_EINVAL;
+    if (!h || !io || !actions_host || !result_host || !ticket_out || (!io->obs_dev && !h->form)) return SSD_EINVAL;
     ON_DEVICE(h);
     REQUIRE_FEAT(h);
     void* obs = nullptr;
@@ -1673,7 +1648,7 @@ int ssd_feat_step_host_async(ssd_handle* h, const ssd_feat_io* io, const void* a
     k.c_done = sl.d_block + h->lay.done_offset;
     k.c_rew8 = reinterpret_cast<int8_t*>(sl.d_block + h->lay.rew_i8_offset);
     k.c_rec = sl.d_block + h->lay.records_offset;
-    feat_kernel_fn(h->cfg.env_kind == SSD_ENV_CLEANUP_FEATURES, false, h->flat_form)<<<h->grid_blocks, FEAT_THREADS, h->feat_smem,
+    feat_kernel_fn(h->cfg.env_kind == SSD_ENV_CLEANUP_FEATURES, false, h->form)<<<h->grid_blocks, FEAT_THREADS, h->feat_smem,
                                                                                        (cudaStream_t)stream>>>(h->fp, k, nullptr);
     if ((rc = check_launch(h, "feat_step_host_async"))) return rc;
     return async_end(h, si, (cudaStream_t)stream, ticket_out);
@@ -1706,7 +1681,7 @@ int ssd_selfdrive_reset(ssd_handle* h, const uint8_t* mask_dev, double* obs_dev,
     CarIO k = {};
     int rc = flat_obs_target(h, "selfdrive_reset", obs_dev, false, &k.obs);
     if (rc) return rc;
-    car_kernel_fn(true, h->flat_form)<<<h->grid_blocks, CAR_THREADS, h->car_smem, (cudaStream_t)stream>>>(h->cp, k, mask_dev);
+    car_kernel_fn(true, h->form)<<<h->grid_blocks, CAR_THREADS, h->car_smem, (cudaStream_t)stream>>>(h->cp, k, mask_dev);
     return check_launch(h, "selfdrive_reset");
 }
 
@@ -1721,14 +1696,14 @@ int ssd_selfdrive_step(ssd_handle* h, const ssd_selfdrive_io* io, void* stream)
     if (!io->actions_dev || !io->rew_dev) return fail(h, SSD_EINVAL, "actions_dev, obs_dev and rew_dev are required");
     if (io->info_dev && (reinterpret_cast<uintptr_t>(io->info_dev) & 31)) return fail(h, SSD_EINVAL, "info_dev must be 32-byte aligned");
     CarIO k = { io->actions_dev, obs, io->rew_dev, io->base_rew_dev, io->transfers_dev, io->info_dev, io->done_dev, io->auto_reset };
-    car_kernel_fn(false, h->flat_form)<<<h->grid_blocks, CAR_THREADS, h->car_smem, (cudaStream_t)stream>>>(h->cp, k, nullptr);
+    car_kernel_fn(false, h->form)<<<h->grid_blocks, CAR_THREADS, h->car_smem, (cudaStream_t)stream>>>(h->cp, k, nullptr);
     return check_launch(h, "selfdrive_step");
 }
 
 int ssd_selfdrive_step_host_async(ssd_handle* h, const ssd_selfdrive_io* io, const void* actions_host, void* result_host,
                                   int64_t* ticket_out, void* stream)
 {
-    if (!h || !io || !actions_host || !result_host || !ticket_out || (!io->obs_dev && !h->flat_form)) return SSD_EINVAL;
+    if (!h || !io || !actions_host || !result_host || !ticket_out || (!io->obs_dev && !h->form)) return SSD_EINVAL;
     ON_DEVICE(h);
     if (h->cfg.env_kind != SSD_ENV_SELFDRIVE) return fail(h, SSD_EINVAL, "selfdrive_step_host_async: handle is not a selfdrive env");
     void* obs = nullptr;
@@ -1745,7 +1720,7 @@ int ssd_selfdrive_step_host_async(ssd_handle* h, const ssd_selfdrive_io* io, con
     k.c_done = sl.d_block + h->lay.done_offset;
     k.c_rew8 = reinterpret_cast<int8_t*>(sl.d_block + h->lay.rew_i8_offset);
     k.c_rec = sl.d_block + h->lay.records_offset;
-    car_kernel_fn(false, h->flat_form)<<<h->grid_blocks, CAR_THREADS, h->car_smem, (cudaStream_t)stream>>>(h->cp, k, nullptr);
+    car_kernel_fn(false, h->form)<<<h->grid_blocks, CAR_THREADS, h->car_smem, (cudaStream_t)stream>>>(h->cp, k, nullptr);
     if ((rc = check_launch(h, "selfdrive_step_host_async"))) return rc;
     return async_end(h, si, (cudaStream_t)stream, ticket_out);
 }
@@ -1815,17 +1790,10 @@ int ssd_checkpoint_load(ssd_handle* h, uint64_t config_tag, const int32_t* env_i
     ck_load_kernel<<<(count + CK_ROWS - 1) / CK_ROWS, CK_THREADS, (size_t)CK_ROWS * h->ck.row_bytes, (cudaStream_t)stream>>>(
         h->ck, env_idx_dev, count, rows_dev, row_ok_dev);
     if ((rc = check_launch(h, "checkpoint_load"))) return rc;
-    if (h->pol_contract) {                                // theta came with the rows: the policy's contract rows follow it
-        policy_contract_refresh_kernel<<<(count + 127) / 128, 128, 0, (cudaStream_t)stream>>>(h->gp, env_idx_dev, count, h->pol_contract,
-                                                                                              h->pol_form - 1);
-        return check_launch(h, "checkpoint_load");
-    }
-    const SolverParams sp = solver_params(h);            // theta came with the rows: the flat policy rows' theta column follows it
-    if (sp.flat.rows) {
-        flat_theta_refresh_kernel<<<(count + 127) / 128, 128, 0, (cudaStream_t)stream>>>(sp, env_idx_dev, count);
-        return check_launch(h, "checkpoint_load");
-    }
-    return SSD_OK;
+    if (!h->theta_rows.rows) return SSD_OK;
+    // theta came with the rows: the policy output's rows that carry it follow
+    theta_rows_refresh_kernel<<<(count + 127) / 128, 128, 0, (cudaStream_t)stream>>>(solver_params(h), env_idx_dev, count);
+    return check_launch(h, "checkpoint_load");
 }
 
 int ssd_enable_timing(ssd_handle* h, int32_t on)

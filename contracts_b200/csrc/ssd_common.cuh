@@ -124,46 +124,44 @@ __device__ __forceinline__ bool negotiate_agreement(uint32_t seed, uint32_t env_
 }
 
 // element types of the policy's input tensors (SSD_POLICY_*: ssd_policy_inputs, ssd_set_policy_output,
-// ssd_set_flat_policy_output); an observation form 1 + POLICY_* writes T = PolicyElem<form>::T
-#define POLICY_F32 0
-#define POLICY_F16 1
-#define POLICY_BF16 2
+// ssd_set_flat_policy_output); an observation form 1 + SSD_POLICY_* writes T = PolicyElem<form>::T
 template <int FORM> struct PolicyElem;
-template <> struct PolicyElem<1 + POLICY_F32> { typedef float T; };
-template <> struct PolicyElem<1 + POLICY_F16> { typedef __half T; };
-template <> struct PolicyElem<1 + POLICY_BF16> { typedef __nv_bfloat16 T; };
+template <> struct PolicyElem<1 + SSD_POLICY_F32> { typedef float T; };
+template <> struct PolicyElem<1 + SSD_POLICY_F16> { typedef __half T; };
+template <> struct PolicyElem<1 + SSD_POLICY_BF16> { typedef __nv_bfloat16 T; };
 
 template <typename T> __device__ __forceinline__ T policy_cast(float v);
 template <> __device__ __forceinline__ float policy_cast<float>(float v) { return v; }
 template <> __device__ __forceinline__ __half policy_cast<__half>(float v) { return __float2half_rn(v); }
 template <> __device__ __forceinline__ __nv_bfloat16 policy_cast<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
 
-// Observation form of the feature-env and selfdrive kernels: OBS_F64 = the float64 rows [E][n][F | D]; 1 + POLICY_* = the
-// policy's flat rows T [E n][W] (ssd_set_flat_policy_output): features ++ [theta, 0] with a contract (W = F + 2), else the
-// features alone (W = F), each value T(float32(x)).
+// Observation form of the feature-env and selfdrive kernels: OBS_F64 = the float64 rows [E][n][F | D]; 1 + SSD_POLICY_* =
+// the policy's flat rows T [E n][W] (ssd_set_flat_policy_output): features ++ [theta, 0] with a contract (W = F + 2), else
+// the features alone (W = F), each value T(float32(x)).
 #define OBS_F64 0
+
+// the rows of a policy output that carry theta: (theta, 0) `reps` times from column `col` of each of an env's n rows,
+// T [E n][width], T by dtype = SSD_POLICY_*; rows == nullptr: none.  A grid world's contract rows are {contract, dtype,
+// 10, 0, 5}, flat rows under a contract {rows, dtype, W, W - 2, 1}.
+struct ThetaRows { void* rows; int dtype, width, col, reps; };
 template <typename T>
-__device__ __forceinline__ void policy_column_rows(T* rows, int n, int width, int col, double theta)
+__device__ __forceinline__ void theta_rows_fill(T* rows, const ThetaRows& r, int n, double theta)
 {
-    const T v = policy_cast<T>(__double2float_rn(theta));
-    for (int a = 0; a < n; a++) rows[(size_t)a * width + col] = v;
+    const T v = policy_cast<T>(__double2float_rn(theta)), z = policy_cast<T>(0.0f);
+    for (int a = 0; a < n; a++)
+        for (int k = 0; k < r.reps; k++) {
+            rows[(size_t)a * r.width + r.col + 2 * k] = v;
+            rows[(size_t)a * r.width + r.col + 2 * k + 1] = z;
+        }
 }
-// Column `col` of the n rows of `env` in a policy tensor T [E n][width] (T by dtype = SSD_POLICY_*) set to theta: what
-// the calls that change theta outside a step do to the flat rows (thread-per-env kernels).
-__device__ __forceinline__ void policy_column_env(void* rows, int dtype, int n, int width, int col, int env, double theta)
+// what the calls that change theta outside a step do to the policy output (thread-per-env kernels)
+__device__ __forceinline__ void theta_rows_env(const ThetaRows& r, int n, int env, double theta)
 {
-    const size_t o = (size_t)env * n * width;
-    if (dtype == POLICY_F32) policy_column_rows(reinterpret_cast<float*>(rows) + o, n, width, col, theta);
-    else if (dtype == POLICY_F16) policy_column_rows(reinterpret_cast<__half*>(rows) + o, n, width, col, theta);
-    else policy_column_rows(reinterpret_cast<__nv_bfloat16*>(rows) + o, n, width, col, theta);
-}
-// The flat policy rows of a feature-env / selfdrive handle as the theta refreshes see them (rows == nullptr: not set).
-struct FlatPolicy {
-    void* rows; int dtype, width;
-};
-__device__ __forceinline__ void flat_policy_theta(const FlatPolicy& f, int n, int env, double theta)
-{
-    if (f.rows) policy_column_env(f.rows, f.dtype, n, f.width, f.width - 2, env, theta);
+    if (!r.rows) return;
+    const size_t o = (size_t)env * n * r.width;
+    if (r.dtype == SSD_POLICY_F32) theta_rows_fill(reinterpret_cast<float*>(r.rows) + o, r, n, theta);
+    else if (r.dtype == SSD_POLICY_F16) theta_rows_fill(reinterpret_cast<__half*>(r.rows) + o, r, n, theta);
+    else theta_rows_fill(reinterpret_cast<__nv_bfloat16*>(r.rows) + o, r, n, theta);
 }
 
 // SSD_STEP_AUTO (ssd_random_actions & co.): counter[0] = step index, counter[1] = CTAs finished.  Every CTA reads

@@ -81,7 +81,7 @@ struct FeatParams {
 
 struct FeatIO {
     const uint8_t* actions;     // [E][n]
-    void* obs;                  // double [E][n][F] (OBS_F64), or the policy's rows T [E n][W] (1 + POLICY_*: feat_policy_row)
+    void* obs;                  // double [E][n][F] (OBS_F64), or the policy's rows T [E n][W] (1 + SSD_POLICY_*: feat_policy_row)
     double* rew; double* base_rew; double* transfers;   // [E][n]
     uint8_t* info;              // [E][n][4]: cleanup (cleaned_squares,0,0,0); harvest (eaten_apples, eaten_close_apples,0,0)
     uint8_t* done;              // [E]
@@ -310,7 +310,7 @@ __device__ __forceinline__ void feat_policy_row(T* o, const double (&v)[FEAT_MAX
 // One launch = one step (or, RESET_ONLY, one masked reset) of every env.
 // Next-step auto-reset (ssd_feat_io.auto_reset): an env that reached its horizon in the previous step starts its next
 // episode in this one — reset observation, zero rewards, done cleared, the actions of this step ignored.
-// FORM: OBS_F64 (float64 rows [E][n][F]) or 1 + POLICY_* (the policy's rows, feat_policy_row).
+// FORM: OBS_F64 (float64 rows [E][n][F]) or 1 + SSD_POLICY_* (the policy's rows, feat_policy_row).
 template <bool CLEANUP, bool RESET_ONLY, int FORM>
 __global__ void __launch_bounds__(FEAT_THREADS, FEAT_MIN_BLOCKS) feat_kernel(const FeatParams p, const FeatIO io, const uint8_t* __restrict__ mask)
 {
@@ -921,14 +921,6 @@ __global__ void feat_get_state_kernel(const FeatParams p, int32_t* pos, int32_t*
     }
     if (theta) theta[env] = *reinterpret_cast<const double*>(rec + FR_THETA);
     if (t) t[env] = (int)rec[FR_T];
-}
-// flat: the policy's rows when they have a theta column (ssd_set_flat_policy_output), kept current
-__global__ void feat_set_theta_kernel(const FeatParams p, const double* theta, const FlatPolicy flat)
-{
-    const int env = blockIdx.x * blockDim.x + threadIdx.x;
-    if (env >= p.E) return;
-    *reinterpret_cast<double*>(p.rec + (size_t)env * FR_WORDS + FR_THETA) = theta[env];
-    flat_policy_theta(flat, p.n, env, theta[env]);
 }
 __global__ void feat_random_actions_kernel(const FeatParams p, uint32_t step_index, uint32_t* counter, int num_actions, uint8_t* actions)
 {

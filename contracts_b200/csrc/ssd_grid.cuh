@@ -19,8 +19,8 @@
 #pragma once
 #include "ssd_common.cuh"
 
-// Observation form written by the observe / reset kernels: OBS_U8 = the uint8 windows [E][n][15][15][3]; 1 + POLICY_* = the
-// policy's image tensor T [E n][3][15][15] (ssd_set_policy_output), the values ssd_policy_inputs would make of the windows.
+// Observation form written by the observe / reset kernels: OBS_U8 = the uint8 windows [E][n][15][15][3]; 1 + SSD_POLICY_* =
+// the policy's image tensor T [E n][3][15][15] (ssd_set_policy_output), the values ssd_policy_inputs would make of the windows.
 #define OBS_U8 0
 template <int FORM> struct ObsForm : PolicyElem<FORM> {};
 template <> struct ObsForm<OBS_U8> { typedef uint8_t T; };
@@ -917,14 +917,6 @@ __device__ __forceinline__ void policy_contract_rows(T* c, int n, double theta, 
 {
     const T v = policy_cast<T>(__double2float_rn(theta)), z = policy_cast<T>(0.0f);
     for (int k = lane; k < n * 10; k += lanes) c[k] = (k & 1) ? z : v;
-}
-// runtime-dtype form for the thread-per-env kernels (negotiation, contract parameters, checkpoint load)
-__device__ __forceinline__ void policy_contract_env(void* c, int dtype, int n, int env, double theta)
-{
-    const size_t o = (size_t)env * n * 10;
-    if (dtype == POLICY_F32) policy_contract_rows(reinterpret_cast<float*>(c) + o, n, theta, 0, 1);
-    else if (dtype == POLICY_F16) policy_contract_rows(reinterpret_cast<__half*>(c) + o, n, theta, 0, 1);
-    else policy_contract_rows(reinterpret_cast<__nv_bfloat16*>(c) + o, n, theta, 0, 1);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -48,7 +48,7 @@ struct CarParams {
 
 struct CarIO {
     const float* actions;   // [E][n]
-    void* obs;              // double [E][n][D] (OBS_F64), or the policy's rows T [E n][W] (1 + POLICY_*: see car_kernel)
+    void* obs;              // double [E][n][D] (OBS_F64), or the policy's rows T [E n][W] (1 + SSD_POLICY_*: see car_kernel)
     double* rew; double* base_rew; double* transfers;   // [E][n]
     double* info;           // [E][n][4]: just_passed, active, ambulance_rank, ambulance_dist_to_front (row of the first acting agent)
     uint8_t* done;          // [E][n+1]
@@ -196,7 +196,7 @@ __device__ __forceinline__ void car_copy_run(uint8_t* dst, const uint8_t* src, i
 // One launch = one step (or, RESET_ONLY, one masked reset) of every env.
 // Next-step auto-reset (ssd_selfdrive_io.auto_reset): an env whose episode ended in the previous step starts its next
 // episode in this one — reset observation, zero rewards, dones cleared, the actions of this step ignored.
-// FORM: OBS_F64 (float64 rows [E][n][D]) or 1 + POLICY_*: the policy's rows T [E n][W], each car's D values ++ [theta, 0]
+// FORM: OBS_F64 (float64 rows [E][n][D]) or 1 + SSD_POLICY_*: the policy's rows T [E n][W], each car's D values ++ [theta, 0]
 // with a contract (W = D + 2), else the D values alone (W = D), each T(float32(x)).  Either form is built in the staging
 // area exactly as it goes out (an env's n rows contiguous, the warp's four envs one after the other) and copied out by
 // car_copy_run.
@@ -493,12 +493,4 @@ __global__ void car_get_state_kernel(const CarParams p, double* pos, double* vel
     if (theta) theta[env] = p.theta[env];
     if (m_transfers) m_transfers[env] = p.m_transfers[env];
     if (t) t[env] = p.t[env];
-}
-// flat: the policy's rows when they have a theta column (ssd_set_flat_policy_output), kept current
-__global__ void car_set_theta_kernel(const CarParams p, const double* theta, const FlatPolicy flat)
-{
-    const int env = blockIdx.x * blockDim.x + threadIdx.x;
-    if (env >= p.E) return;
-    p.theta[env] = theta[env];
-    flat_policy_theta(flat, p.n, env, theta[env]);
 }

@@ -162,8 +162,7 @@ struct SolverParams {
     double low, high;
     const uint8_t* episode; long long episode_stride; uint32_t episode_mask;
     uint8_t* theta; long long theta_stride;
-    void* pol_contract; int pol_dtype;       // gridworld with a policy output (ssd_set_policy_output): its contract rows, else NULL
-    FlatPolicy flat;                         // feature env / selfdrive with flat policy rows that carry theta, else rows NULL
+    ThetaRows rows;                          // the policy output's rows that carry theta (rows NULL: none)
 };
 #define SOLVER_RULE_MAX 0
 #define SOLVER_RULE_MAJORITY 1
@@ -217,8 +216,7 @@ __global__ void solver_choose_kernel(const SolverParams p, int S, int rule, cons
     if (best_param) best_param[env] = theta;
     if (best_idx) best_idx[env] = src;
     *reinterpret_cast<double*>(p.theta + (size_t)env * p.theta_stride) = theta;
-    if (p.pol_contract) policy_contract_env(p.pol_contract, p.pol_dtype, n, env, theta);
-    flat_policy_theta(p.flat, n, env, theta);
+    theta_rows_env(p.rows, n, env, theta);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -228,9 +226,9 @@ __global__ void solver_choose_kernel(const SolverParams p, int S, int rule, cons
 //            quotient that RLlib hands over as float32): uint8 [E][n][15][15][3] -> T [E n][3][15][15],
 //            value = T(float32(float64(x) / 255.0)) through a 256-entry table;
 //   contract `orig_obs["contract"].float().repeat(1, 5)` (vision_net.py:160-161): (theta, 0) five times, T [E n][10].
-// T = float32, float16 or bfloat16 (POLICY_F32 / F16 / BF16).  HBM-bound: 675 B read, 675 sizeof(T) written per agent.
+// T = float32, float16 or bfloat16 (SSD_POLICY_F32 / F16 / BF16).  HBM-bound: 675 B read, 675 sizeof(T) written per agent.
 // One CTA per env; the windows are staged in shared memory, the outputs leave as coalesced element runs.
-// (POLICY_* and policy_cast are in ssd_grid.cuh: the observe / reset kernels write the same tensor with a policy output set.)
+// (PolicyElem and policy_cast are in ssd_common.cuh: the observe / reset kernels write the same tensor with a policy output set.)
 template <typename T>
 __global__ void __launch_bounds__(VIEW_THREADS) policy_inputs_kernel(const GridParams p, const uint8_t* __restrict__ obs, long long obs_stride,
                                                                      T* __restrict__ image, T* __restrict__ contract)

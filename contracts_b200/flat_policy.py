@@ -11,7 +11,6 @@ import ctypes
 import torch
 
 from . import _lib
-from .batched import BatchedGridEnv
 
 
 class FlatPolicyMixin:
@@ -24,12 +23,14 @@ class FlatPolicyMixin:
         self.policy_width = F + (2 if self.contract is not None else 0)
         if policy_dtype is None:
             return False
-        if policy_dtype not in BatchedGridEnv._POLICY_DTYPES:
+        try:
+            code = _lib.policy_dtype_code(policy_dtype)
+        except ValueError:
             self.close()
-            raise ValueError("policy_dtype must be None, torch.float32, torch.float16 or torch.bfloat16, got %r" % (policy_dtype,))
+            raise
         self.policy_obs = torch.zeros((self.E * self.n, self.policy_width), dtype=policy_dtype, device=self.device)
         out = _lib.ssd_flat_policy_out(struct_size=ctypes.sizeof(_lib.ssd_flat_policy_out),
-                                       dtype=BatchedGridEnv._POLICY_DTYPES[policy_dtype], obs_dev=self.policy_obs.data_ptr())
+                                       dtype=code, obs_dev=self.policy_obs.data_ptr())
         _lib.check(self._h, self.lib.ssd_set_flat_policy_output(self._h, ctypes.byref(out)))
         return True
 

@@ -311,6 +311,7 @@ def test_policy_kernel_instantiations_launch():
 
 def test_flat_policy_output_error_surface():
     from contracts_b200 import _lib
+    from contracts_b200.batched import negotiate
     E, n = 16, 4
     stream = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
     for kind in KINDS:
@@ -354,6 +355,11 @@ def test_flat_policy_output_error_surface():
         assert reset(u._h, None, ctypes.c_void_p(u.obs.data_ptr()), stream) == 0
         torch.cuda.synchronize()
         assert torch.equal(stray, u.obs) and torch.equal(q.policy_obs, rows0)
+        # ... and the calls that change theta leave the old rows as they were
+        q.set_contract_params(0.25)
+        negotiate(q, torch.full((E,), 0.5, dtype=torch.float64, device="cuda"), torch.ones((E, n), dtype=torch.float64, device="cuda"))
+        torch.cuda.synchronize()
+        assert torch.equal(q.policy_obs, rows0)
         with pytest.raises(ValueError):
             _make(kind, E, n, torch.int8)
     from contracts_b200.batched import BatchedGridEnv

@@ -344,3 +344,10 @@ def test_policy_output_error_surface():
     assert torch.equal(q.policy_image, u.policy_inputs(torch.float16)[0])
     with pytest.raises(ValueError):
         _make("harvest_new", E, n, torch.int8)
+    # NULL switches the output off: the calls that change theta leave the old tensors as they were
+    img1, con1 = q.policy_image.clone(), q.policy_contract.clone()
+    assert lib.ssd_set_policy_output(q._h, None) == 0
+    q.set_contract_params(0.25)
+    q.negotiate(torch.full((E,), 0.5, dtype=torch.float64, device="cuda"), torch.ones((E, n), dtype=torch.float64, device="cuda"))
+    torch.cuda.synchronize()
+    assert torch.equal(q.policy_image, img1) and torch.equal(q.policy_contract, con1)
