@@ -135,12 +135,20 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
     no uint8 windows (`obs` is None).  reset / step / step_host return `policy_image` in place of `obs`.  The mode is fixed
     for the env's lifetime; the methods that read the uint8 windows (host_snapshot(obs=True), concatenated_obs,
     policy_inputs) raise ValueError in it.
+
+    image_obs=False: the observation is the feature vector (image_obs=False of the reference, cleanup_new.py:193-202,243-254,
+    harvest_new.py:160-168,212-222), written by the device at every step and reset (ssd_set_feature_output) — the same
+    interface as BatchedFeatureEnv: `obs` float64 [E, n, F], or with policy_dtype T the policy's flat rows `policy_obs`
+    T [E*n, policy_width] (features ++ [theta, 0] under a contract, policy_width = F + 2; the features alone without one)
+    and `obs` None.  No uint8 windows are kept: step(want_features=True) and the methods that read windows raise
+    ValueError.
     """
 
     def __init__(self, kind, num_envs, num_agents, ascii_map=None, horizon=1000, contract=None,
                  theta_low=0.0, theta_high=None, null_prob=0.0, seed=73907, first_env_id=0,
                  device=None, padded_obs=False,
-                 use_collective_reward=False, inequity_averse_reward=False, alpha=0.0, beta=0.0, policy_dtype=None):
+                 use_collective_reward=False, inequity_averse_reward=False, alpha=0.0, beta=0.0, policy_dtype=None,
+                 image_obs=True):
         if kind not in ("cleanup_new", "harvest_new"):
             raise ValueError("BatchedGridEnv kind must be cleanup_new or harvest_new, got %r" % (kind,))
         if not torch.cuda.is_available():
@@ -178,7 +186,10 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
         self.F = self.lib.ssd_feature_dim(self._h)
         E, n, dev = self.E, self.n, self.device
         self.policy_dtype, self.policy_image, self.policy_contract = policy_dtype, None, None
-        if policy_dtype is not None:
+        self.image_obs, self.policy_obs, self.policy_width = bool(image_obs), None, None
+        if not self.image_obs:
+            self._init_feature_output(policy_dtype)
+        elif policy_dtype is not None:
             try:
                 code = _lib.policy_dtype_code(policy_dtype)
             except ValueError:
@@ -219,21 +230,52 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
         except Exception:
             pass
 
+    def _init_feature_output(self, policy_dtype):
+        """image_obs=False: the handle writes float64 feature rows to `obs`, or the policy's flat rows to `policy_obs`"""
+        E, n = self.E, self.n
+        try:
+            code = _lib.FEATURE_F64 if policy_dtype is None else _lib.policy_dtype_code(policy_dtype)
+        except ValueError:
+            self.close()
+            raise
+        self.policy_width = self.F + (2 if self.contract is not None else 0)
+        if policy_dtype is None:
+            self.obs = torch.zeros((E, n, self.F), dtype=torch.float64, device=self.device)
+            rows = self.obs
+        else:
+            self.obs = None
+            self.policy_obs = rows = torch.zeros((E * n, self.policy_width), dtype=policy_dtype, device=self.device)
+        out = _lib.ssd_feature_out(struct_size=ctypes.sizeof(_lib.ssd_feature_out), dtype=code, obs_dev=rows.data_ptr())
+        _lib.check(self._h, self.lib.ssd_set_feature_output(self._h, ctypes.byref(out)))
+        self.obs_stride, self._obs_buf = 0, None
+
     def _stream(self):
         return ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
     @property
     def observation(self):
-        """what reset / step return: `obs`, or `policy_image` when the env writes the policy's tensors"""
+        """what reset / step return: `obs`, or `policy_image` when the env writes the policy's tensors (`policy_obs` with
+        image_obs=False)"""
+        if not self.image_obs:
+            return self.obs if self.policy_dtype is None else self.policy_obs
         return self.obs if self.policy_dtype is None else self.policy_image
 
+    def _no_feature_copy(self, want_features):
+        if want_features and not self.image_obs:
+            raise ValueError("want_features: with image_obs=False the observation already is the feature rows (`obs` / policy_obs)")
+
     def _need_windows(self, what):
+        if not self.image_obs:
+            raise ValueError("%s needs the uint8 observation windows; this env observes feature vectors (image_obs=False)" % what)
         if self.policy_dtype is not None:
             raise ValueError("%s needs the uint8 observation windows; this env writes the policy's tensors instead "
                              "(policy_dtype=%s)" % (what, self.policy_dtype))
 
     def _obs_rows(self):
-        """the observation rows checkpoint / restore carry: uint8 [E, n, 15, 15, 3], or T [E, n, 3, 15, 15] in policy mode"""
+        """the observation rows checkpoint / restore carry: uint8 [E, n, 15, 15, 3], or T [E, n, 3, 15, 15] in policy mode;
+        with image_obs=False float64 [E, n, F], or T [E, n, policy_width]"""
+        if not self.image_obs:
+            return self.obs if self.policy_dtype is None else self.policy_obs.view(self.E, self.n, self.policy_width)
         return self.obs if self.policy_dtype is None else self.policy_image.view(self.E, self.n, 3, 15, 15)
 
     def reset(self, mask=None):
@@ -267,6 +309,7 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
         """
         if actions.dtype != torch.uint8 or actions.device != self.device or not actions.is_contiguous():
             actions = actions.to(device=self.device, dtype=torch.uint8).contiguous()
+        self._no_feature_copy(want_features)
         if want_features and self.feature_obs is None:
             self.feature_obs = torch.zeros((self.E, self.n, self.F), dtype=torch.float64, device=self.device)
         io = self._io
@@ -292,6 +335,7 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
                 raise ValueError("step_host needs contiguous CPU tensors: uint8 actions, float64 rewards, uint8 dones")
         if self._host_actions_dev is None:
             self._host_actions_dev = torch.empty((self.E, self.n), dtype=torch.uint8, device=self.device)
+        self._no_feature_copy(want_features)
         if want_features and self.feature_obs is None:
             self.feature_obs = torch.zeros((self.E, self.n, self.F), dtype=torch.float64, device=self.device)
         io = self._io
@@ -319,6 +363,7 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
         dense_rewards=True also writes the float64 [E, n] matrix to self.rew on the device."""
         if actions_host.device.type != "cpu" or actions_host.dtype != torch.uint8 or not actions_host.is_contiguous():
             raise ValueError("step_host_async needs a contiguous CPU uint8 tensor [E, n] (pinned for an asynchronous copy)")
+        self._no_feature_copy(want_features)
         if want_features and self.feature_obs is None:
             self.feature_obs = torch.zeros((self.E, self.n, self.F), dtype=torch.float64, device=self.device)
         io = self._io

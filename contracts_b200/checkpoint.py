@@ -28,8 +28,8 @@ class EnvCheckpoint:
     """Rows of env state with their global ids.  kind: the env kind string; config_tag / row_bytes: the layout the rows
     were saved under (ssd_checkpoint_layout); seed: the handle's seed; env_ids int64 [count]; rows uint8 [count,
     row_bytes]; obs: the observation rows of those envs or None (uint8 [count, n, 15, 15, 3] for the grid worlds, T
-    [count, n, 3, 15, 15] for a grid world with policy_dtype T, float64 [count, n, F | D] for the feature envs and
-    selfdrive, T [count, n, policy_width] for those with policy_dtype T).  The rows themselves do not depend on the
+    [count, n, 3, 15, 15] for a grid world with policy_dtype T, float64 [count, n, F | D] for the feature envs,
+    selfdrive and a grid world with image_obs=False, T [count, n, policy_width] for those with policy_dtype T).  The rows themselves do not depend on the
     observation form."""
 
     def __init__(self, kind, config_tag, row_bytes, seed, env_ids, rows, obs=None):

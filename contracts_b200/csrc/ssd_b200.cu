@@ -68,6 +68,8 @@ struct ssd_handle {
     int form;                // 0: the native form (OBS_U8 / OBS_F64); else 1 + SSD_POLICY_*
     void* pol_rows;          //   the policy image T [E n][3][15][15] (grid worlds) or the flat rows T [E n][W]
     ThetaRows theta_rows;    //   the rows that carry theta: a grid world's contract rows, flat rows under a contract
+    int feat_form;           // ssd_set_feature_output (grid worlds, form 0): 1 + its dtype (SSD_FEATURE_F64 / SSD_POLICY_*), rows at
+                             // pol_rows; 0: off
     char err[512];
     std::vector<void*> dev_allocs;
 };
@@ -105,6 +107,32 @@ static reset_kernel_t reset_kernel_fn(int kind, int form)
     return by_form(form, [&](auto F) -> reset_kernel_t {
         constexpr int FORM = decltype(F)::value;
         return kind == SSD_ENV_CLEANUP ? grid_reset_kernel<SSD_ENV_CLEANUP, FORM> : grid_reset_kernel<SSD_ENV_HARVEST, FORM>;
+    });
+}
+// f(std::integral_constant<int, OUT>()) for the dtype of ssd_set_feature_output (SSD_FEATURE_F64 or SSD_POLICY_*)
+template <typename F>
+static auto by_feature_dtype(int dtype, F f)
+{
+    if (dtype == SSD_POLICY_F32) return f(std::integral_constant<int, SSD_POLICY_F32>());
+    if (dtype == SSD_POLICY_F16) return f(std::integral_constant<int, SSD_POLICY_F16>());
+    if (dtype == SSD_POLICY_BF16) return f(std::integral_constant<int, SSD_POLICY_BF16>());
+    return f(std::integral_constant<int, SSD_FEATURE_F64>());
+}
+typedef void (*feature_kernel_t)(const GridParams, uint32_t*, void*, int);
+static feature_kernel_t feature_kernel_fn(int kind, bool rounds4, int dtype)
+{
+    return by_feature_dtype(dtype, [&](auto O) -> feature_kernel_t {
+        constexpr int OUT = decltype(O)::value;
+        if (kind == SSD_ENV_CLEANUP) return rounds4 ? grid_feature_kernel<SSD_ENV_CLEANUP, 4, OUT> : grid_feature_kernel<SSD_ENV_CLEANUP, MAX_POINT_ROUNDS, OUT>;
+        return rounds4 ? grid_feature_kernel<SSD_ENV_HARVEST, 4, OUT> : grid_feature_kernel<SSD_ENV_HARVEST, MAX_POINT_ROUNDS, OUT>;
+    });
+}
+typedef void (*reset_features_kernel_t)(const GridParams, const uint8_t*, void*, int);
+static reset_features_kernel_t reset_features_kernel_fn(int kind, int dtype)
+{
+    return by_feature_dtype(dtype, [&](auto O) -> reset_features_kernel_t {
+        constexpr int OUT = decltype(O)::value;
+        return kind == SSD_ENV_CLEANUP ? grid_reset_features_kernel<SSD_ENV_CLEANUP, OUT> : grid_reset_features_kernel<SSD_ENV_HARVEST, OUT>;
     });
 }
 typedef void (*feat_kernel_t)(const FeatParams, const FeatIO, const uint8_t*);
@@ -901,9 +929,20 @@ static int set_form(ssd_handle* h, int form, void* pol_rows, ThetaRows theta_row
 {
     if (form) { int rc = set_form_smem(h, form); if (rc) return rc; }
     h->form = form;
+    h->feat_form = 0;
     h->pol_rows = pol_rows;
     h->theta_rows = theta_rows;
     return SSD_OK;
+}
+// elements per row of the feature output: F, + [theta, 0] for the policy dtypes under a contract
+static int feature_width(const ssd_handle* h)
+{
+    return h->gp.F + (h->feat_form != 1 + SSD_FEATURE_F64 && h->cfg.contract_kind != SSD_CONTRACT_NONE ? 2 : 0);
+}
+// the feature output's reset rows of the envs `mask` selects (all when NULL), behind the reset kernel on stream s
+static void launch_reset_features(ssd_handle* h, const uint8_t* mask, cudaStream_t s)
+{
+    reset_features_kernel_fn(h->gp.kind, h->feat_form - 1)<<<h->grid_blocks, GRID_THREADS, 0, s>>>(h->gp, mask, h->pol_rows, feature_width(h));
 }
 
 // =============================================================================================
@@ -1031,6 +1070,16 @@ int ssd_reset(ssd_handle* h, const uint8_t* mask_dev, uint8_t* obs_dev, int64_t 
     ON_DEVICE(h);
     REQUIRE_GRID(h);
     const GridParams& p = h->gp;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (h->feat_form) {                                  // one observation form per handle: the feature rows, no windows
+        if (obs_dev) return fail(h, SSD_EINVAL, "reset: obs_dev must be NULL while a feature output is set (ssd_set_feature_output)");
+        if (p.beam) beam_clear_kernel<<<(p.E + 3) / 4, 128, 0, s>>>(p, mask_dev);
+        reset_kernel_fn(p.kind, OBS_U8)<<<h->grid_blocks, GRID_THREADS, p.g2_smem_bytes, s>>>(p, mask_dev, nullptr, 0, StepIO(), nullptr);
+        int rc = check_launch(h, "reset");
+        if (rc) return rc;
+        launch_reset_features(h, mask_dev, s);
+        return check_launch(h, "reset");
+    }
     long long stride = obs_env_stride ? obs_env_stride : (long long)p.n * SSD_OBS_BYTES;
     if (h->form) {                                       // one observation form per handle: the policy output's
         if (obs_dev) return fail(h, SSD_EINVAL, "reset: obs_dev must be NULL while a policy output is set (ssd_set_policy_output)");
@@ -1038,7 +1087,6 @@ int ssd_reset(ssd_handle* h, const uint8_t* mask_dev, uint8_t* obs_dev, int64_t 
         stride = policy_env_bytes(p, h->form);
     }
     if (stride < (long long)p.n * SSD_OBS_BYTES) return fail(h, SSD_EINVAL, "obs_env_stride too small");
-    cudaStream_t s = (cudaStream_t)stream;
     if (p.beam) beam_clear_kernel<<<(p.E + 3) / 4, 128, 0, s>>>(p, mask_dev);                 // self.beam_pos = [] (map_env.py:316)
     reset_kernel_fn(p.kind, h->form)<<<h->grid_blocks, GRID_THREADS, p.g2_smem_bytes, s>>>(p, mask_dev, obs_dev, stride, StepIO(),
                                                                                             h->theta_rows.rows);
@@ -1054,6 +1102,9 @@ static int make_step_io(ssd_handle* h, const ssd_step_io* io, StepIO& k, bool as
         if (io->obs_dev) return fail(h, SSD_EINVAL, "obs_dev must be NULL while a policy output is set (ssd_set_policy_output)");
         k.obs = (uint8_t*)h->pol_rows;
         k.obs_stride = policy_env_bytes(p, h->form);
+    } else if (h->feat_form) {                           // the feature rows are the observation: no windows, no second copy
+        if (io->obs_dev || io->feature_obs_dev)
+            return fail(h, SSD_EINVAL, "obs_dev and feature_obs_dev must be NULL while a feature output is set (ssd_set_feature_output)");
     } else {
         if (!io->obs_dev) return fail(h, SSD_EINVAL, "obs_dev is required");
         k.obs = io->obs_dev;
@@ -1130,11 +1181,19 @@ static int launch_step(ssd_handle* h, const StepIO& k, cudaStream_t s, const Hos
     if (hc && hc->slot >= 0) CUDA_TRY(h, cudaEventRecord(h->slot[hc->slot].ev_logic, s));   // the slot's actions were read
     if (p.kind == SSD_ENV_CLEANUP) { int rc = copy_rewards(h, k, s, hc); if (rc) return rc; }
     // programmatic dependent launch: the observe CTAs become resident (tables, tiles) as the one-wave logic grid drains
-    const bool dense = h->form || k.obs_stride == (long long)p.n * SSD_OBS_BYTES;       // a policy image is always dense
-    const int lay = (h->obs_lay != 0 && dense && !k.feat) ? h->obs_lay : 0;
-    const obs_kernel_t obs_k = obs_kernel_fn(p.kind, h->rounds4, k.feat != nullptr, lay, h->form);
-    if (h->pdl && !h->timing) CUDA_TRY(h, launch_pdl(obs_k, dim3(h->obs_blocks), dim3(OBS_WARPS * 32), (size_t)p.g2_smem_bytes, s, p, k, h->d_res));
-    else obs_k<<<h->obs_blocks, OBS_WARPS * 32, p.g2_smem_bytes, s>>>(p, k, h->d_res);
+    if (h->feat_form) {          // the feature form: spawn + feature rows in place of the observe kernel
+        const feature_kernel_t fk = feature_kernel_fn(p.kind, h->rounds4, h->feat_form - 1);
+        const int width = feature_width(h);
+        if (h->pdl && !h->timing)
+            CUDA_TRY(h, launch_pdl(fk, dim3(h->obs_blocks), dim3(OBS_WARPS * 32), (size_t)p.g2_smem_bytes, s, p, h->d_res, h->pol_rows, width));
+        else fk<<<h->obs_blocks, OBS_WARPS * 32, p.g2_smem_bytes, s>>>(p, h->d_res, h->pol_rows, width);
+    } else {
+        const bool dense = h->form || k.obs_stride == (long long)p.n * SSD_OBS_BYTES;       // a policy image is always dense
+        const int lay = (h->obs_lay != 0 && dense && !k.feat) ? h->obs_lay : 0;
+        const obs_kernel_t obs_k = obs_kernel_fn(p.kind, h->rounds4, k.feat != nullptr, lay, h->form);
+        if (h->pdl && !h->timing) CUDA_TRY(h, launch_pdl(obs_k, dim3(h->obs_blocks), dim3(OBS_WARPS * 32), (size_t)p.g2_smem_bytes, s, p, k, h->d_res));
+        else obs_k<<<h->obs_blocks, OBS_WARPS * 32, p.g2_smem_bytes, s>>>(p, k, h->d_res);
+    }
     if (p.kind == SSD_ENV_HARVEST) {
         h->launches++;
         if (h->pdl && !h->timing) CUDA_TRY(h, launch_pdl(grid_reward_kernel, dim3(lb), dim3(LOGIC_THREADS), (size_t)0, s, p, k, (const uint32_t*)h->d_res));
@@ -1150,6 +1209,10 @@ static int launch_step(ssd_handle* h, const StepIO& k, cudaStream_t s, const Hos
             CUDA_TRY(h, launch_pdl(reset_k, dim3(h->grid_blocks), dim3(GRID_THREADS), (size_t)p.g2_smem_bytes, s,
                                    p, (const uint8_t*)k.done, k.obs, k.obs_stride, k, h->theta_rows.rows));
         else reset_k<<<h->grid_blocks, GRID_THREADS, p.g2_smem_bytes, s>>>(p, k.done, k.obs, k.obs_stride, k, h->theta_rows.rows);
+        if (h->feat_form) {      // (k.obs is NULL: the reset kernel wrote no windows) the new episodes' reset rows
+            h->launches++;
+            launch_reset_features(h, k.done, s);
+        }
     }
     if (h->timing) cudaEventRecord(h->tev[2], s);
     return check_launch(h, "step");
@@ -1493,6 +1556,29 @@ int ssd_set_policy_output(ssd_handle* h, const ssd_policy_out* out)
     if (reinterpret_cast<uintptr_t>(out->contract_dev) & (esize - 1))
         return fail(h, SSD_EINVAL, "set_policy_output: contract_dev must be aligned to its element size");
     return set_form(h, 1 + out->dtype, out->image_dev, ThetaRows{ out->contract_dev, out->dtype, 10, 0, 5 });
+}
+
+int ssd_set_feature_output(ssd_handle* h, const ssd_feature_out* out)
+{
+    if (!h) return SSD_EINVAL;
+    ON_DEVICE(h);
+    REQUIRE_GRID(h);
+    if (!out) return set_form(h, 0, nullptr, ThetaRows{});
+    if (out->struct_size < (int32_t)sizeof(ssd_feature_out))
+        return fail(h, SSD_EINVAL, "ssd_feature_out.struct_size %d < %d: the caller's declaration of ssd_feature_out is out of date",
+                    out->struct_size, (int)sizeof(ssd_feature_out));
+    if (out->dtype != SSD_FEATURE_F64 && out->dtype != SSD_POLICY_F32 && out->dtype != SSD_POLICY_F16 && out->dtype != SSD_POLICY_BF16)
+        return fail(h, SSD_EINVAL, "set_feature_output: dtype %d is not SSD_FEATURE_F64, SSD_POLICY_F32, _F16 or _BF16", out->dtype);
+    if (!out->obs_dev || (reinterpret_cast<uintptr_t>(out->obs_dev) & 15))
+        return fail(h, SSD_EINVAL, "set_feature_output: obs_dev must be a 16-byte aligned device pointer");
+    CUDA_TRY(h, cudaFuncSetAttribute((const void*)feature_kernel_fn(h->cfg.env_kind, h->rounds4, out->dtype),
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, h->gp.g2_smem_bytes));
+    const bool theta_col = out->dtype != SSD_FEATURE_F64 && h->cfg.contract_kind != SSD_CONTRACT_NONE;
+    const int width = h->gp.F + (theta_col ? 2 : 0);
+    int rc = set_form(h, 0, out->obs_dev, ThetaRows{ theta_col ? out->obs_dev : nullptr, out->dtype, width, width - 2, 1 });
+    if (rc) return rc;
+    h->feat_form = 1 + out->dtype;
+    return SSD_OK;
 }
 
 int ssd_set_flat_policy_output(ssd_handle* h, const ssd_flat_policy_out* out)

@@ -652,10 +652,16 @@ __device__ __forceinline__ uint32_t closest_point(int lane, const uint32_t (&m)[
     }
     return __reduce_min_sync(FULL, best);
 }
-template <int KIND, int MW>
+// element k of a feature row: float64 as it is, a policy element type as T(float32(x))
+template <typename T>
+__device__ __forceinline__ void feat_put(T* f, int k, double x) { f[k] = policy_cast<T>(__double2float_rn(x)); }
+template <>
+__device__ __forceinline__ void feat_put<double>(double* f, int k, double x) { f[k] = x; }
+// out: the env's n rows of `width` elements (0: p.F; columns p.F.. of a wider row are left to the caller)
+template <int KIND, int MW, typename OUT = double>
 __device__ __forceinline__ void write_features(const GridParams& p, const SharedTables& tb, int lane, uint32_t hw /* agent word of lane < n */,
                                                const uint32_t (&am)[MW], const uint32_t (&wm)[MW],
-                                               int cleaned, int total_close, int hcount, double* out)
+                                               int cleaned, int total_close, int hcount, OUT* out, int width = 0)
 {
     const int n = p.n;
     const int my_r = (int)(hw & 255u), my_c = (int)((hw >> 8) & 255u), ori = (int)((hw >> 16) & 3u);
@@ -681,15 +687,16 @@ __device__ __forceinline__ void write_features(const GridParams& p, const Shared
 #pragma unroll
     for (int j = 0; j < SSD_MAXN; j++) cl[j] = __shfl_sync(FULL, cleaned, j);
     if (lane < n) {
-        double* f = out + (size_t)lane * p.F;
-        f[0] = my_r; f[1] = my_c; f[2] = ori; f[3] = cp_r; f[4] = cp_c; f[5] = cp_o; f[6] = ca_r; f[7] = ca_c;
+        OUT* f = out + (size_t)lane * (width ? width : p.F);
+        feat_put(f, 0, my_r); feat_put(f, 1, my_c); feat_put(f, 2, ori); feat_put(f, 3, cp_r); feat_put(f, 4, cp_c);
+        feat_put(f, 5, cp_o); feat_put(f, 6, ca_r); feat_put(f, 7, ca_c);
         if (KIND == SSD_ENV_CLEANUP) {
-            f[8] = cw_r; f[9] = cw_c; f[10] = n_apples; f[11] = hcount;
+            feat_put(f, 8, cw_r); feat_put(f, 9, cw_c); feat_put(f, 10, n_apples); feat_put(f, 11, hcount);
 #pragma unroll
-            for (int j = 0; j < SSD_MAXN; j++) if (j < n) f[12 + j] = cl[j];
+            for (int j = 0; j < SSD_MAXN; j++) if (j < n) feat_put(f, 12 + j, cl[j]);
         } else {
-            f[8] = total_close; f[9] = n_apples;
-            for (int j = 0; j < 2 * n; j++) f[10 + j] = 0.0;
+            feat_put(f, 8, total_close); feat_put(f, 9, n_apples);
+            for (int j = 0; j < 2 * n; j++) feat_put(f, 10 + j, 0.0);
         }
     }
 }

@@ -789,3 +789,146 @@ __global__ void __maxnreg__(OBS_MAXREG) grid_obs_kernel(const GridParams p_in, c
         if (atomicAdd(p.obs_ctr + 1, 1u) == gridDim.x - 1) { p.obs_ctr[0] = 0u; p.obs_ctr[1] = 0u; }
     }
 }
+
+// =============================================================================================
+// FEATURE FORM (ssd_set_feature_output): the observation is infos['feature_obs'] (cleanup_new.py:235-251,
+// harvest_new.py:208-222), written in output form OUT: SSD_FEATURE_F64 (double [E][n][F]) or SSD_POLICY_* (the policy's
+// flat rows T [E n][width], features ++ [theta, 0] under a contract).  No observation windows are built.
+template <int OUT> struct FeatureElem : PolicyElem<1 + OUT> {};
+template <> struct FeatureElem<SSD_FEATURE_F64> { typedef double T; };
+
+// columns F, F + 1 of a policy row under a contract: [theta, 0] (two_stage_train.py:113-121)
+template <typename T>
+__device__ __forceinline__ void feature_theta_cols(T* rows, const GridParams& p, int lane, int width, double theta)
+{
+    if (width > p.F && lane < p.n) { feat_put(rows + (size_t)lane * width, p.F, theta); feat_put(rows + (size_t)lane * width, p.F + 1, 0.0); }
+}
+
+// STEP, in place of the observe kernel behind the logic kernel: one warp per env, grid-stride.  What the observe kernel
+// does for an env apart from painting and the window gather — the env's tile T from the masks, the same spawn on the
+// same draws (masks and #waste written back when it changes them), harvest's total_close_apples into res_g for
+// grid_reward_kernel — then write_features' values.  Shared memory: the observe kernel's layout (T2 unused).
+template <int KIND, int MW, int OUT>
+__global__ void __launch_bounds__(OBS_WARPS * 32) grid_feature_kernel(const GridParams p, uint32_t* __restrict__ res_g, void* out, int width)
+{
+    typedef typename FeatureElem<OUT>::T T;
+    extern __shared__ __align__(16) uint8_t smem[];
+    const SharedTables tb = load_shared_tables(p, smem, true);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    uint8_t* tile = smem + p.sm_warp0 + warp * p.g2_warp_bytes;
+    uint32_t* scratch = reinterpret_cast<uint32_t*>(tile + p.g2_stage);
+    const PointRegs<MW> pr = load_point_regs<MW>(p, lane);
+    init_warp_tiles(p, tile, lane);
+    __syncthreads();                                  // tables visible
+    const int n = p.n, S = p.S;
+    const bool act_lane = lane < n;
+    const uint32_t rot3 = (uint32_t)(lane - 3) & 31u, rot2 = (uint32_t)(lane - 2) & 31u;
+    pdl_launch_dependents();                          // the reward / masked reset kernel behind the step may set up early
+    pdl_wait();                                       // the hot lines and res_g are the logic kernel's output
+    for (int env = blockIdx.x * OBS_WARPS + warp; env < p.E; env += gridDim.x * OBS_WARPS) {
+        uint32_t* hot = reinterpret_cast<uint32_t*>(p.state + (size_t)env * p.rec_stride);
+        const uint32_t hw = hot[lane];
+        uint32_t am[MW], wm[MW];
+#pragma unroll
+        for (int q = 0; q < MW; q++) {
+            am[q] = __shfl_sync(FULL, hw, RO_AMASK / 4 + q);
+            wm[q] = KIND == SSD_ENV_CLEANUP ? __shfl_sync(FULL, hw, RO_WMASK / 4 + q) : 0u;
+        }
+        apply_masks<MW, false>(p, tile, pr, am, wm, rot3, rot2);
+        const uint32_t t = __shfl_sync(FULL, hw, RO_T / 4);               // already incremented by the logic kernel
+        const uint32_t episode = __shfl_sync(FULL, hw, RO_EPISODE / 4);
+        int hcount = (int)__shfl_sync(FULL, hw, RO_HCOUNT / 4);
+        const double theta = __hiloint2double((int)__shfl_sync(FULL, hw, RO_THETA / 4 + 1), (int)__shfl_sync(FULL, hw, RO_THETA / 4));
+        const EnvRng g = { p.seed, p.first_env_id + (uint32_t)env, episode, t };
+        const int ao = act_lane ? ((int)(hw & 255u) + SSD_VIEW) * S + 8 + (int)((hw >> 8) & 255u) : 0;
+        __syncwarp();
+        uint32_t old = 0;
+        if (act_lane) {                               // spawn eligibility: "no agent there" (co-located lanes write the same value)
+            old = tile[ao] & CODE_MASK;
+            tile[ao] = (uint8_t)(old | OCC_BIT);
+        }
+        __syncwarp();
+        bool changed = false;
+        if (KIND == SSD_ENV_CLEANUP) {
+            if (cleanup_spawn_active(tb, hcount)) changed = cleanup_spawn<MW>(p, tb, lane, tile, false, scratch, g, t, hcount, pr, am, wm);
+        } else {
+            changed = harvest_spawn<MW>(p, lane, tile, false, scratch, g, t, pr, am);
+        }
+        if (changed) {                                // the masks (and #waste) go back only when the spawn changed them
+#pragma unroll
+            for (int q = 0; q < MW; q++)
+                if (lane == q) {
+                    hot[RO_AMASK / 4 + q] = am[q];
+                    if (KIND == SSD_ENV_CLEANUP) hot[RO_WMASK / 4 + q] = wm[q];
+                }
+            if (KIND == SSD_ENV_CLEANUP && lane == 0) hot[RO_HCOUNT / 4] = (uint32_t)hcount;
+        }
+        int total_close = 0, cleaned = 0;
+        if (KIND == SSD_ENV_HARVEST && act_lane) {
+            total_close = count_apples_r5(tile, ao, S);
+            res_g[(size_t)env * SSD_MAXN + lane] |= (uint32_t)total_close << RS_CLOSE_SHIFT;
+        }
+        if (KIND == SSD_ENV_CLEANUP && act_lane) cleaned = (int)(res_g[(size_t)env * SSD_MAXN + lane] & RS_CLEANED_MASK);
+        T* rows = reinterpret_cast<T*>(out) + (size_t)env * n * width;
+        write_features<KIND, MW, T>(p, tb, lane, hw, am, wm, cleaned, total_close, hcount, rows, width);
+        feature_theta_cols(rows, p, lane, width, theta);
+        __syncwarp();                                 // every lane's spawn / count reads of T are done
+        if (act_lane) tile[ao] = (uint8_t)old;
+        __syncwarp();
+    }
+}
+
+// RESET ROWS, behind grid_reset_kernel<KIND, 0> (no windows) on the same mask: the reset observation of each reset env from
+// its fresh record (GridWorldEnv._reset_feature_obs, cleanup_new.py:193-202, harvest_new.py:160-168).  One warp per env.
+//   cleanup: custom_reset fills the apple / waste caches BEFORE the reset-time spawn (map_env.py:319-320): no apples
+//            (closest apple [0, 0], 0 apples), the waste list is the map's initial 'H' cells, #waste their count, nothing
+//            cleaned;
+//   harvest: the map after the reset: the record's apples, count_apples_in_radius(5) (j*j + k*k <= 5) as total_close.
+// The theta column (policy rows under a contract) is the record's theta: the negotiated one behind an auto-reset.
+template <int KIND, int OUT>
+__global__ void __launch_bounds__(GRID_THREADS) grid_reset_features_kernel(const GridParams p, const uint8_t* mask, void* out, int width)
+{
+    typedef typename FeatureElem<OUT>::T T;
+    constexpr int MW = MAX_POINT_ROUNDS;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int env0 = blockIdx.x * GRID_WARPS + warp, estride = gridDim.x * GRID_WARPS;
+    const SharedTables tb = { nullptr, nullptr, nullptr, p.apple_rc, p.waste_rc };   // write_features reads only the point lists
+    for (int i0 = 0; env0 + (long long)i0 * estride < p.E; i0 += 32) {
+        const long long el = env0 + (long long)(i0 + lane) * estride;
+        unsigned todo = __ballot_sync(FULL, el < p.E && (!mask || mask[el]));
+        while (todo) {
+            const int env = env0 + (i0 + __ffs(todo) - 1) * estride;
+            todo &= todo - 1;
+            const uint32_t hw = reinterpret_cast<const uint32_t*>(p.state + (size_t)env * p.rec_stride)[lane];
+            uint32_t am[MW], wm[MW];
+#pragma unroll
+            for (int q = 0; q < MW; q++) {
+                am[q] = KIND == SSD_ENV_HARVEST ? __shfl_sync(FULL, hw, RO_AMASK / 4 + q) : 0u;
+                wm[q] = KIND == SSD_ENV_CLEANUP ? p.reset_wmask[q] : 0u;
+            }
+            int total_close = 0;
+            if (KIND == SSD_ENV_HARVEST) {
+                const int my_r = (int)(hw & 255u), my_c = (int)((hw >> 8) & 255u);
+                for (int a = 0; a < p.n; a++) {
+                    const int ar = __shfl_sync(FULL, my_r, a), ac = __shfl_sync(FULL, my_c, a);
+                    int cnt = 0;
+#pragma unroll
+                    for (int q = 0; q < MW; q++) {
+                        bool near = false;
+                        if ((am[q] >> lane) & 1u) {
+                            const uint32_t rc = __ldg(p.apple_rc + lane + 32 * q);
+                            const int dr = (int)(rc >> 8) - ar, dc = (int)(rc & 255u) - ac;
+                            near = dr * dr + dc * dc <= 5;
+                        }
+                        cnt += __popc(__ballot_sync(FULL, near));
+                    }
+                    if (lane == a) total_close = cnt;
+                }
+            }
+            const double theta = __hiloint2double((int)__shfl_sync(FULL, hw, RO_THETA / 4 + 1), (int)__shfl_sync(FULL, hw, RO_THETA / 4));
+            T* rows = reinterpret_cast<T*>(out) + (size_t)env * p.n * width;
+            write_features<KIND, MW, T>(p, tb, lane, hw, am, wm, 0, total_close, p.n_waste_start, rows, width);
+            feature_theta_cols(rows, p, lane, width, theta);
+        }
+    }
+}

@@ -274,6 +274,31 @@ typedef struct ssd_flat_policy_out {
  * aligned obs_dev, or a gridworld handle (those have ssd_set_policy_output).  The caller keeps the tensor alive while it
  * is set. */
 int ssd_set_flat_policy_output(ssd_handle* h, const ssd_flat_policy_out* out);
+/* The grid worlds' feature observation (image_obs=False: cleanup_new.py:193-202,243-254, harvest_new.py:160-168,212-222)
+ * as the handle's observation, written on the device at every step and reset, with no observation windows:
+ *   - SSD_FEATURE_F64: obs_dev double [E][n][F], each value what infos['feature_obs'] (the image_obs=False observation)
+ *     holds; F = ssd_feature_dim(h) = 12 + n (cleanup), 10 + 2n (harvest);
+ *   - SSD_POLICY_F32 / _F16 / _BF16: obs_dev T [E*n][W], the rows of ssd_set_flat_policy_output: W = F + 2 and the row
+ *     features ++ [theta, 0] with a contract, W = F and the features alone without one; each element T(float32(x)).
+ * Grid-world kinds.  While set (sticky; NULL switches the handle back to uint8 windows, and ssd_set_policy_output replaces
+ * it, as it replaces that one), the handle has this one observation form:
+ *   - ssd_reset (masked or not) writes the reset rows of the envs it resets: the reset observation of the reference
+ *     (cleanup: the apple / waste caches from before the reset-time spawn; harvest: the map after it), and ssd_step,
+ *     ssd_step_host, ssd_step_host_async write the step's rows; the auto_reset behind a step writes the new episode's reset
+ *     rows of the envs it restarts.  obs_dev and feature_obs_dev must be NULL in these calls (else SSD_EINVAL);
+ *   - with a policy dtype under a contract, every call that changes theta leaves the theta column of the envs it changes
+ *     current: ssd_reset, auto_reset with negotiation, ssd_negotiate, ssd_set_contract_params, ssd_solver_choose and
+ *     ssd_checkpoint_load (ssd_set_state does not; the next step writes it).
+ * Rewards, dones, infos, state, metrics, episode statistics and the episode log are those of the uint8 form.
+ * Validates before storing anything: SSD_EINVAL for a struct_size too small, an unknown dtype, a NULL or not 16-byte aligned
+ * obs_dev, or a feature-env or selfdrive handle.  The caller keeps the tensor alive while it is set. */
+#define SSD_FEATURE_F64 3        /* accepted by ssd_set_feature_output only */
+typedef struct ssd_feature_out {
+    int32_t struct_size;    /* sizeof(ssd_feature_out) (a smaller value is rejected) */
+    int32_t dtype;          /* SSD_FEATURE_F64, SSD_POLICY_F32 / _F16 / _BF16 */
+    void*   obs_dev;        /* double [E][n][F] or T [E*n][W], 16-byte aligned */
+} ssd_feature_out;
+int ssd_set_feature_output(ssd_handle* h, const ssd_feature_out* out);
 
 /* --- NegotiationSolver (environments/two_stage_train.py:619-776); every env kind ------------------- */
 #define SSD_SOLVER_RULE_MAX 0        /* decision_rule 'max'      (:751-757) */
