@@ -116,6 +116,12 @@ def make_config(**kw):
     return ssd_config(abi_version=SSD_ABI_VERSION, struct_size=ctypes.sizeof(ssd_config), **kw)
 
 
+class ssd_solver_window(ctypes.Structure):
+    _fields_ = [("struct_size", ctypes.c_int32), ("num_samples", ctypes.c_int32), ("capacity", ctypes.c_int32),
+                ("env_dev", ctypes.c_void_p), ("episode_dev", ctypes.c_void_p), ("count_dev", ctypes.c_void_p),
+                ("params_dev", ctypes.c_void_p), ("rows_dev", ctypes.c_void_p)]
+
+
 class ssd_selfdrive_io(ctypes.Structure):
     _fields_ = [(n, ctypes.c_void_p) for n in ("actions_dev", "obs_dev", "rew_dev", "base_rew_dev", "transfers_dev",
                                                "info_dev", "done_dev")] + [("auto_reset", ctypes.c_int32)]
@@ -137,6 +143,7 @@ EXPORTS = [
     "ssd_feat_step_host_async", "ssd_selfdrive_step_host_async",
     "ssd_checkpoint_get_layout", "ssd_checkpoint_save", "ssd_checkpoint_load", "ssd_set_policy_output",
     "ssd_set_episode_log", "ssd_set_flat_policy_output", "ssd_set_feature_output",
+    "ssd_solver_enable", "ssd_solver_rows", "ssd_solver_resolve",
 ]
 
 _LIB = None
@@ -195,6 +202,9 @@ def load():
     L.ssd_set_flat_policy_output.argtypes = [vp, ctypes.POINTER(ssd_flat_policy_out)]
     L.ssd_set_feature_output.argtypes = [vp, ctypes.POINTER(ssd_feature_out)]
     L.ssd_solver_choose.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp]
+    L.ssd_solver_enable.argtypes = [vp, i32]
+    L.ssd_solver_rows.argtypes = [vp, ctypes.POINTER(ssd_solver_window), vp, vp]
+    L.ssd_solver_resolve.argtypes = [vp, ctypes.POINTER(ssd_solver_window), i32, vp, vp, vp, vp, vp]
     L.ssd_feature_dim.argtypes = [vp]
     L.ssd_state_bytes_per_env.argtypes = [vp]
     L.ssd_state_bytes_per_env.restype = i64

@@ -24,6 +24,7 @@
 #include "ssd_selfdrive.cuh"
 #include "ssd_features.cuh"
 #include "ssd_checkpoint.cuh"
+#include "ssd_solver.cuh"
 
 static thread_local char g_create_error[512] = "";
 
@@ -70,6 +71,12 @@ struct ssd_handle {
     ThetaRows theta_rows;    //   the rows that carry theta: a grid world's contract rows, flat rows under a contract
     int feat_form;           // ssd_set_feature_output (grid worlds, form 0): 1 + its dtype (SSD_FEATURE_F64 / SSD_POLICY_*), rows at
                              // pol_rows; 0: off
+    // ssd_solver_enable: the solver queue (ssd_solver.cuh)
+    bool solver_on;
+    uint32_t* d_resolved;    //   [E] episode whose contract the solver chose, SQ_NONE: none
+    uint32_t* d_sq_blocks;   //   [ceil(E / SQ_BLOCK)] pending envs per block of the scan
+    uint8_t* d_sq_ok;        //   checkpoint_load without row_ok_dev: the rows that loaded, [sq_ok_cap]
+    int sq_ok_cap;
     char err[512];
     std::vector<void*> dev_allocs;
 };
@@ -1642,6 +1649,133 @@ int ssd_solver_choose(ssd_handle* h, int32_t num_samples, int32_t rule, const do
     return check_launch(h, "solver_choose");
 }
 
+// ---- the solver queue of a vectorised sampler (ssd_solver.cuh) ----------------------------------------
+// the handle's part of a SolverQueue: where the pending test reads each env, the resolved episodes, the scan's scratch
+static SolverQueue solver_queue_params(ssd_handle* h)
+{
+    SolverQueue q;
+    memset(&q, 0, sizeof(q));
+    q.s = solver_params(h);
+    if (h->cfg.env_kind == SSD_ENV_SELFDRIVE) {
+        q.t = reinterpret_cast<const uint8_t*>(h->cp.t); q.t_stride = 4;
+        q.init = reinterpret_cast<const uint8_t*>(h->cp.meta); q.init_stride = 4;
+    } else if (IS_FEAT(h)) {
+        q.t = reinterpret_cast<const uint8_t*>(h->fp.rec + FR_T); q.t_stride = 4 * FR_WORDS;
+        q.init = reinterpret_cast<const uint8_t*>(h->fp.rec + FR_EPISODE); q.init_stride = 4 * FR_WORDS;
+    } else {
+        q.t = h->gp.state + RO_T; q.t_stride = h->gp.rec_stride;
+        q.init = h->gp.state + RO_FLAGS; q.init_stride = h->gp.rec_stride;
+    }
+    q.resolved = h->d_resolved;
+    q.block_count = h->d_sq_blocks;
+    return q;
+}
+
+// validates the window (before anything is launched) and fills the rest of the SolverQueue
+static int solver_window(ssd_handle* h, const ssd_solver_window* w, const char* what, SolverQueue* q)
+{
+    if (h->cfg.contract_kind == SSD_CONTRACT_NONE) return fail(h, SSD_EINVAL, "%s: the handle has no contract", what);
+    if (!h->solver_on) return fail(h, SSD_EINVAL, "%s: the solver queue is off (ssd_solver_enable)", what);
+    if (!w) return fail(h, SSD_EINVAL, "%s: window is NULL", what);
+    if (w->struct_size < (int32_t)sizeof(ssd_solver_window))
+        return fail(h, SSD_EINVAL, "ssd_solver_window.struct_size %d < %d: the caller's declaration of ssd_solver_window is out of date",
+                    w->struct_size, (int)sizeof(ssd_solver_window));
+    if (w->num_samples < 0) return fail(h, SSD_EINVAL, "%s: num_samples %d < 0", what, w->num_samples);
+    if (w->capacity < 1 || w->capacity > h->cfg.num_envs)
+        return fail(h, SSD_EINVAL, "%s: capacity %d is not in [1, %d]", what, w->capacity, h->cfg.num_envs);
+    if ((long long)w->capacity * (w->num_samples + 1) * h->cfg.num_agents > 0x7FFFFFFFll)
+        return fail(h, SSD_EINVAL, "%s: capacity * (1 + num_samples) * n too large", what);
+    const struct { const void* p; uintptr_t align; const char* name; } ptrs[] = {
+        { w->env_dev, 4, "env_dev" }, { w->episode_dev, 4, "episode_dev" }, { w->count_dev, 4, "count_dev" },
+        { w->params_dev, 8, "params_dev" } };
+    for (const auto& x : ptrs)
+        if (!x.p || (reinterpret_cast<uintptr_t>(x.p) & (x.align - 1)))
+            return fail(h, SSD_EINVAL, "%s: %s must be a %d-byte aligned device pointer", what, x.name, (int)x.align);
+    *q = solver_queue_params(h);
+    q->C = w->capacity; q->S = w->num_samples;
+    q->env = w->env_dev; q->episode = w->episode_dev; q->count = w->count_dev; q->params = w->params_dev;
+    return SSD_OK;
+}
+
+int ssd_solver_enable(ssd_handle* h, int32_t on)
+{
+    if (!h) return SSD_EINVAL;
+    ON_DEVICE(h);
+    if (h->cfg.contract_kind == SSD_CONTRACT_NONE) return fail(h, SSD_EINVAL, "solver_enable: the handle has no contract");
+    if (!on) { h->solver_on = false; return SSD_OK; }
+    const int E = h->cfg.num_envs;
+    int rc;
+    if (!h->d_resolved) {
+        if ((rc = dev_zalloc(h, (size_t)E, &h->d_resolved))) return rc;
+        if ((rc = dev_zalloc(h, (size_t)(E + SQ_BLOCK - 1) / SQ_BLOCK, &h->d_sq_blocks))) return rc;
+    }
+    CUDA_TRY(h, cudaMemset(h->d_resolved, 0xFF, (size_t)E * sizeof(uint32_t)));     // SQ_NONE
+    h->solver_on = true;
+    return SSD_OK;
+}
+
+int ssd_solver_rows(ssd_handle* h, const ssd_solver_window* win, const void* obs_dev, void* stream)
+{
+    if (!h) return SSD_EINVAL;
+    ON_DEVICE(h);
+    SolverQueue q;
+    int rc = solver_window(h, win, "solver_rows", &q);
+    if (rc) return rc;
+    if (!win->rows_dev || (reinterpret_cast<uintptr_t>(win->rows_dev) & 15))
+        return fail(h, SSD_EINVAL, "solver_rows: rows_dev must be a 16-byte aligned device pointer");
+    // the rows of the handle's observation form: layout, element type (SSD_POLICY_* or SSD_FEATURE_F64 = double), width
+    const bool grid = h->cfg.env_kind == SSD_ENV_CLEANUP || h->cfg.env_kind == SSD_ENV_HARVEST;
+    int layout = SQ_ROWS_FLAT, dtype, W, reps = 0, F = 0, src_width = 0;
+    const void* src = nullptr;
+    bool obs_required = false;
+    if (grid && !h->feat_form) {                            // image forms: the contract part alone
+        layout = SQ_ROWS_CONTRACT;
+        if (h->form) { dtype = h->form - 1; W = 10; reps = 5; }
+        else { dtype = SSD_FEATURE_F64; W = 2; reps = 1; }
+    } else {
+        F = ssd_feature_dim(h); W = F + 2;
+        if (grid) { dtype = h->feat_form - 1; src = h->pol_rows; src_width = dtype == SSD_FEATURE_F64 ? F : F + 2; }
+        else if (h->form) { dtype = h->form - 1; src = h->pol_rows; src_width = F + 2; }
+        else { dtype = SSD_FEATURE_F64; src = obs_dev; src_width = F; obs_required = true; }
+    }
+    if (obs_required && (!obs_dev || (reinterpret_cast<uintptr_t>(obs_dev) & 7)))
+        return fail(h, SSD_EINVAL, "solver_rows: obs_dev must be the float64 observation double [E][n][F] (8-byte aligned): the "
+                    "handle's observation is passed per call");
+    if (!obs_required && obs_dev)
+        return fail(h, SSD_EINVAL, "solver_rows: obs_dev must be NULL: the rows are built from the handle's own observation form");
+    cudaStream_t s = (cudaStream_t)stream;
+    const unsigned nb = (unsigned)((q.s.E + SQ_BLOCK - 1) / SQ_BLOCK);
+    solver_count_kernel<<<nb, SQ_BLOCK, 0, s>>>(q);
+    if ((rc = check_launch(h, "solver_rows"))) return rc;
+    solver_scatter_kernel<<<nb, SQ_BLOCK, 0, s>>>(q);
+    if ((rc = check_launch(h, "solver_rows"))) return rc;
+    if (dtype == SSD_FEATURE_F64) launch_solver_rows<double>(q, layout, win->rows_dev, W, reps, src, F, src_width, s);
+    else if (dtype == SSD_POLICY_F32) launch_solver_rows<float>(q, layout, win->rows_dev, W, reps, src, F, src_width, s);
+    else if (dtype == SSD_POLICY_F16) launch_solver_rows<__half>(q, layout, win->rows_dev, W, reps, src, F, src_width, s);
+    else launch_solver_rows<__nv_bfloat16>(q, layout, win->rows_dev, W, reps, src, F, src_width, s);
+    return check_launch(h, "solver_rows");
+}
+
+int ssd_solver_resolve(ssd_handle* h, const ssd_solver_window* win, int32_t rule, const double* vals_dev, double* best_param_dev,
+                       int32_t* best_index_dev, uint32_t* stale_dev, void* stream)
+{
+    if (!h) return SSD_EINVAL;
+    ON_DEVICE(h);
+    if (rule != SOLVER_RULE_MAX && rule != SOLVER_RULE_MAJORITY) return fail(h, SSD_EINVAL, "solver_resolve: unknown decision rule %d", rule);
+    SolverQueue q;
+    int rc = solver_window(h, win, "solver_resolve", &q);
+    if (rc) return rc;
+    if (!vals_dev || (reinterpret_cast<uintptr_t>(vals_dev) & 7))
+        return fail(h, SSD_EINVAL, "solver_resolve: vals_dev must be an 8-byte aligned device pointer");
+    if ((reinterpret_cast<uintptr_t>(best_param_dev) & 7) || (reinterpret_cast<uintptr_t>(best_index_dev) & 3) ||
+        (reinterpret_cast<uintptr_t>(stale_dev) & 3))
+        return fail(h, SSD_EINVAL, "solver_resolve: best_param_dev, best_index_dev and stale_dev must be aligned to their elements");
+    cudaStream_t s = (cudaStream_t)stream;
+    if (stale_dev) CUDA_TRY(h, cudaMemsetAsync(stale_dev, 0, sizeof(uint32_t), s));
+    solver_resolve_kernel<<<(q.C + 127) / 128, 128, 0, s>>>(q, rule, vals_dev, best_param_dev, best_index_dev, stale_dev);
+    return check_launch(h, "solver_resolve");
+}
+
 int ssd_get_state(ssd_handle* h, uint8_t* map_dev, int32_t* pos_dev, int32_t* ori_dev, int32_t* t_dev, double* theta_dev, void* stream)
 {
     if (!h) return SSD_EINVAL;
@@ -1873,12 +2007,25 @@ int ssd_checkpoint_load(ssd_handle* h, uint64_t config_tag, const int32_t* env_i
                     (unsigned long long)config_tag, (unsigned long long)h->config_tag);
     int rc = checkpoint_args(h, "checkpoint_load", env_idx_dev, count, rows_dev);
     if (rc || count == 0) return rc;
+    uint8_t* row_ok = row_ok_dev;
+    if (h->solver_on && !row_ok) {          // the solver queue needs to know which rows loaded
+        if (count > h->sq_ok_cap) {
+            if ((rc = dev_zalloc(h, (size_t)count, &h->d_sq_ok))) return rc;
+            h->sq_ok_cap = count;
+        }
+        row_ok = h->d_sq_ok;
+    }
     ck_load_kernel<<<(count + CK_ROWS - 1) / CK_ROWS, CK_THREADS, (size_t)CK_ROWS * h->ck.row_bytes, (cudaStream_t)stream>>>(
-        h->ck, env_idx_dev, count, rows_dev, row_ok_dev);
+        h->ck, env_idx_dev, count, rows_dev, row_ok);
     if ((rc = check_launch(h, "checkpoint_load"))) return rc;
-    if (!h->theta_rows.rows) return SSD_OK;
-    // theta came with the rows: the policy output's rows that carry it follow
-    theta_rows_refresh_kernel<<<(count + 127) / 128, 128, 0, (cudaStream_t)stream>>>(solver_params(h), env_idx_dev, count);
+    if (h->theta_rows.rows) {
+        // theta came with the rows: the policy output's rows that carry it follow
+        theta_rows_refresh_kernel<<<(count + 127) / 128, 128, 0, (cudaStream_t)stream>>>(solver_params(h), env_idx_dev, count);
+        if ((rc = check_launch(h, "checkpoint_load"))) return rc;
+    }
+    if (!h->solver_on) return SSD_OK;
+    // and so did the contract of their episode: the loaded envs are not pending
+    solver_mark_loaded_kernel<<<(count + 127) / 128, 128, 0, (cudaStream_t)stream>>>(solver_queue_params(h), env_idx_dev, count, row_ok);
     return check_launch(h, "checkpoint_load");
 }
 

@@ -167,29 +167,38 @@ struct SolverParams {
 #define SOLVER_RULE_MAX 0
 #define SOLVER_RULE_MAJORITY 1
 
+// candidate k of `env` in its episode `episode` (solver_sample_kernel, solver_rows_kernel)
+__device__ __forceinline__ double solver_candidate(const SolverParams& p, int env, uint32_t episode, int k)
+{
+    double v = p.low;
+    if (k > 0) {
+        const uint32_t u = draw_u32(p.seed, p.first_env_id + (uint32_t)env, episode, 0u, SITE_SOLVER, 0u, (uint32_t)(k - 1));
+        const double x = __dadd_rn(p.low, __dmul_rn(__dsub_rn(p.high, p.low), (double)u * 2.3283064365386963e-10));
+        v = (double)(float)x;                                       // .astype(np.float32)
+    }
+    return v;
+}
+
 __global__ void solver_sample_kernel(const SolverParams p, int S, double* __restrict__ params)
 {
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;          // one thread per (env, candidate)
     if (idx >= p.E * (S + 1)) return;
     const int env = idx / (S + 1), k = idx - env * (S + 1);
-    double v = p.low;
-    if (k > 0) {
-        const uint32_t episode = *reinterpret_cast<const uint32_t*>(p.episode + (size_t)env * p.episode_stride) & p.episode_mask;
-        const uint32_t u = draw_u32(p.seed, p.first_env_id + (uint32_t)env, episode, 0u, SITE_SOLVER, 0u, (uint32_t)(k - 1));
-        const double x = __dadd_rn(p.low, __dmul_rn(__dsub_rn(p.high, p.low), (double)u * 2.3283064365386963e-10));
-        v = (double)(float)x;                                       // .astype(np.float32)
-    }
-    params[idx] = v;
+    uint32_t episode = 0u;
+    if (k > 0) episode = *reinterpret_cast<const uint32_t*>(p.episode + (size_t)env * p.episode_stride) & p.episode_mask;
+    params[idx] = solver_candidate(p, env, episode, k);
 }
 
-__global__ void solver_choose_kernel(const SolverParams p, int S, int rule, const double* __restrict__ params,
-                                     const double* __restrict__ vals, double* __restrict__ best_param, int* __restrict__ best_idx)
+// compute_best_param for env `env`, whose values / candidates are row `slot` of vals [.][1 + S][n] / params [.][1 + S]: the
+// winner becomes the env's theta (and the policy output's rows that carry it follow) and best_param[slot] / best_idx[slot]
+// (nullable) receive it and its candidate index (solver_choose_kernel: slot = env; solver_resolve_kernel: the window slot)
+__device__ __forceinline__ void solver_choose_env(const SolverParams& p, int S, int rule, const double* __restrict__ params,
+                                                  const double* __restrict__ vals, double* __restrict__ best_param,
+                                                  int* __restrict__ best_idx, int env, int slot)
 {
-    const int env = blockIdx.x * blockDim.x + threadIdx.x;
-    if (env >= p.E) return;
     const int n = p.n;
-    const double* V = vals + (size_t)env * (S + 1) * n;
-    const double* P = params + (size_t)env * (S + 1);
+    const double* V = vals + (size_t)slot * (S + 1) * n;
+    const double* P = params + (size_t)slot * (S + 1);
     int best = 0;                       // the null contract is always a candidate
     double best_w = 0.0;
     for (int a = 0; a < n; a++) best_w = __dadd_rn(best_w, V[a]);
@@ -213,10 +222,18 @@ __global__ void solver_choose_kernel(const SolverParams p, int S, int rule, cons
         }
     }
     const double theta = P[src];
-    if (best_param) best_param[env] = theta;
-    if (best_idx) best_idx[env] = src;
+    if (best_param) best_param[slot] = theta;
+    if (best_idx) best_idx[slot] = src;
     *reinterpret_cast<double*>(p.theta + (size_t)env * p.theta_stride) = theta;
     theta_rows_env(p.rows, n, env, theta);
+}
+
+__global__ void solver_choose_kernel(const SolverParams p, int S, int rule, const double* __restrict__ params,
+                                     const double* __restrict__ vals, double* __restrict__ best_param, int* __restrict__ best_idx)
+{
+    const int env = blockIdx.x * blockDim.x + threadIdx.x;
+    if (env >= p.E) return;
+    solver_choose_env(p, S, rule, params, vals, best_param, best_idx, env, env);
 }
 
 // ---------------------------------------------------------------------------------------------

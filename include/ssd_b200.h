@@ -314,6 +314,48 @@ int ssd_solver_sample(ssd_handle* h, int32_t num_samples, double* params_dev, vo
 int ssd_solver_choose(ssd_handle* h, int32_t num_samples, int32_t rule, const double* params_dev, const double* vals_dev,
                       double* best_param_dev, int32_t* best_index_dev, void* stream);
 
+/* The solver inside a vectorised sampler, where every env is at its own point of its episode and only the envs that were
+ * just reset choose a contract.  An env is PENDING when it is at the start of an episode (reset, t == 0) whose contract the
+ * solver has not chosen yet.  Pending envs are taken in windows of at most `capacity` (C) envs in ascending env order:
+ *   ssd_solver_rows     finds the window, samples its candidates and writes the value-query rows;
+ *   (the caller)        runs its value function on all C x (1 + S) x n rows;
+ *   ssd_solver_resolve  applies compute_best_param (two_stage_train.py:748-776) to the window and clears it from pending.
+ * Each env ends with exactly what ssd_solver_sample + ssd_solver_choose give it on the same values.  Both calls are
+ * asynchronous, synchronise nothing and can be captured in a CUDA graph: (step with auto_reset, rows, value function,
+ * resolve) per step, with C >= the resets of a step; after a full reset, loop windows until pending (count_dev[1]) is 0.
+ * Pending status is read from t and the episode counter, which every reset writes: no step or reset kernel changes. */
+typedef struct ssd_solver_window {
+    int32_t struct_size;      /* sizeof(ssd_solver_window) (a smaller value is rejected) */
+    int32_t num_samples;      /* S >= 0 (contract_samples) */
+    int32_t capacity;         /* C in [1, E] */
+    int32_t* env_dev;         /* int32 [C]: the window's envs (local indices), -1 beyond the window */
+    uint32_t* episode_dev;    /* uint32 [C]: their episode counters when the rows were written */
+    uint32_t* count_dev;      /* uint32 [2]: envs in the window, pending envs in total (window included) */
+    double* params_dev;       /* double [C][1 + S]: the candidates of ssd_solver_sample, 0 beyond the window */
+    void* rows_dev;           /* [C][1 + S][n][W] value-query rows in the handle's observation form (below), 16-byte aligned */
+} ssd_solver_window;
+/* Every env kind with a contract.  on != 0 allocates the per-env record of resolved episodes and marks every env as
+ * having none; 0 switches the queue off.  An env that was never reset is never pending; ssd_checkpoint_load marks the
+ * envs it loads as resolved (their theta comes back with them). */
+int ssd_solver_enable(ssd_handle* h, int32_t on);
+/* Rows [C][1 + S][n][W] by the handle's observation form; row (c, k, a) is agent a of window env c with candidate k:
+ *   - flat forms (feature envs and selfdrive, grid worlds with ssd_set_feature_output), W = F + 2: obs[e][a] ++ [param, 0]
+ *       float64: what NegotiationSolver._obs_with builds (two_stage_train.py:316-325), obs = the float64 observation:
+ *                obs_dev double [E][n][F] for the feature envs and selfdrive, the handle's feature rows for the grid worlds;
+ *       policy dtype T: the handle's policy rows with the feature columns copied bit for bit, then T(float32(param)), 0;
+ *   - image forms (grid worlds): the contract part alone, the image being the same for every candidate:
+ *       uint8 windows: double (param, 0), W = 2;  policy image: T (param, 0) x 5, W = 10 (the contract rows).
+ * obs_dev is required for the float64 form of the feature envs and selfdrive (their observation is passed per call) and
+ * must be NULL otherwise.  Rows, candidates and env ids beyond the window count are zero / zero / -1. */
+int ssd_solver_rows(ssd_handle* h, const ssd_solver_window* win, const void* obs_dev, void* stream);
+/* vals_dev double [C][1 + S][n].  For each env of the window: the chosen parameter becomes its theta (and the policy
+ * output's rows that carry it follow), best_param_dev[c] / best_index_dev[c] (nullable, double [C] / int32 [C]) receive it
+ * and its candidate index, and its episode counts as resolved.  An env that was stepped or reset again since the rows
+ * call is left unchanged: best_index -1, best_param its current theta, and stale_dev (nullable, uint32 [1]) counts it.
+ * Slots beyond the window get best_index -1, best_param 0. */
+int ssd_solver_resolve(ssd_handle* h, const ssd_solver_window* win, int32_t rule, const double* vals_dev, double* best_param_dev,
+                       int32_t* best_index_dev, uint32_t* stale_dev, void* stream);
+
 /* --- state access (parity tests, checkpointing) ---------------------------------------------------- */
 /* map: uint8 chars [E][H][W] (MapEnv.world_map); pos: int32 [E][n][2] (row, col); ori: int32 [E][n]
  * (Agent.int_orientation); t: int32 [E] (MapEnv.timesteps); theta: double [E].  NULL pointers are skipped. */
@@ -466,7 +508,8 @@ int ssd_checkpoint_save(ssd_handle* h, const int32_t* env_idx_dev, int32_t count
  * #waste = popcount of the waste mask, 0 <= t <= horizon (grid worlds); list lengths <= point counts, entries < point
  * counts, each list setting exactly the bits of its presence mask (feature envs); n_crossed <= n, crossing-order entries
  * < n, no entries beyond n_crossed (selfdrive) — and, like a row whose index is outside [0, E), written only when it
- * passes: row_ok_dev[r] (uint8, nullable) = 1 if row r was loaded, else 0.  Duplicate destinations are the caller's error. */
+ * passes: row_ok_dev[r] (uint8, nullable) = 1 if row r was loaded, else 0.  Duplicate destinations are the caller's error.
+ * With the solver queue on (ssd_solver_enable), the loaded envs' episodes count as resolved: their theta came with them. */
 int ssd_checkpoint_load(ssd_handle* h, uint64_t config_tag, const int32_t* env_idx_dev, int32_t count, const uint8_t* rows_dev,
                         uint8_t* row_ok_dev, void* stream);
 
