@@ -562,6 +562,8 @@ static int setup_selfdrive(ssd_handle* h)
         CUDA_TRY(h, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
         CUDA_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)car_kernel_fn(false, OBS_F64), CAR_THREADS, (size_t)h->car_smem));
         h->grid_blocks = std::max(1, std::min((p.E + CAR_ENVS_PER_CTA - 1) / CAR_ENVS_PER_CTA, sms * std::max(per_sm, 1)));
+        if (getenv("SSD_DEBUG")) fprintf(stderr, "[ssd] selfdrive kernel: %d CTAs/SM, %d B smem/CTA, grid %d, %d envs/round\n",
+                                         per_sm, h->car_smem, h->grid_blocks, h->grid_blocks * CAR_ENVS_PER_CTA);
     }
     return SSD_OK;
 }
@@ -691,6 +693,8 @@ static int setup_features(ssd_handle* h)
                                                               (size_t)h->feat_smem));
         const int groups = (p.E + FEAT_ENVS_PER_CTA - 1) / FEAT_ENVS_PER_CTA;
         h->grid_blocks = std::max(1, std::min(groups, sms * std::max(per_sm, 1)));
+        if (getenv("SSD_DEBUG")) fprintf(stderr, "[ssd] feature kernel: %d CTAs/SM, %d B smem/CTA, grid %d, %d envs/round\n",
+                                         per_sm, h->feat_smem, h->grid_blocks, h->grid_blocks * FEAT_ENVS_PER_CTA);
     }
     return SSD_OK;
 }

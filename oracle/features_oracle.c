@@ -377,6 +377,20 @@ void feat_oracle_step(void* h, const int32_t* acts, double* obs, double* rew, do
         env_step(&b->envs[i], acts + (size_t)i * n, obs + (size_t)i * n * b->F, rew + (size_t)i * n, base_rew + (size_t)i * n,
                  transfers + (size_t)i * n, info + (size_t)i * n * 4, done + i);
 }
+/* feat_oracle_step with a per-env skip byte: an env with skip[i] != 0 is not stepped and its output rows are left as the
+   caller passed them (a batch's next-step auto-reset: reset the done envs with a mask, then step the others). */
+void feat_oracle_step_skip(void* h, const int32_t* acts, double* obs, double* rew, double* base_rew, double* transfers,
+                           int32_t* info, uint8_t* done, const uint8_t* skip)
+{
+    fbatch* b = (fbatch*)h;
+    int n = b->n;
+#pragma omp parallel for schedule(static) if (b->E > 1)
+    for (int i = 0; i < b->E; i++) {
+        if (skip && skip[i]) continue;
+        env_step(&b->envs[i], acts + (size_t)i * n, obs + (size_t)i * n * b->F, rew + (size_t)i * n, base_rew + (size_t)i * n,
+                 transfers + (size_t)i * n, info + (size_t)i * n * 4, done + i);
+    }
+}
 /* metrics [E][8 + 4*8]: dirt, raw, transfers, apples, low_density, 0, 0, 0, sum_raw[8], tsum_raw[8], sum_tr[8], tsum_tr[8] */
 void feat_oracle_get_metrics(void* h, double* out)
 {

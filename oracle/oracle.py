@@ -60,6 +60,7 @@ def lib():
         L.feat_oracle_dim.argtypes = [vp]
         L.feat_oracle_reset.argtypes = [vp] * 4
         L.feat_oracle_step.argtypes = [vp] * 8
+        L.feat_oracle_step_skip.argtypes = [vp] * 9
         L.feat_oracle_get_metrics.argtypes = [vp, vp]
         L.feat_oracle_get_state.argtypes = [vp] * 6
         L.car_oracle_create.restype = vp
@@ -68,6 +69,7 @@ def lib():
         L.car_oracle_obs_dim.argtypes = [vp]
         L.car_oracle_reset.argtypes = [vp] * 4
         L.car_oracle_step.argtypes = [vp] * 8
+        L.car_oracle_step_skip.argtypes = [vp] * 9
         L.car_oracle_get_state.argtypes = [vp] * 6
         L.car_oracle_set_theta.argtypes = [vp, vp]
         L.oracle_philox4x32_10.argtypes = [vp, vp, vp]
@@ -82,6 +84,13 @@ def set_num_threads(n):
 
 def _p(a):
     return None if a is None else a.ctypes.data_as(ctypes.c_void_p)
+
+
+def _skip_bytes(skip, E):
+    s = np.ascontiguousarray(skip, dtype=np.uint8).reshape(-1)
+    if s.shape[0] != E:
+        raise ValueError(f"skip has {s.shape[0]} entries for {E} envs")
+    return s
 
 
 def philox4x32_10(ctr, key):
@@ -271,13 +280,20 @@ class CarOracle:
         lib().car_oracle_reset(self._h, _p(m), _p(ep), _p(obs))
         return obs
 
-    def step(self, actions):
+    def step(self, actions, skip=None):
+        """Steps every env whose `skip` byte is zero (all of them without `skip`).  A skipped env keeps its state and its
+        output rows stay zero, so `reset(mask)` followed by `step(a, skip=mask)` is a batch's next-step auto-reset."""
         a = np.ascontiguousarray(actions, dtype=np.float32).reshape(self.E, self.n)
         E, n = self.E, self.n
         out = {"obs": np.zeros((E, n, self.D)), "rew": np.zeros((E, n)), "base_rew": np.zeros((E, n)),
                "transfers": np.zeros((E, n)), "info": np.zeros((E, n, 4)), "done": np.zeros((E, n + 1), np.uint8)}
-        lib().car_oracle_step(self._h, _p(a), _p(out["obs"]), _p(out["rew"]), _p(out["base_rew"]), _p(out["transfers"]),
-                              _p(out["info"]), _p(out["done"]))
+        args = (self._h, _p(a), _p(out["obs"]), _p(out["rew"]), _p(out["base_rew"]), _p(out["transfers"]),
+                _p(out["info"]), _p(out["done"]))
+        if skip is None:
+            lib().car_oracle_step(*args)
+        else:
+            sk = _skip_bytes(skip, E)
+            lib().car_oracle_step_skip(*args, _p(sk))
         return out
 
     def get_state(self):
@@ -328,13 +344,20 @@ class FeatOracle:
         lib().feat_oracle_reset(self._h, _p(m), _p(ep), _p(obs))
         return obs
 
-    def step(self, actions):
+    def step(self, actions, skip=None):
+        """Steps every env whose `skip` byte is zero (all of them without `skip`).  A skipped env keeps its state and its
+        output rows stay zero, so `reset(mask)` followed by `step(a, skip=mask)` is a batch's next-step auto-reset."""
         a = np.ascontiguousarray(actions, dtype=np.int32).reshape(self.E, self.n)
         E, n = self.E, self.n
         out = {"obs": np.zeros((E, n, self.F)), "rew": np.zeros((E, n)), "base_rew": np.zeros((E, n)),
                "transfers": np.zeros((E, n)), "info": np.zeros((E, n, 4), np.int32), "done": np.zeros(E, np.uint8)}
-        lib().feat_oracle_step(self._h, _p(a), _p(out["obs"]), _p(out["rew"]), _p(out["base_rew"]), _p(out["transfers"]),
-                               _p(out["info"]), _p(out["done"]))
+        args = (self._h, _p(a), _p(out["obs"]), _p(out["rew"]), _p(out["base_rew"]), _p(out["transfers"]),
+                _p(out["info"]), _p(out["done"]))
+        if skip is None:
+            lib().feat_oracle_step(*args)
+        else:
+            sk = _skip_bytes(skip, E)
+            lib().feat_oracle_step_skip(*args, _p(sk))
         return out
 
     def metrics_raw(self):

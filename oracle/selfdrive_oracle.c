@@ -250,6 +250,20 @@ void car_oracle_step(void* h, const float* acts, double* obs, double* rew, doubl
         env_step(&b->envs[i], acts + (size_t)i * n, obs + (size_t)i * n * D, rew + (size_t)i * n, base_rew + (size_t)i * n,
                  transfers + (size_t)i * n, info + (size_t)i * n * 4, done + (size_t)i * (n + 1));
 }
+/* car_oracle_step with a per-env skip byte: an env with skip[i] != 0 is not stepped and its output rows are left as the
+   caller passed them (a batch's next-step auto-reset: reset the done envs with a mask, then step the others). */
+void car_oracle_step_skip(void* h, const float* acts, double* obs, double* rew, double* base_rew, double* transfers,
+                          double* info, uint8_t* done, const uint8_t* skip)
+{
+    car_batch* b = (car_batch*)h;
+    int n = b->n, D = obs_dim(n);
+#pragma omp parallel for schedule(static) if (b->E > 1)
+    for (int i = 0; i < b->E; i++) {
+        if (skip && skip[i]) continue;
+        env_step(&b->envs[i], acts + (size_t)i * n, obs + (size_t)i * n * D, rew + (size_t)i * n, base_rew + (size_t)i * n,
+                 transfers + (size_t)i * n, info + (size_t)i * n * 4, done + (size_t)i * (n + 1));
+    }
+}
 /* state: pos [E][n], vel [E][n], theta [E], transfers metric [E], t [E] */
 void car_oracle_get_state(void* h, double* pos, double* vel, double* theta, double* m_transfers, int32_t* t)
 {

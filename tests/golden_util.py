@@ -211,6 +211,18 @@ def replay(backend, fx, check_features=True):
         check_episode_metrics(kind, n, bool(fx["contract"]), backend.metrics_raw(), want, "ep %d" % ep)
 
 
+def auto_reset_step(orc, actions, done_prev):
+    """One step of a batch with the next-step auto-reset, on a FeatOracle / CarOracle of all its envs: the envs that
+    finished in the previous step (done_prev, bool [E]) restart instead of stepping (reset observation, zero rewards,
+    transfers and infos, done cleared, their actions ignored); the others step.  Returns the step's outputs."""
+    done_prev = np.asarray(done_prev, dtype=bool)
+    restart = orc.reset(done_prev) if done_prev.any() else None
+    o = orc.step(actions, skip=done_prev)
+    if restart is not None:
+        o["obs"][done_prev] = restart[done_prev]
+    return o
+
+
 class OracleBackend:
     def __init__(self, oracle_mod, fx):
         self.o = oracle_mod.GridOracle(str(fx["kind"]), 1, int(fx["n"]), [str(r) for r in fx["ascii_map"]],
