@@ -73,8 +73,13 @@ class ssd_feature_out(ctypes.Structure):
     _fields_ = [("struct_size", ctypes.c_int32), ("dtype", ctypes.c_int32), ("obs_dev", ctypes.c_void_p)]
 
 
+class ssd_global_out(ctypes.Structure):
+    _fields_ = [("struct_size", ctypes.c_int32), ("dtype", ctypes.c_int32), ("obs_dev", ctypes.c_void_p)]
+
+
 POLICY_DTYPE = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}     # SSD_POLICY_F32 / _F16 / _BF16
 FEATURE_F64 = 3                                                           # SSD_FEATURE_F64 (ssd_set_feature_output)
+GLOBAL_U8 = 4                                                             # SSD_GLOBAL_U8 (ssd_set_global_output)
 
 
 def policy_dtype_code(dtype):
@@ -142,7 +147,7 @@ EXPORTS = [
     "ssd_step_host_async", "ssd_step_host_wait", "ssd_host_result_layout", "ssd_host_result_expand", "ssd_set_episode_stats",
     "ssd_feat_step_host_async", "ssd_selfdrive_step_host_async",
     "ssd_checkpoint_get_layout", "ssd_checkpoint_save", "ssd_checkpoint_load", "ssd_set_policy_output",
-    "ssd_set_episode_log", "ssd_set_flat_policy_output", "ssd_set_feature_output",
+    "ssd_set_episode_log", "ssd_set_flat_policy_output", "ssd_set_feature_output", "ssd_set_global_output",
     "ssd_solver_enable", "ssd_solver_rows", "ssd_solver_resolve",
 ]
 
@@ -201,6 +206,7 @@ def load():
     L.ssd_set_policy_output.argtypes = [vp, ctypes.POINTER(ssd_policy_out)]
     L.ssd_set_flat_policy_output.argtypes = [vp, ctypes.POINTER(ssd_flat_policy_out)]
     L.ssd_set_feature_output.argtypes = [vp, ctypes.POINTER(ssd_feature_out)]
+    L.ssd_set_global_output.argtypes = [vp, ctypes.POINTER(ssd_global_out)]
     L.ssd_solver_choose.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp]
     L.ssd_solver_enable.argtypes = [vp, i32]
     L.ssd_solver_rows.argtypes = [vp, ctypes.POINTER(ssd_solver_window), vp, vp]

@@ -142,15 +142,29 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
     T [E*n, policy_width] (features ++ [theta, 0] under a contract, policy_width = F + 2; the features alone without one)
     and `obs` None.  No uint8 windows are kept: step(want_features=True) and the methods that read windows raise
     ValueError.
+
+    global_obs=True: the observation is JointEnv's global view (global_obs=True of the reference, two_stage_train.py:572-617:
+    get_global_obs() = global_view() / 255, cleanup_new.py:299-300), written by the device at every step and reset
+    (ssd_set_global_output): `obs` uint8 [E, H, W, 3], what global_view() returns, or with policy_dtype T `policy_obs`
+    T [E, 3, H, W] = (u8 / 255).float().permute(0, 3, 1, 2).to(T) — VisionNetwork.forward's input — and `obs` None.  No
+    contract (JointEnv wraps the bare base env) and image_obs=True.  No uint8 windows are kept: step(want_features=True)
+    and the methods that read windows raise ValueError; global_view() and render() still work.
+    (The concatenated JointEnv variant needs no form of its own: `policy_image.view(E, 3 n, 15, 15)` of a policy_dtype env
+    without a contract is (concatenated_obs() / 255).float().permute(0, 3, 1, 2), the channel index 3 a + c being
+    agent-major.)
     """
 
     def __init__(self, kind, num_envs, num_agents, ascii_map=None, horizon=1000, contract=None,
                  theta_low=0.0, theta_high=None, null_prob=0.0, seed=73907, first_env_id=0,
                  device=None, padded_obs=False,
                  use_collective_reward=False, inequity_averse_reward=False, alpha=0.0, beta=0.0, policy_dtype=None,
-                 image_obs=True):
+                 image_obs=True, global_obs=False):
         if kind not in ("cleanup_new", "harvest_new"):
             raise ValueError("BatchedGridEnv kind must be cleanup_new or harvest_new, got %r" % (kind,))
+        if global_obs and not image_obs:
+            raise ValueError("global_obs=True observes the colour map: it does not go with image_obs=False")
+        if global_obs and contract is not None:
+            raise ValueError("global_obs=True is JointEnv's observation of the bare base env: no contract (got %r)" % (contract,))
         if not torch.cuda.is_available():
             raise _lib.SsdError("CUDA device required: contracts_b200 has no CPU fallback")
         self.lib = _lib.load()
@@ -187,8 +201,11 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
         E, n, dev = self.E, self.n, self.device
         self.policy_dtype, self.policy_image, self.policy_contract = policy_dtype, None, None
         self.image_obs, self.policy_obs, self.policy_width = bool(image_obs), None, None
+        self.global_obs = bool(global_obs)
         if not self.image_obs:
             self._init_feature_output(policy_dtype)
+        elif self.global_obs:
+            self._init_global_output(policy_dtype)
         elif policy_dtype is not None:
             try:
                 code = _lib.policy_dtype_code(policy_dtype)
@@ -249,33 +266,56 @@ class BatchedGridEnv(HostResultMixin, CheckpointMixin, EpisodeLogMixin):
         _lib.check(self._h, self.lib.ssd_set_feature_output(self._h, ctypes.byref(out)))
         self.obs_stride, self._obs_buf = 0, None
 
+    def _init_global_output(self, policy_dtype):
+        """global_obs=True: the handle writes the global view uint8 [E, H, W, 3] to `obs`, or T [E, 3, H, W] to `policy_obs`"""
+        try:
+            code = _lib.GLOBAL_U8 if policy_dtype is None else _lib.policy_dtype_code(policy_dtype)
+        except ValueError:
+            self.close()
+            raise
+        if policy_dtype is None:
+            self.obs = rows = torch.zeros((self.E, self.H, self.W, 3), dtype=torch.uint8, device=self.device)
+        else:
+            self.obs = None
+            self.policy_obs = rows = torch.zeros((self.E, 3, self.H, self.W), dtype=policy_dtype, device=self.device)
+        out = _lib.ssd_global_out(struct_size=ctypes.sizeof(_lib.ssd_global_out), dtype=code, obs_dev=rows.data_ptr())
+        _lib.check(self._h, self.lib.ssd_set_global_output(self._h, ctypes.byref(out)))
+        self.obs_stride, self._obs_buf = 0, None
+
     def _stream(self):
         return ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
     @property
     def observation(self):
         """what reset / step return: `obs`, or `policy_image` when the env writes the policy's tensors (`policy_obs` with
-        image_obs=False)"""
-        if not self.image_obs:
+        image_obs=False or global_obs=True)"""
+        if not self.image_obs or self.global_obs:
             return self.obs if self.policy_dtype is None else self.policy_obs
         return self.obs if self.policy_dtype is None else self.policy_image
 
     def _no_feature_copy(self, want_features):
         if want_features and not self.image_obs:
             raise ValueError("want_features: with image_obs=False the observation already is the feature rows (`obs` / policy_obs)")
+        if want_features and self.global_obs:
+            raise ValueError("want_features: a global_obs=True env writes the global view and no feature rows")
 
     def _need_windows(self, what):
         if not self.image_obs:
             raise ValueError("%s needs the uint8 observation windows; this env observes feature vectors (image_obs=False)" % what)
+        if self.global_obs:
+            raise ValueError("%s needs the uint8 observation windows; this env observes the global view (global_obs=True)" % what)
         if self.policy_dtype is not None:
             raise ValueError("%s needs the uint8 observation windows; this env writes the policy's tensors instead "
                              "(policy_dtype=%s)" % (what, self.policy_dtype))
 
     def _obs_rows(self):
         """the observation rows checkpoint / restore carry: uint8 [E, n, 15, 15, 3], or T [E, n, 3, 15, 15] in policy mode;
-        with image_obs=False float64 [E, n, F], or T [E, n, policy_width]"""
+        with image_obs=False float64 [E, n, F], or T [E, n, policy_width]; with global_obs=True uint8 [E, H, W, 3], or
+        T [E, 3, H, W]"""
         if not self.image_obs:
             return self.obs if self.policy_dtype is None else self.policy_obs.view(self.E, self.n, self.policy_width)
+        if self.global_obs:
+            return self.obs if self.policy_dtype is None else self.policy_obs
         return self.obs if self.policy_dtype is None else self.policy_image.view(self.E, self.n, 3, 15, 15)
 
     def reset(self, mask=None):

@@ -29,8 +29,9 @@ class EnvCheckpoint:
     were saved under (ssd_checkpoint_layout); seed: the handle's seed; env_ids int64 [count]; rows uint8 [count,
     row_bytes]; obs: the observation rows of those envs or None (uint8 [count, n, 15, 15, 3] for the grid worlds, T
     [count, n, 3, 15, 15] for a grid world with policy_dtype T, float64 [count, n, F | D] for the feature envs,
-    selfdrive and a grid world with image_obs=False, T [count, n, policy_width] for those with policy_dtype T).  The rows themselves do not depend on the
-    observation form."""
+    selfdrive and a grid world with image_obs=False, T [count, n, policy_width] for those with policy_dtype T; uint8
+    [count, H, W, 3] for a grid world with global_obs=True, T [count, 3, H, W] with policy_dtype T too).  The rows
+    themselves do not depend on the observation form."""
 
     def __init__(self, kind, config_tag, row_bytes, seed, env_ids, rows, obs=None):
         self.kind, self.config_tag, self.row_bytes, self.seed = str(kind), int(config_tag), int(row_bytes), int(seed)

@@ -69,8 +69,10 @@ struct ssd_handle {
     int form;                // 0: the native form (OBS_U8 / OBS_F64); else 1 + SSD_POLICY_*
     void* pol_rows;          //   the policy image T [E n][3][15][15] (grid worlds) or the flat rows T [E n][W]
     ThetaRows theta_rows;    //   the rows that carry theta: a grid world's contract rows, flat rows under a contract
-    int feat_form;           // ssd_set_feature_output (grid worlds, form 0): 1 + its dtype (SSD_FEATURE_F64 / SSD_POLICY_*), rows at
-                             // pol_rows; 0: off
+    // ssd_set_feature_output / ssd_set_global_output (grid worlds, form 0): the kernels that replace the observe kernel and
+    // write the reset envs' rows, rows at pol_rows
+    int alt_form;            //   0: off; ALT_FEATURES, ALT_GLOBAL
+    int alt_dtype;           //   the rows' element type: SSD_FEATURE_F64 / SSD_GLOBAL_U8 (the form's own) or SSD_POLICY_*
     // ssd_solver_enable: the solver queue (ssd_solver.cuh)
     bool solver_on;
     uint32_t* d_resolved;    //   [E] episode whose contract the solver chose, SQ_NONE: none
@@ -116,32 +118,49 @@ static reset_kernel_t reset_kernel_fn(int kind, int form)
         return kind == SSD_ENV_CLEANUP ? grid_reset_kernel<SSD_ENV_CLEANUP, FORM> : grid_reset_kernel<SSD_ENV_HARVEST, FORM>;
     });
 }
-// f(std::integral_constant<int, OUT>()) for the dtype of ssd_set_feature_output (SSD_FEATURE_F64 or SSD_POLICY_*)
-template <typename F>
-static auto by_feature_dtype(int dtype, F f)
+// the observation forms that replace the observe kernel (ssd_handle::alt_form)
+#define ALT_FEATURES 1           // ssd_set_feature_output: grid_feature_kernel / grid_reset_features_kernel
+#define ALT_GLOBAL 2             // ssd_set_global_output: grid_global_kernel / grid_reset_global_kernel
+// f(std::integral_constant<int, OUT>()) for the dtype of such a form: SSD_POLICY_*, else the form's own NATIVE dtype
+// (SSD_FEATURE_F64 / SSD_GLOBAL_U8)
+template <int NATIVE, typename F>
+static auto by_out_dtype(int dtype, F f)
 {
     if (dtype == SSD_POLICY_F32) return f(std::integral_constant<int, SSD_POLICY_F32>());
     if (dtype == SSD_POLICY_F16) return f(std::integral_constant<int, SSD_POLICY_F16>());
     if (dtype == SSD_POLICY_BF16) return f(std::integral_constant<int, SSD_POLICY_BF16>());
-    return f(std::integral_constant<int, SSD_FEATURE_F64>());
+    return f(std::integral_constant<int, NATIVE>());
 }
-typedef void (*feature_kernel_t)(const GridParams, uint32_t*, void*, int);
-static feature_kernel_t feature_kernel_fn(int kind, bool rounds4, int dtype)
+typedef void (*alt_kernel_t)(const GridParams, uint32_t*, void*, int);
+static alt_kernel_t alt_kernel_fn(int kind, bool rounds4, int alt, int dtype)
 {
-    return by_feature_dtype(dtype, [&](auto O) -> feature_kernel_t {
+    if (alt == ALT_GLOBAL)
+        return by_out_dtype<SSD_GLOBAL_U8>(dtype, [&](auto O) -> alt_kernel_t {
+            constexpr int OUT = decltype(O)::value;
+            if (kind == SSD_ENV_CLEANUP) return rounds4 ? grid_global_kernel<SSD_ENV_CLEANUP, 4, OUT> : grid_global_kernel<SSD_ENV_CLEANUP, MAX_POINT_ROUNDS, OUT>;
+            return rounds4 ? grid_global_kernel<SSD_ENV_HARVEST, 4, OUT> : grid_global_kernel<SSD_ENV_HARVEST, MAX_POINT_ROUNDS, OUT>;
+        });
+    return by_out_dtype<SSD_FEATURE_F64>(dtype, [&](auto O) -> alt_kernel_t {
         constexpr int OUT = decltype(O)::value;
         if (kind == SSD_ENV_CLEANUP) return rounds4 ? grid_feature_kernel<SSD_ENV_CLEANUP, 4, OUT> : grid_feature_kernel<SSD_ENV_CLEANUP, MAX_POINT_ROUNDS, OUT>;
         return rounds4 ? grid_feature_kernel<SSD_ENV_HARVEST, 4, OUT> : grid_feature_kernel<SSD_ENV_HARVEST, MAX_POINT_ROUNDS, OUT>;
     });
 }
-typedef void (*reset_features_kernel_t)(const GridParams, const uint8_t*, void*, int);
-static reset_features_kernel_t reset_features_kernel_fn(int kind, int dtype)
+typedef void (*alt_reset_kernel_t)(const GridParams, const uint8_t*, void*, int);
+static alt_reset_kernel_t alt_reset_kernel_fn(int kind, int alt, int dtype)
 {
-    return by_feature_dtype(dtype, [&](auto O) -> reset_features_kernel_t {
+    if (alt == ALT_GLOBAL)
+        return by_out_dtype<SSD_GLOBAL_U8>(dtype, [&](auto O) -> alt_reset_kernel_t {
+            constexpr int OUT = decltype(O)::value;
+            return kind == SSD_ENV_CLEANUP ? grid_reset_global_kernel<SSD_ENV_CLEANUP, OUT> : grid_reset_global_kernel<SSD_ENV_HARVEST, OUT>;
+        });
+    return by_out_dtype<SSD_FEATURE_F64>(dtype, [&](auto O) -> alt_reset_kernel_t {
         constexpr int OUT = decltype(O)::value;
         return kind == SSD_ENV_CLEANUP ? grid_reset_features_kernel<SSD_ENV_CLEANUP, OUT> : grid_reset_features_kernel<SSD_ENV_HARVEST, OUT>;
     });
 }
+// dynamic shared memory of the reset-row kernel of form `alt`: grid_reset_global_kernel holds one map per warp
+static int alt_reset_smem(const GridParams& p, int alt) { return alt == ALT_GLOBAL ? GRID_WARPS * p.map_bytes : 0; }
 typedef void (*feat_kernel_t)(const FeatParams, const FeatIO, const uint8_t*);
 // form: OBS_F64 or the flat policy form of ssd_set_flat_policy_output (1 + SSD_POLICY_*)
 static feat_kernel_t feat_kernel_fn(bool cleanup, bool reset_only, int form)
@@ -299,8 +318,9 @@ static int dev_zalloc(ssd_handle* h, size_t count, T** out)
 }
 
 // the dynamic shared-memory limit of every kernel of the handle's step and reset in observation form `form` (0 at create,
-// the policy form when an output is set)
-static int set_form_smem(ssd_handle* h, int form)
+// the policy form when an output is set), or, for a grid world, of the kernels of form `alt` (ALT_* with element type
+// alt_dtype) that replace the observe kernel (grid_reset_kernel<KIND, 0> keeps its limit from create)
+static int set_form_smem(ssd_handle* h, int form, int alt = 0, int alt_dtype = 0)
 {
     const int kind = h->cfg.env_kind;
     if (kind == SSD_ENV_SELFDRIVE) {
@@ -310,6 +330,11 @@ static int set_form_smem(ssd_handle* h, int form)
         for (int q = 0; q < 2; q++)
             CUDA_TRY(h, cudaFuncSetAttribute((const void*)feat_kernel_fn(kind == SSD_ENV_CLEANUP_FEATURES, q != 0, form),
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, h->feat_smem));
+    } else if (alt) {
+        CUDA_TRY(h, cudaFuncSetAttribute((const void*)alt_kernel_fn(kind, h->rounds4, alt, alt_dtype),
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, h->gp.g2_smem_bytes));
+        CUDA_TRY(h, cudaFuncSetAttribute((const void*)alt_reset_kernel_fn(kind, alt, alt_dtype),
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, alt_reset_smem(h->gp, alt)));
     } else {
         const int smem = h->gp.g2_smem_bytes;
         CUDA_TRY(h, cudaFuncSetAttribute((const void*)reset_kernel_fn(kind, form), cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
@@ -935,25 +960,30 @@ static int check_policy_out(ssd_handle* h, const Out* out, const char* type, con
         return fail(h, SSD_EINVAL, "%s: %s must be a 16-byte aligned device pointer", what, ptr_name);
     return SSD_OK;
 }
-// the handle's observation form and what it writes; form 0 (the native form) clears the policy output
-static int set_form(ssd_handle* h, int form, void* pol_rows, ThetaRows theta_rows)
+// the handle's observation form and what it writes: every setter replaces all of it.  form 0 (the native form) with alt 0
+// clears the output; alt (ALT_*, element type alt_dtype; form 0) selects the kernels that replace the observe kernel
+static int set_form(ssd_handle* h, int form, void* pol_rows, ThetaRows theta_rows, int alt = 0, int alt_dtype = 0)
 {
-    if (form) { int rc = set_form_smem(h, form); if (rc) return rc; }
+    if (form || alt) { int rc = set_form_smem(h, form, alt, alt_dtype); if (rc) return rc; }
     h->form = form;
-    h->feat_form = 0;
+    h->alt_form = alt;
+    h->alt_dtype = alt_dtype;
     h->pol_rows = pol_rows;
     h->theta_rows = theta_rows;
     return SSD_OK;
 }
-// elements per row of the feature output: F, + [theta, 0] for the policy dtypes under a contract
-static int feature_width(const ssd_handle* h)
+// the width argument of the alt kernels: elements per row of the feature output (F, + [theta, 0] for the policy dtypes
+// under a contract); 0 for the global view
+static int alt_width(const ssd_handle* h)
 {
-    return h->gp.F + (h->feat_form != 1 + SSD_FEATURE_F64 && h->cfg.contract_kind != SSD_CONTRACT_NONE ? 2 : 0);
+    if (h->alt_form != ALT_FEATURES) return 0;
+    return h->gp.F + (h->alt_dtype != SSD_FEATURE_F64 && h->cfg.contract_kind != SSD_CONTRACT_NONE ? 2 : 0);
 }
-// the feature output's reset rows of the envs `mask` selects (all when NULL), behind the reset kernel on stream s
-static void launch_reset_features(ssd_handle* h, const uint8_t* mask, cudaStream_t s)
+// the alt form's reset rows of the envs `mask` selects (all when NULL), behind the reset kernel on stream s
+static void launch_reset_alt(ssd_handle* h, const uint8_t* mask, cudaStream_t s)
 {
-    reset_features_kernel_fn(h->gp.kind, h->feat_form - 1)<<<h->grid_blocks, GRID_THREADS, 0, s>>>(h->gp, mask, h->pol_rows, feature_width(h));
+    alt_reset_kernel_fn(h->gp.kind, h->alt_form, h->alt_dtype)<<<h->grid_blocks, GRID_THREADS, alt_reset_smem(h->gp, h->alt_form), s>>>(
+        h->gp, mask, h->pol_rows, alt_width(h));
 }
 
 // =============================================================================================
@@ -1082,13 +1112,14 @@ int ssd_reset(ssd_handle* h, const uint8_t* mask_dev, uint8_t* obs_dev, int64_t 
     REQUIRE_GRID(h);
     const GridParams& p = h->gp;
     cudaStream_t s = (cudaStream_t)stream;
-    if (h->feat_form) {                                  // one observation form per handle: the feature rows, no windows
-        if (obs_dev) return fail(h, SSD_EINVAL, "reset: obs_dev must be NULL while a feature output is set (ssd_set_feature_output)");
+    if (h->alt_form) {                                   // one observation form per handle: the feature rows / global view, no windows
+        if (obs_dev) return fail(h, SSD_EINVAL, "reset: obs_dev must be NULL while a feature or global output is set "
+                                                "(ssd_set_feature_output / ssd_set_global_output)");
         if (p.beam) beam_clear_kernel<<<(p.E + 3) / 4, 128, 0, s>>>(p, mask_dev);
         reset_kernel_fn(p.kind, OBS_U8)<<<h->grid_blocks, GRID_THREADS, p.g2_smem_bytes, s>>>(p, mask_dev, nullptr, 0, StepIO(), nullptr);
         int rc = check_launch(h, "reset");
         if (rc) return rc;
-        launch_reset_features(h, mask_dev, s);
+        launch_reset_alt(h, mask_dev, s);
         return check_launch(h, "reset");
     }
     long long stride = obs_env_stride ? obs_env_stride : (long long)p.n * SSD_OBS_BYTES;
@@ -1113,9 +1144,10 @@ static int make_step_io(ssd_handle* h, const ssd_step_io* io, StepIO& k, bool as
         if (io->obs_dev) return fail(h, SSD_EINVAL, "obs_dev must be NULL while a policy output is set (ssd_set_policy_output)");
         k.obs = (uint8_t*)h->pol_rows;
         k.obs_stride = policy_env_bytes(p, h->form);
-    } else if (h->feat_form) {                           // the feature rows are the observation: no windows, no second copy
+    } else if (h->alt_form) {                            // the feature rows / global view are the observation: no windows, no copy
         if (io->obs_dev || io->feature_obs_dev)
-            return fail(h, SSD_EINVAL, "obs_dev and feature_obs_dev must be NULL while a feature output is set (ssd_set_feature_output)");
+            return fail(h, SSD_EINVAL, "obs_dev and feature_obs_dev must be NULL while a feature or global output is set "
+                                       "(ssd_set_feature_output / ssd_set_global_output)");
     } else {
         if (!io->obs_dev) return fail(h, SSD_EINVAL, "obs_dev is required");
         k.obs = io->obs_dev;
@@ -1192,9 +1224,9 @@ static int launch_step(ssd_handle* h, const StepIO& k, cudaStream_t s, const Hos
     if (hc && hc->slot >= 0) CUDA_TRY(h, cudaEventRecord(h->slot[hc->slot].ev_logic, s));   // the slot's actions were read
     if (p.kind == SSD_ENV_CLEANUP) { int rc = copy_rewards(h, k, s, hc); if (rc) return rc; }
     // programmatic dependent launch: the observe CTAs become resident (tables, tiles) as the one-wave logic grid drains
-    if (h->feat_form) {          // the feature form: spawn + feature rows in place of the observe kernel
-        const feature_kernel_t fk = feature_kernel_fn(p.kind, h->rounds4, h->feat_form - 1);
-        const int width = feature_width(h);
+    if (h->alt_form) {           // the feature / global form: spawn + its rows in place of the observe kernel
+        const alt_kernel_t fk = alt_kernel_fn(p.kind, h->rounds4, h->alt_form, h->alt_dtype);
+        const int width = alt_width(h);
         if (h->pdl && !h->timing)
             CUDA_TRY(h, launch_pdl(fk, dim3(h->obs_blocks), dim3(OBS_WARPS * 32), (size_t)p.g2_smem_bytes, s, p, h->d_res, h->pol_rows, width));
         else fk<<<h->obs_blocks, OBS_WARPS * 32, p.g2_smem_bytes, s>>>(p, h->d_res, h->pol_rows, width);
@@ -1220,9 +1252,9 @@ static int launch_step(ssd_handle* h, const StepIO& k, cudaStream_t s, const Hos
             CUDA_TRY(h, launch_pdl(reset_k, dim3(h->grid_blocks), dim3(GRID_THREADS), (size_t)p.g2_smem_bytes, s,
                                    p, (const uint8_t*)k.done, k.obs, k.obs_stride, k, h->theta_rows.rows));
         else reset_k<<<h->grid_blocks, GRID_THREADS, p.g2_smem_bytes, s>>>(p, k.done, k.obs, k.obs_stride, k, h->theta_rows.rows);
-        if (h->feat_form) {      // (k.obs is NULL: the reset kernel wrote no windows) the new episodes' reset rows
+        if (h->alt_form) {       // (k.obs is NULL: the reset kernel wrote no windows) the new episodes' reset rows
             h->launches++;
-            launch_reset_features(h, k.done, s);
+            launch_reset_alt(h, k.done, s);
         }
     }
     if (h->timing) cudaEventRecord(h->tev[2], s);
@@ -1582,14 +1614,28 @@ int ssd_set_feature_output(ssd_handle* h, const ssd_feature_out* out)
         return fail(h, SSD_EINVAL, "set_feature_output: dtype %d is not SSD_FEATURE_F64, SSD_POLICY_F32, _F16 or _BF16", out->dtype);
     if (!out->obs_dev || (reinterpret_cast<uintptr_t>(out->obs_dev) & 15))
         return fail(h, SSD_EINVAL, "set_feature_output: obs_dev must be a 16-byte aligned device pointer");
-    CUDA_TRY(h, cudaFuncSetAttribute((const void*)feature_kernel_fn(h->cfg.env_kind, h->rounds4, out->dtype),
-                                     cudaFuncAttributeMaxDynamicSharedMemorySize, h->gp.g2_smem_bytes));
     const bool theta_col = out->dtype != SSD_FEATURE_F64 && h->cfg.contract_kind != SSD_CONTRACT_NONE;
     const int width = h->gp.F + (theta_col ? 2 : 0);
-    int rc = set_form(h, 0, out->obs_dev, ThetaRows{ theta_col ? out->obs_dev : nullptr, out->dtype, width, width - 2, 1 });
-    if (rc) return rc;
-    h->feat_form = 1 + out->dtype;
-    return SSD_OK;
+    return set_form(h, 0, out->obs_dev, ThetaRows{ theta_col ? out->obs_dev : nullptr, out->dtype, width, width - 2, 1 },
+                    ALT_FEATURES, out->dtype);
+}
+
+int ssd_set_global_output(ssd_handle* h, const ssd_global_out* out)
+{
+    if (!h) return SSD_EINVAL;
+    ON_DEVICE(h);
+    REQUIRE_GRID(h);
+    if (!out) return set_form(h, 0, nullptr, ThetaRows{});
+    if (out->struct_size < (int32_t)sizeof(ssd_global_out))
+        return fail(h, SSD_EINVAL, "ssd_global_out.struct_size %d < %d: the caller's declaration of ssd_global_out is out of date",
+                    out->struct_size, (int)sizeof(ssd_global_out));
+    if (out->dtype != SSD_GLOBAL_U8 && out->dtype != SSD_POLICY_F32 && out->dtype != SSD_POLICY_F16 && out->dtype != SSD_POLICY_BF16)
+        return fail(h, SSD_EINVAL, "set_global_output: dtype %d is not SSD_GLOBAL_U8, SSD_POLICY_F32, _F16 or _BF16", out->dtype);
+    if (!out->obs_dev || (reinterpret_cast<uintptr_t>(out->obs_dev) & 15))
+        return fail(h, SSD_EINVAL, "set_global_output: obs_dev must be a 16-byte aligned device pointer");
+    if (h->cfg.contract_kind != SSD_CONTRACT_NONE)
+        return fail(h, SSD_EINVAL, "set_global_output: the handle has a contract (JointEnv's global observation is of the bare base env)");
+    return set_form(h, 0, out->obs_dev, ThetaRows{}, ALT_GLOBAL, out->dtype);
 }
 
 int ssd_set_flat_policy_output(ssd_handle* h, const ssd_flat_policy_out* out)
@@ -1732,13 +1778,13 @@ int ssd_solver_rows(ssd_handle* h, const ssd_solver_window* win, const void* obs
     int layout = SQ_ROWS_FLAT, dtype, W, reps = 0, F = 0, src_width = 0;
     const void* src = nullptr;
     bool obs_required = false;
-    if (grid && !h->feat_form) {                            // image forms: the contract part alone
+    if (grid && h->alt_form != ALT_FEATURES) {              // image forms: the contract part alone
         layout = SQ_ROWS_CONTRACT;
         if (h->form) { dtype = h->form - 1; W = 10; reps = 5; }
         else { dtype = SSD_FEATURE_F64; W = 2; reps = 1; }
     } else {
         F = ssd_feature_dim(h); W = F + 2;
-        if (grid) { dtype = h->feat_form - 1; src = h->pol_rows; src_width = dtype == SSD_FEATURE_F64 ? F : F + 2; }
+        if (grid) { dtype = h->alt_dtype; src = h->pol_rows; src_width = dtype == SSD_FEATURE_F64 ? F : F + 2; }
         else if (h->form) { dtype = h->form - 1; src = h->pol_rows; src_width = F + 2; }
         else { dtype = SSD_FEATURE_F64; src = obs_dev; src_width = F; obs_required = true; }
     }

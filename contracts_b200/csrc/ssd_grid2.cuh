@@ -932,3 +932,178 @@ __global__ void __launch_bounds__(GRID_THREADS) grid_reset_features_kernel(const
         }
     }
 }
+
+// =============================================================================================
+// GLOBAL FORM (ssd_set_global_output): the observation is JointEnv's global view, MapEnv.global_view() (map_env.py:394-395;
+// global_view_kernel's output), written in output form OUT: SSD_GLOBAL_U8 (uint8 [E][H][W][3]) or SSD_POLICY_* (T
+// [E][3][H][W], T(float32(u8 / 255.0)): get_global_obs() as VisionNetwork.forward feeds it).  No observation windows are built.
+template <int OUT> struct GlobalElem : PolicyElem<1 + OUT> {};
+template <> struct GlobalElem<SSD_GLOBAL_U8> { typedef uint8_t T; };
+
+// One env's view from a map of cell codes (cell (r, c) at m[r * stride + c]; an agent painted as PAINT_CODE; OCC_BIT ignored)
+// to `dst`, the env's block.  inv_w = 1.0f / W: (cell + 0.5) * inv_w stays within 4e-4 of the exact quotient for the
+// cells of a 48 x 64 map, so its truncation is cell / W.  Stores are coalesced:
+//   uint8: the 3 H W bytes as aligned words (lane = word; a word spans two cells: its four bytes are picked from their
+//          colours with one byte permute), the unaligned head and tail as bytes — a block starts on any byte;
+//   T:     three planes of H W elements, lane = cell, the palette's T entries (load_policy_palette) per channel.
+template <int OUT>
+__device__ __forceinline__ void write_global_view(const GridParams& p, int lane, const uint8_t* m, int stride, float inv_w,
+                                                  const uint32_t* pal, void* dst)
+{
+    typedef typename GlobalElem<OUT>::T T;
+    const int W = p.W, HW = p.H * p.W;
+    auto cell_off = [&](int cell, int& c) -> int {
+        const int r = __float2int_rz(__fmul_rn(__int2float_rn(cell) + 0.5f, inv_w));
+        c = cell - r * W;
+        return r * stride + c;
+    };
+    if constexpr (OUT == SSD_GLOBAL_U8) {
+        const uint8_t* pb = reinterpret_cast<const uint8_t*>(pal);     // a code is the byte offset of its palette entry
+        uint8_t* g = reinterpret_cast<uint8_t*>(dst);
+        const int L = 3 * HW;
+        const int head = min((int)((0u - (uint32_t)reinterpret_cast<uintptr_t>(g)) & 3u), L);
+        const int nw = (L - head) >> 2, tail0 = head + 4 * nw;
+        auto byte_at = [&](int b) -> uint8_t {
+            const int cell = (int)(((uint32_t)b * 0xAAABu) >> 17), ch = b - 3 * cell;     // b / 3 for b < 2^17
+            int c;
+            return pb[(m[cell_off(cell, c)] & CODE_MASK) + ch];
+        };
+        if (lane < head) g[lane] = byte_at(lane);
+        if (lane < L - tail0) g[tail0 + lane] = byte_at(tail0 + lane);
+        uint32_t* gw = reinterpret_cast<uint32_t*>(g + head);
+        for (int w = lane; w < nw; w += 32) {
+            const int b0 = head + 4 * w;
+            const int cell = (int)(((uint32_t)b0 * 0xAAABu) >> 17), ch = b0 - 3 * cell;
+            int c;
+            const int o0 = cell_off(cell, c), o1 = c + 1 < W ? o0 + 1 : o0 - c + stride;   // the next cell (next row's first)
+            const uint32_t c0 = pal[(m[o0] & CODE_MASK) >> 2], c1 = pal[(m[o1] & CODE_MASK) >> 2];
+            gw[w] = __byte_perm(c0 | (c1 << 24), c1 >> 8, 0x3210u + 0x1111u * (uint32_t)ch);    // bytes ch .. ch + 3 of c0 ++ c1
+        }
+    } else {
+        const T* ppal = policy_palette<T>();
+        T* o = reinterpret_cast<T*>(dst);
+        for (int cell = lane; cell < HW; cell += 32) {
+            int c;
+            const int code = m[cell_off(cell, c)] & CODE_MASK;
+            o[cell] = ppal[code]; o[HW + cell] = ppal[code + 1]; o[2 * HW + cell] = ppal[code + 2];
+        }
+    }
+}
+
+// STEP, in place of the observe kernel behind the logic kernel: one warp per env, grid-stride.  grid_feature_kernel's env
+// work — the env's tile T from the masks, the same spawn on the same draws (masks and #waste written back when it changes
+// them), harvest's total_close_apples into res_g for grid_reward_kernel — then the agents painted into T in agent order
+// (the highest index wins a shared cell; t > 0 after a step, so they always show) and the view written from T's map rows.
+// Shared memory: the observe kernel's layout (T2 unused).  `width` is unused (grid_feature_kernel's signature).
+template <int KIND, int MW, int OUT>
+__global__ void __launch_bounds__(OBS_WARPS * 32) grid_global_kernel(const GridParams p, uint32_t* __restrict__ res_g, void* out, int width)
+{
+    typedef typename GlobalElem<OUT>::T T;
+    extern __shared__ __align__(16) uint8_t smem[];
+    const SharedTables tb = load_shared_tables(p, smem, false);
+    if constexpr (OUT != SSD_GLOBAL_U8) load_policy_palette<T>(p);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    uint8_t* tile = smem + p.sm_warp0 + warp * p.g2_warp_bytes;
+    uint32_t* scratch = reinterpret_cast<uint32_t*>(tile + p.g2_stage);
+    const PointRegs<MW> pr = load_point_regs<MW>(p, lane);
+    init_warp_tiles(p, tile, lane);
+    __syncthreads();                                  // tables visible
+    const int n = p.n, S = p.S;
+    const bool act_lane = lane < n;
+    const uint32_t rot3 = (uint32_t)(lane - 3) & 31u, rot2 = (uint32_t)(lane - 2) & 31u;
+    const float inv_w = __frcp_rn((float)p.W);
+    const size_t env_elems = (size_t)3 * p.H * p.W;
+    pdl_launch_dependents();                          // the reward / masked reset kernel behind the step may set up early
+    pdl_wait();                                       // the hot lines and res_g are the logic kernel's output
+    for (int env = blockIdx.x * OBS_WARPS + warp; env < p.E; env += gridDim.x * OBS_WARPS) {
+        uint32_t* hot = reinterpret_cast<uint32_t*>(p.state + (size_t)env * p.rec_stride);
+        const uint32_t hw = hot[lane];
+        uint32_t am[MW], wm[MW];
+#pragma unroll
+        for (int q = 0; q < MW; q++) {
+            am[q] = __shfl_sync(FULL, hw, RO_AMASK / 4 + q);
+            wm[q] = KIND == SSD_ENV_CLEANUP ? __shfl_sync(FULL, hw, RO_WMASK / 4 + q) : 0u;
+        }
+        apply_masks<MW, false>(p, tile, pr, am, wm, rot3, rot2);
+        const uint32_t t = __shfl_sync(FULL, hw, RO_T / 4);               // already incremented by the logic kernel
+        const uint32_t episode = __shfl_sync(FULL, hw, RO_EPISODE / 4);
+        int hcount = (int)__shfl_sync(FULL, hw, RO_HCOUNT / 4);
+        const EnvRng g = { p.seed, p.first_env_id + (uint32_t)env, episode, t };
+        const int ao = act_lane ? ((int)(hw & 255u) + SSD_VIEW) * S + 8 + (int)((hw >> 8) & 255u) : 0;
+        __syncwarp();
+        uint32_t old = 0;
+        if (act_lane) {                               // spawn eligibility: "no agent there" (co-located lanes write the same value)
+            old = tile[ao] & CODE_MASK;
+            tile[ao] = (uint8_t)(old | OCC_BIT);
+        }
+        __syncwarp();
+        bool changed = false;
+        if (KIND == SSD_ENV_CLEANUP) {
+            if (cleanup_spawn_active(tb, hcount)) changed = cleanup_spawn<MW>(p, tb, lane, tile, false, scratch, g, t, hcount, pr, am, wm);
+        } else {
+            changed = harvest_spawn<MW>(p, lane, tile, false, scratch, g, t, pr, am);
+        }
+        if (changed) {                                // the masks (and #waste) go back only when the spawn changed them
+#pragma unroll
+            for (int q = 0; q < MW; q++)
+                if (lane == q) {
+                    hot[RO_AMASK / 4 + q] = am[q];
+                    if (KIND == SSD_ENV_CLEANUP) hot[RO_WMASK / 4 + q] = wm[q];
+                }
+            if (KIND == SSD_ENV_CLEANUP && lane == 0) hot[RO_HCOUNT / 4] = (uint32_t)hcount;
+        }
+        if (KIND == SSD_ENV_HARVEST && act_lane)
+            res_g[(size_t)env * SSD_MAXN + lane] |= (uint32_t)count_apples_r5(tile, ao, S) << RS_CLOSE_SHIFT;
+        // ---- paint agents in agent order: the highest index wins a shared cell (map_env.py:257-261)
+        const unsigned grp = __match_any_sync(FULL, act_lane ? (uint32_t)ao : (0x40000000u | (uint32_t)lane));
+        __syncwarp();                                 // every lane's spawn / count reads of T are done
+        if (act_lane && lane == 31 - __clz(grp)) tile[ao] = (uint8_t)PAINT_CODE(lane);
+        __syncwarp();
+        write_global_view<OUT>(p, lane, tile + SSD_VIEW * S + 8, S, inv_w, tb.pal, reinterpret_cast<T*>(out) + (size_t)env * env_elems);
+        __syncwarp();                                 // the view's reads of T are done
+        if (act_lane) tile[ao] = (uint8_t)old;
+        __syncwarp();
+    }
+}
+
+// RESET VIEW, behind grid_reset_kernel<KIND, 0> (no windows) on the same mask: the view of each reset env from its fresh
+// record — the static map with the record's apples and (cleanup) waste, no agents (t == 0: MapEnv.reset does not paint them).  One
+// warp per env; dynamic shared memory: one map (map_bytes, rows of Wp cells) per warp.  `width` is unused.
+template <int KIND, int OUT>
+__global__ void __launch_bounds__(GRID_THREADS) grid_reset_global_kernel(const GridParams p, const uint8_t* mask, void* out, int width)
+{
+    typedef typename GlobalElem<OUT>::T T;
+    extern __shared__ __align__(16) uint8_t smem[];
+    __shared__ uint32_t s_pal[16];
+    if (threadIdx.x < 16) s_pal[threadIdx.x] = __ldg(p.pal + threadIdx.x);
+    if constexpr (OUT != SSD_GLOBAL_U8) load_policy_palette<T>(p);
+    __syncthreads();
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int env0 = blockIdx.x * GRID_WARPS + warp, estride = gridDim.x * GRID_WARPS;
+    uint8_t* m = smem + warp * p.map_bytes;
+    const float inv_w = __frcp_rn((float)p.W);
+    const size_t env_elems = (size_t)3 * p.H * p.W;
+    for (int i0 = 0; env0 + (long long)i0 * estride < p.E; i0 += 32) {
+        const long long el = env0 + (long long)(i0 + lane) * estride;
+        unsigned todo = __ballot_sync(FULL, el < p.E && (!mask || mask[el]));
+        while (todo) {
+            const int env = env0 + (i0 + __ffs(todo) - 1) * estride;
+            todo &= todo - 1;
+            const uint32_t hw = reinterpret_cast<const uint32_t*>(p.state + (size_t)env * p.rec_stride)[lane];
+            for (int i = lane; i < (p.map_bytes >> 4); i += 32)
+                reinterpret_cast<uint4*>(m)[i] = __ldg(reinterpret_cast<const uint4*>(p.base_map) + i);
+            __syncwarp();
+#pragma unroll
+            for (int q = 0; q < MAX_POINT_ROUNDS; q++) {   // point 32 q + lane: the cell takes its code when its mask bit is set
+                const uint32_t aq = __shfl_sync(FULL, hw, RO_AMASK / 4 + q);
+                const uint32_t wq = KIND == SSD_ENV_CLEANUP ? __shfl_sync(FULL, hw, RO_WMASK / 4 + q) : 0u;
+                const int j = 32 * q + lane;
+                if (j < p.n_apple && ((aq >> lane) & 1u)) m[__ldg(p.apple_c + j)] = (uint8_t)C_APPLE;
+                if (KIND == SSD_ENV_CLEANUP && j < p.n_waste && ((wq >> lane) & 1u)) m[__ldg(p.waste_c + j)] = (uint8_t)C_WASTE;
+            }
+            __syncwarp();
+            write_global_view<OUT>(p, lane, m, p.Wp, inv_w, s_pal, reinterpret_cast<T*>(out) + (size_t)env * env_elems);
+            __syncwarp();                                  // the view's reads of m are done
+        }
+    }
+}

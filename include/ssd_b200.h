@@ -280,8 +280,8 @@ int ssd_set_flat_policy_output(ssd_handle* h, const ssd_flat_policy_out* out);
  *     holds; F = ssd_feature_dim(h) = 12 + n (cleanup), 10 + 2n (harvest);
  *   - SSD_POLICY_F32 / _F16 / _BF16: obs_dev T [E*n][W], the rows of ssd_set_flat_policy_output: W = F + 2 and the row
  *     features ++ [theta, 0] with a contract, W = F and the features alone without one; each element T(float32(x)).
- * Grid-world kinds.  While set (sticky; NULL switches the handle back to uint8 windows, and ssd_set_policy_output replaces
- * it, as it replaces that one), the handle has this one observation form:
+ * Grid-world kinds.  While set (sticky; NULL switches the handle back to uint8 windows, and ssd_set_policy_output or
+ * ssd_set_global_output replaces it, as it replaces them), the handle has this one observation form:
  *   - ssd_reset (masked or not) writes the reset rows of the envs it resets: the reset observation of the reference
  *     (cleanup: the apple / waste caches from before the reset-time spawn; harvest: the map after it), and ssd_step,
  *     ssd_step_host, ssd_step_host_async write the step's rows; the auto_reset behind a step writes the new episode's reset
@@ -299,6 +299,31 @@ typedef struct ssd_feature_out {
     void*   obs_dev;        /* double [E][n][F] or T [E*n][W], 16-byte aligned */
 } ssd_feature_out;
 int ssd_set_feature_output(ssd_handle* h, const ssd_feature_out* out);
+/* JointEnv's global observation (global_obs=True: two_stage_train.py:572-617, get_global_obs = global_view() / 255,
+ * cleanup_new.py:299-300, harvest_new.py:178-179) as the handle's observation, written on the device at every step and
+ * reset, with no observation windows:
+ *   - SSD_GLOBAL_U8: obs_dev uint8 [E][H][W][3], byte for byte what ssd_global_view returns for the same state;
+ *   - SSD_POLICY_F32 / _F16 / _BF16: obs_dev T [E][3][H][W], each element T(float32(u8 / 255.0)) of that view (the
+ *     rounding of ssd_policy_inputs: VisionNetwork.forward's preprocessing of get_global_obs()).
+ * Grid-world kinds without a contract (JointEnv wraps the bare base env).  While set (sticky; NULL switches the handle back
+ * to uint8 windows, and each of ssd_set_policy_output / ssd_set_feature_output replaces it, as this call replaces them),
+ * the handle has this one observation form:
+ *   - ssd_reset (masked or not) writes the view of the envs it resets (the agents are not painted at t == 0, as
+ *     MapEnv.reset leaves them out of the colour map), ssd_step, ssd_step_host and ssd_step_host_async write the view after
+ *     the step, and the auto_reset behind a step writes the reset view of the envs it restarts.  obs_dev and
+ *     feature_obs_dev must be NULL in these calls (else SSD_EINVAL).
+ * Rewards, dones, infos, state, metrics, episode statistics, the episode log, ssd_global_view, ssd_render and beam recording
+ * are those of the uint8 form.
+ * Validates before storing anything: SSD_EINVAL for a struct_size too small, an unknown dtype, a NULL or not 16-byte aligned
+ * obs_dev, a handle with a contract, or a feature-env or selfdrive handle.  The caller keeps the tensor alive while it is
+ * set. */
+#define SSD_GLOBAL_U8 4          /* accepted by ssd_set_global_output only */
+typedef struct ssd_global_out {
+    int32_t struct_size;    /* sizeof(ssd_global_out) (a smaller value is rejected) */
+    int32_t dtype;          /* SSD_GLOBAL_U8, SSD_POLICY_F32 / _F16 / _BF16 */
+    void*   obs_dev;        /* uint8 [E][H][W][3] or T [E][3][H][W], 16-byte aligned */
+} ssd_global_out;
+int ssd_set_global_output(ssd_handle* h, const ssd_global_out* out);
 
 /* --- NegotiationSolver (environments/two_stage_train.py:619-776); every env kind ------------------- */
 #define SSD_SOLVER_RULE_MAX 0        /* decision_rule 'max'      (:751-757) */
