@@ -542,8 +542,12 @@ static int setup_grid(ssd_handle* h)
     CUDA_TRY(h, cudaFuncSetAttribute((const void*)logic_kernel_fn(c.env_kind, 0), cudaFuncAttributeMaxDynamicSharedMemorySize, h->logic_smem));
     if (h->logic_lay)
         CUDA_TRY(h, cudaFuncSetAttribute((const void*)logic_kernel_fn(c.env_kind, h->logic_lay), cudaFuncAttributeMaxDynamicSharedMemorySize, h->logic_smem));
-    if (getenv("SSD_DEBUG")) fprintf(stderr, "[ssd] observe kernel: %d warps/CTA, %d CTAs/SM, %d B smem/CTA, grid %d; logic smem %d B\n",
-                                     OBS_WARPS, per_sm2, p.g2_smem_bytes, h->obs_blocks, h->logic_smem);
+    if (getenv("SSD_DEBUG"))
+        fprintf(stderr, "[ssd] observe kernel: %d warps/CTA, %d CTAs/SM, %d B smem/CTA, grid %d; logic smem %d B; "
+                        "reset kernel: %d CTAs x %d warps = %d warps; octet logic kernel: %d CTAs x %d envs = %d envs/round\n",
+                OBS_WARPS, per_sm2, p.g2_smem_bytes, h->obs_blocks, h->logic_smem,
+                h->grid_blocks, GRID_WARPS, h->grid_blocks * GRID_WARPS,
+                h->logic8_blocks, L8_ENVS_PER_CTA, h->logic8_blocks * L8_ENVS_PER_CTA);
     if ((rc = dev_zalloc(h, (size_t)p.E * SSD_MAXN, &h->d_res))) return rc;
     if ((rc = dev_zalloc(h, 2, &p.obs_ctr))) return rc;
     h->pdl = !(getenv("SSD_NO_PDL") && atoi(getenv("SSD_NO_PDL")) != 0);

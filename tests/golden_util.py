@@ -317,3 +317,21 @@ def policy_image(want_u8, dtype, chunk=8192):
         x = want_u8[e0:e0 + chunk]
         out.append((x.double() / 255).float().to(dtype).reshape(-1, 15, 15, 3).permute(0, 3, 1, 2))
     return torch.cat(out)
+
+
+
+def profiled_names(fn):
+    """names of the records torch.profiler (CUDA activities) takes while fn runs twice, each time until its work finishes.
+
+    Late in a long test process the records of a profiling window's first launches have been missing: every kernel of
+    the first of a list of handles driven in turn (reset and three steps), the later handles' records present, and the
+    same with fn starting half a second into the window.  The second run makes each of fn's launches again after those,
+    so a launch that fn makes is recorded whichever of the window's first records are lost."""
+    import torch
+    from torch.profiler import ProfilerActivity, profile
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(2):
+            fn()
+            torch.cuda.synchronize()
+    return {e.name for e in prof.events()}

@@ -292,25 +292,39 @@ def test_variant_matches_oracle(oracle_lib, monkeypatch, v, form):
 # ---- the observe kernel's schedule: static grid-stride envs, then a dynamic tail from a global counter that the last CTA
 # re-arms; sizes chosen relative to the persistent grid (W = grid x 8 warps)
 _GRID = {}
+_RESET_LINE = re.compile(r"reset kernel: \d+ CTAs x \d+ warps = (\d+) warps; octet logic kernel: \d+ CTAs x \d+ envs = (\d+) envs/round")
 
 
-def _persistent_warps(capfd, monkeypatch):
-    """warps of the observe kernel's persistent grid for stock cleanup n = 8 (SSD_DEBUG prints the grid at create)"""
-    if "W" not in _GRID:
+def persistent_grids(capfd, monkeypatch, v):
+    """(W, Wr, G8) of the configuration of VARIANTS row v: the observe kernel's warps, the reset kernels' warps and the
+    octet logic kernel's envs per round, from the line SSD_DEBUG prints at create (a probe batch larger than every grid;
+    the grids depend on kind, agents and map, not on the observation form)"""
+    key = (v.kind, v.n, v.map)
+    if key not in _GRID:
         from contracts_b200.batched import BatchedGridEnv
         monkeypatch.setenv("SSD_DEBUG", "1")
         E = 1 << 16
         capfd.readouterr()
-        probe = BatchedGridEnv("cleanup_new", E, 8, contract="CleanupContract")
+        probe = BatchedGridEnv(v.kind + "_new", E, v.n, _map(v), contract=CONTRACT[v.kind] if v.n >= 2 else None)
         err = capfd.readouterr().err
         probe.close()
         monkeypatch.delenv("SSD_DEBUG")
         m = re.search(r"observe kernel: (\d+) warps/CTA, .* grid (\d+);", err)
         assert m, "SSD_DEBUG printed no observe-kernel grid: %r" % err
-        W = int(m.group(1)) * int(m.group(2))
-        assert W < E, "the probe batch does not fill the persistent grid"
-        _GRID["W"] = W
-    return _GRID["W"]
+        r = _RESET_LINE.search(err)
+        assert r, "SSD_DEBUG printed no reset / octet grid: %r" % err
+        grids = (int(m.group(1)) * int(m.group(2)), int(r.group(1)), int(r.group(2)))
+        assert max(grids) < E, "the probe batch does not fill the persistent grids %r" % (grids,)
+        with capfd.disabled():
+            print("[persistent grids] %s n=%d %s map: W = %d observe warps, Wr = %d reset warps, G8 = %d octet envs/round" %
+                  ((v.kind, v.n, v.map) + grids))
+        _GRID[key] = grids
+    return _GRID[key]
+
+
+def _persistent_warps(capfd, monkeypatch, v=VARIANTS[0]):
+    """warps of the observe kernel's persistent grid (stock cleanup n = 8 unless another VARIANTS row is given)"""
+    return persistent_grids(capfd, monkeypatch, v)[0]
 
 
 SIZES = {"1": lambda W: 1, "W-1": lambda W: W - 1, "W": lambda W: W, "W+1": lambda W: W + 1, "2W+1": lambda W: 2 * W + 1,
@@ -327,11 +341,19 @@ def obs_static_pct(request, monkeypatch):
     return request.param
 
 
-@pytest.mark.parametrize("size", list(SIZES))
+# the observe kernel's layouts: stock cleanup n = 8 (LAY = 1; its sizes carry no prefix), stock harvest n = 4 (LAY = 2) and
+# the generic kernel with 8 mask words (LAY = 0, MW = 8)
+SCHEDULE_ROWS = ("cleanup_n8_stock", "harvest_n4_stock", "cleanup_n8_big44x60")
+
+
+@pytest.mark.parametrize("size", [(row + "/" if row != SCHEDULE_ROWS[0] else "") + s for row in SCHEDULE_ROWS for s in SIZES])
 def test_observe_schedule_matches_oracle(oracle_lib, capfd, monkeypatch, obs_static_pct, size):
-    """stock cleanup n = 8, uint8 and bf16: 20 back-to-back auto-reset steps, every env compared with the oracle"""
-    E = SIZES[size](_persistent_warps(capfd, monkeypatch))
-    r = Rollout(oracle_lib, "cleanup", 8, _map(VARIANTS[0]), E, 7, ("u8", "bf16"), 25, seed=77)
+    """each layout of the observe kernel, uint8 and bf16: 20 back-to-back auto-reset steps, every env compared with the
+    oracle; E relative to that configuration's own persistent grid"""
+    row, _, size = size.rpartition("/")
+    v = next(x for x in VARIANTS if x.name == (row or SCHEDULE_ROWS[0]))
+    E = SIZES[size](_persistent_warps(capfd, monkeypatch, v))
+    r = Rollout(oracle_lib, v.kind, v.n, _map(v), E, 7, ("u8", "bf16"), 25, seed=77)
     r.reset()
     r.set_t((24 - np.arange(E)) % 25)                # env e finishes in step e mod 25
     for t in range(20):

@@ -386,18 +386,16 @@ def test_launched_kernels():
     """torch.profiler: the feature form launches grid_feature_kernel and (reset / auto-reset) grid_reset_features_kernel
     in every output form on the stock maps (cleanup: 4 mask words, harvest's 155 apple points: 8) — and never
     grid_obs_kernel."""
-    from torch.profiler import ProfilerActivity, profile
     forms = [(None, 3)] + [(DTYPES[d], o) for o, d in enumerate(("f32", "f16", "bf16"))]
     envs = [(_make(kind, 256, 4, horizon=3, policy_dtype=dt), kind) for kind in ("cleanup", "harvest") for dt, _ in forms]
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+
+    def run():
         for env, kind in envs:
             env.reset()
             a = env.random_actions(None, 8)
             for _ in range(4):
                 env.step(env.random_actions(None, 8, out=a), auto_reset=True)
-        torch.cuda.synchronize()
-    names = {e.name for e in prof.events()}
+    names = gu.profiled_names(run)
     for k in (0, 1):
         for _, o in forms:
             for want in ("grid_feature_kernel<%d, %d, %d>" % (k, 4 if k == 0 else 8, o), "grid_reset_features_kernel<%d, %d>" % (k, o)):

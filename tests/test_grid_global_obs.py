@@ -384,18 +384,16 @@ def test_launched_kernels():
     """torch.profiler: the global form launches grid_global_kernel and (reset / auto-reset) grid_reset_global_kernel in
     every output form on the stock maps (cleanup: 4 mask words; harvest's 155 apple points: 8) — and never grid_obs_kernel.
     (The other mask-word variants run in test_oracle_rollout's big maps.)"""
-    from torch.profiler import ProfilerActivity, profile
     forms = [(None, 4)] + [(DTYPES[d], o) for o, d in enumerate(("f32", "f16", "bf16"))]
     envs = [(_make(kind, 256, 4, horizon=3, policy_dtype=dt), kind) for kind in ("cleanup", "harvest") for dt, _ in forms]
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+
+    def run():
         for env, kind in envs:
             env.reset()
             a = env.random_actions(None, 8)
             for _ in range(4):
                 env.step(env.random_actions(None, 8, out=a), auto_reset=True)
-        torch.cuda.synchronize()
-    names = {e.name for e in prof.events()}
+    names = gu.profiled_names(run)
     for k in (0, 1):
         for _, o in forms:
             for want in ("grid_global_kernel<%d, %d, %d>" % (k, 4 if k == 0 else 8, o), "grid_reset_global_kernel<%d, %d>" % (k, o)):
@@ -410,18 +408,16 @@ def test_other_mask_words_launch():
     """torch.profiler: a big cleanup map runs the 8-word cleanup variant and a small harvest map the 4-word one, in every
     output form; their views equal global_view()."""
     from test_cuda_vs_oracle import CRAMPED_HARVEST
-    from torch.profiler import ProfilerActivity, profile
     forms = [(None, 4)] + [(DTYPES[d], o) for o, d in enumerate(("f32", "f16", "bf16"))]
     maps = (("cleanup", gu.big_map("cleanup", 40, 50, 3), 8), ("harvest", CRAMPED_HARVEST, 4))
     envs = [(_make(kind, 64, 3, amap, policy_dtype=dt), kind, mw, o) for kind, amap, mw in maps for dt, o in forms]
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+
+    def run():
         for env, kind, _, _ in envs:
             env.reset()
             for _ in range(3):
                 env.step(env.random_actions(None, NACT[kind]))
-        torch.cuda.synchronize()
-    names = {e.name for e in prof.events()}
+    names = gu.profiled_names(run)
     for env, kind, mw, o in envs:
         want = "grid_global_kernel<%d, %d, %d>" % (0 if kind == "cleanup" else 1, mw, o)
         assert any(want in s for s in names), (want, sorted(s for s in names if "kernel<" in s))
